@@ -6,7 +6,8 @@
     python bench.py --impl reference --gpus N --steps K --warmup W
 
 A "step" is one full sweep (k T-steps and k W-steps) over the whole data set.  Prints ONE JSON line.
-See DESIGN.md "Measurement" for what each key means.
+See DESIGN.md "Measurement" for what each key means.  --dump-outputs DIR also writes the factors W and T of the
+last timed step (the inputs are seeded, so two builds run with the same arguments can be compared output for output).
 """
 import argparse
 import json
@@ -49,7 +50,12 @@ def parse():
     ap.add_argument('--cpu-rows', type=int, default=None)
     ap.add_argument('--masked', default='dense', choices=['dense', 'sparse'], help='config 4: data layout of the observed entries')
     ap.add_argument('--refresh-every', type=int, default=1, help='config 4 sparse: residual restart period (sweeps)')
+    ap.add_argument('--dump-outputs', metavar='DIR', default=None,
+                    help='write the factors the timed sweeps produced as DIR/W.npy and DIR/T.npy (at most 64 MB; '
+                         'a fixed seeded sample of the rows of W when it does not fit)')
     a = ap.parse_args()
+    if a.steps < 1:
+        ap.error('--steps must be at least 1')
     if a.order is None:
         a.order = 'rri' if a.config == 'cfg4' else 'hals'
     return a
@@ -131,6 +137,37 @@ class ClockSampler(object):
                 'power_w_max': max(pw) if pw else None, 'reasons': sorted(reasons), 'samples': len(sm)}
 
 
+DUMP_BYTES = 64 * 10 ** 6
+
+
+def _dump_sample(count, keep, seed):
+    """indices 0..count-1, or a fixed seeded sorted sample of `keep` of them"""
+    import numpy as np
+    return np.arange(count) if keep >= count else np.sort(np.random.RandomState(seed).choice(count, keep, replace=False))
+
+
+def dump_outputs(dirname, n, row0, W, T, dist=None):
+    """--dump-outputs: W and T (NumPy, float32 or float64) as the timed sweeps left them, written to DIR/W.npy and
+    DIR/T.npy.  When the two exceed DUMP_BYTES, W.npy holds the rows of a fixed seeded sample (sorted), the same for
+    every run of the same configuration; T.npy likewise holds a sample of T's columns when T alone exceeds half of
+    DUMP_BYTES.  With row shards every rank passes its rows [row0, row0 + len(W)) of the n global ones (collective)
+    and rank 0 writes."""
+    import numpy as np
+    T = T[:, _dump_sample(T.shape[1], (DUMP_BYTES // 2) // (T.shape[0] * T.itemsize), 1)]
+    keep = (DUMP_BYTES - T.nbytes - 4096) // (W.shape[1] * W.itemsize)       # 4 KB for the two .npy headers
+    rows = _dump_sample(n, keep, 0)
+    Ws = W[rows[(rows >= row0) & (rows < row0 + W.shape[0])] - row0]
+    if dist is not None:
+        parts = [None] * dist.get_world_size()
+        dist.all_gather_object(parts, Ws)
+        if dist.get_rank() != 0:
+            return
+        Ws = np.concatenate(parts)
+    os.makedirs(dirname, exist_ok=True)
+    np.save(os.path.join(dirname, 'W.npy'), Ws)
+    np.save(os.path.join(dirname, 'T.npy'), T)
+
+
 GEN_BLOCK = 8192
 
 
@@ -199,11 +236,12 @@ def _load_cpu_arm():
     return 'port', run, orc
 
 
-def cpu_reference_sweeps(cfg, rows, sweeps, warm=1):
+def cpu_reference_sweeps(cfg, rows, sweeps, warm=1, dump=None):
     """Time the reference's sweep (per-topic GEMVs over X, nmf.py:415-476, interleaved order -- the only order it
     has) on ALL host cores, on a row sample of the configuration; its cost is exactly linear in n, so the
     full-size figure is the sample's rate scaled by rows/n.  BLAS threads are forced to the number of available
-    cores whatever OMP_NUM_THREADS says (torch.distributed.run exports OMP_NUM_THREADS=1)."""
+    cores whatever OMP_NUM_THREADS says (torch.distributed.run exports OMP_NUM_THREADS=1).  dump: directory that
+    receives the sample's W and T after the timed sweeps (dump_outputs)."""
     import numpy as np
     from threadpoolctl import threadpool_info, threadpool_limits
     ncores = len(os.sched_getaffinity(0))
@@ -226,6 +264,8 @@ def cpu_reference_sweeps(cfg, rows, sweeps, warm=1):
         t0 = time.perf_counter()
         W, T = run(X, cfg['k'], W, T, sweeps, M) if M is not None else run(X, cfg['k'], W, T, sweeps)
         dtm = (time.perf_counter() - t0) / sweeps
+    if dump:
+        dump_outputs(dump, rows, 0, W, T)
     full = dtm * cfg['n'] / rows
     what = ('the UNMODIFIED reference nmf() (oracle/_ref copy of src/rri_nmf, py3 shim, logger at WARNING)'
             if kind == 'reference' else 'the NumPy port oracle/rri_oracle.py of the reference sweep')
@@ -260,13 +300,9 @@ def main_reference(args):
     cfg = dict(CONFIGS[args.config])
     if args.rows:
         cfg['n'] = args.rows
-    steps = max(1, args.steps)
     # bounded sample: K timed sweeps (+ warm-up) stay around a minute of CPU time
-    rows = args.cpu_rows or cpu_sample_rows(cfg, steps + min(args.warmup, 1), 60.0)
-    if cfg.get('density'):
-        steps = min(steps, 5)                    # the masked reference costs ~10 ms per row and sweep
-        rows = args.cpu_rows or cpu_sample_rows(cfg, steps + 1, 60.0)
-    cb = cpu_reference_sweeps(cfg, rows, sweeps=steps, warm=max(0, min(args.warmup, 1)))
+    rows = args.cpu_rows or cpu_sample_rows(cfg, args.steps + min(args.warmup, 1), 60.0)
+    cb = cpu_reference_sweeps(cfg, rows, sweeps=args.steps, warm=max(0, min(args.warmup, 1)), dump=args.dump_outputs)
     line = {
         'impl': 'reference', 'metric': 'RRI sweeps/sec', 'value': cb['value'], 'unit': 'sweeps/s', 'n_gpus': args.gpus,
         'steps': args.steps, 'warmup': args.warmup, 'ms_per_step': 1e3 / cb['value'], 'higher_is_better': True,
@@ -341,6 +377,8 @@ def main_ours(args):
     barrier()
     th1 = time.time()
     ms = ev0.elapsed_time(ev1)
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, n, b, W.cpu().numpy(), T.cpu().numpy(), dist if world > 1 else None)
     clocks = None
     if rank == 0:
         time.sleep(0.12)
@@ -596,6 +634,8 @@ def main_masked(args):
     torch.cuda.synchronize()
     th1 = time.time()
     ms_per_step = ev0.elapsed_time(ev1) / args.steps
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, n, 0, W.cpu().numpy(), T.cpu().numpy())
     time.sleep(0.12)
     clocks = sampler.window(th0, th1)
     sampler.stop()

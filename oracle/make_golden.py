@@ -4,6 +4,9 @@ TEST INFRASTRUCTURE ONLY.  Run in the build container (needs /root/reference):
 
     python oracle/make_golden.py
 
+(`python oracle/make_golden.py live-pins` writes the one file that does not come from the reference: see
+live_case_pins.)
+
 All cases pass explicit W_in/T_in (so sklearn's randomized_svd stream is not part of the
 golden), `reset_topic_method=None`, logger at WARNING (SURVEY.md F4).  Inputs are stored in the
 file when they are not reproducible from a NumPy RandomState seed.
@@ -227,5 +230,42 @@ def main():
         print('  %-32s %8d B' % (f, os.path.getsize(os.path.join(OUT, f))))
 
 
+# the inputs of the live-reference tests (tests/test_oracle.py, tests/test_abi_cpu.py)
+LIVE_RANDOM_CASES = ((64, 40, 5, False), (33, 57, 4, False), (40, 30, 4, True))
+
+
+def live_case_pins():
+    """tests/golden/live_cases_f64.npz: what the ORACLE (and, for the host helpers, rri_nmf_b200._host) returns on the
+    inputs of the tests that compare with the live reference, so that those tests check every checkout, also one
+    without the reference.  These values are not the reference's own: the reference sources are not part of the
+    repository.  With the reference present the same tests also compare with it directly.
+
+        python oracle/make_golden.py live-pins
+    """
+    sys.path.insert(0, os.path.join(HERE, '..'))
+    from rri_nmf_b200._host import initialize_nmf, normalize, tfidf
+    d = {}
+    for n, dd, k, masked in LIVE_RANDOM_CASES:
+        rs = np.random.RandomState(n + dd)
+        X, W0, T0 = rs.rand(n, dd), rs.rand(n, k), rs.rand(k, dd)
+        M = (rs.rand(n, dd) < 0.4).astype(float) if masked else None
+        o = orc.nmf_oracle(X, k, W0, T0, max_iter=5, W_mat=M, compute_obj_each_iter=True, eps_stop=-1.0)
+        key = '%d_%d_%d_%d' % (n, dd, k, masked)
+        d['W_' + key], d['T_' + key], d['obj_' + key] = o['W'], o['T'], np.array(o['obj_history'])
+    rs = np.random.RandomState(1)
+    X, W0, T0 = rs.rand(60, 50), rs.rand(60, 4), rs.rand(4, 50)
+    o = orc.nmf_oracle(X, 4, W0, T0, max_iter=200, compute_obj_each_iter=True, eps_stop=1e-3)
+    d['stop_len'] = np.array([len(o['obj_history'])])
+    rs = np.random.RandomState(0)
+    X = rs.rand(40, 30) * (rs.rand(40, 30) < 0.3)
+    d['tfidf'], d['normalize'] = tfidf(X), normalize(X)
+    for init in ('random', 'smart_random', 'nndsvd', 'nndsvda', 'nndsvdar'):
+        d['W_' + init], d['T_' + init] = initialize_nmf(X, 5, init, random_state=3)
+    np.savez_compressed(os.path.join(OUT, 'live_cases_f64.npz'), **d)
+
+
 if __name__ == '__main__':
-    main()
+    if sys.argv[1:] == ['live-pins']:
+        live_case_pins()
+    else:
+        main()

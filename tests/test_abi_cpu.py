@@ -78,19 +78,26 @@ def test_nndsvd_known_answer():
 
 
 def test_host_helpers_against_reference_when_present():
+    """against tests/golden/live_cases_f64.npz (these helpers' own outputs, oracle/make_golden.py live-pins) and,
+    when the reference is present, against its matrixops / initialization directly"""
     import refshim
-    if not refshim.available():
-        pytest.skip('/root/reference not present')
-    ref = refshim.load()
+    from conftest import golden
     from rri_nmf_b200._host import initialize_nmf, normalize, tfidf
     rs = np.random.RandomState(0)
     X = rs.rand(40, 30) * (rs.rand(40, 30) < 0.3)
-    assert np.allclose(tfidf(X), ref.matrixops.tfidf(X))
-    assert np.allclose(normalize(X), ref.matrixops.normalize(X))
-    for init in ('random', 'smart_random', 'nndsvd', 'nndsvda', 'nndsvdar'):
-        a = initialize_nmf(X, 5, init, random_state=3)
-        b = ref.initialization.initialize_nmf(X, 5, init, random_state=3)
-        assert np.allclose(a[0], b[0]) and np.allclose(a[1], b[1]), init
+    g = golden('live_cases_f64.npz')
+    inits = ('random', 'smart_random', 'nndsvd', 'nndsvda', 'nndsvdar')
+    expected = [(g['tfidf'], g['normalize'], {i: (g['W_' + i], g['T_' + i]) for i in inits})]
+    if refshim.available():
+        ref = refshim.load()
+        expected.append((ref.matrixops.tfidf(X), ref.matrixops.normalize(X),
+                         {i: ref.initialization.initialize_nmf(X, 5, i, random_state=3) for i in inits}))
+    for tf, nm, init_out in expected:
+        assert np.allclose(tfidf(X), tf)
+        assert np.allclose(normalize(X), nm)
+        for init in inits:
+            a, b = initialize_nmf(X, 5, init, random_state=3), init_out[init]
+            assert np.allclose(a[0], b[0]) and np.allclose(a[1], b[1]), init
 
 
 def test_estimator_surface():

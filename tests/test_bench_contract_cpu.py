@@ -4,6 +4,8 @@ import os
 import subprocess
 import sys
 
+import numpy as np
+
 from conftest import ROOT
 
 
@@ -39,6 +41,47 @@ def test_reference_arm_full_threads_under_torchrun_env():
     assert r.returncode == 0, r.stderr[-2000:]
     j = json.loads([l for l in r.stdout.splitlines() if l.startswith('{')][0])
     assert j['cpu_baseline']['cores'] == len(os.sched_getaffinity(0)) and j['cpu_baseline']['kind'] == 'port'
+
+
+def test_reference_arm_dump_outputs(tmp_path):
+    """--dump-outputs: W and T after the last timed sweep, the same from run to run; --steps sets how many sweeps"""
+    args = ('--impl', 'reference', '--config', 'cfg1', '--warmup', '1', '--dump-outputs')
+    for name, steps in (('a', '2'), ('b', '2'), ('c', '3')):
+        _run('--steps', steps, *(args + (str(tmp_path / name),)))
+
+    def ld(run, f):
+        return np.load(str(tmp_path / run / f))
+    W, T = ld('a', 'W.npy'), ld('a', 'T.npy')
+    assert W.shape == (500, 10) and T.shape == (10, 300) and W.dtype == T.dtype == np.float64
+    assert np.allclose(W, ld('b', 'W.npy'), rtol=1e-12, atol=0) and np.allclose(T, ld('b', 'T.npy'), rtol=1e-12, atol=0)
+    assert not np.allclose(W, ld('c', 'W.npy'))
+
+
+def test_dump_outputs_samples_rows_beyond_the_cap(tmp_path):
+    import bench
+    n, k = 150000, 64
+    W = np.random.RandomState(1).rand(n, k)
+    W[:, 0] = np.arange(n)
+    T = np.random.RandomState(2).rand(k, 2000)
+    for name in ('a', 'b'):
+        bench.dump_outputs(str(tmp_path / name), n, 0, W, T)
+    files = [str(tmp_path / 'a' / f) for f in ('W.npy', 'T.npy')]
+    assert sum(os.path.getsize(f) for f in files) <= bench.DUMP_BYTES
+    Ws = np.load(files[0])
+    rows = Ws[:, 0].astype(np.int64)
+    assert 0 < len(rows) < n and np.all(np.diff(rows) > 0) and np.array_equal(Ws, W[rows])
+    assert np.array_equal(Ws, np.load(str(tmp_path / 'b' / 'W.npy')))
+    assert np.array_equal(np.load(files[1]), T)
+    # a T larger than the cap by itself: a sample of its columns, and W still fits next to it
+    T = np.random.RandomState(3).rand(k, 200000)
+    T[0] = np.arange(T.shape[1])
+    bench.dump_outputs(str(tmp_path / 'c'), 1000, 0, W[:1000], T)
+    files = [str(tmp_path / 'c' / f) for f in ('W.npy', 'T.npy')]
+    assert sum(os.path.getsize(f) for f in files) <= bench.DUMP_BYTES
+    Ts = np.load(files[1])
+    cols = Ts[0].astype(np.int64)
+    assert 0 < len(cols) < T.shape[1] and np.all(np.diff(cols) > 0) and np.array_equal(Ts, T[:, cols])
+    assert np.array_equal(np.load(files[0]), W[:1000])
 
 
 def test_reference_arm_other_ranks_exit_quietly():

@@ -1,5 +1,5 @@
 """The NumPy oracle against the golden vectors produced by the unmodified reference
-(oracle/make_golden.py) and -- when /root/reference is present -- against the live reference."""
+(oracle/make_golden.py) and -- when the reference is present -- against the live reference."""
 import numpy as np
 import pytest
 
@@ -131,43 +131,48 @@ def test_text_topic_model_simplex():
     assert relfro(out['W'], g['W_est']) < 1e-10 and relfro(out['T'], g['T_est']) < 1e-10
 
 
-# ------------------------------------------------------------------ live reference (container only)
-needs_ref = pytest.mark.skipif(not refshim.available(), reason='/root/reference not present')
+# ------------------------------------------------------------------ cases run against the live reference
+# The reference sources are not part of the repository.  tests/golden/live_cases_f64.npz pins what the oracle returns
+# on these inputs (oracle/make_golden.py live-pins), so every checkout checks them; with the reference present
+# (RRI_REFERENCE_ROOT) the tests also compare with it directly, at the same tolerances.
 
 
-@needs_ref
 @pytest.mark.parametrize('n,d,k,masked', [(64, 40, 5, False), (33, 57, 4, False), (40, 30, 4, True)])
 def test_live_reference_random(n, d, k, masked):
-    ref = refshim.load()
     rs = np.random.RandomState(n + d)
     X, W0, T0 = rs.rand(n, d), rs.rand(n, k), rs.rand(k, d)
     M = (rs.rand(n, d) < 0.4).astype(float) if masked else None
-    r = ref.nmf.nmf(X, k, W_in=W0, T_in=T0, max_iter=5, W_mat=M, reset_topic_method=None,
-                    compute_obj_each_iter=True, eps_stop=-1.0)
     o = orc.nmf_oracle(X, k, W0, T0, max_iter=5, W_mat=M, compute_obj_each_iter=True, eps_stop=-1.0)
-    assert relfro(o['W'], r['W']) < TOL and relfro(o['T'], r['T']) < TOL
-    assert np.allclose(o['obj_history'], r['obj_history'], rtol=1e-11)
+    g = golden('live_cases_f64.npz')
+    key = '%d_%d_%d_%d' % (n, d, k, masked)
+    expected = [(g['W_' + key], g['T_' + key], g['obj_' + key])]
+    if refshim.available():
+        r = refshim.load().nmf.nmf(X, k, W_in=W0, T_in=T0, max_iter=5, W_mat=M, reset_topic_method=None,
+                                   compute_obj_each_iter=True, eps_stop=-1.0)
+        expected.append((r['W'], r['T'], r['obj_history']))
+    for W, T, obj in expected:
+        assert relfro(o['W'], W) < TOL and relfro(o['T'], T) < TOL
+        assert np.allclose(o['obj_history'], obj, rtol=1e-11)
 
 
-@needs_ref
 def test_live_reference_stopping_rule():
-    ref = refshim.load()
     rs = np.random.RandomState(1)
     X, W0, T0 = rs.rand(60, 50), rs.rand(60, 4), rs.rand(4, 50)
-    r = ref.nmf.nmf(X, 4, W_in=W0, T_in=T0, max_iter=200, reset_topic_method=None,
-                    compute_obj_each_iter=True, eps_stop=1e-3)
     o = orc.nmf_oracle(X, 4, W0, T0, max_iter=200, compute_obj_each_iter=True, eps_stop=1e-3)
-    assert len(o['obj_history']) == len(r['obj_history']) < 200
+    assert len(o['obj_history']) == int(golden('live_cases_f64.npz')['stop_len'][0]) < 200
+    if refshim.available():
+        r = refshim.load().nmf.nmf(X, 4, W_in=W0, T_in=T0, max_iter=200, reset_topic_method=None,
+                                   compute_obj_each_iter=True, eps_stop=1e-3)
+        assert len(o['obj_history']) == len(r['obj_history'])
 
 
-@needs_ref
 def test_live_reference_zero_topic_raises():
     """A topic that collapses to zero with resets disabled: the T row is all-zero -> nt = 0 ->
     the W-step takes qf_min's c<=0 branch without bounds and raises (optimization.py:60-67,105-107)."""
-    ref = refshim.load()
     rs = np.random.RandomState(33 + 57)
     X, W0, T0 = rs.rand(33, 57), rs.rand(33, 8), rs.rand(8, 57)
     with pytest.raises(ValueError):
-        ref.nmf.nmf(X, 8, W_in=W0, T_in=T0, max_iter=5, reset_topic_method=None)
-    with pytest.raises(ValueError):
         orc.nmf_oracle(X, 8, W0, T0, max_iter=5)
+    if refshim.available():
+        with pytest.raises(ValueError):
+            refshim.load().nmf.nmf(X, 8, W_in=W0, T_in=T0, max_iter=5, reset_topic_method=None)
