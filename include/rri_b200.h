@@ -33,7 +33,9 @@ enum {
     RRI_FLAG_ZERO_T    = 1,   /* some sum(T[t,:]) <= 1e-10          nmf.py:757-758 */
     RRI_FLAG_ZERO_W    = 2,   /* some sum(W[:,t]) <= 1e-10          nmf.py:793-794, assert :476 */
     RRI_FLAG_UNBOUNDED = 4,   /* denominator <= 0 with no bound     optimization.py:60-67, :76-77, :105-107 */
-    RRI_FLAG_NONFINITE = 8    /* NaN/Inf produced */
+    RRI_FLAG_NONFINITE = 8,   /* NaN/Inf produced */
+    RRI_FLAG_NOT_IMPLEMENTED = 16  /* project_T_each_iter, block order: a denominator <= 0 with t_row_sum != 1
+                                      (optimization.py:60-74 raises NotImplementedError) */
 };
 
 /* keyword arguments of nmf() that reach the hot path (nmf.py:98-108) */

@@ -14,6 +14,7 @@ RRI_MATH_IEEE, RRI_MATH_TF32 = 0, 1
 RRI_ORDER_RRI, RRI_ORDER_HALS = 0, 1
 RRI_MASK_NONE, RRI_MASK_REAL, RRI_MASK_U8 = 0, 1, 2
 FLAG_ZERO_T, FLAG_ZERO_W, FLAG_UNBOUNDED, FLAG_NONFINITE = 1, 2, 4, 8
+FLAG_NOT_IMPLEMENTED = 16
 
 
 class RriParams(C.Structure):

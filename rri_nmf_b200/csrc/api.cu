@@ -156,6 +156,7 @@ struct rri_handle_s {
     void *Wt = nullptr, *Tt = nullptr, *Cpart = nullptr, *cg = nullptr /* [max(n,d)*k | k*k] */, *Hm = nullptr;
     void *gram_part = nullptr, *colsum_part = nullptr;
     int splits_t = 1, splits_w = 1, ub_blocks_t = 1, ub_blocks_w = 1, gchunks_w = 1, gchunks_t = 1;
+    double* sx_slots = nullptr;        // grid-reduction scratch of the constrained T update (simplex_T)
     Tf32Gemm* tf32 = nullptr;
     bool fixT_cached = false;
     // masked
@@ -521,6 +522,7 @@ static int bind_impl(rri_handle_t h, cudaStream_t st)
         // K-contiguous operands
         const int64_t v = 16 / (int64_t)es;
         h->ldxt = (n + v - 1) / v * v;
+        if (!h->sx_slots && ws_alloc(h, (void**)&h->sx_slots, sizeof(double) * (size_t)simplex_T_slots(d))) return 1;
         if (h->Xt_ext) {
             if (h->ldxt_ext < h->ldxt || h->ldxt_ext % v != 0 || (reinterpret_cast<uintptr_t>(h->Xt_ext) & 15) != 0)
                 return fail("caller-provided X' storage needs a 16-byte aligned base and a row stride >= %lld, multiple of %lld",
@@ -703,13 +705,9 @@ static int check_params(rri_handle_t h, const rri_params_t* p)
     if (!h->X) return fail("rri_bind has not been called");
     if (p->fix_W && p->fix_T) return fail("fix_W and fix_T both set: nothing to update");
     if (p->fix_W) return fail("fix_W=True is not supported on the device path (the reference's T-only sweep also rescales W, nmf.py:450-452)");
-    if (p->simplex_T) {
-        // unmasked: Euclidean projection of the row onto the simplex (optimization.py:58-59); masked / observed
-        // entries: the vector-c branch rescales the clipped solution to the sum (optimization.py:85-87)
-        if (h->mk == MK_NONE && h->order != RRI_ORDER_RRI)
-            return fail("project_T_each_iter couples the columns of T: it needs update_order='rri'");
-        if (!(p->ub_t > 0)) return fail("simplex_T needs t_row_sum > 0");
-    }
+    // simplex_T, unmasked: Euclidean projection of the row onto the simplex (optimization.py:58-59); masked / observed
+    // entries: the vector-c branch rescales the clipped solution to the sum (optimization.py:85-87)
+    if (p->simplex_T && !(p->ub_t > 0)) return fail("simplex_T needs t_row_sum > 0");
     return 0;
 }
 
@@ -841,8 +839,9 @@ static int hals_W_half(rri_handle_t h, T* W, const T* Tk, int64_t ldtk, const rr
     return 0;
 }
 
+// Tk [k, ldtk]: where T is written (the caller's T, or this rank's replica inside the peer-exchange buffer)
 template <typename T>
-static int hals_T_half(rri_handle_t h, T* W, T* Tm, const rri_params_t* p, cudaStream_t st)
+static int hals_T_half(rri_handle_t h, T* W, T* Tk, int64_t ldtk, const rri_params_t* p, cudaStream_t st)
 {
     const int k = h->k;
     const int64_t n = h->n, d = h->d;
@@ -850,7 +849,7 @@ static int hals_T_half(rri_handle_t h, T* W, T* Tm, const rri_params_t* p, cudaS
     T* G = cg + (size_t)d * k;
     const bool tc_gram = gram_in_contraction(h);
     const int psplits = h->math == RRI_MATH_TF32 ? 1 : h->splits_t;
-    if (h->world > 1 && h->p2p) {
+    if (h->world > 1 && h->p2p && !p->simplex_T) {
         // Exchange over NVLink peer memory fused with the update: this rank's partials [X_i'W_i | W_i'W_i] are
         // produced straight into its exported slot, then ONE kernel publishes / waits, adds the slices it owns over
         // all ranks in rank order, updates those rows of T' and stores them into every rank's replicas.
@@ -884,8 +883,20 @@ static int hals_T_half(rri_handle_t h, T* W, T* Tm, const rri_params_t* p, cudaS
         if (allreduce(h, cg, (size_t)d * k + (size_t)k * k, st)) return 1;
         C = cg; parts = 1;
     }
+    if (p->simplex_T) {
+        // the projection couples the columns of T: one cooperative launch, or a chain of per-topic launches where
+        // the grid cannot be co-resident or k is outside the fused kernel's register range (RRI_SIMPLEX_FUSED=0
+        // forces the chain; read per call so that one process can time both)
+        const char* e = getenv("RRI_SIMPLEX_FUSED");
+        int nl = 0;
+        const int rc = launch_simplex_T_update<T>((T*)h->Tt, d, k, C, parts, d * k, G, solve_args(p, true), p->ub_t, Tk,
+                                                  ldtk, h->sx_slots, h->flags, h->sm_count, !(e && *e == '0'), &nl, st);
+        if (rc) return fail("constrained T update failed: %s", cudaGetErrorString((cudaError_t)rc));
+        h->launches += nl;
+        return 0;
+    }
     // Tt (d x k) is updated in place; its transpose is written straight into the caller's T (k x d)
-    launch_update_rows<T>((T*)h->Tt, d, k, C, parts, d * k, nullptr, G, solve_args(p, true), Tm, d, (T*)h->colsum_part,
+    launch_update_rows<T>((T*)h->Tt, d, k, C, parts, d * k, nullptr, G, solve_args(p, true), Tk, ldtk, (T*)h->colsum_part,
                           h->flags, h->ub_blocks_t, ColsumOut{nullptr, 0, 0, h->counters + 2}, st);
     h->launches++;
     CKL();
@@ -895,13 +906,13 @@ static int hals_T_half(rri_handle_t h, T* W, T* Tm, const rri_params_t* p, cudaS
 // Once per call: sum(T[t,:]) and sum(W[:,t]) (nmf.py:757, :793) with the zero-topic flags, from the rows of T and of
 // W' -- a topic that empties inside a call makes the next half-step's denominator zero and raises the unbounded flag
 // anyway, so nothing is lost by not looking after every half-step.  On row shards the test on W is over ALL rows: the
-// shard sums are all-reduced.  (T sums: the peer exchange finalises them itself.)
+// shard sums are all-reduced.  t_sums: take the T sums here (false where the peer exchange finalised them itself).
 template <typename T>
-static int hals_finish_sums(rri_handle_t h, const T* Tm, bool t_updated, cudaStream_t st)
+static int hals_finish_sums(rri_handle_t h, const T* Tm, bool t_sums, cudaStream_t st)
 {
     launch_rowsum_flag<T>((const T*)h->Wt, h->k, h->n, h->ldwt, h->sums, h->k, h->world > 1 ? 0 : 2, h->flags, st);
     h->launches++;
-    if (t_updated && !(h->world > 1 && h->p2p)) {
+    if (t_sums) {
         launch_rowsum_flag<T>(Tm, h->k, h->d, h->d, h->sums, 0, 1, h->flags, st);
         h->launches++;
     }
@@ -1214,13 +1225,13 @@ static int sweeps_impl(rri_handle_t h, T* W, T* Tm, int n_sweeps, const rri_para
         if (px) CK(cudaMemcpy2DAsync(Tk, (size_t)ldtk * sizeof(T), Tm, (size_t)d * sizeof(T), (size_t)d * sizeof(T), (size_t)k,
                                      cudaMemcpyDeviceToDevice, st));
         for (int s = 0; s < n_sweeps; ++s) {
-            if (hals_T_half<T>(h, W, Tm, p, st)) return 1;
+            if (hals_T_half<T>(h, W, Tk, ldtk, p, st)) return 1;
             if (hals_W_half<T>(h, W, Tk, ldtk, p, true, st)) return 1;
         }
         if (px) CK(cudaMemcpy2DAsync(Tm, (size_t)d * sizeof(T), Tk, (size_t)ldtk * sizeof(T), (size_t)d * sizeof(T), (size_t)k,
                                      cudaMemcpyDeviceToDevice, st));
         h->c2_valid = n_sweeps > 0;            // Cpart = X T' for the T just written, Tt = its transpose
-        return n_sweeps > 0 ? hals_finish_sums<T>(h, Tm, true, st) : 0;
+        return n_sweeps > 0 ? hals_finish_sums<T>(h, Tm, !(px && !p->simplex_T), st) : 0;
     }
     if (rri_prologue<T>(h, W, 0, p, st)) return 1;
     for (int s = 0; s < n_sweeps; ++s)
@@ -1594,7 +1605,7 @@ static int profile_impl(rri_handle_t h, int which, const T* W, const T* Tm, int 
             if (contraction<T>(h, (const T*)h->Xt, h->ldxt, (const T*)h->Wt, h->ldwt, (T*)h->Cpart, d, k, n, h->splits_t, st)) return 1;
         } else if (which == 3) {
             // the whole T half-step (contraction + Gram + exchange + update); collective on row shards
-            if (hals_T_half<T>(h, const_cast<T*>(W), const_cast<T*>(Tm), &prm, st)) return 1;
+            if (hals_T_half<T>(h, const_cast<T*>(W), Tk, ldtk, &prm, st)) return 1;
         } else if (which == 4) {
             if (hals_W_half<T>(h, const_cast<T*>(W), Tk, ldtk, &prm, true, st)) return 1;
         } else {

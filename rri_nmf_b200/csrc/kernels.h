@@ -202,6 +202,17 @@ void launch_flag_from_sums(const double* sums, int off, int k, int zero_flag, in
 // matrixops.py:5-69 computes the same threshold by sorting)
 template <typename T>
 void launch_project_rows_simplex(T* A, int64_t rows, int64_t cols, double s, cudaStream_t st);
+
+// Block-order T half-step with the projection of every updated row of T onto the simplex of radius s
+// (project_T_each_iter, nmf.py:420-447 + :759-761), from the contraction C = sum of `parts` slices [d, k] and the Gram
+// matrix G [k, k]: updates T' = Tt [d, k] in place and writes T = Tout [k, ldo].  allow_fused: one cooperative launch
+// when k and the grid fit it (else, and with allow_fused false, a chain of 2k + 1 launches).  Returns 0 or a
+// cudaError_t; *launches = kernels launched.  slots: simplex_T_slots(d) doubles of scratch.
+int simplex_T_slots(int64_t d);
+template <typename T>
+int launch_simplex_T_update(T* Tt, int64_t d, int k, const T* C, int parts, int64_t pstride, const T* G, const SolveArgs& a,
+                            double s, T* Tout, int64_t ldo, double* slots, int* flags, int sm_count, bool allow_fused,
+                            int* launches, cudaStream_t st);
 }  // namespace rri
 
 namespace rri {

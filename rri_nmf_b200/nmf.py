@@ -575,6 +575,9 @@ def _solve(engine, Xd, W, T, rtv, a):
             # transform(): the reference would re-seed topic t (T row included!) when no new document uses it
             # (nmf.py:796-816 runs under fix_T as well).  Here T is left alone and the column stays zero.
             flags &= ~_lib.FLAG_ZERO_W
+        if flags & _lib.FLAG_NOT_IMPLEMENTED:
+            # block order with project_T_each_iter: a T denominator <= 0 and t_row_sum != 1 (optimization.py:60-74)
+            raise NotImplementedError('s={} is not yet implemented'.format(t_row_sum))
         _raise_on_flags(flags, engine, reset_topic_method if not (can_reset or fix_T) else None)
         iter_no += ns
         if project_W_each_iter and not a['fix_W'] and w_row_sum is not None:      # nmf.py:481-484
