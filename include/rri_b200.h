@@ -109,6 +109,19 @@ int rri_bind(rri_handle_t h, const void* X_dev, int64_t ldX,
 int rri_bind_csr(rri_handle_t h, int64_t nnz, const int64_t* rowptr_dev, const int32_t* col_dev,
                  const void* val_dev, const void* weight_dev, void* stream);
 
+/* Zero-filled sparse binding: the CSR matrix is an ordinary non-negative matrix stored sparsely (a tf-idf
+ * document-term matrix); every entry is fitted, the unstored ones as 0.  Same CSR contract as rri_bind_csr
+ * (int64 rowptr, int32 strictly ascending columns, nnz < 2^31, the three arrays stay alive while the handle is
+ * used).  Only handles created with RRI_ORDER_HALS and RRI_MATH_IEEE (fp32 or fp64).  The column orientation and
+ * the chunk plan of long rows / columns are built once (synchronises `stream`); the workspace grows with nnz and
+ * (n + d) * k, never with n * d.  The block-order half-steps then take X T' and X' W from a sparse x dense
+ * contraction.  On such a handle: rri_sweeps (block order and fix_T), rri_objective and rri_objective_contraction
+ * (both through the identity, ||X||^2 from the stored values in fp64), rri_partials_T (nw of length 1),
+ * rri_topic_sums, rri_stats and rri_profile_kernel (which = 1 / 2: the W- / T-half contraction, 3 / 4: the whole
+ * half-steps).  rri_topics and rri_peer_export refuse it; row shards use the NCCL all-reduce. */
+int rri_bind_csr_zero(rri_handle_t h, int64_t nnz, const int64_t* rowptr_dev, const int32_t* col_dev,
+                      const void* val_dev, void* stream);
+
 /* Run n_sweeps full sweeps in place on W_dev[n_local,k], T_dev[k,d]:  nmf.py:377, :415-476
  * (+ masked branches :687-701, :735-746; qf_min optimization.py:51-59, :75-87).
  * flags_host (may be NULL): receives the OR of RRI_FLAG_* over all sweeps (forces a stream sync).

@@ -76,7 +76,11 @@ def initialize_nmf(X, n_components, init=None, eps=1e-6, random_state=None, row_
 
 def normalize(X, dim=1, zero_sum_fix=True):
     """Scale rows (dim=1) or columns (dim=0) to sum to 1; all-zero vectors become uniform
-    (matrixops.py:124-163)."""
+    (matrixops.py:124-163).  A scipy.sparse X gives a CSR matrix equal to the dense result (an all-zero row then
+    stores its d uniform entries)."""
+    import scipy.sparse as sp
+    if sp.issparse(X):
+        return _normalize_sparse(X, dim, zero_sum_fix)
     X = np.asarray(X, dtype=float)
     if dim == 0:
         return normalize(X.T, 1, zero_sum_fix).T
@@ -89,8 +93,39 @@ def normalize(X, dim=1, zero_sum_fix=True):
     return out
 
 
+def _normalize_sparse(X, dim, zero_sum_fix):
+    import scipy.sparse as sp
+    if dim == 0:
+        return _normalize_sparse(X.T, 1, zero_sum_fix).T.tocsr()
+    if dim != 1:
+        raise Exception('Unknown dim=%r' % (dim,))
+    X = sp.csr_matrix(X, dtype=float, copy=True)
+    n, d = X.shape
+    s = np.asarray(X.sum(1)).ravel() + np.spacing(1)
+    X.data = X.data / np.repeat(s, np.diff(X.indptr))
+    if not zero_sum_fix:
+        return X
+    zero = np.flatnonzero(s < 1e-10)
+    if zero.size == 0:
+        return X
+    keep = np.ones(n)
+    keep[zero] = 0.0
+    uni = sp.csr_matrix((np.full(zero.size * d, 1.0 / d), (np.repeat(zero, d), np.tile(np.arange(d), zero.size))),
+                        shape=(n, d))
+    out = (sp.diags(keep) @ X + uni).tocsr()
+    out.sort_indices()
+    return out
+
+
 def tfidf(X, return_idf=False):
-    """tf-idf with idf = log(n / df) (matrixops.py:166-179); dense input."""
+    """tf-idf with idf = log(n / df) (matrixops.py:166-179).  A scipy.sparse X gives a CSR matrix equal to the dense
+    result."""
+    import scipy.sparse as sp
+    if sp.issparse(X):
+        X = sp.csr_matrix(X)
+        idf = np.log(X.shape[0] / (np.asarray((X > 0).sum(0)).ravel() + np.spacing(1)))
+        out = X.multiply(idf[None, :]).tocsr()
+        return (out, idf) if return_idf else out
     X = np.asarray(X)
     n = X.shape[0]
     idf = np.log(n / ((X > 0).sum(0) + np.spacing(1)))

@@ -42,6 +42,7 @@ SYMBOLS = {
     'rri_set_transpose_storage': (C.c_int, [_vp, _vp, _i64]),
     'rri_bind': (C.c_int, [_vp, _vp, _i64, _vp, _i32, _i64, _vp]),
     'rri_bind_csr': (C.c_int, [_vp, _i64, _vp, _vp, _vp, _vp, _vp]),
+    'rri_bind_csr_zero': (C.c_int, [_vp, _i64, _vp, _vp, _vp, _vp]),
     'rri_sweeps': (C.c_int, [_vp, _vp, _vp, _i32, C.POINTER(RriParams), C.POINTER(_i32), _vp]),
     'rri_topics': (C.c_int, [_vp, _vp, _vp, _i32, _i32, C.POINTER(RriParams), C.POINTER(_i32), _vp]),
     'rri_topic_sums': (C.c_int, [_vp, C.POINTER(C.c_double), C.POINTER(C.c_double), _vp]),

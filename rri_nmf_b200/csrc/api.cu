@@ -175,6 +175,10 @@ struct rri_handle_s {
     bool sp_refresh_v2 = true;         // residual restart: row copy from the factors, column copy gathered from it
     bool sp_batched_sums = true;       // per-topic sums once per sweep (2 launches) instead of once per half-step (2k)
     int* sp_err = nullptr;
+    // zero-filled sparse binding (rri_bind_csr_zero): the rows and the columns with their chunk plans; the block-order
+    // half-steps take X T' / X' W from launch_spmm instead of the dense contraction
+    bool zero_csr = false;
+    SpmmPlan zrow{}, zcol{};
     // common
     double* sums = nullptr;    // [2k] device
     int* flags = nullptr;      // device
@@ -288,6 +292,7 @@ extern "C" int rri_peer_export(rri_handle_t h, char handle_out[64])
     if (!h) return fail("null handle");
     if (!h->X) return fail("rri_bind has not been called");
     if (h->order != RRI_ORDER_HALS || h->mk != MK_NONE) return fail("the peer-memory exchange serves unmasked hals handles");
+    if (h->zero_csr) return fail("the peer-memory exchange serves dense data; zero-filled sparse handles use the NCCL all-reduce");
     if (!peer_rank_supported(h)) return fail("the fused peer-memory T update supports k <= 128 (f32) / 64 (f64)");
     CK(cudaSetDevice(h->device));
     if (!h->xbuf) {
@@ -448,6 +453,39 @@ static int allreduce(rri_handle_t h, void* buf, size_t count, cudaStream_t st)
     return 0;
 }
 
+// Workspace of the block-order half-steps downstream of the contraction (and of the contraction's output): both the
+// dense binding and the zero-filled sparse one.  splits_w / splits_t (K-slices of the two contractions) are set first.
+static int alloc_halfstep_ws(rri_handle_t h)
+{
+    const int64_t n = h->n, d = h->d;
+    const int k = h->k;
+    const size_t es = h->es;
+    const size_t a = (size_t)h->splits_w * n * k, b = (size_t)h->splits_t * d * k;
+    if (ws_alloc(h, &h->Cpart, es * (a > b ? a : b))) return 1;
+    const int64_t m = n > d ? n : d;
+    if (ws_alloc(h, &h->cg, es * ((size_t)m * k + (size_t)k * k))) return 1;
+    if (ws_alloc(h, &h->Hm, es * (size_t)k * k)) return 1;
+    {   // rows of W' are TMA operands in tf32 mode: keep them 16-byte aligned
+        const int64_t v = 16 / (int64_t)es;
+        h->ldwt = (n + v - 1) / v * v;
+    }
+    if (ws_alloc(h, &h->Wt, es * (size_t)k * h->ldwt) || ws_alloc(h, &h->Tt, es * (size_t)d * k)) return 1;
+    h->gchunks_w = gram_chunks(n, k, h->sm_count);
+    h->gchunks_t = gram_chunks(d, k, h->sm_count);
+    const int gc = h->gchunks_w > h->gchunks_t ? h->gchunks_w : h->gchunks_t;
+    if (ws_alloc(h, &h->gram_part, es * (size_t)gc * k * k)) return 1;
+    h->ub_blocks_w = update_rows_blocks(n, h->sm_count);
+    h->ub_blocks_t = update_rows_blocks(d, h->sm_count);
+    int ubm = h->ub_blocks_w > h->ub_blocks_t ? h->ub_blocks_w : h->ub_blocks_t;
+    {   // the multi-GPU T update works in 32-row blocks (peer_update_blocks)
+        const int pb = peer_update_blocks(d, h->sm_count);
+        if (pb > ubm) ubm = pb;
+    }
+    if (ws_alloc(h, &h->colsum_part, es * (size_t)ubm * k)) return 1;
+    if (h->order == RRI_ORDER_HALS && ws_alloc(h, (void**)&h->sx_slots, sizeof(double) * (size_t)simplex_T_slots(d))) return 1;
+    return 0;
+}
+
 template <typename T>
 static int bind_impl(rri_handle_t h, cudaStream_t st)
 {
@@ -488,28 +526,7 @@ static int bind_impl(rri_handle_t h, cudaStream_t st)
         h->splits_w = simt_gemm_splits(n, d, h->sm_count);
         h->splits_t = simt_gemm_splits(d, n, h->sm_count);
         if (h->math == RRI_MATH_TF32) { h->splits_w = 1; h->splits_t = 1; }
-        const size_t a = (size_t)h->splits_w * n * k, b = (size_t)h->splits_t * d * k;
-        if (ws_alloc(h, &h->Cpart, es * (a > b ? a : b))) return 1;
-        const int64_t m = n > d ? n : d;
-        if (ws_alloc(h, &h->cg, es * ((size_t)m * k + (size_t)k * k))) return 1;
-        if (ws_alloc(h, &h->Hm, es * (size_t)k * k)) return 1;
-        {   // rows of W' are TMA operands in tf32 mode: keep them 16-byte aligned
-            const int64_t v = 16 / (int64_t)es;
-            h->ldwt = (n + v - 1) / v * v;
-        }
-        if (ws_alloc(h, &h->Wt, es * (size_t)k * h->ldwt) || ws_alloc(h, &h->Tt, es * (size_t)d * k)) return 1;
-        h->gchunks_w = gram_chunks(n, k, h->sm_count);
-        h->gchunks_t = gram_chunks(d, k, h->sm_count);
-        const int gc = h->gchunks_w > h->gchunks_t ? h->gchunks_w : h->gchunks_t;
-        if (ws_alloc(h, &h->gram_part, es * (size_t)gc * k * k)) return 1;
-        h->ub_blocks_w = update_rows_blocks(n, h->sm_count);
-        h->ub_blocks_t = update_rows_blocks(d, h->sm_count);
-        int ubm = h->ub_blocks_w > h->ub_blocks_t ? h->ub_blocks_w : h->ub_blocks_t;
-        {   // the multi-GPU T update works in 32-row blocks (peer_update_blocks)
-            const int pb = peer_update_blocks(d, h->sm_count);
-            if (pb > ubm) ubm = pb;
-        }
-        if (ws_alloc(h, &h->colsum_part, es * (size_t)ubm * k)) return 1;
+        if (alloc_halfstep_ws(h)) return 1;
         if (h->math == RRI_MATH_TF32) {
             std::string err;
             // (k + 16: the device-resident NNDSVD runs its randomized SVD with k + 10 columns through this kernel)
@@ -522,7 +539,6 @@ static int bind_impl(rri_handle_t h, cudaStream_t st)
         // K-contiguous operands
         const int64_t v = 16 / (int64_t)es;
         h->ldxt = (n + v - 1) / v * v;
-        if (!h->sx_slots && ws_alloc(h, (void**)&h->sx_slots, sizeof(double) * (size_t)simplex_T_slots(d))) return 1;
         if (h->Xt_ext) {
             if (h->ldxt_ext < h->ldxt || h->ldxt_ext % v != 0 || (reinterpret_cast<uintptr_t>(h->Xt_ext) & 15) != 0)
                 return fail("caller-provided X' storage needs a 16-byte aligned base and a row stride >= %lld, multiple of %lld",
@@ -569,6 +585,7 @@ extern "C" int rri_bind(rri_handle_t h, const void* X_dev, int64_t ldX, const vo
     if (mask_kind != RRI_MASK_NONE && ldM < h->d) return fail("ldM < d");
     if (mask_kind < 0 || mask_kind > 2) return fail("bad mask kind %d", mask_kind);
     if (h->sparse) return fail("this handle is bound to observed-entries (CSR) data; create a new one for dense data");
+    if (h->zero_csr) return fail("this handle is bound to zero-filled sparse (CSR) data; create a new one for dense data");
     if (h->X && ((h->mk != MK_NONE) != (mask_kind != RRI_MASK_NONE)))
         return fail("a handle cannot switch between masked and unmasked data; create a new one");
     CK(cudaSetDevice(h->device));
@@ -683,6 +700,101 @@ extern "C" int rri_bind_csr(rri_handle_t h, int64_t nnz, const int64_t* rowptr_d
     if (rc) return rc;
     h->sparse = true;
     h->mk = MK_SPARSE;
+    h->X = val_dev ? val_dev : (const void*)rowptr_dev;      // "bound" marker; the dense kernels never see it
+    return 0;
+}
+
+// -------------------------------------------------------------------------------------------------
+// zero-filled sparse binding: the block order with a sparse x dense contraction (spmm_kernels.cu)
+// -------------------------------------------------------------------------------------------------
+// Chunk plan of one orientation: segments longer than SPMM_CHUNK are cut into chunks whose partials are added in chunk
+// order by the last one to arrive.  Built on the host from the segment pointers, once per binding.
+static int build_spmm_plan(rri_handle_t h, SpmmPlan& pl, int64_t nseg, const int64_t* ptr_dev, const int32_t* idx,
+                           const void* val)
+{
+    std::vector<int64_t> ptr((size_t)nseg + 1);
+    CK(cudaMemcpy(ptr.data(), ptr_dev, sizeof(int64_t) * ptr.size(), cudaMemcpyDeviceToHost));
+    std::vector<int32_t> lseg;
+    std::vector<int64_t> lslot;
+    std::vector<int2> litem;
+    for (int64_t s = 0; s < nseg; ++s) {
+        const int64_t len = ptr[s + 1] - ptr[s];
+        if (len <= SPMM_CHUNK) continue;
+        const int j = (int)lseg.size();
+        lseg.push_back((int32_t)s);
+        lslot.push_back((int64_t)litem.size());
+        for (int64_t c = 0; c * SPMM_CHUNK < len; ++c) litem.push_back(make_int2(j, (int)c));
+    }
+    pl = SpmmPlan{};
+    pl.nseg = nseg; pl.ptr = ptr_dev; pl.idx = idx; pl.val = val;
+    pl.nlong_items = (int64_t)litem.size();
+    void *a = nullptr, *b = nullptr, *c = nullptr;
+    if (ws_alloc(h, &a, sizeof(int2) * litem.size()) || ws_alloc(h, &b, sizeof(int32_t) * lseg.size()) ||
+        ws_alloc(h, &c, sizeof(int64_t) * lslot.size()) || ws_alloc(h, &pl.slots, h->es * litem.size() * (size_t)h->k) ||
+        ws_alloc(h, (void**)&pl.counters, sizeof(unsigned) * lseg.size()))
+        return 1;
+    CK(cudaStreamSynchronize(0));          // (the zero-fills above ran on the legacy default stream)
+    if (!litem.empty()) {
+        CK(cudaMemcpy(a, litem.data(), sizeof(int2) * litem.size(), cudaMemcpyHostToDevice));
+        CK(cudaMemcpy(b, lseg.data(), sizeof(int32_t) * lseg.size(), cudaMemcpyHostToDevice));
+        CK(cudaMemcpy(c, lslot.data(), sizeof(int64_t) * lslot.size(), cudaMemcpyHostToDevice));
+    }
+    pl.litem = (const int2*)a; pl.lseg = (const int32_t*)b; pl.lslot = (const int64_t*)c;
+    return 0;
+}
+
+template <typename T>
+static int bind_csr_zero_impl(rri_handle_t h, const int64_t* rowptr, const int32_t* col, const T* val, cudaStream_t st)
+{
+    const int64_t n = h->n, d = h->d, nnz = h->nnz;
+    const size_t ne = (size_t)(nnz > 0 ? nnz : 1);
+    size_t op = 8 * (size_t)h->sm_count;
+    if (op < 512) op = 512;
+    if (ws_alloc(h, (void**)&h->obj_part, sizeof(double) * op) || ws_alloc(h, (void**)&h->obj_out, sizeof(double) * 16)) return 1;
+    void *csc_row = nullptr, *x_csc = nullptr, *colptr = nullptr;
+    if (ws_alloc(h, &csc_row, sizeof(int32_t) * ne) || ws_alloc(h, &x_csc, sizeof(T) * ne) ||
+        ws_alloc(h, &colptr, sizeof(int64_t) * (size_t)(d + 1)) || ws_alloc(h, (void**)&h->sp_err, sizeof(int)))
+        return 1;
+    h->splits_w = 1; h->splits_t = 1;
+    if (alloc_halfstep_ws(h)) return 1;
+    CK(cudaStreamSynchronize(0));
+    // the CSR position of every CSC entry is only needed while the column orientation is built
+    uint32_t* perm = nullptr;
+    CK(cudaMalloc(&perm, sizeof(uint32_t) * ne));
+    const int rc = sp_build_csc<T>(rowptr, col, val, nullptr, n, d, nnz, (int64_t*)colptr, (int32_t*)csc_row, (T*)x_csc,
+                                   nullptr, perm, h->sm_count, h->sp_err, st);
+    cudaFree(perm);
+    if (rc < 0)
+        return fail("malformed CSR input:%s%s%s", (-rc & 1) ? " rowptr is not a monotone [0..nnz] sequence;" : "",
+                    (-rc & 2) ? " column index outside [0,d);" : "",
+                    (-rc & 4) ? " column indices must be strictly ascending inside every row (sort and merge duplicates);" : "");
+    if (rc > 0) return fail("building the column orientation failed: %s", cudaGetErrorString((cudaError_t)rc));
+    h->launches += 8;
+    if (build_spmm_plan(h, h->zrow, n, rowptr, col, val) ||
+        build_spmm_plan(h, h->zcol, d, (const int64_t*)colptr, (const int32_t*)csc_row, x_csc))
+        return 1;
+    CKL();
+    CK(cudaStreamSynchronize(st));
+    return 0;
+}
+
+extern "C" int rri_bind_csr_zero(rri_handle_t h, int64_t nnz, const int64_t* rowptr_dev, const int32_t* col_dev,
+                                 const void* val_dev, void* stream)
+{
+    if (!h) return fail("null handle");
+    if (h->X) return fail("the handle is already bound; create a new one");
+    if (nnz < 0 || nnz >= ((int64_t)1 << 31)) return fail("nnz must be in [0, 2^31) (got %lld)", (long long)nnz);
+    if (!rowptr_dev) return fail("rowptr is null");
+    if (nnz > 0 && (!col_dev || !val_dev)) return fail("col/val is null");
+    if (h->order != RRI_ORDER_HALS) return fail("zero-filled sparse data runs in block order: create the handle with RRI_ORDER_HALS");
+    if (h->math != RRI_MATH_IEEE) return fail("zero-filled sparse data runs with RRI_MATH_IEEE (the sparse contraction is not compute-bound)");
+    CK(cudaSetDevice(h->device));
+    h->nnz = nnz;
+    cudaStream_t st = (cudaStream_t)stream;
+    const int rc = h->dtype == RRI_F32 ? bind_csr_zero_impl<float>(h, rowptr_dev, col_dev, (const float*)val_dev, st)
+                                       : bind_csr_zero_impl<double>(h, rowptr_dev, col_dev, (const double*)val_dev, st);
+    if (rc) return rc;
+    h->zero_csr = true;
     h->X = val_dev ? val_dev : (const void*)rowptr_dev;      // "bound" marker; the dense kernels never see it
     return 0;
 }
@@ -826,7 +938,12 @@ static int hals_W_half(rri_handle_t h, T* W, const T* Tk, int64_t ldtk, const rr
         // C2 = X T' and H = T T' (from the d x k transposed copy, or as the Gram tile of the contraction)
         const bool tc_gram = gram_in_contraction(h);
         if (!tc_gram) { launch_gram<T>((const T*)h->Tt, d, k, (T*)h->gram_part, h->gchunks_t, (T*)h->Hm, st); h->launches += 2; }
-        if (contraction<T>(h, (const T*)h->X, h->ldx, Tk, ldtk, (T*)h->Cpart, n, k, d, h->splits_w, st, tc_gram ? (T*)h->Hm : nullptr)) return 1;
+        if (h->zero_csr) {
+            launch_spmm<T>(h->zrow, (const T*)h->Tt, k, (T*)h->Cpart, st);
+            h->launches++;
+        } else if (contraction<T>(h, (const T*)h->X, h->ldx, Tk, ldtk, (T*)h->Cpart, n, k, d, h->splits_w, st, tc_gram ? (T*)h->Hm : nullptr)) {
+            return 1;
+        }
     }
     const int parts = h->math == RRI_MATH_TF32 ? 1 : h->splits_w;
     // the zero-column test of nmf.py:793 is over ALL rows: with row shards the sums are all-reduced once per call
@@ -874,8 +991,13 @@ static int hals_T_half(rri_handle_t h, T* W, T* Tk, int64_t ldtk, const rri_para
     if (!tc_gram) { launch_gram<T>(W, n, k, (T*)h->gram_part, h->gchunks_w, G, st); h->launches += 2; }
     // (one rank, TF32: the Gram tile lands right behind the contraction output, as the all-reduce wants it)
     T* Cout = (h->world > 1 && psplits == 1) ? cg : (T*)h->Cpart;
-    if (contraction<T>(h, (const T*)h->Xt, h->ldxt, (const T*)h->Wt, h->ldwt, Cout, d, k, n, h->splits_t, st,
-                       tc_gram ? G : nullptr)) return 1;
+    if (h->zero_csr) {
+        launch_spmm<T>(h->zcol, W, k, Cout, st);
+        h->launches++;
+    } else if (contraction<T>(h, (const T*)h->Xt, h->ldxt, (const T*)h->Wt, h->ldwt, Cout, d, k, n, h->splits_t, st,
+                              tc_gram ? G : nullptr)) {
+        return 1;
+    }
     const T* C = Cout;
     int parts = psplits;
     if (h->world > 1) {
@@ -1293,6 +1415,7 @@ extern "C" int rri_topics(rri_handle_t h, void* W_dev, void* T_dev, int32_t t_be
     if (!h) return fail("null handle");
     if (!W_dev || !T_dev) return fail("W or T is null");
     if (check_params(h, p)) return 1;
+    if (h->zero_csr) return fail("rri_topics does not serve zero-filled sparse handles (block order only)");
     if (h->order != RRI_ORDER_RRI) return fail("rri_topics needs a handle created with RRI_ORDER_RRI");
     if (p->fix_T) return fail("rri_topics does not take fix_T");
     if (t_begin < 0 || t_end > h->k || t_begin >= t_end) return fail("bad topic range [%d,%d)", t_begin, t_end);
@@ -1320,8 +1443,12 @@ extern "C" int rri_topic_sums(rri_handle_t h, double* sum_T_host, double* sum_W_
 // objective, partial statistic, misc
 // -------------------------------------------------------------------------------------------------
 template <typename T>
+static int objective_contraction_impl(rri_handle_t h, const T* W, const T* Tm, bool reuse, cudaStream_t st);
+
+template <typename T>
 static int objective_impl(rri_handle_t h, const T* W, const T* Tm, cudaStream_t st)
 {
+    if (h->zero_csr) return objective_contraction_impl<T>(h, W, Tm, false, st);     // (no pass over n x d entries)
     if (h->sparse) {
         launch_transpose<T>(Tm, h->k, h->d, h->d, (T*)h->Tt, h->sp_ldt, st);
         sp_refresh<T>(h, true, false, W, st);
@@ -1368,17 +1495,23 @@ static int objective_contraction_impl(rri_handle_t h, const T* W, const T* Tm, b
     CK(cudaStreamSynchronize(0));
     double* acc = h->obj_out + 8;                       // {||X||^2, <X T', W>}
     if (!h->xsq_valid) {
-        launch_sumsq_rows<T>((const T*)h->X, n, d, h->ldx, h->obj_part, acc, h->sm_count, st);
+        if (h->zero_csr) launch_sumsq_rows<T>((const T*)h->zrow.val, 1, h->nnz, h->nnz, h->obj_part, acc, h->sm_count, st);
+        else launch_sumsq_rows<T>((const T*)h->X, n, d, h->ldx, h->obj_part, acc, h->sm_count, st);
         h->xsq_valid = true;
         h->launches += 2;
     }
     if (!(reuse && h->c2_valid)) {
         launch_transpose<T>(Tm, k, d, d, (T*)h->Tt, k, st);
         h->launches++;
-        if (contraction<T>(h, (const T*)h->X, h->ldx, Tm, d, (T*)h->Cpart, n, k, d, h->splits_w, st)) return 1;
+        if (h->zero_csr) {
+            launch_spmm<T>(h->zrow, (const T*)h->Tt, k, (T*)h->Cpart, st);
+            h->launches++;
+        } else if (contraction<T>(h, (const T*)h->X, h->ldx, Tm, d, (T*)h->Cpart, n, k, d, h->splits_w, st)) {
+            return 1;
+        }
         h->c2_valid = false;                            // (the caller's T may change before the next call)
     }
-    const int parts = h->math == RRI_MATH_TF32 ? 1 : h->splits_w;
+    const int parts = h->math == RRI_MATH_TF32 ? 1 : h->splits_w;      // (1 on zero-filled sparse handles)
     launch_dot_parts<T>((const T*)h->Cpart, parts, n * k, W, n * k, h->obj_part, acc + 1, h->sm_count, st);
     T* G = (T*)h->Gobj;
     T* H = G + (size_t)k * k;
@@ -1412,18 +1545,20 @@ extern "C" int rri_objective_contraction(rri_handle_t h, const void* W_dev, cons
     return 0;
 }
 
+// p[c * pstride] = (X' w_t)[c], g[j] = (W' w_t)[j]
 template <typename T>
-__global__ void partials_unmasked_kernel(const T* __restrict__ stat, const T* __restrict__ Tm, int64_t d, int k,
-                                         int t, T* __restrict__ wR, T* __restrict__ nw)
+__global__ void partials_unmasked_kernel(const T* __restrict__ p, int64_t pstride, const T* __restrict__ g,
+                                         const T* __restrict__ Tm, int64_t d, int k, int t, T* __restrict__ wR,
+                                         T* __restrict__ nw)
 {
     const int64_t c = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
     if (c < d) {
         T dot = T(0);
         for (int j = 0; j < k; ++j)
-            if (j != t) dot = fma(stat[d + j], Tm[(int64_t)j * d + c], dot);     // nmf.py:674-675
-        wR[c] = stat[c] - dot;
+            if (j != t) dot = fma(g[j], Tm[(int64_t)j * d + c], dot);            // nmf.py:674-675
+        wR[c] = p[c * pstride] - dot;
     }
-    if (c == 0) nw[0] = stat[d + t];                                                // nmf.py:676
+    if (c == 0) nw[0] = g[t];                                                       // nmf.py:676
 }
 
 template <typename T>
@@ -1445,6 +1580,18 @@ static int partials_impl(rri_handle_t h, const T* W, const T* Tm, int t, T* wR, 
         CKL();
         return 0;
     }
+    if (h->zero_csr) {
+        // X' W and W'W of the T half-step, then the statistic of topic t from column t of both
+        const int k = h->k;
+        T* G = (T*)h->cg + (size_t)d * k;
+        launch_spmm<T>(h->zcol, W, k, (T*)h->Cpart, st);
+        launch_gram<T>(W, h->n, k, (T*)h->gram_part, h->gchunks_w, G, st);
+        partials_unmasked_kernel<T><<<(unsigned)((d + 255) / 256), 256, 0, st>>>((const T*)h->Cpart + t, k, G + (size_t)t * k,
+                                                                                  Tm, d, k, t, wR, nw);
+        h->launches += 4;
+        CKL();
+        return 0;
+    }
     if (h->mk != MK_NONE) {
         launch_wrri_tstats<T>((const T*)h->X, h->ldx, h->M, h->mk, h->ldm, W, Tm, h->n, d, h->k, t,
                               (T*)h->numer_part, (T*)h->denom_part, h->tpl, st);
@@ -1455,7 +1602,8 @@ static int partials_impl(rri_handle_t h, const T* W, const T* Tm, int t, T* wR, 
         if (h->order != RRI_ORDER_RRI) return fail("rri_partials_T (unmasked) needs a handle created with RRI_ORDER_RRI");
         if (rri_prologue<T>(h, const_cast<T*>(W), t, &p, st)) return 1;     // prologue does not write W
         launch_reduce_stat<T>((const T*)h->ppart, h->pp.rg, d, (const T*)h->gpart, h->gbw, h->k, (T*)h->stat, st);
-        partials_unmasked_kernel<T><<<(unsigned)((d + 255) / 256), 256, 0, st>>>((const T*)h->stat, Tm, d, h->k, t, wR, nw);
+        partials_unmasked_kernel<T><<<(unsigned)((d + 255) / 256), 256, 0, st>>>((const T*)h->stat, 1, (const T*)h->stat + d,
+                                                                                  Tm, d, h->k, t, wR, nw);
         h->launches += 2;
     }
     CKL();
@@ -1553,6 +1701,10 @@ static int profile_impl(rri_handle_t h, int which, const T* W, const T* Tm, int 
         launch_transpose<T>(W, n, k, k, (T*)h->Wt, h->ldwt, st);
         h->launches++;
     }
+    if (which == 1 && h->zero_csr) {              // the W-half contraction gathers rows of T'
+        launch_transpose<T>(Tm, k, d, d, (T*)h->Tt, k, st);
+        h->launches++;
+    }
     rri_params_t prm;
     memset(&prm, 0, sizeof(prm));
     prm.eps = 1.7763568394002505e-15;
@@ -1599,9 +1751,11 @@ static int profile_impl(rri_handle_t h, int which, const T* W, const T* Tm, int 
             h->launches++;
         } else if (which == 1) {
             if (h->mk != MK_NONE) return fail("which=1 needs an unmasked handle");
+            if (h->zero_csr) { launch_spmm<T>(h->zrow, (const T*)h->Tt, k, (T*)h->Cpart, st); h->launches++; continue; }
             if (contraction<T>(h, (const T*)h->X, h->ldx, Tm, d, (T*)h->Cpart, n, k, d, h->splits_w, st)) return 1;
         } else if (which == 2) {
             if (h->mk != MK_NONE || h->order != RRI_ORDER_HALS) return fail("which=2 needs an unmasked hals-order handle");
+            if (h->zero_csr) { launch_spmm<T>(h->zcol, W, k, (T*)h->Cpart, st); h->launches++; continue; }
             if (contraction<T>(h, (const T*)h->Xt, h->ldxt, (const T*)h->Wt, h->ldwt, (T*)h->Cpart, d, k, n, h->splits_t, st)) return 1;
         } else if (which == 3) {
             // the whole T half-step (contraction + Gram + exchange + update); collective on row shards

@@ -274,3 +274,25 @@ int launch_sp_pass(const SpSide& s, const void* quad, const T* own_po, const T* 
 template <typename T>
 void launch_sp_objective(const SpSide& s, int64_t nnz, double* part, double* out, cudaStream_t st);
 }  // namespace rri
+
+namespace rri {
+// ---------------------------------------------------------------------------------------------
+// sparse x dense contraction on zero-filled sparse data (block order)          (spmm_kernels.cu)
+// ---------------------------------------------------------------------------------------------
+constexpr int SPMM_CHUNK = 1024;    // longest segment taken by one lane group; longer ones are cut into chunks
+struct SpmmPlan {                   // one compressed orientation and its chunk plan (built once at bind time)
+    int64_t nseg;                   // rows (CSR) or columns (CSC)
+    const int64_t* ptr;             // [nseg + 1]
+    const int32_t* idx;             // [nnz] column (CSR) / row (CSC) of every entry
+    const void* val;                // [nnz]
+    int64_t nlong_items;            // chunks of the segments longer than SPMM_CHUNK
+    const int2* litem;              // [nlong_items] {long segment, chunk}
+    const int32_t* lseg;            // [nlong] segment of long segment j
+    const int64_t* lslot;           // [nlong] first partial slot of long segment j
+    void* slots;                    // [nlong_items][k] chunk partials
+    unsigned* counters;             // [nlong] arrivals, zero between launches
+};
+// C[r, :] = sum_{e in segment r} val[e] * B[idx[e], :]   (B [., k] and C [nseg, k] row-major, one launch)
+template <typename T>
+void launch_spmm(const SpmmPlan& p, const T* B, int k, T* C, cudaStream_t st);
+}  // namespace rri

@@ -52,13 +52,15 @@ class RRIEngine(object):
 
     X: torch tensor [n_local, d] on a CUDA device, float32 or float64, row-major (a row stride >= d
     is allowed).  W_mat: optional weights, same shape (same dtype, or uint8 0/1 mask).
-    X may also be a torch sparse CSR tensor: its stored entries are the observed ones (the recommender
-    setting, never densified); W_mat is then an optional 1-D tensor of nnz entry weights.
+    X may also be a torch sparse CSR tensor (never densified).  unstored='missing' (default): its stored entries are
+    the observed ones (the recommender setting); W_mat is then an optional 1-D tensor of nnz entry weights.
+    unstored='zero': X is an ordinary non-negative matrix stored sparsely (a tf-idf document-term matrix), every entry
+    is fitted, the unstored ones as 0 (rri_bind_csr_zero: order='hals', math='ieee', no W_mat).
     order: 'rri' (reference-exact interleaved order, nmf.py:415-476) or 'hals' (block order).
     math : 'ieee' or 'tf32' (tcgen05 tensor-core contraction; float32 + hals only).
     """
 
-    def __init__(self, X, k, W_mat=None, order='rri', math='ieee', comm=None):
+    def __init__(self, X, k, W_mat=None, order='rri', math='ieee', comm=None, unstored='missing'):
         if not isinstance(X, torch.Tensor) or not X.is_cuda:
             raise _lib.RriError('RRIEngine needs X resident on a CUDA device (no CPU fallback)')
         if X.dim() != 2:
@@ -68,6 +70,16 @@ class RRIEngine(object):
         self.sparse = X.layout == torch.sparse_csr
         if not self.sparse and X.layout != torch.strided:
             raise ValueError('X must be a dense (strided) or a sparse CSR tensor')
+        if unstored not in ('missing', 'zero'):
+            raise ValueError("unstored must be 'missing' or 'zero'")
+        if unstored == 'zero' and self.sparse:
+            if order != 'hals':
+                raise NotImplementedError("zero-filled sparse X runs in block order: use order='hals' (or X.to_dense())")
+            if math != 'ieee':
+                raise ValueError("zero-filled sparse X runs with math='ieee' (the sparse contraction is not compute-bound)")
+            if W_mat is not None:
+                raise ValueError('zero-filled sparse X takes no W_mat (weights on every entry would be a dense n x d object)')
+        self.unstored = unstored if self.sparse else 'missing'
         if not self.sparse and X.stride(1) != 1:
             X = X.contiguous()
         self.lib = _lib.load()
@@ -128,13 +140,19 @@ class RRIEngine(object):
 
     def _bind_csr(self, X, weights):
         """Observed-entries binding (rri_bind_csr): X is a torch sparse CSR tensor whose stored entries are the
-        observed ones; `weights` (optional) is a 1-D tensor of nnz entry weights in the order of X.values()."""
+        observed ones; `weights` (optional) is a 1-D tensor of nnz entry weights in the order of X.values().
+        With unstored='zero': the zero-filled binding (rri_bind_csr_zero)."""
         if self.math != 'ieee':
             raise ValueError("sparse (observed-entries) data runs with math='ieee'")
         self.crow = X.crow_indices().to(torch.int64).contiguous()
         self.col = X.col_indices().to(torch.int32).contiguous()
         self.val = X.values().contiguous()
         self.nnz = int(self.val.numel())
+        if self.unstored == 'zero':
+            self.entry_weights = None
+            check(self.lib.rri_bind_csr_zero(self.h, self.nnz, _ptr(self.crow), _ptr(self.col), _ptr(self.val),
+                                             self._stream()))
+            return
         self.entry_weights = None
         if weights is not None:
             if weights.dim() != 1 or int(weights.numel()) != self.nnz:
@@ -157,7 +175,7 @@ class RRIEngine(object):
     @property
     def masked(self):
         """True when only a subset of the entries is fitted (dense W_mat or sparse observed entries)"""
-        return self.sparse or self.W_mat is not None
+        return (self.sparse and self.unstored == 'missing') or self.W_mat is not None
 
     def _setup_peer_exchange(self, comm):
         """Map every rank's exchange buffer (CUDA IPC over NVLink) so that the T half-step reads the shard

@@ -26,9 +26,17 @@ Additional keyword-only arguments select the device path:
                   sklearn, as the reference does), None (default) = on the device when X is already a CUDA tensor or
                   has 2^26 or more elements, on the host otherwise.  Sparse X is always initialised on the host.
 
-X may also be a scipy.sparse matrix or a torch sparse CSR tensor: its STORED entries are the observed ones (the
-recommender setting of sklearn_interface.py:78-102 without densifying the (i, j, rating) triples and without a
-dense W_mat); W_mat is then None or a sparse matrix of the same structure holding entry weights.
+X may also be a scipy.sparse matrix or a torch sparse CSR tensor, never densified.  What its unstored entries mean is
+set by the keyword-only argument `unstored`:
+    'missing' (default)  the STORED entries are the observed ones (the recommender setting of
+                  sklearn_interface.py:78-102 without densifying the (i, j, rating) triples and without a dense W_mat);
+                  W_mat is then None or a sparse matrix of the same structure holding entry weights.
+    'zero'        X is an ordinary non-negative matrix stored sparsely (a tf-idf document-term matrix): every entry is
+                  fitted, the unstored ones as 0 -- the result equals nmf(X.toarray(), ..., update_order='hals',
+                  math='ieee') up to the summation order.  Needs update_order='hals' (fix_T=True runs in either order),
+                  math='ieee' and no W_mat; the block-order half-steps take X T' and X' W from a sparse x dense
+                  contraction whose traffic grows with the stored entries, not with n * d.  Topic reset is not applied
+                  (an emptied topic raises, as on the dense block order).
 """
 import logging
 import time
@@ -67,14 +75,16 @@ class DeviceObjective(object):
                                              reuse_last_sweep=self._after_sweep, **self.regs)
             self._after_sweep = False
         elif self._rebuild is not None:
-            X, W_mat, device, dtype, order = self._rebuild
+            X, W_mat, device, dtype, order, unstored = self._rebuild
             device = torch.device(device)
             with torch.cuda.device(device):
                 if _is_sparse(X):
                     Xd, Md = _sparse_to_device(X, W_mat, device, dtype)
                 else:
                     Xd, Md = _to_device(X, device, dtype), _mask_to_device(W_mat, device, dtype)
-                eng = RRIEngine(Xd, int(np.shape(self.W)[1]), W_mat=Md, order='rri')
+                # (the zero-filled sparse binding exists in block order only; every other binding evaluates in 'rri')
+                eng = RRIEngine(Xd, int(np.shape(self.W)[1]), W_mat=Md, order='hals' if unstored == 'zero' else 'rri',
+                                unstored=unstored)
                 try:
                     self.obj = eng.objective(_to_device(self.W, device, dtype).contiguous(),
                                              _to_device(self.T, device, dtype).contiguous(), **self.regs)
@@ -82,11 +92,11 @@ class DeviceObjective(object):
                     eng.close()
         return self.obj
 
-    def _detach(self, X, W_mat, W, T, device, dtype, order):
+    def _detach(self, X, W_mat, W, T, device, dtype, order, unstored='missing'):
         """called by nmf() before it closes the engine"""
         self.engine = None
         self.W, self.T = W, T
-        self._rebuild = (X, W_mat, str(device), dtype, order)
+        self._rebuild = (X, W_mat, str(device), dtype, order, unstored)
 
     def __getstate__(self):
         st = dict(self.__dict__)
@@ -286,7 +296,8 @@ def nmf(X, k, w_row=None, W_mat=None, fix_W=False, fix_T=False, random_state=Non
         n_resets=23, reg_w_l2=0, reg_t_l2=0, reg_w_l1=0, reg_t_l1=0, diagnostics=[], store_gradients=False,
         ind_rows_to_store=None, eps_gauss_t=None, delta_gauss_t=None,
         *, device=None, update_order='rri', math='ieee', comm=None, engine=None, sweeps_per_call=16,
-        init_on_device=None, return_reconstruction_err=False, sparse_refresh_every=1, objective='auto'):
+        init_on_device=None, return_reconstruction_err=False, sparse_refresh_every=1, objective='auto',
+        unstored='missing'):
     """Non-negative factorisation X ~ W T by rank-one residue iteration.  See the reference docstring
     (nmf.py:109-269) for the arguments; returns {'W', 'T', 'iter_cputime', 'random_state'[, 'obj_history',
     'obj_calculator', 'diagnostics']} (nmf.py:551-560).  W and T come back as the kind of array X was
@@ -295,6 +306,19 @@ def nmf(X, k, w_row=None, W_mat=None, fix_W=False, fix_T=False, random_state=Non
     del lib
     if update_order not in ('rri', 'hals'):
         raise ValueError("update_order must be 'rri' or 'hals'")
+    if unstored not in ('missing', 'zero'):
+        raise ValueError("unstored must be 'missing' or 'zero'")
+    zero_filled = unstored == 'zero' and _is_sparse(X)
+    if zero_filled:
+        if W_mat is not None:
+            raise ValueError("unstored='zero' takes no W_mat: weights on a zero-filled matrix would be a dense n x d object")
+        if math != 'ieee':
+            raise ValueError("unstored='zero' runs with math='ieee' (the sparse contraction is not compute-bound)")
+        if fix_W:
+            raise NotImplementedError("fix_W=True is not available with unstored='zero'")
+        if update_order != 'hals' and not fix_T:
+            raise NotImplementedError("unstored='zero' runs in block order: use update_order='hals', or densify with "
+                                      "X.toarray() for the interleaved order")
     n, d = X.shape
     rtv = {}
     numpy_io = not isinstance(X, torch.Tensor)
@@ -423,7 +447,9 @@ def nmf(X, k, w_row=None, W_mat=None, fix_W=False, fix_T=False, random_state=Non
         _t1 = time.perf_counter()
         own_engine = engine is None
         if engine is None:
-            engine = RRIEngine(Xd, k, W_mat=Md, order=update_order, math=math, comm=comm)
+            # (fix_T: the W-only sweeps are the same in both orders; the zero-filled binding is a block-order one)
+            engine = RRIEngine(Xd, k, W_mat=Md, order='hals' if zero_filled else update_order, math=math, comm=comm,
+                               unstored=unstored)
         timing['engine_setup_s'] = time.perf_counter() - _t1       # workspace, transposed copy of X, peer mapping
         try:
             if init_on_device:
@@ -457,7 +483,8 @@ def nmf(X, k, w_row=None, W_mat=None, fix_W=False, fix_T=False, random_state=Non
                 out['reconstruction_err'] = float(np.sqrt(2.0 * engine.objective_terms(Wd, Td)[0]))
             if 'obj_calculator' in out and own_engine:
                 # the calculator outlives this call without pinning device memory (and stays picklable)
-                out['obj_calculator']._detach(X, W_mat_user, out['W'], out['T'], device, dtype, update_order)
+                out['obj_calculator']._detach(X, W_mat_user, out['W'], out['T'], device, dtype, engine.order,
+                                              engine.unstored)
             return out
         finally:
             if own_engine:

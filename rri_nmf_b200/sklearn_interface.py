@@ -7,6 +7,10 @@ plus the sklearn-conventional read-only aliases `components_` (= T), `n_componen
 Additional constructor arguments: `device`, `update_order`, `math` (forwarded to `nmf`); `NMF_RS_Estimator` also
 takes `sparse=True` to keep the (i, j, rating) triples sparse all the way to the device (observed-entries engine,
 traffic proportional to the number of ratings) instead of densifying them as the reference does.
+
+`NMF_TM_Estimator` takes scipy.sparse document-term matrices in fit, fit_transform, one_iter, transform and score.  With
+update_order='hals' X stays sparse all the way to the device (nmf(..., unstored='zero'): unstored entries are zeros);
+with the default update_order='rri' the estimator densifies X and runs the reference-exact interleaved order.
 """
 import numpy as np
 import scipy.sparse as sp
@@ -24,6 +28,18 @@ _EMPTY = np.array([])
 
 def _np(a):
     return a.detach().cpu().numpy() if isinstance(a, torch.Tensor) else a
+
+
+def _r2_sparse(X, W, T):
+    """1 - SSE / SST of sklearn_interface.py:339-345 for a scipy.sparse X without an n x d temporary, in fp64:
+    SST = ||X||^2 - n ||mean||^2,  SSE = ||X||^2 - 2 <X T', W> + <W'W, T T'>"""
+    W = np.asarray(W, dtype=np.float64)
+    T = np.asarray(T, dtype=np.float64)
+    xsq = float(X.multiply(X).sum())
+    mean = np.asarray(X.mean(axis=0)).ravel()
+    SST = xsq - X.shape[0] * float(mean @ mean)
+    SSE = xsq - 2.0 * float(np.sum(np.asarray(X @ T.T) * W)) + float(np.sum((W.T @ W) * (T @ T.T)))
+    return 1 - SSE / SST
 
 
 class _FactorMixin(object):
@@ -81,8 +97,22 @@ class NMF_TM_Estimator(_FactorMixin, sklearn.base.BaseEstimator, sklearn.base.Tr
         self.do_final_project_W = do_final_project_W
         self.device, self.update_order, self.math = device, update_order, math
 
+    def _keep_sparse(self, X):
+        """sparse X goes to the device as it is in block order; the interleaved order runs on its dense form"""
+        return sp.issparse(X) and self.update_order == 'hals'
+
     def _prep(self, X, fit):
-        X = np.asarray(_np(X))
+        if self._keep_sparse(X):
+            X = sp.csr_matrix(X)
+            if self.handle_tfidf:
+                if fit:
+                    X, self.idf = tfidf(X, return_idf=True)
+                else:
+                    X = X.multiply(self.idf[None, :]).tocsr()
+            if self.handle_normalization:
+                X = normalize(X)
+            return X
+        X = np.asarray(X.toarray() if sp.issparse(X) else _np(X))
         if self.handle_tfidf:
             if fit:
                 X, self.idf = tfidf(X, return_idf=True)
@@ -96,6 +126,8 @@ class NMF_TM_Estimator(_FactorMixin, sklearn.base.BaseEstimator, sklearn.base.Tr
         W_in, T_in = self._warm_start()
         X = self._prep(X, fit=True)
         kw = dict(self._device_kwargs())
+        if sp.issparse(X):
+            kw['unstored'] = 'zero'
         kw.update(self.nmf_kwargs)
         # sklearn_interface.py:269-276 / :300-308
         soln = nmf(X, self.k, max_iter=max_iter, max_time=max_time, project_W_each_iter=False, w_row_sum=1.0,
@@ -111,7 +143,8 @@ class NMF_TM_Estimator(_FactorMixin, sklearn.base.BaseEstimator, sklearn.base.Tr
         return self
 
     def fit_transform(self, X, y=None):
-        assert np.all(np.asarray(_np(X)) >= 0), 'X must be non-negative'      # sklearn_interface.py:251
+        Xv = X.data if sp.issparse(X) else np.asarray(_np(X))
+        assert np.all(Xv >= 0), 'X must be non-negative'                      # sklearn_interface.py:251
         self._run(X, self.max_iter, 7200)
         return self.W
 
@@ -126,18 +159,23 @@ class NMF_TM_Estimator(_FactorMixin, sklearn.base.BaseEstimator, sklearn.base.Tr
     def transform(self, Xnew):
         """express Xnew in terms of the fitted topics: 4 W-only sweeps (sklearn_interface.py:320-334)"""
         Xnew = self._prep(Xnew, fit=False)
+        kw = dict(self._device_kwargs(), unstored='zero') if sp.issparse(Xnew) else self._device_kwargs()
         soln = nmf(Xnew, self.k, max_iter=4, max_time=7200, project_W_each_iter=False, w_row_sum=1.0,
                    t_row_sum=1.0, T_in=self.T, do_final_project_W=self.do_final_project_W, fix_T=True,
                    reg_w_l1=self.wr1, reg_w_l2=self.wr2, reg_t_l1=self.tr1, reg_t_l2=self.tr2,
-                   random_state=self.random_state, **self._device_kwargs())
+                   random_state=self.random_state, **kw)
         return soln['W']
 
     def constrained_transform(self, X):
         return self.transform(X)
 
     def score(self, X, y=None):
-        """R^2 of the reconstruction of new X (sklearn_interface.py:339-345)"""
-        X = np.asarray(_np(X))
+        """R^2 of the reconstruction of new X (sklearn_interface.py:339-345).  Sparse X in block order: no n x d array
+        is formed -- SST = ||X||^2 - n ||mean||^2 and SSE = ||X||^2 - 2 <X T', W> + <W'W, T T'>, in fp64 on the host."""
+        if self._keep_sparse(X):
+            X = sp.csr_matrix(X, dtype=np.float64)
+            return _r2_sparse(X, self.transform(X), self.T)
+        X = np.asarray(X.toarray() if sp.issparse(X) else _np(X))
         SST = ((X - np.mean(X, axis=0)) ** 2).sum()
         W = self.transform(X)
         SSE = ((X - np.dot(W, self.T)) ** 2).sum()
