@@ -122,6 +122,19 @@ int rri_bind_csr(rri_handle_t h, int64_t nnz, const int64_t* rowptr_dev, const i
 int rri_bind_csr_zero(rri_handle_t h, int64_t nnz, const int64_t* rowptr_dev, const int32_t* col_dev,
                       const void* val_dev, void* stream);
 
+/* Sparse x dense product on a sparse handle (rri_bind_csr or rri_bind_csr_zero), for the randomized SVD of the NNDSVD
+ * initialisation (nmf.py:840-843 initialises on W_mat o X):
+ *     transpose = 0:  C[n_local, width] = X  B[d, width]        (over the CSR rows)
+ *     transpose = 1:  C[d, width]       = X' B[n_local, width]  (over the CSC columns)
+ * B and C are row-major with leading dimensions ldb, ldc >= width (in elements), element type of the handle, device
+ * memory.  X is the zero-filled matrix of the stored entries; on an observed-entries handle with entry weights it is
+ * w o x.  Operands wider than 256 columns run as panels of 256 columns, one launch each.  Summation order is fixed
+ * (no float atomics): repeated calls give identical bits.  An observed-entries handle builds its chunk plans (and, with
+ * weights, a weighted copy of the values: 2 * nnz elements, freed with the handle) on its first call, which
+ * synchronises `stream`.  Calls and sweeps on one handle must be issued on one stream. */
+int rri_spmm(rri_handle_t h, int32_t transpose, const void* B_dev, int64_t ldb, void* C_dev, int64_t ldc, int32_t width,
+             void* stream);
+
 /* Run n_sweeps full sweeps in place on W_dev[n_local,k], T_dev[k,d]:  nmf.py:377, :415-476
  * (+ masked branches :687-701, :735-746; qf_min optimization.py:51-59, :75-87).
  * flags_host (may be NULL): receives the OR of RRI_FLAG_* over all sweeps (forces a stream sync).

@@ -8,6 +8,11 @@ streaming passes over it run through the engine's own contraction kernel (rri_ge
 GEMMs only when no engine is at hand: CPU tensors, the masked product W_mat o X), the small factorisations are
 `torch.linalg.qr/svd`.  The same torch code runs on CPU tensors, which is how it is checked
 against `_host.initialize_nmf` without a GPU (tests/test_device_init_cpu.py).
+
+X may also be a torch sparse CSR tensor.  It is never densified: shape, dtype and device come from the tensor, the means
+of 'nndsvda' / 'nndsvdar' / 'smart_random' are (sum of the stored values) / (n*d), and on a CUDA device the products
+must come from the sweep engine (`RRIEngine.products` on a sparse handle: rri_spmm, the SpMM kernel of the zero-filled
+block order).  The workspace is O((n + d) * (k + 10) + nnz).
 """
 import numpy as np
 import torch
@@ -24,10 +29,23 @@ def _span_normalize(A):
     return Q
 
 
+def _is_sparse(M):
+    return M.layout != torch.strided
+
+
+def _mean(M):
+    """mean over all n*d entries; the unstored entries of a sparse M are zeros"""
+    if _is_sparse(M):
+        return M.values().sum() / (M.shape[0] * M.shape[1])
+    return M.mean()
+
+
 class _TorchProducts(object):
     """the two streaming products of the randomized SVD as library GEMMs (CPU tensors, or no engine at hand)"""
 
     def __init__(self, M):
+        if _is_sparse(M) and M.is_cuda:
+            raise ValueError('a sparse X on a CUDA device needs the engine products (RRIEngine.products: rri_spmm)')
         self.M = M
 
     def right(self, Q):          # M @ Q      [n, r]
@@ -41,8 +59,8 @@ def randomized_svd_torch(M, n_components, random_state=None, n_oversamples=10, p
     """sklearn.utils.extmath.randomized_svd(M, n_components, random_state=...) with its defaults
     (n_iter='auto', transpose='auto', flip_sign=True; the power iterations are re-orthonormalised by a thin QR where
     sklearn's 'auto' uses LU -- same subspace) on M's device.
-    M: dense 2-D torch tensor (float32 or float64); it is only ever used as a GEMM operand (no copy, no transpose
-    materialised).  `products` (optional): object with right(Q) = M @ Q and left(Q) = M' @ Q -- the sweep engine's
+    M: dense 2-D torch tensor (float32 or float64) or sparse CSR tensor; it is only ever used as a product operand (no
+    copy, no transpose materialised).  `products` (optional): object with right(Q) = M @ Q and left(Q) = M' @ Q -- the sweep engine's
     own streaming contraction (`RRIEngine.products`, rri_gemm_nt: the tcgen05 kernel in TF32 mode, the IEEE SIMT
     kernel otherwise) -- so that the 2*n_iter + 2 passes over X run through the repo's kernels.
     Returns (U[n,k], s[k], Vt[k,d])."""
@@ -65,10 +83,21 @@ def randomized_svd_torch(M, n_components, random_state=None, n_oversamples=10, p
         Q = normalize(A_mm(Q))
         Q = normalize(At_mm(Q))
     Q, _ = torch.linalg.qr(A_mm(Q), mode='reduced')
-    B = At_mm(Q).t()                         # Q'A as the transpose of A'Q
-    Uhat, s, Vt = torch.linalg.svd(B, full_matrices=False)
-    del B
+    Bt = At_mm(Q)                            # A'Q, the transpose of Q'A
+    if _is_sparse(M):
+        # The factors of a sparse X can be far larger than X: the SVD of the r x A_cols matrix Q'A through a thin QR
+        # of its transpose, A'Q = Qb Rb, and the r x r SVD of Rb' (a library SVD of the wide matrix itself needs
+        # several copies of it).  Same factorisation up to rounding; the signs are fixed by svd_flip below.
+        Qb, Rb = torch.linalg.qr(Bt, mode='reduced')
+        del Bt
+        Uhat, s, Vrt = torch.linalg.svd(Rb.t())
+        Vt = Vrt @ Qb.t()
+        del Qb
+    else:
+        Uhat, s, Vt = torch.linalg.svd(Bt.t(), full_matrices=False)
+        del Bt
     U = Q @ Uhat
+    del Q
     # svd_flip: u_based_decision unless transposed (then the rows of Vt are the columns of the caller's U)
     if not transpose:
         idx = U.abs().argmax(dim=0)
@@ -76,8 +105,8 @@ def randomized_svd_torch(M, n_components, random_state=None, n_oversamples=10, p
     else:
         idx = Vt.abs().argmax(dim=1)
         signs = torch.sign(Vt[torch.arange(Vt.shape[0], device=Vt.device), idx])
-    U = U * signs[None, :]
-    Vt = Vt * signs[:, None]
+    U.mul_(signs[None, :])
+    Vt.mul_(signs[:, None])
     k = n_components
     if transpose:
         return Vt[:k, :].t(), s[:k], U[:, :k].t()
@@ -85,7 +114,7 @@ def randomized_svd_torch(M, n_components, random_state=None, n_oversamples=10, p
 
 
 def initialize_nmf_torch(X, n_components, init=None, eps=1e-6, random_state=None, products=None):
-    """initialize_nmf (initialization.py:9-163, `_host.initialize_nmf`) for a dense torch tensor X on any device;
+    """initialize_nmf (initialization.py:9-163, `_host.initialize_nmf`) for a dense or sparse CSR torch tensor X on any device;
     returns torch tensors (W[n,k], T[k,d]) on X's device.  'random' / 'smart_random' draw from the NumPy generator
     on the host exactly like the reference (n*k + k*d numbers) and upload."""
     n, d = X.shape
@@ -100,7 +129,7 @@ def initialize_nmf_torch(X, n_components, init=None, eps=1e-6, random_state=None
         return torch.from_numpy(W).to(dev), torch.from_numpy(T).to(dev)
     if init == 'smart_random':
         rng = _rng(random_state)
-        scale = float(torch.sqrt(X.mean() / k))
+        scale = float(torch.sqrt(_mean(X) / k))
         T = np.abs(scale * rng.randn(k, d))
         W = np.abs(scale * rng.randn(n, k))
         return torch.from_numpy(W).to(dev), torch.from_numpy(T).to(dev)
@@ -111,29 +140,27 @@ def initialize_nmf_torch(X, n_components, init=None, eps=1e-6, random_state=None
     U, Vt = U.contiguous(), Vt.contiguous()
     # every singular pair is split into its positive and negative parts; per component the sign pattern carrying
     # more mass is kept (initialization.py:113-139); the leading pair is used as is up to sign (:108-109)
-    Up, Un = U.clamp(min=0), (-U).clamp(min=0)
-    Vp, Vn = Vt.clamp(min=0), (-Vt).clamp(min=0)
-    nup, nun = torch.linalg.norm(Up, dim=0), torch.linalg.norm(Un, dim=0)
-    nvp, nvn = torch.linalg.norm(Vp, dim=1), torch.linalg.norm(Vn, dim=1)
+    # (one n x k / k x d temporary at a time: the factors of a sparse X can be far larger than X)
+    nup, nun = torch.linalg.norm(U.clamp(min=0), dim=0), torch.linalg.norm((-U).clamp(min=0), dim=0)
+    nvp, nvn = torch.linalg.norm(Vt.clamp(min=0), dim=1), torch.linalg.norm((-Vt).clamp(min=0), dim=1)
     mp, mn = nup * nvp, nun * nvn
     pos = mp > mn
     tiny = torch.finfo(dt).tiny
-    u = torch.where(pos[None, :], Up / nup.clamp(min=tiny)[None, :], Un / nun.clamp(min=tiny)[None, :])
-    v = torch.where(pos[:, None], Vp / nvp.clamp(min=tiny)[:, None], Vn / nvn.clamp(min=tiny)[:, None])
+    sgn = torch.where(pos, 1.0, -1.0).to(dt)
     lam = torch.sqrt(S * torch.where(pos, mp, mn))
-    W = u * lam[None, :]
-    T = v * lam[:, None]
+    W = (U * sgn[None, :]).clamp_(min=0).div_(torch.where(pos, nup, nun).clamp(min=tiny)[None, :]).mul_(lam[None, :])
+    T = (Vt * sgn[:, None]).clamp_(min=0).div_(torch.where(pos, nvp, nvn).clamp(min=tiny)[:, None]).mul_(lam[:, None])
     W[:, 0] = torch.sqrt(S[0]) * U[:, 0].abs()
     T[0, :] = torch.sqrt(S[0]) * Vt[0, :].abs()
     W[W < eps] = 0
     T[T < eps] = 0
     if init == 'nndsvda':
-        avg = X.mean()
+        avg = _mean(X)
         W[W == 0] = avg
         T[T == 0] = avg
     elif init == 'nndsvdar':
         rng = _rng(random_state)
-        avg = float(X.mean())
+        avg = float(_mean(X))
         zw, zt = W == 0, T == 0
         # the reference fills W's zeros first, then T's, in C order (initialization.py:150-151)
         W[zw] = torch.from_numpy(np.abs(avg * rng.randn(int(zw.sum())) / 100)).to(device=dev, dtype=dt)

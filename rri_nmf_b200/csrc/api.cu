@@ -179,6 +179,10 @@ struct rri_handle_s {
     // half-steps take X T' / X' W from launch_spmm instead of the dense contraction
     bool zero_csr = false;
     SpmmPlan zrow{}, zcol{};
+    // rri_spmm: chunk plans of an observed-entries handle (built on its first call, over w o x when weights were given)
+    // and chunk slots for panels wider than k ([max chunks][spmm_slot_w], grown on demand)
+    bool spmm_planned = false;
+    void* spmm_slots = nullptr; int spmm_slot_w = 0;
     // common
     double* sums = nullptr;    // [2k] device
     int* flags = nullptr;      // device
@@ -198,6 +202,16 @@ static int ws_alloc(rri_handle_t h, void** p, size_t bytes)
     h->allocs.push_back(*p);
     h->ws_bytes += (int64_t)bytes;
     return 0;
+}
+
+// returns one ws_alloc block to the device block cache (nothing of this handle may still use it)
+static void ws_release(rri_handle_t h, void* p, size_t bytes)
+{
+    if (bytes == 0) bytes = 16;
+    for (size_t i = 0; i < h->allocs.size(); ++i)
+        if (h->allocs[i] == p) { h->allocs.erase(h->allocs.begin() + (long)i); break; }
+    cached_free(p);
+    h->ws_bytes -= (int64_t)bytes;
 }
 
 extern "C" int rri_create(rri_handle_t* out, int64_t n_local, int64_t d, int32_t k, int32_t dtype,
@@ -799,6 +813,83 @@ extern "C" int rri_bind_csr_zero(rri_handle_t h, int64_t nnz, const int64_t* row
     return 0;
 }
 
+// -------------------------------------------------------------------------------------------------
+// rri_spmm: the sparse x dense products of a randomized SVD (NNDSVD initialisation) through launch_spmm
+// -------------------------------------------------------------------------------------------------
+// An observed-entries handle gets the chunk plans of the zero-filled binding on its first call, built by the same code
+// over its CSR and CSC.  With entry weights the plans run over a weighted copy of the values (w o x in both
+// orientations, 2 * nnz elements, freed with the handle): the product is then the reference's W_mat o X.
+template <typename T>
+static int spmm_plan_observed(rri_handle_t h, cudaStream_t st)
+{
+    const void* vrow = h->csr.x;
+    const void* vcol = h->csc.x;
+    if (h->csr.wgt) {
+        void *wr = nullptr, *wc = nullptr;
+        const size_t ne = (size_t)(h->nnz > 0 ? h->nnz : 1);
+        if (ws_alloc(h, &wr, sizeof(T) * ne) || ws_alloc(h, &wc, sizeof(T) * ne)) return 1;
+        CK(cudaStreamSynchronize(0));          // (the zero-fills above ran on the legacy default stream)
+        launch_spmm_weighted_values<T>((const T*)h->csr.x, (const T*)h->csr.wgt, h->nnz, (T*)wr, h->sm_count, st);
+        launch_spmm_weighted_values<T>((const T*)h->csc.x, (const T*)h->csc.wgt, h->nnz, (T*)wc, h->sm_count, st);
+        h->launches += 2;
+        CKL();
+        vrow = wr; vcol = wc;
+    }
+    if (build_spmm_plan(h, h->zrow, h->n, h->csr.ptr, h->csr.idx, vrow) ||
+        build_spmm_plan(h, h->zcol, h->d, h->csc.ptr, h->csc.idx, vcol))
+        return 1;
+    h->spmm_planned = true;
+    return 0;
+}
+
+template <typename T>
+static int spmm_impl(rri_handle_t h, int transpose, const T* B, int64_t ldb, T* C, int64_t ldc, int width, cudaStream_t st)
+{
+    if (!h->zero_csr && !h->spmm_planned && spmm_plan_observed<T>(h, st)) return 1;
+    SpmmPlan pl = transpose ? h->zcol : h->zrow;
+    const int pw = width < SPMM_PANEL ? width : SPMM_PANEL;
+    if (pw > h->k) {
+        // the plan's own slots are [chunks][k]: wider panels use the handle's second slot buffer
+        if (pw > h->spmm_slot_w) {
+            const int64_t items = h->zrow.nlong_items > h->zcol.nlong_items ? h->zrow.nlong_items : h->zcol.nlong_items;
+            if (h->spmm_slots) {
+                CK(cudaStreamSynchronize(st));
+                ws_release(h, h->spmm_slots, sizeof(T) * (size_t)items * (size_t)h->spmm_slot_w);
+                h->spmm_slots = nullptr; h->spmm_slot_w = 0;
+            }
+            if (ws_alloc(h, &h->spmm_slots, sizeof(T) * (size_t)items * (size_t)pw)) return 1;
+            CK(cudaStreamSynchronize(0));
+            h->spmm_slot_w = pw;
+        }
+        pl.slots = h->spmm_slots;
+    }
+    launch_spmm<T>(pl, B, ldb, width, C, ldc, st);
+    h->launches += (width + SPMM_PANEL - 1) / SPMM_PANEL;
+    CKL();
+    return 0;
+}
+
+extern "C" int rri_spmm(rri_handle_t h, int32_t transpose, const void* B_dev, int64_t ldb, void* C_dev, int64_t ldc,
+                        int32_t width, void* stream)
+{
+    if (!h) return fail("null handle");
+    if (!h->X) return fail("rri_bind_csr / rri_bind_csr_zero has not been called");
+    if (!h->sparse && !h->zero_csr)
+        return fail("rri_spmm serves sparse handles (rri_bind_csr or rri_bind_csr_zero); this handle holds dense data");
+    if (transpose != 0 && transpose != 1) return fail("transpose must be 0 or 1 (got %d)", transpose);
+    if (width < 1) return fail("width must be at least 1 (got %d)", width);
+    if (!B_dev || !C_dev) return fail("B and C must not be null");
+    if (ldb < width || ldc < width)
+        return fail("ldb and ldc must be at least width = %d (got %lld, %lld)", width, (long long)ldb, (long long)ldc);
+    if (ldb >= ((int64_t)1 << 31) || ldc >= ((int64_t)1 << 31)) return fail("ldb and ldc must be below 2^31");
+    if (((uintptr_t)B_dev % h->es) || ((uintptr_t)C_dev % h->es))
+        return fail("B and C must be aligned to their %d-byte elements", (int)h->es);
+    CK(cudaSetDevice(h->device));
+    cudaStream_t st = (cudaStream_t)stream;
+    return h->dtype == RRI_F32 ? spmm_impl<float>(h, transpose, (const float*)B_dev, ldb, (float*)C_dev, ldc, width, st)
+                               : spmm_impl<double>(h, transpose, (const double*)B_dev, ldb, (double*)C_dev, ldc, width, st);
+}
+
 static SolveArgs solve_args(const rri_params_t* p, bool forT)
 {
     SolveArgs a;
@@ -939,7 +1030,7 @@ static int hals_W_half(rri_handle_t h, T* W, const T* Tk, int64_t ldtk, const rr
         const bool tc_gram = gram_in_contraction(h);
         if (!tc_gram) { launch_gram<T>((const T*)h->Tt, d, k, (T*)h->gram_part, h->gchunks_t, (T*)h->Hm, st); h->launches += 2; }
         if (h->zero_csr) {
-            launch_spmm<T>(h->zrow, (const T*)h->Tt, k, (T*)h->Cpart, st);
+            launch_spmm<T>(h->zrow, (const T*)h->Tt, k, k, (T*)h->Cpart, k, st);
             h->launches++;
         } else if (contraction<T>(h, (const T*)h->X, h->ldx, Tk, ldtk, (T*)h->Cpart, n, k, d, h->splits_w, st, tc_gram ? (T*)h->Hm : nullptr)) {
             return 1;
@@ -992,7 +1083,7 @@ static int hals_T_half(rri_handle_t h, T* W, T* Tk, int64_t ldtk, const rri_para
     // (one rank, TF32: the Gram tile lands right behind the contraction output, as the all-reduce wants it)
     T* Cout = (h->world > 1 && psplits == 1) ? cg : (T*)h->Cpart;
     if (h->zero_csr) {
-        launch_spmm<T>(h->zcol, W, k, Cout, st);
+        launch_spmm<T>(h->zcol, W, k, k, Cout, k, st);
         h->launches++;
     } else if (contraction<T>(h, (const T*)h->Xt, h->ldxt, (const T*)h->Wt, h->ldwt, Cout, d, k, n, h->splits_t, st,
                               tc_gram ? G : nullptr)) {
@@ -1504,7 +1595,7 @@ static int objective_contraction_impl(rri_handle_t h, const T* W, const T* Tm, b
         launch_transpose<T>(Tm, k, d, d, (T*)h->Tt, k, st);
         h->launches++;
         if (h->zero_csr) {
-            launch_spmm<T>(h->zrow, (const T*)h->Tt, k, (T*)h->Cpart, st);
+            launch_spmm<T>(h->zrow, (const T*)h->Tt, k, k, (T*)h->Cpart, k, st);
             h->launches++;
         } else if (contraction<T>(h, (const T*)h->X, h->ldx, Tm, d, (T*)h->Cpart, n, k, d, h->splits_w, st)) {
             return 1;
@@ -1584,7 +1675,7 @@ static int partials_impl(rri_handle_t h, const T* W, const T* Tm, int t, T* wR, 
         // X' W and W'W of the T half-step, then the statistic of topic t from column t of both
         const int k = h->k;
         T* G = (T*)h->cg + (size_t)d * k;
-        launch_spmm<T>(h->zcol, W, k, (T*)h->Cpart, st);
+        launch_spmm<T>(h->zcol, W, k, k, (T*)h->Cpart, k, st);
         launch_gram<T>(W, h->n, k, (T*)h->gram_part, h->gchunks_w, G, st);
         partials_unmasked_kernel<T><<<(unsigned)((d + 255) / 256), 256, 0, st>>>((const T*)h->Cpart + t, k, G + (size_t)t * k,
                                                                                   Tm, d, k, t, wR, nw);
@@ -1751,11 +1842,11 @@ static int profile_impl(rri_handle_t h, int which, const T* W, const T* Tm, int 
             h->launches++;
         } else if (which == 1) {
             if (h->mk != MK_NONE) return fail("which=1 needs an unmasked handle");
-            if (h->zero_csr) { launch_spmm<T>(h->zrow, (const T*)h->Tt, k, (T*)h->Cpart, st); h->launches++; continue; }
+            if (h->zero_csr) { launch_spmm<T>(h->zrow, (const T*)h->Tt, k, k, (T*)h->Cpart, k, st); h->launches++; continue; }
             if (contraction<T>(h, (const T*)h->X, h->ldx, Tm, d, (T*)h->Cpart, n, k, d, h->splits_w, st)) return 1;
         } else if (which == 2) {
             if (h->mk != MK_NONE || h->order != RRI_ORDER_HALS) return fail("which=2 needs an unmasked hals-order handle");
-            if (h->zero_csr) { launch_spmm<T>(h->zcol, W, k, (T*)h->Cpart, st); h->launches++; continue; }
+            if (h->zero_csr) { launch_spmm<T>(h->zcol, W, k, k, (T*)h->Cpart, k, st); h->launches++; continue; }
             if (contraction<T>(h, (const T*)h->Xt, h->ldxt, (const T*)h->Wt, h->ldwt, (T*)h->Cpart, d, k, n, h->splits_t, st)) return 1;
         } else if (which == 3) {
             // the whole T half-step (contraction + Gram + exchange + update); collective on row shards

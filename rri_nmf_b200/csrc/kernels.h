@@ -280,6 +280,7 @@ namespace rri {
 // sparse x dense contraction on zero-filled sparse data (block order)          (spmm_kernels.cu)
 // ---------------------------------------------------------------------------------------------
 constexpr int SPMM_CHUNK = 1024;    // longest segment taken by one lane group; longer ones are cut into chunks
+constexpr int SPMM_PANEL = 256;     // widest operand panel of one launch (accumulators in registers)
 struct SpmmPlan {                   // one compressed orientation and its chunk plan (built once at bind time)
     int64_t nseg;                   // rows (CSR) or columns (CSC)
     const int64_t* ptr;             // [nseg + 1]
@@ -289,10 +290,14 @@ struct SpmmPlan {                   // one compressed orientation and its chunk 
     const int2* litem;              // [nlong_items] {long segment, chunk}
     const int32_t* lseg;            // [nlong] segment of long segment j
     const int64_t* lslot;           // [nlong] first partial slot of long segment j
-    void* slots;                    // [nlong_items][k] chunk partials
+    void* slots;                    // [nlong_items][panel width] chunk partials
     unsigned* counters;             // [nlong] arrivals, zero between launches
 };
-// C[r, :] = sum_{e in segment r} val[e] * B[idx[e], :]   (B [., k] and C [nseg, k] row-major, one launch)
+// C[r, :width] = sum_{e in segment r} val[e] * B[idx[e], :width]   (B [., ldb] and C [nseg, ldc] row-major; one launch per
+// panel of at most SPMM_PANEL columns, in ascending order; p.slots holds [nlong_items][min(width, SPMM_PANEL)])
 template <typename T>
-void launch_spmm(const SpmmPlan& p, const T* B, int k, T* C, cudaStream_t st);
+void launch_spmm(const SpmmPlan& p, const T* B, int64_t ldb, int width, T* C, int64_t ldc, cudaStream_t st);
+// out[i] = w[i] * x[i]
+template <typename T>
+void launch_spmm_weighted_values(const T* x, const T* w, int64_t nnz, T* out, int sm_count, cudaStream_t st);
 }  // namespace rri

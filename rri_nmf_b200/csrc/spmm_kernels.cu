@@ -14,6 +14,10 @@
 // that arrives last (arrival counter, zero between launches) adds the slots in chunk order and writes the output row.
 // Every output entry is therefore summed in an order fixed by the plan: N sweeps in one call equal N calls of one
 // sweep, bit for bit.  One launch per half-step whatever k is.
+//
+// B and C have leading dimensions (ldb, ldc >= k), so that a column panel of a wider operand is computed in place:
+// rri_spmm takes operands of up to k + 10 columns (the randomized SVD of the NNDSVD initialisation) as panels of at most
+// SPMM_PANEL columns, one launch each, in ascending order.  The chunk slots of a panel are [chunks, panel width].
 #include "common.cuh"
 #include "kernels.h"
 
@@ -42,7 +46,7 @@ RRI_DEVINL void st_units(T* p, const T* v)
 // W elements per load (Vec<T>::N or 1); NV loads per lane and entry
 template <typename T, int W, int NV>
 __global__ void __launch_bounds__(256)
-spmm_kernel(SpmmPlan p, const T* __restrict__ B, int k, int G, T* __restrict__ C)
+spmm_kernel(SpmmPlan p, const T* __restrict__ B, int ldb, int k, int G, T* __restrict__ C, int ldc)
 {
     // entries whose gathers are in flight together (2 for the widest fp64 rows: 4 spills there)
     constexpr int U = NV * W * sizeof(T) > 32 ? 2 : 4;
@@ -82,7 +86,7 @@ spmm_kernel(SpmmPlan p, const T* __restrict__ B, int k, int G, T* __restrict__ C
         for (int u = 0; u < U; ++u)
 #pragma unroll
             for (int v = 0; v < NV; ++v)
-                if (lane + G * v < units) ld_units<T, W>(B + (int64_t)jj[u] * k + (lane + G * v) * W, &bv[u][v * W]);
+                if (lane + G * v < units) ld_units<T, W>(B + (int64_t)jj[u] * ldb + (lane + G * v) * W, &bv[u][v * W]);
 #pragma unroll
         for (int u = 0; u < U; ++u)
 #pragma unroll
@@ -98,12 +102,12 @@ spmm_kernel(SpmmPlan p, const T* __restrict__ B, int k, int G, T* __restrict__ C
         for (int v = 0; v < NV; ++v)
             if (lane + G * v < units) {
                 T bq[W];
-                ld_units<T, W>(B + (int64_t)jq * k + (lane + G * v) * W, bq);
+                ld_units<T, W>(B + (int64_t)jq * ldb + (lane + G * v) * W, bq);
 #pragma unroll
                 for (int w = 0; w < W; ++w) acc[v * W + w] = fma(xq, bq[w], acc[v * W + w]);
             }
     }
-    T* out = j < 0 ? C + seg * k : static_cast<T*>(p.slots) + (p.lslot[j] + c) * k;
+    T* out = j < 0 ? C + seg * ldc : static_cast<T*>(p.slots) + (p.lslot[j] + c) * k;
 #pragma unroll
     for (int v = 0; v < NV; ++v)
         if (lane + G * v < units) st_units<T, W>(out + (lane + G * v) * W, &acc[v * W]);
@@ -131,39 +135,64 @@ spmm_kernel(SpmmPlan p, const T* __restrict__ B, int k, int G, T* __restrict__ C
 #pragma unroll
                 for (int w = 0; w < W; ++w) s[w] += t[w];
             }
-            st_units<T, W>(C + seg * k + off, s);
+            st_units<T, W>(C + seg * ldc + off, s);
         }
     if (lane == 0) p.counters[j] = 0u;
 }
 
 template <typename T>
-void launch_spmm(const SpmmPlan& p, const T* B, int k, T* C, cudaStream_t st)
+void launch_spmm(const SpmmPlan& p, const T* B, int64_t ldb, int width, T* C, int64_t ldc, cudaStream_t st)
 {
     constexpr int VN = Vec<T>::N;
-    const bool vec = (k % VN) == 0 && (reinterpret_cast<uintptr_t>(B) & 15) == 0 &&
-                     (reinterpret_cast<uintptr_t>(C) & 15) == 0 && (reinterpret_cast<uintptr_t>(p.slots) & 15) == 0;
-    const int units = vec ? k / VN : k;
-    int G = 1;
-    while (G < units && G < 32) G <<= 1;
-    const int nv = (units + G - 1) / G;
     const int64_t items = p.nlong_items + p.nseg;
-    const unsigned blocks = (unsigned)((items + 256 / G - 1) / (256 / G));
-    if (blocks == 0) return;
-#define RRI_SPMM(W, NV) spmm_kernel<T, W, NV><<<blocks, 256, 0, st>>>(p, B, k, G, C)
-    if (vec) {
-        if (nv <= 1) RRI_SPMM(VN, 1);
-        else if (nv <= 2) RRI_SPMM(VN, 2);
-        else if constexpr (sizeof(T) == 8) RRI_SPMM(VN, 4);      // (fp64, k > 128; fp32 needs at most 2)
-    } else {
-        if (nv <= 1) RRI_SPMM(1, 1);
-        else if (nv <= 2) RRI_SPMM(1, 2);
-        else if (nv <= 4) RRI_SPMM(1, 4);
-        else RRI_SPMM(1, 8);
-    }
+    for (int off = 0; off < width; off += SPMM_PANEL) {
+        const int k = width - off < SPMM_PANEL ? width - off : SPMM_PANEL;
+        const T* Bp = B + off;
+        T* Cp = C + off;
+        const bool vec = (k % VN) == 0 && (ldb % VN) == 0 && (ldc % VN) == 0 &&
+                         (reinterpret_cast<uintptr_t>(Bp) & 15) == 0 && (reinterpret_cast<uintptr_t>(Cp) & 15) == 0 &&
+                         (reinterpret_cast<uintptr_t>(p.slots) & 15) == 0;
+        const int units = vec ? k / VN : k;
+        int G = 1;
+        while (G < units && G < 32) G <<= 1;
+        const int nv = (units + G - 1) / G;
+        const unsigned blocks = (unsigned)((items + 256 / G - 1) / (256 / G));
+        if (blocks == 0) return;
+        const int lb = (int)ldb, lc = (int)ldc;
+#define RRI_SPMM(W, NV) spmm_kernel<T, W, NV><<<blocks, 256, 0, st>>>(p, Bp, lb, k, G, Cp, lc)
+        if (vec) {
+            if (nv <= 1) RRI_SPMM(VN, 1);
+            else if (nv <= 2) RRI_SPMM(VN, 2);
+            else if constexpr (sizeof(T) == 8) RRI_SPMM(VN, 4);      // (fp64, k > 128; fp32 needs at most 2)
+        } else {
+            if (nv <= 1) RRI_SPMM(1, 1);
+            else if (nv <= 2) RRI_SPMM(1, 2);
+            else if (nv <= 4) RRI_SPMM(1, 4);
+            else RRI_SPMM(1, 8);
+        }
 #undef RRI_SPMM
+    }
 }
 
-template void launch_spmm<float>(const SpmmPlan&, const float*, int, float*, cudaStream_t);
-template void launch_spmm<double>(const SpmmPlan&, const double*, int, double*, cudaStream_t);
+// w o x of an observed-entries binding, the values rri_spmm applies there (built once, on the first call)
+template <typename T>
+__global__ void spmm_weighted_values_kernel(const T* __restrict__ x, const T* __restrict__ w, int64_t nnz, T* __restrict__ out)
+{
+    for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < nnz; i += (int64_t)gridDim.x * blockDim.x)
+        out[i] = w[i] * x[i];
+}
+
+template <typename T>
+void launch_spmm_weighted_values(const T* x, const T* w, int64_t nnz, T* out, int sm_count, cudaStream_t st)
+{
+    if (nnz <= 0) return;
+    const int64_t want = (nnz + 255) / 256, cap = (int64_t)sm_count * 8;
+    spmm_weighted_values_kernel<T><<<(unsigned)(want < cap ? want : cap), 256, 0, st>>>(x, w, nnz, out);
+}
+
+template void launch_spmm<float>(const SpmmPlan&, const float*, int64_t, int, float*, int64_t, cudaStream_t);
+template void launch_spmm<double>(const SpmmPlan&, const double*, int64_t, int, double*, int64_t, cudaStream_t);
+template void launch_spmm_weighted_values<float>(const float*, const float*, int64_t, float*, int, cudaStream_t);
+template void launch_spmm_weighted_values<double>(const double*, const double*, int64_t, double*, int, cudaStream_t);
 
 }  // namespace rri

@@ -326,9 +326,33 @@ class RRIEngine(object):
         """The two streaming products of a randomized SVD of X through the engine's contraction kernel (used by the
         device-resident NNDSVD initialisation, SURVEY.md §8 f3): right(Q) = X @ Q, left(Q) = X' @ Q.  The transposed
         product needs the engine's K-contiguous copy of X' (block-order handles); without it that one product is
-        a library GEMM."""
+        a library GEMM.  On a sparse handle both products are rri_spmm (the zero-filled matrix of the stored entries,
+        times the entry weights when given); Q is padded to a 16-byte row internally."""
         eng = self
         v = 16 // self.X.element_size()
+        if self.sparse:
+            def spmm(Q, transpose):
+                rows_in, rows_out = (eng.n, eng.d) if transpose else (eng.d, eng.n)
+                if Q.dim() != 2 or int(Q.shape[0]) != rows_in:
+                    raise ValueError('the operand must have %d rows' % rows_in)
+                r = int(Q.shape[1])
+                ld = (r + v - 1) // v * v
+                B = Q.to(device=eng.device, dtype=eng.dtype)
+                if ld != r or not B.is_contiguous():
+                    Bp = torch.zeros((rows_in, ld), dtype=eng.dtype, device=eng.device)
+                    Bp[:, :r] = B
+                    B = Bp
+                Cm = torch.empty((rows_out, ld), dtype=eng.dtype, device=eng.device)
+                check(eng.lib.rri_spmm(eng.h, int(transpose), _ptr(B), ld, _ptr(Cm), ld, ld, eng._stream()))
+                return Cm[:, :r]
+
+            class _S(object):
+                def right(self, Q):
+                    return spmm(Q, 0)
+
+                def left(self, Q):
+                    return spmm(Q, 1)
+            return _S()
 
         def kmajor(Q):
             """Q' [r, K] with a 16-byte aligned row stride (a legal TMA operand)"""

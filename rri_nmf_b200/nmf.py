@@ -24,7 +24,9 @@ Additional keyword-only arguments select the device path:
     init_on_device  where the NNDSVD initialisation runs when W_in/T_in are not both given: True = on the GPU that
                   holds X (`_device_init.py`; X never returns to the host), False = on the host (`_host.py`, NumPy /
                   sklearn, as the reference does), None (default) = on the device when X is already a CUDA tensor or
-                  has 2^26 or more elements, on the host otherwise.  Sparse X is always initialised on the host.
+                  has 2^26 or more elements (n * d, stored or not), on the host otherwise.  Sparse X follows the same
+                  rule; on the device its products go through rri_spmm and it is never densified.  Row-sharded runs
+                  (comm=...) take W_in / T_in and initialise nothing.
 
 X may also be a scipy.sparse matrix or a torch sparse CSR tensor, never densified.  What its unstored entries mean is
 set by the keyword-only argument `unstored`:
@@ -197,9 +199,15 @@ def _normalize_rows(A):
 def _initialize_on_device(Xd, W_mat, k, init, random_state, t_row_sum, w_row_sum, products=None):
     """nmf.py:840-850 (initialize_nmf on W_mat o X, then the row normalisations) with X staying on its device:
     initialization.py:80-163 through `_device_init.initialize_nmf_torch`.  products: the engine's streaming
-    contraction for the passes over X (unmasked data only: with W_mat the matrix being factorised is W_mat o X)."""
+    contraction for the passes over X (dense data: unmasked only, with W_mat the matrix being factorised is W_mat o X;
+    sparse data: always, the engine applies the entry weights).  A sparse Xd with entry weights W_mat (1-D) is handed
+    on as the CSR tensor of w o x (nnz values) for the means."""
     Xi = Xd
-    if W_mat is not None:
+    if Xd.layout == torch.sparse_csr:
+        if W_mat is not None:
+            Xi = torch.sparse_csr_tensor(Xd.crow_indices(), Xd.col_indices(), Xd.values() * W_mat, size=tuple(Xd.shape),
+                                         check_invariants=False)
+    elif W_mat is not None:
         Mi = W_mat if isinstance(W_mat, torch.Tensor) else torch.from_numpy(np.ascontiguousarray(W_mat))
         Xi = Xd * Mi.to(device=Xd.device, dtype=Xd.dtype)
         products = None
@@ -396,7 +404,7 @@ def nmf(X, k, w_row=None, W_mat=None, fix_W=False, fix_T=False, random_state=Non
     need_init = _is_empty(W_in) or _is_empty(T_in)
     if init_on_device is None:
         init_on_device = (isinstance(X, torch.Tensor) and X.is_cuda) or n * d >= (1 << 26)
-    init_on_device = bool(init_on_device) and need_init and not sparse_in and comm is None
+    init_on_device = bool(init_on_device) and need_init and comm is None
     W0 = T0 = None
     if need_init and not init_on_device:
         if sparse_in:
@@ -456,7 +464,7 @@ def nmf(X, k, w_row=None, W_mat=None, fix_W=False, fix_T=False, random_state=Non
                 # NNDSVD where X lives; its passes over X go through the engine's own contraction kernel
                 _ti = time.perf_counter()
                 Wi, Ti = _initialize_on_device(Xd, W_mat, k, init, random_state, t_row_sum, w_row_sum,
-                                               products=engine.products() if Md is None else None)
+                                               products=engine.products() if (Md is None or sparse_in) else None)
                 torch.cuda.current_stream(device).synchronize()
                 timing['init_on_device_s'] = time.perf_counter() - _ti
                 W0 = Wi if W0 is None else W0
