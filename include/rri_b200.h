@@ -90,13 +90,22 @@ int rri_peer_close(rri_handle_t h);
 
 /* Optional, before rri_bind on a hals handle: storage [d, ldXt] (ldXt >= n rounded up to 16 bytes) owned by the
  * caller for the engine's transposed copy of X, so that it comes from the caller's allocator (torch's caching
- * allocator: no cudaMalloc/cudaFree of a data-sized buffer per fit). */
+ * allocator: no cudaMalloc/cudaFree of a data-sized buffer per fit).
+ * With RRI_MATH_TF32 the same storage can hold, instead, 16-bit copies of X and X': fp16(tf32(x) * 2^e) with one
+ * power-of-two scale, exact when every nonzero TF32 value of X lies within 30 binades of fp16's normal range under
+ * that scale and X holds no inf / nan.  The block-order contractions then read half the bytes and see the same
+ * operands.  rri_bind checks the data and takes that form when it is exact and the storage holds
+ * 2 * (n * d8 + d * n8) bytes (d8, n8: d, n rounded up to 8); otherwise it builds the fp32 copy.  Environment
+ * RRI_X16=0 (read at every rri_bind) keeps the fp32 copy.  rri_x_operand_bits reports the choice. */
 int rri_set_transpose_storage(rri_handle_t h, void* Xt_dev, int64_t ldXt);
 
 /* Bind the data (and optional elementwise weights W_mat) resident in device memory.  In hals order
  * the engine builds its own transposed copy of X (one extra pass, once).  nmf.py:98 (X, W_mat). */
 int rri_bind(rri_handle_t h, const void* X_dev, int64_t ldX,
              const void* mask_dev, int32_t mask_kind, int64_t ldM, void* stream);
+/* The storage of X the contractions of the block order read: 16 (the 16-bit copies described above), or the bits of
+ * the handle's element type. */
+int rri_x_operand_bits(rri_handle_t h, int32_t* bits);
 
 /* Observed-entries binding for the recommender setting (SURVEY.md §8 f4): the (i, j, rating) triples of
  * sklearn_interface.py:78-83 as a CSR matrix of the LOCAL rows, instead of the densified X and the dense 0/1
@@ -189,6 +198,15 @@ int rri_stats(rri_handle_t h, int64_t* kernel_launches, int64_t* workspace_bytes
  * C[M,N] = A[M,K] * B[N,K]^T, row-major, math as in rri_create (TF32 tcgen05 or IEEE SIMT). */
 int rri_gemm_nt(rri_handle_t h, const void* A_dev, int64_t lda, const void* B_dev, int64_t ldb,
                 void* C_dev, int64_t ldc, int64_t M, int32_t N, int64_t K, void* stream);
+
+/* The streaming product of a block-order half-step on a dense, unmasked hals handle, through the operand copies
+ * the sweeps read (the 16-bit ones where rri_x_operand_bits says 16):
+ *     transpose = 0:  C[n_local, N] = X  B[N, d]'          transpose = 1:  C[d, N] = X' B[N, n_local]'
+ * B row-major with leading dimension ldb (a multiple of 16 bytes in TF32 math), C row-major [., N]; 1 <= N <= k + 16
+ * (at most 256).  With 16-bit copies B is rounded to TF32 and scaled into fp16 by a power of two taken from its
+ * maximum; entries below ~2^-29 of that maximum become fp16 subnormals. */
+int rri_contract_x(rri_handle_t h, int32_t transpose, const void* B_dev, int64_t ldb, int32_t N, void* C_dev,
+                   void* stream);
 
 /* Roofline hook for bench.py: launch the dominant streaming kernel of this handle `iters` times on
  * `stream` between two CUDA events and return the average launch duration in milliseconds.

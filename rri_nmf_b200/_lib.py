@@ -41,6 +41,7 @@ SYMBOLS = {
     'rri_peer_close': (C.c_int, [_vp]),
     'rri_set_transpose_storage': (C.c_int, [_vp, _vp, _i64]),
     'rri_bind': (C.c_int, [_vp, _vp, _i64, _vp, _i32, _i64, _vp]),
+    'rri_x_operand_bits': (C.c_int, [_vp, C.POINTER(_i32)]),
     'rri_bind_csr': (C.c_int, [_vp, _i64, _vp, _vp, _vp, _vp, _vp]),
     'rri_bind_csr_zero': (C.c_int, [_vp, _i64, _vp, _vp, _vp, _vp]),
     'rri_spmm': (C.c_int, [_vp, _i32, _vp, _i64, _vp, _i64, _i32, _vp]),
@@ -54,6 +55,7 @@ SYMBOLS = {
     'rri_cache_trim': (C.c_int, [_i32]),
     'rri_stats': (C.c_int, [_vp, C.POINTER(_i64), C.POINTER(_i64)]),
     'rri_profile_kernel': (C.c_int, [_vp, _i32, _vp, _vp, _i32, C.POINTER(C.c_float), _vp]),
+    'rri_contract_x': (C.c_int, [_vp, _i32, _vp, _i64, _i32, _vp, _vp]),
     'rri_gemm_nt': (C.c_int, [_vp, _vp, _i64, _vp, _i64, _vp, _i64, _i64, _i32, _i64, _vp]),
 }
 

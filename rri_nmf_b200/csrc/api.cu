@@ -153,6 +153,12 @@ struct rri_handle_s {
     // hals order
     void *Xt = nullptr; int64_t ldxt = 0, ldwt = 0;
     void* Xt_ext = nullptr; int64_t ldxt_ext = 0;      // caller-provided storage for the transposed copy (optional)
+    // TF32 math with data whose TF32 values fit fp16's normal range under one power-of-two scale 2^x_exp: the storage of
+    // X' holds 16-bit copies X16 [n, ldx16] and X16' [d, ldxt16] instead, and the contractions read those (x16_kernels.cu)
+    bool x16 = false; int x_exp = 0;
+    void *X16 = nullptr, *Xt16 = nullptr; int64_t ldx16 = 0, ldxt16 = 0;
+    void* F16 = nullptr;               // fp16 copy of the factor operand of a contraction [<= k + 16 rows, max(n, d) cols]
+    unsigned *x16_scan = nullptr, *f16_part = nullptr; int* f16_exp = nullptr;
     void *Wt = nullptr, *Tt = nullptr, *Cpart = nullptr, *cg = nullptr /* [max(n,d)*k | k*k] */, *Hm = nullptr;
     void *gram_part = nullptr, *colsum_part = nullptr;
     int splits_t = 1, splits_w = 1, ub_blocks_t = 1, ub_blocks_w = 1, gchunks_w = 1, gchunks_t = 1;
@@ -546,6 +552,10 @@ static int bind_impl(rri_handle_t h, cudaStream_t st)
             // (k + 16: the device-resident NNDSVD runs its randomized SVD with k + 10 columns through this kernel)
             h->tf32 = tf32_gemm_create(h->sm_count, k + 16 < 256 ? k + 16 : 256, err);
             if (!h->tf32) return fail("tf32 contraction unavailable: %s", err.c_str());
+            if (ws_alloc(h, (void**)&h->x16_scan, 4 * sizeof(unsigned)) || ws_alloc(h, (void**)&h->f16_exp, sizeof(int)) ||
+                ws_alloc(h, (void**)&h->f16_part, sizeof(unsigned) * (size_t)f16_factor_parts(h->sm_count)))
+                return 1;
+            CK(cudaStreamSynchronize(0));
         }
     }
     if (h->order == RRI_ORDER_HALS) {
@@ -553,17 +563,48 @@ static int bind_impl(rri_handle_t h, cudaStream_t st)
         // K-contiguous operands
         const int64_t v = 16 / (int64_t)es;
         h->ldxt = (n + v - 1) / v * v;
+        // the 16-bit copies: rows of 16-byte multiples, the same bytes as X' in fp32 but for that rounding
+        const int64_t ldx16 = (d + 7) / 8 * 8, ldxt16 = (n + 7) / 8 * 8;
+        const size_t bytes16 = 2 * ((size_t)n * ldx16 + (size_t)d * ldxt16);
+        size_t cap;
         if (h->Xt_ext) {
             if (h->ldxt_ext < h->ldxt || h->ldxt_ext % v != 0 || (reinterpret_cast<uintptr_t>(h->Xt_ext) & 15) != 0)
                 return fail("caller-provided X' storage needs a 16-byte aligned base and a row stride >= %lld, multiple of %lld",
                             (long long)h->ldxt, (long long)v);
             h->Xt = h->Xt_ext; h->ldxt = h->ldxt_ext;
-        } else if (!h->Xt) {
-            CK(cached_malloc(&h->Xt, es * (size_t)d * h->ldxt));    // (no memset: fully overwritten by the transpose)
-            h->allocs.push_back(h->Xt);
-            h->ws_bytes += (int64_t)(es * (size_t)d * h->ldxt);
+            cap = es * (size_t)d * h->ldxt;
+        } else {
+            cap = es * (size_t)d * h->ldxt > bytes16 ? es * (size_t)d * h->ldxt : bytes16;
+            if (!h->Xt) {
+                CK(cached_malloc(&h->Xt, cap));    // (no memset: fully overwritten by the transpose or the 16-bit copies)
+                h->allocs.push_back(h->Xt);
+                h->ws_bytes += (int64_t)cap;
+            }
         }
-        launch_transpose<T>((const T*)h->X, n, d, h->ldx, (T*)h->Xt, h->ldxt, st);
+        // RRI_X16=0 keeps fp32 storage (read per bind: one process can build both kinds of handle)
+        const char* ev = getenv("RRI_X16");
+        h->x16 = false;
+        if (h->math == RRI_MATH_TF32 && !(ev && *ev == '0') && bytes16 <= cap) {
+            launch_x16_scan((const float*)h->X, n, d, h->ldx, h->x16_scan, h->sm_count, st);
+            h->launches++;
+            unsigned scan[3];
+            CK(cudaMemcpyAsync(scan, h->x16_scan, sizeof(scan), cudaMemcpyDeviceToHost, st));
+            CK(cudaStreamSynchronize(st));
+            h->x16 = x16_exponent(scan, &h->x_exp);
+        }
+        if (h->x16) {
+            if (!h->F16) {
+                const int64_t m = n > d ? n : d;
+                const int rows = k + 16 < 256 ? k + 16 : 256;
+                if (ws_alloc(h, &h->F16, 2 * (size_t)rows * (size_t)((m + 7) / 8 * 8))) return 1;
+                CK(cudaStreamSynchronize(0));
+            }
+            h->X16 = h->Xt; h->ldx16 = ldx16;
+            h->Xt16 = (char*)h->Xt + 2 * (size_t)n * ldx16; h->ldxt16 = ldxt16;
+            launch_x16_copy((const float*)h->X, n, d, h->ldx, h->x_exp, h->X16, ldx16, h->Xt16, ldxt16, st);
+        } else {
+            launch_transpose<T>((const T*)h->X, n, d, h->ldx, (T*)h->Xt, h->ldxt, st);
+        }
         h->launches++;
         CKL();
     } else {
@@ -1020,6 +1061,32 @@ static bool gram_in_contraction(rri_handle_t h)
     return h->math == RRI_MATH_TF32 && !off;
 }
 
+// C = A B' over the data of a block-order half-step: A = X (transpose = false, n x d) or X' (d x n), B [N, K] factor
+// rows, plus the Gram tile G = B B' when G is given.  A handle holding 16-bit copies of X contracts them against an fp16
+// copy of B made here (convert = false: the copy of the previous call is still current).
+template <typename T>
+static int data_contraction(rri_handle_t h, bool transpose, const T* B, int64_t ldb, int N, T* C, cudaStream_t st,
+                            T* G = nullptr, bool convert = true)
+{
+    const int64_t M = transpose ? h->d : h->n, K = transpose ? h->n : h->d;
+    if (!h->x16)
+        return transpose ? contraction<T>(h, (const T*)h->Xt, h->ldxt, B, ldb, C, M, N, K, h->splits_t, st, G)
+                         : contraction<T>(h, (const T*)h->X, h->ldx, B, ldb, C, M, N, K, h->splits_w, st, G);
+    const int64_t ldf = (K + 7) / 8 * 8;
+    if (convert) {
+        launch_f16_factor((const float*)B, N, K, ldb, h->f16_part, f16_factor_parts(h->sm_count), h->F16, ldf, h->f16_exp, st);
+        h->launches += 2;
+    }
+    const __half* F = (const __half*)h->F16;
+    std::string err;
+    const int nl = f16_gemm_run(h->tf32, (const __half*)(transpose ? h->Xt16 : h->X16), transpose ? h->ldxt16 : h->ldx16,
+                                h->x_exp, F, ldf, h->f16_exp, (float*)C, N, M, N, K, st, err, G ? F : nullptr, ldf, G ? N : 0,
+                                (float*)G, N);
+    if (nl < 0) return fail("16-bit contraction failed: %s", err.c_str());
+    h->launches += nl;
+    return 0;
+}
+
 template <typename T>
 static int hals_W_half(rri_handle_t h, T* W, const T* Tk, int64_t ldtk, const rri_params_t* p, bool recompute, cudaStream_t st)
 {
@@ -1032,7 +1099,7 @@ static int hals_W_half(rri_handle_t h, T* W, const T* Tk, int64_t ldtk, const rr
         if (h->zero_csr) {
             launch_spmm<T>(h->zrow, (const T*)h->Tt, k, k, (T*)h->Cpart, k, st);
             h->launches++;
-        } else if (contraction<T>(h, (const T*)h->X, h->ldx, Tk, ldtk, (T*)h->Cpart, n, k, d, h->splits_w, st, tc_gram ? (T*)h->Hm : nullptr)) {
+        } else if (data_contraction<T>(h, false, Tk, ldtk, k, (T*)h->Cpart, st, tc_gram ? (T*)h->Hm : nullptr)) {
             return 1;
         }
     }
@@ -1067,8 +1134,7 @@ static int hals_T_half(rri_handle_t h, T* W, T* Tk, int64_t ldtk, const rri_para
         T* myG = myC + (size_t)d * k;
         if (!tc_gram) { launch_gram<T>(W, n, k, (T*)h->gram_part, h->gchunks_w, myG, st); h->launches += 2; }
         T* Cdst = psplits == 1 ? myC : (T*)h->Cpart;
-        if (contraction<T>(h, (const T*)h->Xt, h->ldxt, (const T*)h->Wt, h->ldwt, Cdst, d, k, n, h->splits_t, st,
-                           tc_gram ? myG : nullptr)) return 1;
+        if (data_contraction<T>(h, true, (const T*)h->Wt, h->ldwt, k, Cdst, st, tc_gram ? myG : nullptr)) return 1;
         if (psplits > 1) { launch_reduce_parts<T>((const T*)h->Cpart, psplits, d * k, d * k, myC, st); h->launches++; }
         const PeerExchange px = peer_args(h, e);
         const int blocks = peer_update_blocks(px.row_hi - px.row_lo, h->sm_count);
@@ -1085,8 +1151,7 @@ static int hals_T_half(rri_handle_t h, T* W, T* Tk, int64_t ldtk, const rri_para
     if (h->zero_csr) {
         launch_spmm<T>(h->zcol, W, k, k, Cout, k, st);
         h->launches++;
-    } else if (contraction<T>(h, (const T*)h->Xt, h->ldxt, (const T*)h->Wt, h->ldwt, Cout, d, k, n, h->splits_t, st,
-                              tc_gram ? G : nullptr)) {
+    } else if (data_contraction<T>(h, true, (const T*)h->Wt, h->ldwt, k, Cout, st, tc_gram ? G : nullptr)) {
         return 1;
     }
     const T* C = Cout;
@@ -1751,6 +1816,43 @@ extern "C" int rri_stats(rri_handle_t h, int64_t* kernel_launches, int64_t* work
     return 0;
 }
 
+extern "C" int rri_x_operand_bits(rri_handle_t h, int32_t* bits)
+{
+    if (!h || !bits) return fail("null argument");
+    *bits = h->x16 ? 16 : 8 * (int32_t)h->es;
+    return 0;
+}
+
+template <typename T>
+static int contract_x_impl(rri_handle_t h, bool transpose, const T* B, int64_t ldb, int N, T* C, cudaStream_t st)
+{
+    if (h->math == RRI_MATH_TF32) return data_contraction<T>(h, transpose, B, ldb, N, C, st);
+    const int64_t M = transpose ? h->d : h->n, K = transpose ? h->n : h->d;
+    launch_simt_gemm_nt<T>(transpose ? (const T*)h->Xt : (const T*)h->X, transpose ? h->ldxt : h->ldx, B, ldb, C, M, N, K, 1, st);
+    h->launches++;
+    return 0;
+}
+
+extern "C" int rri_contract_x(rri_handle_t h, int32_t transpose, const void* B_dev, int64_t ldb, int32_t N, void* C_dev,
+                              void* stream)
+{
+    if (!h) return fail("null handle");
+    if (!h->X) return fail("rri_bind has not been called");
+    if (h->order != RRI_ORDER_HALS || h->mk != MK_NONE || !h->Xt)
+        return fail("rri_contract_x needs a dense, unmasked handle created with RRI_ORDER_HALS");
+    const int nmax = h->k + 16 < 256 ? h->k + 16 : 256;
+    if (N < 1 || N > nmax) return fail("N must be in [1, %d] (got %d)", nmax, N);
+    if (!B_dev || !C_dev || ldb < (transpose ? h->n : h->d)) return fail("bad operand");
+    CK(cudaSetDevice(h->device));
+    cudaStream_t st = (cudaStream_t)stream;
+    const int rc = h->dtype == RRI_F32
+                       ? contract_x_impl<float>(h, transpose != 0, (const float*)B_dev, ldb, N, (float*)C_dev, st)
+                       : contract_x_impl<double>(h, transpose != 0, (const double*)B_dev, ldb, N, (double*)C_dev, st);
+    if (rc) return rc;
+    CKL();
+    return 0;
+}
+
 extern "C" int rri_gemm_nt(rri_handle_t h, const void* A_dev, int64_t lda, const void* B_dev, int64_t ldb,
                            void* C_dev, int64_t ldc, int64_t M, int32_t N, int64_t K, void* stream)
 {
@@ -1843,11 +1945,12 @@ static int profile_impl(rri_handle_t h, int which, const T* W, const T* Tm, int 
         } else if (which == 1) {
             if (h->mk != MK_NONE) return fail("which=1 needs an unmasked handle");
             if (h->zero_csr) { launch_spmm<T>(h->zrow, (const T*)h->Tt, k, k, (T*)h->Cpart, k, st); h->launches++; continue; }
-            if (contraction<T>(h, (const T*)h->X, h->ldx, Tm, d, (T*)h->Cpart, n, k, d, h->splits_w, st)) return 1;
+            // (a 16-bit handle converts T in the untimed warm-up launch only: the timed launches are the contraction)
+            if (data_contraction<T>(h, false, Tm, d, k, (T*)h->Cpart, st, nullptr, it < 0)) return 1;
         } else if (which == 2) {
             if (h->mk != MK_NONE || h->order != RRI_ORDER_HALS) return fail("which=2 needs an unmasked hals-order handle");
             if (h->zero_csr) { launch_spmm<T>(h->zcol, W, k, k, (T*)h->Cpart, k, st); h->launches++; continue; }
-            if (contraction<T>(h, (const T*)h->Xt, h->ldxt, (const T*)h->Wt, h->ldwt, (T*)h->Cpart, d, k, n, h->splits_t, st)) return 1;
+            if (data_contraction<T>(h, true, (const T*)h->Wt, h->ldwt, k, (T*)h->Cpart, st, nullptr, it < 0)) return 1;
         } else if (which == 3) {
             // the whole T half-step (contraction + Gram + exchange + update); collective on row shards
             if (hals_T_half<T>(h, const_cast<T*>(W), Tk, ldtk, &prm, st)) return 1;

@@ -30,7 +30,9 @@
 //   * optional auxiliary tile: one more row super-tile whose A operand is a second matrix A2 (in practice the
 //     factor itself, so the tile is the k x k Gram matrix B B' of the same half-step) written to its own
 //     output -- the Gram product of BASELINE.json's kernel group (2) rides on the streaming contraction
-//     instead of costing two more launches per half-step.
+//     instead of costing two more launches per half-step;
+//   * 16-bit operands (f16_gemm_run): exact fp16 copies of TF32 values under a power-of-two scale (x16_kernels.cu) go
+//     through the same kernel with kind::f16 MMAs -- half the bytes per K, the same swizzle, split, fix-up and flush.
 #include <cuda.h>
 #include <cuda_runtime.h>
 #include <stdio.h>
@@ -45,10 +47,10 @@ namespace rri {
 namespace {
 
 constexpr int BM = 128;            // rows per UMMA (M of the instruction, cta_group::1)
-constexpr int BK = 32;             // fp32 elements per 128-byte swizzle row
-constexpr int UK = 8;              // K of one tcgen05.mma kind::tf32
+constexpr int BK = 32;             // fp32 elements per 128-byte swizzle row (64 for 16-bit operands)
+constexpr int ROW_BYTES = 128;     // one swizzle row: the K extent of a stage in bytes, whatever the element type
 constexpr int FLUSH = 4;            // K-chunks (x32 floats = 128 K) accumulated in TMEM before a flush into registers
-constexpr int A_TILE_BYTES = BM * BK * 4;      // 16 KB
+constexpr int A_TILE_BYTES = BM * ROW_BYTES;   // 16 KB
 constexpr int SMEM_LIMIT = 227 * 1024;
 
 struct GemmParams {
@@ -68,6 +70,10 @@ struct GemmParams {
     int nbuf;                      // TMEM accumulator buffers (2 when 2*MT*NPAD <= 512 columns)
     int flush;                     // K-chunks per TMEM accumulation run
     int reverse_tail;              // tails of split tiles stream K downward (see the producer)
+    // 16-bit operands (F16): A holds fp16(a * 2^a_exp), B and A2 fp16(b * 2^(*b_exp)), exponents in [-126, 126]; the
+    // epilogue scales the sums back
+    int a_exp;
+    const int* b_exp;
 };
 
 using namespace tc;
@@ -89,17 +95,21 @@ __host__ __device__ __forceinline__ int64_t part_of(int64_t units, int parts, in
 // main kernel
 // ------------------------------------------------------------------------------------------------
 // EWQ = epilogue warps per TMEM lane quarter (each takes NPAD/EWQ accumulator columns of every tile): 2 for
-// k <= 64, 4 for wider ranks so that a thread never holds more than 64 accumulators
-template <int MT, int NPAD, int EWQ>
+// k <= 64, 4 for wider ranks so that a thread never holds more than 64 accumulators.
+// F16: fp16 operands and tcgen05.mma kind::f16 (fp32 accumulators) instead of fp32 operands rounded to TF32 on the way
+// into shared memory.  A stage then holds 64 K-elements per row instead of 32, in the same bytes and the same swizzle.
+template <int MT, int NPAD, int EWQ, bool F16>
 __global__ void __launch_bounds__(64 + 128 * EWQ, 1)
 tf32_gemm_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CUtensorMap tmB,
                  const __grid_constant__ CUtensorMap tmA2, GemmParams p, int* err)
 {
+    constexpr int BKE = F16 ? 2 * BK : BK;     // K-elements per chunk (one 128-byte swizzle row)
+    constexpr int UK = F16 ? 16 : 8;           // K of one tcgen05.mma: 32 bytes of a row either way
     extern __shared__ __align__(1024) uint8_t smem_raw[];
     // carve: [A stages][B stages][barriers][tmem ptr]
     uint8_t* smem = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~(uintptr_t)1023);
     constexpr int a_stage = MT * A_TILE_BYTES;
-    constexpr int b_stage = NPAD * BK * 4;
+    constexpr int b_stage = NPAD * ROW_BYTES;
     uint8_t* smA = smem;
     uint8_t* smB = smem + (size_t)p.stages * a_stage;
     uint64_t* full = reinterpret_cast<uint64_t*>(smB + (size_t)p.stages * b_stage);
@@ -151,11 +161,11 @@ tf32_gemm_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant_
                     mbar_wait(&empty[stage], phase ^ 1, err, 1);
                     mbar_expect_tx(&full[stage], (uint32_t)(a_stage + b_stage));
                     if (s < p.n_super_main)
-                        tma_load_2d(&tmA, smA + (size_t)stage * a_stage, &full[stage], (int)(kc * BK), (int)(s * MT * BM), polA);
+                        tma_load_2d(&tmA, smA + (size_t)stage * a_stage, &full[stage], (int)(kc * BKE), (int)(s * MT * BM), polA);
                     else        // auxiliary tile: rows of A2 (rows beyond M2 are zero-filled by TMA)
-                        tma_load_2d(&tmA2, smA + (size_t)stage * a_stage, &full[stage], (int)(kc * BK),
+                        tma_load_2d(&tmA2, smA + (size_t)stage * a_stage, &full[stage], (int)(kc * BKE),
                                     (int)((s - p.n_super_main) * MT * BM), polB);
-                    tma_load_2d(&tmB, smB + (size_t)stage * b_stage, &full[stage], (int)(kc * BK), 0, polB);
+                    tma_load_2d(&tmB, smB + (size_t)stage * b_stage, &full[stage], (int)(kc * BKE), 0, polB);
                     if (++stage == p.stages) { stage = 0; phase ^= 1; }
                 }
                 u += len;
@@ -164,7 +174,7 @@ tf32_gemm_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant_
     } else if (warp == 1) {
         // ===================================== MMA issuer =======================================
         if (lane == 0) {
-            const uint32_t idesc = make_idesc_tf32(BM, NPAD);
+            const uint32_t idesc = F16 ? make_idesc_f16(BM, NPAD) : make_idesc_tf32(BM, NPAD);
             int stage = 0; uint32_t phase = 0;
             uint32_t run = 0;                                     // accumulation runs issued so far
             for (int64_t u = u_begin; u < u_end;) {
@@ -185,10 +195,12 @@ tf32_gemm_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant_
 #pragma unroll
                         for (int mt = 0; mt < MT; ++mt) {
 #pragma unroll
-                            for (int ks = 0; ks < BK / UK; ++ks) {
-                                const uint64_t ad = make_desc(a0 + mt * A_TILE_BYTES + ks * UK * 4);
-                                const uint64_t bd = make_desc(b0 + ks * UK * 4);
-                                umma_tf32(tacc + (uint32_t)(mt * NPAD), ad, bd, idesc, (i > i0 || ks > 0) ? 1u : 0u);
+                            for (int ks = 0; ks < BKE / UK; ++ks) {
+                                const uint64_t ad = make_desc(a0 + mt * A_TILE_BYTES + ks * 32);
+                                const uint64_t bd = make_desc(b0 + ks * 32);
+                                const uint32_t accum = (i > i0 || ks > 0) ? 1u : 0u;
+                                if (F16) umma_f16(tacc + (uint32_t)(mt * NPAD), ad, bd, idesc, accum);
+                                else umma_tf32(tacc + (uint32_t)(mt * NPAD), ad, bd, idesc, accum);
                             }
                         }
                         umma_commit(&empty[stage]);               // frees the smem slot when the MMAs retire
@@ -239,6 +251,14 @@ tf32_gemm_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant_
             // ---- the segment is done: a full K range goes straight to its output tile; a partial one goes to this
             // CTA's slot, and whichever contributor arrives last at the tile adds all slots in CTA order
             const bool aux = s >= p.n_super_main;
+            if (F16) {
+                // undo the operands' power-of-two scales (both exponents lie in [-126, 126]): exact, so slots scaled one
+                // by one add up to the scaled sum
+                const float sb = __int_as_float((127 - *p.b_exp) << 23);
+                const float sa = aux ? sb : __int_as_float((127 - p.a_exp) << 23);
+#pragma unroll
+                for (int i = 0; i < NACC; ++i) acc[i] = acc[i] * sa * sb;
+            }
             float* out = aux ? p.C2 : p.C;
             const int64_t out_ld = aux ? p.ldc2 : p.ldc;
             const int64_t out_row0 = (aux ? s - p.n_super_main : s) * MT * BM;
@@ -403,18 +423,21 @@ void tf32_gemm_destroy(Tf32Gemm* g)
     delete g;
 }
 
-static bool encode_2d(Tf32Gemm* g, CUtensorMap* tm, const float* base, int64_t rows, int64_t cols, int64_t ld,
-                      int box_rows, std::string& err)
+// f16: a matrix of fp16 elements (box of 64 per 128-byte row), otherwise fp32 (the handle's TFLOAT32 / FLOAT32 map)
+static bool encode_2d(Tf32Gemm* g, CUtensorMap* tm, const void* base, int64_t rows, int64_t cols, int64_t ld,
+                      int box_rows, bool f16, std::string& err)
 {
-    if ((reinterpret_cast<uintptr_t>(base) & 15) != 0 || (ld * 4) % 16 != 0) {
-        err = "TMA needs 16-byte aligned rows (leading dimension multiple of 4 floats, base 16-byte aligned)";
+    const int es = f16 ? 2 : 4;
+    if ((reinterpret_cast<uintptr_t>(base) & 15) != 0 || (ld * es) % 16 != 0) {
+        err = "TMA needs 16-byte aligned rows (leading dimension a multiple of 16 bytes, base 16-byte aligned)";
         return false;
     }
     cuuint64_t gdim[2] = {(cuuint64_t)cols, (cuuint64_t)rows};
-    cuuint64_t gstr[1] = {(cuuint64_t)ld * 4};
-    cuuint32_t box[2] = {(cuuint32_t)BK, (cuuint32_t)box_rows};
+    cuuint64_t gstr[1] = {(cuuint64_t)(ld * es)};
+    cuuint32_t box[2] = {(cuuint32_t)(ROW_BYTES / es), (cuuint32_t)box_rows};
     cuuint32_t estr[2] = {1, 1};
-    CUresult r = g->encode(tm, g->dtype, 2, const_cast<float*>(base), gdim, gstr, box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE,
+    CUresult r = g->encode(tm, f16 ? CU_TENSOR_MAP_DATA_TYPE_FLOAT16 : g->dtype, 2, const_cast<void*>(base), gdim, gstr, box,
+                           estr, CU_TENSOR_MAP_INTERLEAVE_NONE,
                            CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
     if (r != CUDA_SUCCESS) {
         char buf[128];
@@ -426,11 +449,11 @@ static bool encode_2d(Tf32Gemm* g, CUtensorMap* tm, const float* base, int64_t r
     return true;
 }
 
-template <int MT, int NPAD>
+template <int MT, int NPAD, bool F16>
 static int run_cfg(Tf32Gemm* g, const CUtensorMap& tmA, const CUtensorMap& tmB, const CUtensorMap& tmA2, GemmParams p,
                    cudaStream_t st, std::string& err)
 {
-    const int a_stage = MT * A_TILE_BYTES, b_stage = NPAD * BK * 4;
+    const int a_stage = MT * A_TILE_BYTES, b_stage = NPAD * ROW_BYTES;
     const int bar_bytes = 4096;       // mbarriers, TMEM slot, fix-up scratch (one slot pointer per CTA of the grid)
     int stages = (SMEM_LIMIT - 1024 /*alignment slack*/ - bar_bytes) / (a_stage + b_stage);
     if (stages > 8) stages = 8;
@@ -441,14 +464,15 @@ static int run_cfg(Tf32Gemm* g, const CUtensorMap& tmA, const CUtensorMap& tmB, 
     int cols = 32;
     while (cols < p.nbuf * MT * NPAD) cols <<= 1;
     p.tmem_cols = cols;
-    p.flush = g->flush > 0 ? g->flush : (1 << 30);
+    // the flush period is a K length (RRI_GEMM_FLUSH counts 32-wide chunks): two 64-wide chunks of 16-bit operands
+    p.flush = g->flush > 0 ? (F16 ? (g->flush + 1) / 2 : g->flush) : (1 << 30);
     // Measured (profiles/r02_gemm_reverse_tail_ab.txt): the shared B stream wins where B is half of A's traffic (k = 128:
     // T half-step of a config-5 shard 1.91 -> 1.76 ms) and loses where it is a quarter (k = 64: 2.49 -> 2.71 ms; streaming
     // all CTAs through the same columns at the same time costs more than the re-reads it saves).
     p.reverse_tail = g->reverse_tail >= 0 ? g->reverse_tail : (NPAD >= 128 ? 1 : 0);
     int64_t grid = p.units < g->sm_count ? p.units : g->sm_count;
     constexpr int EWQ = NPAD >= 128 ? 4 : 2;
-    auto kern = tf32_gemm_kernel<MT, NPAD, EWQ>;
+    auto kern = tf32_gemm_kernel<MT, NPAD, EWQ, F16>;
     if (cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem) != cudaSuccess) {
         err = "cudaFuncSetAttribute(max dynamic smem) failed";
         return -1;
@@ -459,9 +483,9 @@ static int run_cfg(Tf32Gemm* g, const CUtensorMap& tmA, const CUtensorMap& tmB, 
     return 1;
 }
 
-int tf32_gemm_run(Tf32Gemm* g, const float* A, int64_t lda, const float* B, int64_t ldb, float* C, int64_t ldc,
-                  int64_t M, int N, int64_t K, cudaStream_t st, std::string& err, const float* A2, int64_t lda2, int M2,
-                  float* C2, int64_t ldc2)
+static int gemm_run(Tf32Gemm* g, bool f16, const void* A, int64_t lda, int a_exp, const void* B, int64_t ldb,
+                    const int* b_exp, float* C, int64_t ldc, int64_t M, int N, int64_t K, cudaStream_t st, std::string& err,
+                    const void* A2, int64_t lda2, int M2, float* C2, int64_t ldc2)
 {
     if (!g) { err = "null contraction handle"; return -1; }
     if (N < 1 || N > 256) { err = "N must be in [1,256]"; return -1; }
@@ -476,16 +500,17 @@ int tf32_gemm_run(Tf32Gemm* g, const float* A, int64_t lda, const float* B, int6
     if (npad <= 64 && (M + 2 * BM - 1) / (2 * BM) < g->sm_count && (int64_t)npad * K * 4 <= ((int64_t)16 << 20)) mt = 1;
     if (g->force_mt == 1 || (g->force_mt == 2 && npad < 256)) mt = g->force_mt;
     CUtensorMap tmA, tmB, tmA2;
-    if (!encode_2d(g, &tmA, A, M, K, lda, mt * BM, err)) return -1;
-    if (!encode_2d(g, &tmB, B, N, K, ldb, npad, err)) return -1;
+    if (!encode_2d(g, &tmA, A, M, K, lda, mt * BM, f16, err)) return -1;
+    if (!encode_2d(g, &tmB, B, N, K, ldb, npad, f16, err)) return -1;
     const bool aux = A2 != nullptr && M2 > 0 && C2 != nullptr;
-    if (aux) { if (!encode_2d(g, &tmA2, A2, M2, K, lda2, mt * BM, err)) return -1; }
+    if (aux) { if (!encode_2d(g, &tmA2, A2, M2, K, lda2, mt * BM, f16, err)) return -1; }
     else tmA2 = tmA;
     GemmParams p;
     p.M = M; p.K = K; p.N = N; p.NPAD = npad;
     p.n_super_main = (M + (int64_t)mt * BM - 1) / ((int64_t)mt * BM);
     p.n_super = p.n_super_main + (aux ? (M2 + mt * BM - 1) / (mt * BM) : 0);
-    p.nk = (K + BK - 1) / BK;
+    const int bke = f16 ? 2 * BK : BK;
+    p.nk = (K + bke - 1) / bke;
     p.units = p.n_super * p.nk;
     p.C = C; p.ldc = ldc; p.ws = g->ws;
     p.C2 = aux ? C2 : C; p.ldc2 = aux ? ldc2 : ldc; p.M2 = aux ? M2 : 0;
@@ -501,12 +526,30 @@ int tf32_gemm_run(Tf32Gemm* g, const float* A, int64_t lda, const float* B, int6
     p.ctr = g->ctr;
     p.stages = 0; p.tmem_cols = 0;
     p.nbuf = 1; p.flush = 0;
-#define RRI_GEMM_CASE(MTv, NP) if (mt == MTv && npad == NP) return run_cfg<MTv, NP>(g, tmA, tmB, tmA2, p, st, err)
+    p.a_exp = a_exp; p.b_exp = b_exp;
+#define RRI_GEMM_CASE(MTv, NP)                                                                              \
+    if (mt == MTv && npad == NP)                                                                            \
+        return f16 ? run_cfg<MTv, NP, true>(g, tmA, tmB, tmA2, p, st, err) : run_cfg<MTv, NP, false>(g, tmA, tmB, tmA2, p, st, err)
     RRI_GEMM_CASE(2, 32); RRI_GEMM_CASE(2, 64); RRI_GEMM_CASE(2, 128);
     RRI_GEMM_CASE(1, 32); RRI_GEMM_CASE(1, 64); RRI_GEMM_CASE(1, 128); RRI_GEMM_CASE(1, 256);
 #undef RRI_GEMM_CASE
     err = "no contraction kernel for this shape";
     return -1;
+}
+
+int tf32_gemm_run(Tf32Gemm* g, const float* A, int64_t lda, const float* B, int64_t ldb, float* C, int64_t ldc,
+                  int64_t M, int N, int64_t K, cudaStream_t st, std::string& err, const float* A2, int64_t lda2, int M2,
+                  float* C2, int64_t ldc2)
+{
+    return gemm_run(g, false, A, lda, 0, B, ldb, nullptr, C, ldc, M, N, K, st, err, A2, lda2, M2, C2, ldc2);
+}
+
+int f16_gemm_run(Tf32Gemm* g, const __half* A, int64_t lda, int a_exp, const __half* B, int64_t ldb, const int* b_exp,
+                 float* C, int64_t ldc, int64_t M, int N, int64_t K, cudaStream_t st, std::string& err, const __half* A2,
+                 int64_t lda2, int M2, float* C2, int64_t ldc2)
+{
+    if (!b_exp) { err = "16-bit contraction without the factor's scale"; return -1; }
+    return gemm_run(g, true, A, lda, a_exp, B, ldb, b_exp, C, ldc, M, N, K, st, err, A2, lda2, M2, C2, ldc2);
 }
 
 }  // namespace rri

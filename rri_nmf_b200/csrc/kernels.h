@@ -128,6 +128,22 @@ void launch_colsum_finalize(const T* colsum_part, int blocks, int k, double* sum
 template <typename T>
 void launch_transpose(const T* A, int64_t rows, int64_t cols, int64_t lda, T* B, int64_t ldb,
                       cudaStream_t st);
+
+// ---------------------------------------------------------------------------------------------
+// 16-bit copies of TF32 operands for the block-order contraction (f16_gemm_run)      (x16_kernels.cu)
+// ---------------------------------------------------------------------------------------------
+// out[3] <- {bits of max |tf32(x)|, bits of the smallest nonzero |tf32(x)|, 1 if any value is inf / nan} over X
+void launch_x16_scan(const float* X, int64_t rows, int64_t cols, int64_t ld, unsigned* out, int sm_count, cudaStream_t st);
+// host: true (and the scale exponent e) when fp16(tf32(x) * 2^e) is exact for every x the scan saw
+bool x16_exponent(const unsigned scan[3], int* e);
+// Y[r, c] = Yt[c, r] = fp16(tf32(X[r, c]) * 2^e)  (Y [rows, ldy], Yt [cols, ldyt])
+void launch_x16_copy(const float* X, int64_t rows, int64_t cols, int64_t ldx, int e, void* Y, int64_t ldy, void* Yt,
+                     int64_t ldyt, cudaStream_t st);
+// out [rows, ldo] = fp16(tf32(F) * 2^e) with e (written to *e_out) putting max |tf32(F)| into [2^15, 2^16);
+// part: nparts = f16_factor_parts() block maxima
+int f16_factor_parts(int sm_count);
+void launch_f16_factor(const float* F, int rows, int64_t cols, int64_t ld, unsigned* part, int nparts, void* out,
+                       int64_t ldo, int* e_out, cudaStream_t st);
 }  // namespace rri
 
 namespace rri {

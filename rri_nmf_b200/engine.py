@@ -127,9 +127,14 @@ class RRIEngine(object):
             ldm = int(W_mat.stride(0))
         if order == 'hals' and self.W_mat is None:
             # the transposed copy of X lives in a torch tensor: allocation and release go through the caching
-            # allocator instead of a cudaMalloc/cudaFree of a data-sized buffer per engine
+            # allocator instead of a cudaMalloc/cudaFree of a data-sized buffer per engine.  With math='tf32' the library
+            # may keep 16-bit copies of X and X' there instead (rri_set_transpose_storage): the row stride leaves room
+            # for them where n or d is not a multiple of 8
             v = 16 // X.element_size()
             ldxt = (self.n + v - 1) // v * v
+            if math == 'tf32':
+                b16 = 2 * (self.n * ((self.d + 7) // 8 * 8) + self.d * ((self.n + 7) // 8 * 8))
+                ldxt = max(ldxt, (-(-b16 // (4 * self.d)) + v - 1) // v * v)
             self.Xt = torch.empty((self.d, ldxt), dtype=self.dtype, device=self.device)
             check(self.lib.rri_set_transpose_storage(self.h, _ptr(self.Xt), ldxt))
         check(self.lib.rri_bind(self.h, _ptr(self.X), int(self.X.stride(0)), _ptr(self.W_mat), mk, ldm,
@@ -322,6 +327,18 @@ class RRIEngine(object):
                                    M, N, K, self._stream()))
         return Cm
 
+    def contract_x(self, B, transpose=False):
+        """C = X @ B.T (transpose=False) or X.T @ B.T (True) through the operand copies the block-order sweeps read
+        (rri_contract_x; dense unmasked hals engines).  B [N, K] with unit column stride, N <= k + 16."""
+        K = self.n if transpose else self.d
+        if B.dim() != 2 or int(B.shape[1]) != K or B.stride(1) != 1:
+            raise ValueError('B must be [N, %d] with unit column stride' % K)
+        N = int(B.shape[0])
+        Cm = torch.empty((self.d if transpose else self.n), N, dtype=self.dtype, device=self.device)
+        check(self.lib.rri_contract_x(self.h, int(bool(transpose)), _ptr(B), int(B.stride(0)), N, _ptr(Cm),
+                                      self._stream()))
+        return Cm
+
     def products(self):
         """The two streaming products of a randomized SVD of X through the engine's contraction kernel (used by the
         device-resident NNDSVD initialisation, SURVEY.md §8 f3): right(Q) = X @ Q, left(Q) = X' @ Q.  The transposed
@@ -373,7 +390,7 @@ class RRIEngine(object):
             def left(self, Q):
                 if eng.Xt is None or Q.shape[1] > 256:
                     return eng.X.t() @ Q.to(eng.dtype)
-                return eng.gemm_nt(eng.Xt[:, :eng.n], kmajor(Q))
+                return eng.contract_x(kmajor(Q), transpose=True)
         return _P()
 
     def profile_kernel(self, which, W, T, iters=5):
@@ -389,4 +406,6 @@ class RRIEngine(object):
     def stats(self):
         a, b = C.c_int64(0), C.c_int64(0)
         check(self.lib.rri_stats(self.h, C.byref(a), C.byref(b)))
-        return {'kernel_launches': int(a.value), 'workspace_bytes': int(b.value)}
+        bits = C.c_int32(0)
+        check(self.lib.rri_x_operand_bits(self.h, C.byref(bits)))
+        return {'kernel_launches': int(a.value), 'workspace_bytes': int(b.value), 'x_operand': 'f%d' % bits.value}
