@@ -121,13 +121,16 @@ int rri_bind_csr(rri_handle_t h, int64_t nnz, const int64_t* rowptr_dev, const i
 /* Zero-filled sparse binding: the CSR matrix is an ordinary non-negative matrix stored sparsely (a tf-idf
  * document-term matrix); every entry is fitted, the unstored ones as 0.  Same CSR contract as rri_bind_csr
  * (int64 rowptr, int32 strictly ascending columns, nnz < 2^31, the three arrays stay alive while the handle is
- * used).  Only handles created with RRI_ORDER_HALS and RRI_MATH_IEEE (fp32 or fp64).  The column orientation and
- * the chunk plan of long rows / columns are built once (synchronises `stream`); the workspace grows with nnz and
- * (n + d) * k, never with n * d.  The block-order half-steps then take X T' and X' W from a sparse x dense
- * contraction.  On such a handle: rri_sweeps (block order and fix_T), rri_objective and rri_objective_contraction
- * (both through the identity, ||X||^2 from the stored values in fp64), rri_partials_T (nw of length 1),
- * rri_topic_sums, rri_stats and rri_profile_kernel (which = 1 / 2: the W- / T-half contraction, 3 / 4: the whole
- * half-steps).  rri_topics and rri_peer_export refuse it; row shards use the NCCL all-reduce. */
+ * used).  Handles created with RRI_MATH_IEEE (fp32 or fp64), in either order.  The column orientation and the chunk
+ * plan of long rows / columns are built once (synchronises `stream`); the workspace grows with nnz and (n + d) * k,
+ * never with n * d.  RRI_ORDER_HALS: the block-order half-steps take X T' and X' W from a sparse x dense contraction.
+ * RRI_ORDER_RRI: the interleaved order of the dense path with one fused pass over the rows and the columns per topic
+ * (y = X T_t', p = w_t+1' X), three launches per topic.  On such a handle: rri_sweeps (either order, and fix_T, which
+ * runs the block-order W half), rri_objective and rri_objective_contraction (both through the identity, ||X||^2 from
+ * the stored values in fp64), rri_partials_T (nw of length 1), rri_topic_sums, rri_stats, rri_spmm and
+ * rri_profile_kernel (which = 0: the fused pass of an rri-order handle, 1 / 2: the W- / T-half contraction, 3 / 4:
+ * the whole half-steps of a block-order handle).  rri_topics serves the rri-order handles and refuses the block-order
+ * ones; rri_peer_export refuses both: row shards use the NCCL all-reduce. */
 int rri_bind_csr_zero(rri_handle_t h, int64_t nnz, const int64_t* rowptr_dev, const int32_t* col_dev,
                       const void* val_dev, void* stream);
 
@@ -152,7 +155,8 @@ int rri_sweeps(rri_handle_t h, void* W_dev, void* T_dev, int32_t n_sweeps,
                const rri_params_t* p, int32_t* flags_host, void* stream);
 
 /* Run topics [t_begin, t_end) of ONE rri-order sweep (the body of the loop at nmf.py:415) so a host
- * policy (topic reset, nmf.py:762-783, :796-816) can act between topics.  rri order only. */
+ * policy (topic reset, nmf.py:762-783, :796-816) can act between topics.  rri order only (dense, masked,
+ * observed-entries or zero-filled sparse data). */
 int rri_topics(rri_handle_t h, void* W_dev, void* T_dev, int32_t t_begin, int32_t t_end,
                const rri_params_t* p, int32_t* flags_host, void* stream);
 
@@ -210,7 +214,8 @@ int rri_contract_x(rri_handle_t h, int32_t transpose, const void* B_dev, int64_t
 
 /* Roofline hook for bench.py: launch the dominant streaming kernel of this handle `iters` times on
  * `stream` between two CUDA events and return the average launch duration in milliseconds.
- *   which = 0: the rri-order fused pass (y = X T_t', p = w_t' X)      -- reads X[n,d] once
+ *   which = 0: the rri-order fused pass (y = X T_t', p = w_t' X)      -- reads X[n,d] once (zero-filled sparse
+ *              handles: the stored entries once in each orientation)
  *   which = 1: the W half-step contraction  X T'  (n x d -> n x k)     -- reads X once
  *   which = 2: the T half-step contraction  X' W  (d x n -> d x k)     -- reads X' once (hals handles)
  *   which = 3 / 4: one whole T / W half-step of the block order (contraction, Gram, exchange, update); these

@@ -185,6 +185,7 @@ struct rri_handle_s {
     // half-steps take X T' / X' W from launch_spmm instead of the dense contraction
     bool zero_csr = false;
     SpmmPlan zrow{}, zcol{};
+    SparsePassPlan spp{};              // RRI_ORDER_RRI: the fused pass over both orientations (sparse_rri_kernels.cu)
     // rri_spmm: chunk plans of an observed-entries handle (built on its first call, over w o x when weights were given)
     // and chunk slots for panels wider than k ([max chunks][spmm_slot_w], grown on demand)
     bool spmm_planned = false;
@@ -828,6 +829,20 @@ static int bind_csr_zero_impl(rri_handle_t h, const int64_t* rowptr, const int32
     if (build_spmm_plan(h, h->zrow, n, rowptr, col, val) ||
         build_spmm_plan(h, h->zcol, d, (const int64_t*)colptr, (const int32_t*)csc_row, x_csc))
         return 1;
+    if (h->order == RRI_ORDER_RRI) {
+        // the interleaved order's partials at ct = 1 / rg = 1: the sparse pass writes y [n] and p [d] directly, and the
+        // dense order's T-step, W-step and statistic reduction read them unchanged
+        h->spp = plan_sparse_rri_pass<T>(h->zrow, h->zcol, nnz, h->sm_count);
+        h->pp = PassPlan{1, 1, 1, 1, d};
+        h->hb = tstep_blocks(d);
+        h->gbw = wstep_blocks(n, h->sm_count);
+        const int ks = h->k + 1;
+        if (ws_alloc(h, &h->ypart, sizeof(T) * (size_t)n) || ws_alloc(h, &h->ppart, sizeof(T) * (size_t)d) ||
+            ws_alloc(h, &h->gpart, sizeof(T) * (size_t)h->gbw * ks) || ws_alloc(h, &h->hpart, sizeof(T) * (size_t)h->hb * ks) ||
+            ws_alloc(h, &h->stat, sizeof(T) * (size_t)(d + ks)))
+            return 1;
+        CK(cudaStreamSynchronize(0));
+    }
     CKL();
     CK(cudaStreamSynchronize(st));
     return 0;
@@ -841,7 +856,6 @@ extern "C" int rri_bind_csr_zero(rri_handle_t h, int64_t nnz, const int64_t* row
     if (nnz < 0 || nnz >= ((int64_t)1 << 31)) return fail("nnz must be in [0, 2^31) (got %lld)", (long long)nnz);
     if (!rowptr_dev) return fail("rowptr is null");
     if (nnz > 0 && (!col_dev || !val_dev)) return fail("col/val is null");
-    if (h->order != RRI_ORDER_HALS) return fail("zero-filled sparse data runs in block order: create the handle with RRI_ORDER_HALS");
     if (h->math != RRI_MATH_IEEE) return fail("zero-filled sparse data runs with RRI_MATH_IEEE (the sparse contraction is not compute-bound)");
     CK(cudaSetDevice(h->device));
     h->nnz = nnz;
@@ -958,15 +972,27 @@ static int check_params(rri_handle_t h, const rri_params_t* p)
 // -------------------------------------------------------------------------------------------------
 // rri order, unmasked
 // -------------------------------------------------------------------------------------------------
+// y = X T_t' (the W-step's statistic, do_y) and p = w_tn' X (the next T-step's, do_p) in one pass over X: the dense
+// streaming pass, or on a zero-filled sparse handle the pass over its rows and columns (ct = rg = 1)
+template <typename T>
+static void rri_pass(rri_handle_t h, const T* tvec, const T* W, int tn, bool do_y, bool do_p, cudaStream_t st)
+{
+    if (h->zero_csr)
+        launch_sparse_rri_pass<T>(h->spp, h->zrow, h->zcol, tvec, W, h->k, tn, (T*)h->ypart, (T*)h->ppart, do_y, do_p, st);
+    else
+        launch_rri_pass<T>((const T*)h->X, h->ldx, h->n, h->d, tvec, W, h->k, tn, (T*)h->ypart, (T*)h->ppart, do_y, do_p,
+                           h->pp, st);
+    h->launches++;
+}
+
 template <typename T>
 static int rri_prologue(rri_handle_t h, T* W, int t0, const rri_params_t* p, cudaStream_t st)
 {
     // p = w_t0' X and g = w_t0' W for the first T-step (nmf.py:672-673)
-    launch_rri_pass<T>((const T*)h->X, h->ldx, h->n, h->d, nullptr, W, h->k, t0, (T*)h->ypart, (T*)h->ppart,
-                       false, true, h->pp, st);
+    rri_pass<T>(h, nullptr, W, t0, false, true, st);
     launch_rri_wstep<T>(W, h->n, h->k, 0, t0, (const T*)h->ypart, h->pp.ct, h->n, (const T*)h->hpart, h->hb,
                         solve_args(p, false), (T*)h->gpart, h->sums, h->flags, false, h->gbw, st);
-    h->launches += 2;
+    h->launches++;
     CKL();
     return 0;
 }
@@ -1017,11 +1043,10 @@ static int rri_topic_range(rri_handle_t h, T* W, T* Tm, int t0, int t1, bool fir
         }
         // k == 1: the look-ahead statistic p = w_tn'X would be taken from the column this very topic is
         // about to overwrite, so it is recomputed after the W-step instead
-        launch_rri_pass<T>((const T*)h->X, h->ldx, n, d, Tm + (int64_t)t * d, W, k, tn, (T*)h->ypart,
-                           (T*)h->ppart, true, k > 1, h->pp, st);
+        rri_pass<T>(h, Tm + (int64_t)t * d, W, tn, true, k > 1, st);
         launch_rri_wstep<T>(W, n, k, t, tn, (const T*)h->ypart, h->pp.ct, n, (const T*)h->hpart, h->hb, aw,
                             (T*)h->gpart, h->sums, h->flags, true, h->gbw, st);
-        h->launches += 3;
+        h->launches += 2;
         if (k == 1) {
             if (rri_finish<T>(h, 0, st)) return 1;
             if (rri_prologue<T>(h, W, 0, p, st)) return 1;
@@ -1571,7 +1596,8 @@ extern "C" int rri_topics(rri_handle_t h, void* W_dev, void* T_dev, int32_t t_be
     if (!h) return fail("null handle");
     if (!W_dev || !T_dev) return fail("W or T is null");
     if (check_params(h, p)) return 1;
-    if (h->zero_csr) return fail("rri_topics does not serve zero-filled sparse handles (block order only)");
+    if (h->zero_csr && h->order != RRI_ORDER_RRI)
+        return fail("rri_topics does not serve zero-filled sparse handles of the block order (create one with RRI_ORDER_RRI)");
     if (h->order != RRI_ORDER_RRI) return fail("rri_topics needs a handle created with RRI_ORDER_RRI");
     if (p->fix_T) return fail("rri_topics does not take fix_T");
     if (t_begin < 0 || t_end > h->k || t_begin >= t_end) return fail("bad topic range [%d,%d)", t_begin, t_end);
@@ -1940,8 +1966,7 @@ static int profile_impl(rri_handle_t h, int which, const T* W, const T* Tm, int 
         }
         if (which == 0) {
             if (h->mk != MK_NONE || h->order != RRI_ORDER_RRI) return fail("which=0 needs an unmasked rri-order handle");
-            launch_rri_pass<T>((const T*)h->X, h->ldx, n, d, Tm, W, k, 1 % k, (T*)h->ypart, (T*)h->ppart, true, true, h->pp, st);
-            h->launches++;
+            rri_pass<T>(h, Tm, W, 1 % k, true, true, st);
         } else if (which == 1) {
             if (h->mk != MK_NONE) return fail("which=1 needs an unmasked handle");
             if (h->zero_csr) { launch_spmm<T>(h->zrow, (const T*)h->Tt, k, k, (T*)h->Cpart, k, st); h->launches++; continue; }

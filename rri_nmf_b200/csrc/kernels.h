@@ -316,4 +316,20 @@ void launch_spmm(const SpmmPlan& p, const T* B, int64_t ldb, int width, T* C, in
 // out[i] = w[i] * x[i]
 template <typename T>
 void launch_spmm_weighted_values(const T* x, const T* w, int64_t nnz, T* out, int sm_count, cudaStream_t st);
+
+// ---------------------------------------------------------------------------------------------
+// interleaved-order pass on zero-filled sparse data: both statistics of rri_pass_kernel in one launch
+//                                                                             (sparse_rri_kernels.cu)
+// ---------------------------------------------------------------------------------------------
+struct SparsePassPlan {
+    int gy, gp;            // lanes per work item over the rows / the columns
+    int blocks;            // resident blocks of one launch
+    int blocks_y, blocks_p;    // their split between the orientations when both statistics are computed
+};
+template <typename T>
+SparsePassPlan plan_sparse_rri_pass(const SpmmPlan& rows, const SpmmPlan& cols, int64_t nnz, int sm_count);
+// y[i] = sum_{e in row i} val[e] * trow[col[e]]   (do_y)   and   p[j] = sum_{e in col j} val[e] * W[row[e] * k + tn]   (do_p)
+template <typename T>
+void launch_sparse_rri_pass(const SparsePassPlan& pl, const SpmmPlan& rows, const SpmmPlan& cols, const T* trow,
+                            const T* W, int k, int tn, T* y, T* p, bool do_y, bool do_p, cudaStream_t st);
 }  // namespace rri

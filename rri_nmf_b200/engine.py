@@ -55,7 +55,8 @@ class RRIEngine(object):
     X may also be a torch sparse CSR tensor (never densified).  unstored='missing' (default): its stored entries are
     the observed ones (the recommender setting); W_mat is then an optional 1-D tensor of nnz entry weights.
     unstored='zero': X is an ordinary non-negative matrix stored sparsely (a tf-idf document-term matrix), every entry
-    is fitted, the unstored ones as 0 (rri_bind_csr_zero: order='hals', math='ieee', no W_mat).
+    is fitted, the unstored ones as 0 (rri_bind_csr_zero: math='ieee', no W_mat; order='hals' contracts X T' / X' W,
+    order='rri' makes one pass over the rows and the columns per topic).
     order: 'rri' (reference-exact interleaved order, nmf.py:415-476) or 'hals' (block order).
     math : 'ieee' or 'tf32' (tcgen05 tensor-core contraction; float32 + hals only).
     """
@@ -73,8 +74,6 @@ class RRIEngine(object):
         if unstored not in ('missing', 'zero'):
             raise ValueError("unstored must be 'missing' or 'zero'")
         if unstored == 'zero' and self.sparse:
-            if order != 'hals':
-                raise NotImplementedError("zero-filled sparse X runs in block order: use order='hals' (or X.to_dense())")
             if math != 'ieee':
                 raise ValueError("zero-filled sparse X runs with math='ieee' (the sparse contraction is not compute-bound)")
             if W_mat is not None:

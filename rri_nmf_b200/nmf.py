@@ -5,8 +5,10 @@ early stop, topic reset, return dict -- same names, meaning and error behaviour 
 
 Additional keyword-only arguments select the device path:
     device        torch device (default 'cuda'); there is NO CPU fallback
-    update_order  'rri'  -- the reference's interleaved order (default; exact drop-in), or
-                  'hals' -- block order: all T-steps then all W-steps (2 passes over X per sweep)
+    update_order  'rri'  -- the reference's interleaved order (exact drop-in), or
+                  'hals' -- block order: all T-steps then all W-steps (2 passes over X per sweep), or
+                  None   -- the default: 'rri' for every input except zero-filled sparse data (unstored='zero'), where
+                            the caller names the order (the two cost very different amounts there, see below)
     math          'ieee' (default) or 'tf32' (tcgen05 tensor-core contractions; float32 + 'hals')
     comm          engine.NcclComm for a row-sharded multi-GPU run (X, W_in, W_mat are the local shards)
     objective     how `obj_history` is evaluated: 'exact' = an explicit pass over X per evaluation (the reference's
@@ -34,11 +36,17 @@ set by the keyword-only argument `unstored`:
                   sklearn_interface.py:78-102 without densifying the (i, j, rating) triples and without a dense W_mat);
                   W_mat is then None or a sparse matrix of the same structure holding entry weights.
     'zero'        X is an ordinary non-negative matrix stored sparsely (a tf-idf document-term matrix): every entry is
-                  fitted, the unstored ones as 0 -- the result equals nmf(X.toarray(), ..., update_order='hals',
-                  math='ieee') up to the summation order.  Needs update_order='hals' (fix_T=True runs in either order),
-                  math='ieee' and no W_mat; the block-order half-steps take X T' and X' W from a sparse x dense
-                  contraction whose traffic grows with the stored entries, not with n * d.  Topic reset is not applied
-                  (an emptied topic raises, as on the dense block order).
+                  fitted, the unstored ones as 0 -- the result equals nmf(X.toarray(), ..., update_order=<the same>,
+                  math='ieee') up to the summation order.  Needs math='ieee', no W_mat, and an explicit update_order
+                  (fix_T=True runs the W-only sweeps whatever the order):
+                  'hals'  the block-order half-steps take X T' and X' W from a sparse x dense contraction; the fast
+                          choice (two passes over the stored entries per sweep).  Topic reset is not applied (an
+                          emptied topic raises, as on the dense block order).
+                  'rri'   the reference's interleaved order: per topic one pass over the stored entries in both
+                          orientations (k passes per sweep, an order of magnitude slower than 'hals', an order of
+                          magnitude faster than the densified matrix).  Topic reset works as on dense data: the
+                          residual document is found over the stored entries, never densifying X.
+                  Traffic grows with the stored entries, not with n * d.
 """
 import logging
 import time
@@ -84,8 +92,8 @@ class DeviceObjective(object):
                     Xd, Md = _sparse_to_device(X, W_mat, device, dtype)
                 else:
                     Xd, Md = _to_device(X, device, dtype), _mask_to_device(W_mat, device, dtype)
-                # (the zero-filled sparse binding exists in block order only; every other binding evaluates in 'rri')
-                eng = RRIEngine(Xd, int(np.shape(self.W)[1]), W_mat=Md, order='hals' if unstored == 'zero' else 'rri',
+                # (a zero-filled sparse binding evaluates in the order of the fit; every other binding in 'rri')
+                eng = RRIEngine(Xd, int(np.shape(self.W)[1]), W_mat=Md, order=order if unstored == 'zero' else 'rri',
                                 unstored=unstored)
                 try:
                     self.obj = eng.objective(_to_device(self.W, device, dtype).contiguous(),
@@ -303,7 +311,7 @@ def nmf(X, k, w_row=None, W_mat=None, fix_W=False, fix_T=False, random_state=Non
         t_row_sum=None, early_stop=None, reset_topic_method='max_resid_document', fix_reset_seed=False,
         n_resets=23, reg_w_l2=0, reg_t_l2=0, reg_w_l1=0, reg_t_l1=0, diagnostics=[], store_gradients=False,
         ind_rows_to_store=None, eps_gauss_t=None, delta_gauss_t=None,
-        *, device=None, update_order='rri', math='ieee', comm=None, engine=None, sweeps_per_call=16,
+        *, device=None, update_order=None, math='ieee', comm=None, engine=None, sweeps_per_call=16,
         init_on_device=None, return_reconstruction_err=False, sparse_refresh_every=1, objective='auto',
         unstored='missing'):
     """Non-negative factorisation X ~ W T by rank-one residue iteration.  See the reference docstring
@@ -312,8 +320,8 @@ def nmf(X, k, w_row=None, W_mat=None, fix_W=False, fix_T=False, random_state=Non
     (NumPy in -> NumPy out, torch tensor in -> torch tensors on the device)."""
     lib = _lib.load()           # fail loudly before doing anything if the CUDA library is missing
     del lib
-    if update_order not in ('rri', 'hals'):
-        raise ValueError("update_order must be 'rri' or 'hals'")
+    if update_order not in (None, 'rri', 'hals'):
+        raise ValueError("update_order must be 'rri', 'hals' or None")
     if unstored not in ('missing', 'zero'):
         raise ValueError("unstored must be 'missing' or 'zero'")
     zero_filled = unstored == 'zero' and _is_sparse(X)
@@ -324,9 +332,12 @@ def nmf(X, k, w_row=None, W_mat=None, fix_W=False, fix_T=False, random_state=Non
             raise ValueError("unstored='zero' runs with math='ieee' (the sparse contraction is not compute-bound)")
         if fix_W:
             raise NotImplementedError("fix_W=True is not available with unstored='zero'")
-        if update_order != 'hals' and not fix_T:
-            raise NotImplementedError("unstored='zero' runs in block order: use update_order='hals', or densify with "
-                                      "X.toarray() for the interleaved order")
+        if update_order is None and not fix_T:
+            raise NotImplementedError("unstored='zero' needs an explicit order: update_order='hals' (block order, fast) or "
+                                      "update_order='rri' (the reference's interleaved order, k passes per sweep), or "
+                                      "densify with X.toarray()")
+    if update_order is None:
+        update_order = 'rri'
     n, d = X.shape
     rtv = {}
     numpy_io = not isinstance(X, torch.Tensor)
@@ -455,9 +466,10 @@ def nmf(X, k, w_row=None, W_mat=None, fix_W=False, fix_T=False, random_state=Non
         _t1 = time.perf_counter()
         own_engine = engine is None
         if engine is None:
-            # (fix_T: the W-only sweeps are the same in both orders; the zero-filled binding is a block-order one)
-            engine = RRIEngine(Xd, k, W_mat=Md, order='hals' if zero_filled else update_order, math=math, comm=comm,
-                               unstored=unstored)
+            # (fix_T: the W-only sweeps are the same in both orders; on zero-filled data they run on a block-order
+            # binding, which holds no interleaved-order partials)
+            engine = RRIEngine(Xd, k, W_mat=Md, order='hals' if zero_filled and fix_T else update_order, math=math,
+                               comm=comm, unstored=unstored)
         timing['engine_setup_s'] = time.perf_counter() - _t1       # workspace, transposed copy of X, peer mapping
         try:
             if init_on_device:
@@ -734,9 +746,14 @@ def _sweep_with_resets(engine, Xd, W, T, params, a, state):
     def reset(t):
         state['n_resets_remaining'] -= 1
         if method == 'max_resid_document':
-            R = (Xd - W @ T).clamp_(min=0)
-            mi = int(torch.argmax((R ** 2).sum(1)))
-            T[t, :] = R[mi, :]
+            if engine.sparse:
+                mi, cols, vals = max_resid_document_sparse(engine.crow, engine.col, engine.val, W, T)
+                T[t, :] = 0
+                T[t, cols] = vals
+            else:
+                R = (Xd - W @ T).clamp_(min=0)
+                mi = int(torch.argmax((R ** 2).sum(1)))
+                T[t, :] = R[mi, :]
             W[:, t] = 0
             W[mi, t] = 1.0
         elif method == 'random':
@@ -772,14 +789,37 @@ def _sweep_with_resets(engine, Xd, W, T, params, a, state):
     return flags_all
 
 
+def max_resid_document_sparse(crow, col, val, W, T, chunk_entries=None):
+    """(i, columns, values) for zero-filled sparse X given as CSR (crow, col, val): i is the first row of
+    max(X - W T, 0) with the largest sum of squares (the reference's 'max_resid_document', nmf.py:766-770), columns and
+    values are that row's stored entries of the clamped residual.  With W, T >= 0 every unstored entry of
+    max(X - W T, 0) is max(-W[i] . T[:, j], 0) = 0, so the sums run over the stored entries only, in chunks of
+    entries: no n x d array is formed."""
+    nnz = int(val.numel())
+    step = chunk_entries or max(1, (1 << 22) // max(int(W.shape[1]), 1))
+    col = col.to(torch.int64)
+    r = torch.empty(nnz, dtype=W.dtype, device=W.device)
+    for a in range(0, nnz, step):
+        b = min(a + step, nnz)
+        rows = torch.searchsorted(crow, torch.arange(a, b, device=crow.device), right=True) - 1
+        pred = (W[rows] * T[:, col[a:b]].t()).sum(1)
+        r[a:b] = (val[a:b].to(W.dtype) - pred).clamp_(min=0)
+    # (one fixed summation order per row)
+    ss = torch.segment_reduce(r * r, 'sum', lengths=crow.diff(), unsafe=True)
+    mi = int(torch.argmax(ss))
+    lo, hi = int(crow[mi]), int(crow[mi + 1])
+    return mi, col[lo:hi], r[lo:hi]
+
+
 def _w_step_only(engine, W, T, t, params):
     """W-step of topic t alone (nmf.py:462-469 with the current T), used only on the rare reset path right after
-    a topic was re-seeded; plain torch ops on the device tensors."""
+    a topic was re-seeded; plain torch ops on the device tensors (X T_t' of sparse data through rri_spmm)."""
     Tt = T[t, :]
     h = T @ Tt
     nt = float(h[t])
     h[t] = 0
-    numer = engine.X @ Tt - W @ h - params.reg_w_l1
+    xt = engine.products().right(Tt.reshape(-1, 1))[:, 0] if engine.sparse else engine.X @ Tt
+    numer = xt - W @ h - params.reg_w_l1
     denom = nt + params.reg_w_l2
     if denom > 0:
         W[:, t] = numer.clamp(min=0) / (denom + params.eps)

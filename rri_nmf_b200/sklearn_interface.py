@@ -6,11 +6,13 @@ plus the sklearn-conventional read-only aliases `components_` (= T), `n_componen
 
 Additional constructor arguments: `device`, `update_order`, `math` (forwarded to `nmf`); `NMF_RS_Estimator` also
 takes `sparse=True` to keep the (i, j, rating) triples sparse all the way to the device (observed-entries engine,
-traffic proportional to the number of ratings) instead of densifying them as the reference does.
+traffic proportional to the number of ratings) instead of densifying them as the reference does; `NMF_TM_Estimator`
+takes `sparse=True` to keep scipy.sparse document-term matrices sparse in the interleaved order (see below).
 
 `NMF_TM_Estimator` takes scipy.sparse document-term matrices in fit, fit_transform, one_iter, transform and score.  With
-update_order='hals' X stays sparse all the way to the device (nmf(..., unstored='zero'): unstored entries are zeros);
-with the default update_order='rri' the estimator densifies X and runs the reference-exact interleaved order.
+update_order='hals' X stays sparse all the way to the device (nmf(..., unstored='zero'): unstored entries are zeros).
+With the default update_order='rri' the estimator densifies X and runs the reference-exact interleaved order, unless it
+was built with `sparse=True`: then X stays sparse in that order too (one pass over the stored entries per topic).
 """
 import numpy as np
 import scipy.sparse as sp
@@ -85,7 +87,7 @@ class NMF_TM_Estimator(_FactorMixin, sklearn.base.BaseEstimator, sklearn.base.Tr
 
     def __init__(self, n, d, k, wr1=0, wr2=0, tr1=0, tr2=0, random_state=0, handle_tfidf=False,
                  handle_normalization=False, max_iter=300, W=_EMPTY, T=_EMPTY, nmf_kwargs={},
-                 do_final_project_W=True, device=None, update_order='rri', math='ieee'):
+                 do_final_project_W=True, device=None, update_order='rri', math='ieee', sparse=False):
         self.n, self.d, self.k = n, d, k
         self.wr1, self.wr2, self.tr1, self.tr2 = wr1, wr2, tr1, tr2
         self.random_state = random_state
@@ -96,10 +98,12 @@ class NMF_TM_Estimator(_FactorMixin, sklearn.base.BaseEstimator, sklearn.base.Tr
         self.nmf_kwargs = nmf_kwargs
         self.do_final_project_W = do_final_project_W
         self.device, self.update_order, self.math = device, update_order, math
+        self.sparse = sparse
 
     def _keep_sparse(self, X):
-        """sparse X goes to the device as it is in block order; the interleaved order runs on its dense form"""
-        return sp.issparse(X) and self.update_order == 'hals'
+        """sparse X goes to the device as it is in block order, and in the interleaved order with sparse=True;
+        otherwise the interleaved order runs on its dense form"""
+        return sp.issparse(X) and (self.update_order == 'hals' or self.sparse)
 
     def _prep(self, X, fit):
         if self._keep_sparse(X):
@@ -170,8 +174,8 @@ class NMF_TM_Estimator(_FactorMixin, sklearn.base.BaseEstimator, sklearn.base.Tr
         return self.transform(X)
 
     def score(self, X, y=None):
-        """R^2 of the reconstruction of new X (sklearn_interface.py:339-345).  Sparse X in block order: no n x d array
-        is formed -- SST = ||X||^2 - n ||mean||^2 and SSE = ||X||^2 - 2 <X T', W> + <W'W, T T'>, in fp64 on the host."""
+        """R^2 of the reconstruction of new X (sklearn_interface.py:339-345).  Sparse X kept sparse (block order, or
+        sparse=True): no n x d array is formed -- SST = ||X||^2 - n ||mean||^2 and SSE = ||X||^2 - 2 <X T', W> + <W'W, T T'>, in fp64 on the host."""
         if self._keep_sparse(X):
             X = sp.csr_matrix(X, dtype=np.float64)
             return _r2_sparse(X, self.transform(X), self.T)
