@@ -88,6 +88,17 @@ int rri_peer_enable(rri_handle_t h, int32_t on);
 /* unmap the peers' buffers; all ranks call it (and synchronise) BEFORE any rank destroys its handle */
 int rri_peer_close(rri_handle_t h);
 
+/* Several models of one matrix on one binding (restarts, consensus runs): after rri_create, whose k is the total width
+ * models * k_m <= 256, and before rri_bind.  Needs RRI_ORDER_HALS, world == 1 and k % models == 0; dense unmasked data
+ * (rri_bind refuses a mask, rri_bind_csr / rri_bind_csr_zero refuse the handle).  Each block-order half-step makes one
+ * contraction over the stacked factor operand (one read of X for all models) and one row-update launch for all models,
+ * each at rank k_m; with RRI_MATH_IEEE every model is bit-identical to a handle of its own.  Layouts:
+ *     W_dev [models][n_local][k_m],   T_dev [models][k_m][d]  (= the stacked [k, d] operand of the W half-step).
+ * Per model: rri_sweeps writes `models` flag words to flags_host, rri_topic_sums returns k sums per factor (model-major),
+ * rri_objective and rri_objective_contraction write 6 doubles per model.  rri_topics, rri_partials_T and the peer-memory
+ * entry points refuse the handle; sweeps take no simplex_T.  models == 1 is a handle as rri_create makes it. */
+int rri_set_models(rri_handle_t h, int32_t models);
+
 /* Optional, before rri_bind on a hals handle: storage [d, ldXt] (ldXt >= n rounded up to 16 bytes) owned by the
  * caller for the engine's transposed copy of X, so that it comes from the caller's allocator (torch's caching
  * allocator: no cudaMalloc/cudaFree of a data-sized buffer per fit).

@@ -123,6 +123,9 @@ struct PeerGroup {
 struct rri_handle_s {
     int64_t n = 0, d = 0;
     int k = 0, dtype = 0, math = 0, order = 0, device = 0, sm_count = 148;
+    // several models of rank km = k / models on one binding (rri_set_models): W [models][n][km], T [models][km][d] (the
+    // stacked [k, d] operand of the W-half contraction), Tt [models][d][km], Wt the stacked [k, ldwt]
+    int models = 1, km = 0;
     size_t es = 4;
     // data
     const void* X = nullptr; int64_t ldx = 0;
@@ -242,7 +245,7 @@ extern "C" int rri_create(rri_handle_t* out, int64_t n_local, int64_t d, int32_t
     if (prop.major != 10)
         return fail("device %d is sm_%d%d; this build contains sm_100a code only", device, prop.major, prop.minor);
     rri_handle_t h = new rri_handle_s();
-    h->n = n_local; h->d = d; h->k = k; h->dtype = dtype; h->math = math; h->order = order;
+    h->n = n_local; h->d = d; h->k = k; h->km = k; h->dtype = dtype; h->math = math; h->order = order;
     h->device = device; h->sm_count = prop.multiProcessorCount;
     h->es = dtype == RRI_F32 ? 4 : 8;
     if (ws_alloc(h, (void**)&h->sums, sizeof(double) * 2 * k) || ws_alloc(h, (void**)&h->flags, sizeof(int) * 4) ||
@@ -275,6 +278,7 @@ extern "C" int rri_destroy(rri_handle_t h)
 extern "C" int rri_set_comm(rri_handle_t h, void* nccl_comm, int32_t rank, int32_t world, const char* nccl_lib_path)
 {
     if (!h) return fail("null handle");
+    if (world > 1 && h->models > 1) return fail("a handle of several models runs on one GPU (world == 1)");
     if (world > 1) {
         if (!nccl_comm) return fail("world > 1 needs a communicator");
         if (nccl_load(nccl_lib_path)) return 1;
@@ -314,6 +318,7 @@ extern "C" int rri_peer_export(rri_handle_t h, char handle_out[64])
     if (!h->X) return fail("rri_bind has not been called");
     if (h->order != RRI_ORDER_HALS || h->mk != MK_NONE) return fail("the peer-memory exchange serves unmasked hals handles");
     if (h->zero_csr) return fail("the peer-memory exchange serves dense data; zero-filled sparse handles use the NCCL all-reduce");
+    if (h->models > 1) return fail("the peer-memory exchange does not serve a handle of several models");
     if (!peer_rank_supported(h)) return fail("the fused peer-memory T update supports k <= 128 (f32) / 64 (f64)");
     CK(cudaSetDevice(h->device));
     if (!h->xbuf) {
@@ -348,6 +353,7 @@ extern "C" int rri_peer_export(rri_handle_t h, char handle_out[64])
 extern "C" int rri_peer_import(rri_handle_t h, const char* handles, int32_t rank, int32_t world)
 {
     if (!h) return fail("null handle");
+    if (h->models > 1) return fail("the peer-memory exchange does not serve a handle of several models");
     if (!h->xbuf) return fail("rri_peer_export must be called first");
     if (world < 2 || world > 16 || rank < 0 || rank >= world) return fail("bad rank/world %d/%d", rank, world);
     CK(cudaSetDevice(h->device));
@@ -424,6 +430,7 @@ extern "C" int rri_peer_close(rri_handle_t h)
 extern "C" int rri_peer_enable(rri_handle_t h, int32_t on)
 {
     if (!h) return fail("null handle");
+    if (h->models > 1) return fail("the peer-memory exchange does not serve a handle of several models");
     if (on && !h->peer_mapped) return fail("rri_peer_import has not succeeded on this rank");
     h->p2p = on != 0;
     // with the exchange on, the T' copy of this handle IS its replica inside the exchange buffer (the peers write
@@ -491,10 +498,11 @@ static int alloc_halfstep_ws(rri_handle_t h)
         h->ldwt = (n + v - 1) / v * v;
     }
     if (ws_alloc(h, &h->Wt, es * (size_t)k * h->ldwt) || ws_alloc(h, &h->Tt, es * (size_t)d * k)) return 1;
-    h->gchunks_w = gram_chunks(n, k, h->sm_count);
-    h->gchunks_t = gram_chunks(d, k, h->sm_count);
+    // (IEEE Gram products: per model, chunked as a handle of one model of rank km would chunk them)
+    h->gchunks_w = gram_chunks(n, h->km, h->sm_count);
+    h->gchunks_t = gram_chunks(d, h->km, h->sm_count);
     const int gc = h->gchunks_w > h->gchunks_t ? h->gchunks_w : h->gchunks_t;
-    if (ws_alloc(h, &h->gram_part, es * (size_t)gc * k * k)) return 1;
+    if (ws_alloc(h, &h->gram_part, es * (size_t)gc * k * h->km)) return 1;
     h->ub_blocks_w = update_rows_blocks(n, h->sm_count);
     h->ub_blocks_t = update_rows_blocks(d, h->sm_count);
     int ubm = h->ub_blocks_w > h->ub_blocks_t ? h->ub_blocks_w : h->ub_blocks_t;
@@ -518,7 +526,9 @@ static int bind_impl(rri_handle_t h, cudaStream_t st)
         size_t op = 2 * (size_t)(h->oblocks > 256 ? h->oblocks : 256);
         if (op < (size_t)8 * h->sm_count) op = (size_t)8 * h->sm_count;
         if (ws_alloc(h, (void**)&h->obj_part, sizeof(double) * op)) return 1;
-        if (ws_alloc(h, (void**)&h->obj_out, sizeof(double) * 16)) return 1;
+        // model z's six numbers at obj_out + 8 z, then ||X||^2 and one <X T', W> per model (obj_slots)
+        const size_t oo = (size_t)9 * h->models + 1;
+        if (ws_alloc(h, (void**)&h->obj_out, sizeof(double) * (oo > 16 ? oo : 16))) return 1;
     }
     if (h->mk != MK_NONE) {
         if (!h->numer_part) {
@@ -623,6 +633,25 @@ static int bind_impl(rri_handle_t h, cudaStream_t st)
     return 0;
 }
 
+extern "C" int rri_set_models(rri_handle_t h, int32_t models)
+{
+    if (!h) return fail("null handle");
+    if (h->X) return fail("rri_set_models must be called before the data are bound");
+    if (models < 1) return fail("models must be >= 1 (got %d)", models);
+    if (h->order != RRI_ORDER_HALS) return fail("several models per handle need RRI_ORDER_HALS");
+    if (h->world != 1) return fail("several models per handle run on one GPU (world == 1)");
+    if (h->k % models != 0) return fail("k (%d) must be a multiple of models (%d)", h->k, models);
+    if (models > 4) {       // one flags word per model (rri_create allocates 4)
+        ws_release(h, h->flags, sizeof(int) * 4);
+        h->flags = nullptr;
+        if (ws_alloc(h, (void**)&h->flags, sizeof(int) * (size_t)models)) return 1;
+        CK(cudaStreamSynchronize(0));
+    }
+    h->models = models;
+    h->km = h->k / models;
+    return 0;
+}
+
 extern "C" int rri_set_transpose_storage(rri_handle_t h, void* Xt_dev, int64_t ldXt)
 {
     if (!h) return fail("null handle");
@@ -644,6 +673,7 @@ extern "C" int rri_bind(rri_handle_t h, const void* X_dev, int64_t ldX, const vo
     if (h->zero_csr) return fail("this handle is bound to zero-filled sparse (CSR) data; create a new one for dense data");
     if (h->X && ((h->mk != MK_NONE) != (mask_kind != RRI_MASK_NONE)))
         return fail("a handle cannot switch between masked and unmasked data; create a new one");
+    if (h->models > 1 && mask_kind != RRI_MASK_NONE) return fail("a handle of several models takes unmasked data");
     CK(cudaSetDevice(h->device));
     h->X = X_dev; h->ldx = ldX;
     h->M = mask_kind == RRI_MASK_NONE ? nullptr : mask_dev;
@@ -743,6 +773,7 @@ extern "C" int rri_bind_csr(rri_handle_t h, int64_t nnz, const int64_t* rowptr_d
 {
     if (!h) return fail("null handle");
     if (h->X) return fail("the handle is already bound; create a new one");
+    if (h->models > 1) return fail("a handle of several models takes dense data (rri_bind)");
     if (nnz < 0 || nnz >= ((int64_t)1 << 31)) return fail("nnz must be in [0, 2^31) (got %lld)", (long long)nnz);
     if (!rowptr_dev) return fail("rowptr is null");
     if (nnz > 0 && (!col_dev || !val_dev)) return fail("col/val is null");
@@ -853,6 +884,7 @@ extern "C" int rri_bind_csr_zero(rri_handle_t h, int64_t nnz, const int64_t* row
 {
     if (!h) return fail("null handle");
     if (h->X) return fail("the handle is already bound; create a new one");
+    if (h->models > 1) return fail("a handle of several models takes dense data (rri_bind)");
     if (nnz < 0 || nnz >= ((int64_t)1 << 31)) return fail("nnz must be in [0, 2^31) (got %lld)", (long long)nnz);
     if (!rowptr_dev) return fail("rowptr is null");
     if (nnz > 0 && (!col_dev || !val_dev)) return fail("col/val is null");
@@ -966,6 +998,7 @@ static int check_params(rri_handle_t h, const rri_params_t* p)
     // simplex_T, unmasked: Euclidean projection of the row onto the simplex (optimization.py:58-59); masked / observed
     // entries: the vector-c branch rescales the clipped solution to the sum (optimization.py:85-87)
     if (p->simplex_T && !(p->ub_t > 0)) return fail("simplex_T needs t_row_sum > 0");
+    if (p->simplex_T && h->models > 1) return fail("simplex_T is not available on a handle of several models");
     return 0;
 }
 
@@ -1112,15 +1145,51 @@ static int data_contraction(rri_handle_t h, bool transpose, const T* B, int64_t 
     return 0;
 }
 
+// Tt [models][d][km] <- the transpose of every model's T [km, d]
+template <typename T>
+static void transpose_T(rri_handle_t h, const T* Tm, cudaStream_t st)
+{
+    const int km = h->km;
+    for (int z = 0; z < h->models; ++z)
+        launch_transpose<T>(Tm + (int64_t)z * km * h->d, km, h->d, h->d, (T*)h->Tt + (int64_t)z * h->d * km, km, st);
+    h->launches += h->models;
+}
+
+// Wt [k, ldwt] (stacked, model-major rows) <- the transpose of every model's W [n, km]
+template <typename T>
+static void transpose_W(rri_handle_t h, const T* W, cudaStream_t st)
+{
+    const int km = h->km;
+    for (int z = 0; z < h->models; ++z)
+        launch_transpose<T>(W + (int64_t)z * h->n * km, h->n, km, km, (T*)h->Wt + (int64_t)z * km * h->ldwt, h->ldwt, st);
+    h->launches += h->models;
+}
+
+// The row updates of all models of a handle in one launch: model z reads the column block z*km of the stacked contraction
+// and its Gram matrix -- the diagonal block z of the k x k Gram tile of the tensor-core contraction, or the z-th of the
+// per-model IEEE Gram products
+static RowBatch row_batch(rri_handle_t h, bool tc_gram)
+{
+    RowBatch rb;
+    rb.models = h->models;
+    rb.ldc = h->k;
+    rb.lds = tc_gram ? h->k : h->km;
+    rb.s_stride = tc_gram ? (int64_t)h->km * (h->k + 1) : (int64_t)h->km * h->km;
+    return rb;
+}
+
 template <typename T>
 static int hals_W_half(rri_handle_t h, T* W, const T* Tk, int64_t ldtk, const rri_params_t* p, bool recompute, cudaStream_t st)
 {
-    const int k = h->k;
+    const int k = h->k, km = h->km;
     const int64_t n = h->n, d = h->d;
+    const bool tc_gram = gram_in_contraction(h);
     if (recompute) {
         // C2 = X T' and H = T T' (from the d x k transposed copy, or as the Gram tile of the contraction)
-        const bool tc_gram = gram_in_contraction(h);
-        if (!tc_gram) { launch_gram<T>((const T*)h->Tt, d, k, (T*)h->gram_part, h->gchunks_t, (T*)h->Hm, st); h->launches += 2; }
+        if (!tc_gram) {
+            launch_gram<T>((const T*)h->Tt, d, km, (T*)h->gram_part, h->gchunks_t, (T*)h->Hm, st, h->models, d * km);
+            h->launches += 2;
+        }
         if (h->zero_csr) {
             launch_spmm<T>(h->zrow, (const T*)h->Tt, k, k, (T*)h->Cpart, k, st);
             h->launches++;
@@ -1131,9 +1200,9 @@ static int hals_W_half(rri_handle_t h, T* W, const T* Tk, int64_t ldtk, const rr
     const int parts = h->math == RRI_MATH_TF32 ? 1 : h->splits_w;
     // the zero-column test of nmf.py:793 is over ALL rows: with row shards the sums are all-reduced once per call
     // (the per-topic sums and the zero-topic flags are taken once per call from W' and T: hals_finish_sums)
-    launch_update_rows<T>(W, n, k, (const T*)h->Cpart, parts, n * k, nullptr, (const T*)h->Hm, solve_args(p, false),
+    launch_update_rows<T>(W, n, km, (const T*)h->Cpart, parts, n * k, nullptr, (const T*)h->Hm, solve_args(p, false),
                           (T*)h->Wt, h->ldwt, (T*)h->colsum_part, h->flags, h->ub_blocks_w,
-                          ColsumOut{nullptr, k, 0, h->counters + 0}, st);
+                          ColsumOut{nullptr, k, 0, h->counters + 0}, row_batch(h, tc_gram), st);
     h->launches++;
     CKL();
     return 0;
@@ -1170,7 +1239,7 @@ static int hals_T_half(rri_handle_t h, T* W, T* Tk, int64_t ldtk, const rri_para
         CKL();
         return 0;
     }
-    if (!tc_gram) { launch_gram<T>(W, n, k, (T*)h->gram_part, h->gchunks_w, G, st); h->launches += 2; }
+    if (!tc_gram) { launch_gram<T>(W, n, h->km, (T*)h->gram_part, h->gchunks_w, G, st, h->models, n * h->km); h->launches += 2; }
     // (one rank, TF32: the Gram tile lands right behind the contraction output, as the all-reduce wants it)
     T* Cout = (h->world > 1 && psplits == 1) ? cg : (T*)h->Cpart;
     if (h->zero_csr) {
@@ -1199,8 +1268,8 @@ static int hals_T_half(rri_handle_t h, T* W, T* Tk, int64_t ldtk, const rri_para
         return 0;
     }
     // Tt (d x k) is updated in place; its transpose is written straight into the caller's T (k x d)
-    launch_update_rows<T>((T*)h->Tt, d, k, C, parts, d * k, nullptr, G, solve_args(p, true), Tk, ldtk, (T*)h->colsum_part,
-                          h->flags, h->ub_blocks_t, ColsumOut{nullptr, 0, 0, h->counters + 2}, st);
+    launch_update_rows<T>((T*)h->Tt, d, h->km, C, parts, d * k, nullptr, G, solve_args(p, true), Tk, ldtk, (T*)h->colsum_part,
+                          h->flags, h->ub_blocks_t, ColsumOut{nullptr, 0, 0, h->counters + 2}, row_batch(h, tc_gram), st);
     h->launches++;
     CKL();
     return 0;
@@ -1213,10 +1282,10 @@ static int hals_T_half(rri_handle_t h, T* W, T* Tk, int64_t ldtk, const rri_para
 template <typename T>
 static int hals_finish_sums(rri_handle_t h, const T* Tm, bool t_sums, cudaStream_t st)
 {
-    launch_rowsum_flag<T>((const T*)h->Wt, h->k, h->n, h->ldwt, h->sums, h->k, h->world > 1 ? 0 : 2, h->flags, st);
+    launch_rowsum_flag<T>((const T*)h->Wt, h->k, h->n, h->ldwt, h->sums, h->k, h->world > 1 ? 0 : 2, h->flags, st, h->km);
     h->launches++;
     if (t_sums) {
-        launch_rowsum_flag<T>(Tm, h->k, h->d, h->d, h->sums, 0, 1, h->flags, st);
+        launch_rowsum_flag<T>(Tm, h->k, h->d, h->d, h->sums, 0, 1, h->flags, st, h->km);
         h->launches++;
     }
     if (h->world <= 1) return 0;
@@ -1489,7 +1558,7 @@ template <typename T>
 static int sweeps_impl(rri_handle_t h, T* W, T* Tm, int n_sweeps, const rri_params_t* p, cudaStream_t st)
 {
     const int k = h->k;
-    const int64_t n = h->n, d = h->d;
+    const int64_t d = h->d;
     if (h->sparse) return sp_sweeps<T>(h, W, Tm, n_sweeps, p, st);
     if (h->mk != MK_NONE) {
         if (h->wtc) { wrri_tc_load_factors(h->wtc, (const float*)W, (const float*)Tm, st); h->launches += 2; }
@@ -1510,16 +1579,14 @@ static int sweeps_impl(rri_handle_t h, T* W, T* Tm, int n_sweeps, const rri_para
     if (p->fix_T) {
         // W-only sweeps (transform(): sklearn_interface.py:327-334): X T' and T T' are constant, so
         // one pass over X serves every sweep; both update orders coincide here
-        launch_transpose<T>(Tm, k, d, d, (T*)h->Tt, k, st);
-        h->launches++;
+        transpose_T<T>(h, Tm, st);
         for (int s = 0; s < n_sweeps; ++s)
             if (hals_W_half<T>(h, W, Tm, d, p, s == 0, st)) return 1;
         return n_sweeps > 0 ? hals_finish_sums<T>(h, Tm, false, st) : 0;
     }
     if (h->order == RRI_ORDER_HALS) {
-        launch_transpose<T>(Tm, k, d, d, (T*)h->Tt, k, st);
-        launch_transpose<T>(W, n, k, k, (T*)h->Wt, h->ldwt, st);
-        h->launches += 2;
+        transpose_T<T>(h, Tm, st);
+        transpose_W<T>(h, W, st);
         const bool px = h->world > 1 && h->p2p;
         // with the peer exchange the current T lives in this rank's replica inside the exchange buffer (the peers
         // store the rows they update into it); the caller's T is loaded into it here and read back at the end
@@ -1545,7 +1612,7 @@ static int sweeps_impl(rri_handle_t h, T* W, T* Tm, int n_sweeps, const rri_para
 static int read_flags(rri_handle_t h, int32_t* flags_host, cudaStream_t st)
 {
     if (!flags_host) return 0;
-    CK(cudaMemcpyAsync(flags_host, h->flags, sizeof(int), cudaMemcpyDeviceToHost, st));
+    CK(cudaMemcpyAsync(flags_host, h->flags, sizeof(int) * (size_t)h->models, cudaMemcpyDeviceToHost, st));
     CK(cudaStreamSynchronize(st));
     return 0;
 }
@@ -1559,7 +1626,7 @@ extern "C" int rri_sweeps(rri_handle_t h, void* W_dev, void* T_dev, int32_t n_sw
     if (check_params(h, p)) return 1;
     CK(cudaSetDevice(h->device));
     cudaStream_t st = (cudaStream_t)stream;
-    CK(cudaMemsetAsync(h->flags, 0, sizeof(int), st));
+    CK(cudaMemsetAsync(h->flags, 0, sizeof(int) * (size_t)h->models, st));
     h->c2_valid = false;
     if (n_sweeps > 0) {
         int rc = h->dtype == RRI_F32 ? sweeps_impl<float>(h, (float*)W_dev, (float*)T_dev, n_sweeps, p, st)
@@ -1641,12 +1708,29 @@ static int objective_impl(rri_handle_t h, const T* W, const T* Tm, cudaStream_t 
         CKL();
         return 0;
     }
-    launch_objective<T>((const T*)h->X, h->ldx, h->M, h->mk, h->ldm, W, Tm, h->n, h->d, h->k, h->obj_part,
-                        h->oblocks, h->obj_out, st);
-    launch_norms<T>(W, h->n * h->k, h->obj_part, h->obj_out + 2, st);
-    launch_norms<T>(Tm, (int64_t)h->k * h->d, h->obj_part, h->obj_out + 4, st);
-    h->launches += 6;
+    // one explicit pass per model over its own W and T, as separate fits make it
+    const int km = h->km;
+    for (int z = 0; z < h->models; ++z) {
+        const T* Wz = W + (int64_t)z * h->n * km;
+        const T* Tz = Tm + (int64_t)z * km * h->d;
+        double* out = h->obj_out + 8 * z;
+        launch_objective<T>((const T*)h->X, h->ldx, h->M, h->mk, h->ldm, Wz, Tz, h->n, h->d, km, h->obj_part,
+                            h->oblocks, out, st);
+        launch_norms<T>(Wz, h->n * km, h->obj_part, out + 2, st);
+        launch_norms<T>(Tz, (int64_t)km * h->d, h->obj_part, out + 4, st);
+        h->launches += 6;
+    }
     CKL();
+    return 0;
+}
+
+// the six numbers of every model (model z's at obj_out + 8 z) -> out_host[6 z ..]
+static int copy_objective(rri_handle_t h, double* out_host, cudaStream_t st)
+{
+    std::vector<double> v((size_t)8 * h->models);
+    CK(cudaMemcpyAsync(v.data(), h->obj_out, sizeof(double) * v.size(), cudaMemcpyDeviceToHost, st));
+    CK(cudaStreamSynchronize(st));
+    for (int z = 0; z < h->models; ++z) memcpy(out_host + 6 * z, v.data() + 8 * z, sizeof(double) * 6);
     return 0;
 }
 
@@ -1660,9 +1744,7 @@ extern "C" int rri_objective(rri_handle_t h, const void* W_dev, const void* T_de
     int rc = h->dtype == RRI_F32 ? objective_impl<float>(h, (const float*)W_dev, (const float*)T_dev, st)
                                  : objective_impl<double>(h, (const double*)W_dev, (const double*)T_dev, st);
     if (rc) return rc;
-    CK(cudaMemcpyAsync(out_host, h->obj_out, sizeof(double) * 6, cudaMemcpyDeviceToHost, st));
-    CK(cudaStreamSynchronize(st));
-    return 0;
+    return copy_objective(h, out_host, st);
 }
 
 // Objective through the contraction (unmasked dense data):  ||X - W T||^2 = ||X||^2 - 2 <X T', W> + <W'W, T T'>.
@@ -1672,19 +1754,19 @@ template <typename T>
 static int objective_contraction_impl(rri_handle_t h, const T* W, const T* Tm, bool reuse, cudaStream_t st)
 {
     const int64_t n = h->n, d = h->d;
-    const int k = h->k;
+    const int k = h->k, km = h->km, models = h->models;
     if (!h->Gobj && ws_alloc(h, &h->Gobj, sizeof(T) * 2 * (size_t)k * k)) return 1;
     CK(cudaStreamSynchronize(0));
-    double* acc = h->obj_out + 8;                       // {||X||^2, <X T', W>}
+    double* xsq = h->obj_out + 8 * models;              // ||X||^2, then <X T', W> of every model
+    double* cross = xsq + 1;
     if (!h->xsq_valid) {
-        if (h->zero_csr) launch_sumsq_rows<T>((const T*)h->zrow.val, 1, h->nnz, h->nnz, h->obj_part, acc, h->sm_count, st);
-        else launch_sumsq_rows<T>((const T*)h->X, n, d, h->ldx, h->obj_part, acc, h->sm_count, st);
+        if (h->zero_csr) launch_sumsq_rows<T>((const T*)h->zrow.val, 1, h->nnz, h->nnz, h->obj_part, xsq, h->sm_count, st);
+        else launch_sumsq_rows<T>((const T*)h->X, n, d, h->ldx, h->obj_part, xsq, h->sm_count, st);
         h->xsq_valid = true;
         h->launches += 2;
     }
     if (!(reuse && h->c2_valid)) {
-        launch_transpose<T>(Tm, k, d, d, (T*)h->Tt, k, st);
-        h->launches++;
+        transpose_T<T>(h, Tm, st);
         if (h->zero_csr) {
             launch_spmm<T>(h->zrow, (const T*)h->Tt, k, k, (T*)h->Cpart, k, st);
             h->launches++;
@@ -1694,15 +1776,22 @@ static int objective_contraction_impl(rri_handle_t h, const T* W, const T* Tm, b
         h->c2_valid = false;                            // (the caller's T may change before the next call)
     }
     const int parts = h->math == RRI_MATH_TF32 ? 1 : h->splits_w;      // (1 on zero-filled sparse handles)
-    launch_dot_parts<T>((const T*)h->Cpart, parts, n * k, W, n * k, h->obj_part, acc + 1, h->sm_count, st);
+    // model z: its column block of X T' against its own W
+    for (int z = 0; z < models; ++z)
+        launch_dot_parts<T>((const T*)h->Cpart + (int64_t)z * km, parts, n * k, W + (int64_t)z * n * km, n * km, h->obj_part,
+                            cross + z, h->sm_count, st, k, km);
     T* G = (T*)h->Gobj;
     T* H = G + (size_t)k * k;
-    launch_gram<T>(W, n, k, (T*)h->gram_part, h->gchunks_w, G, st);                 // IEEE Gram products
-    launch_gram<T>((const T*)h->Tt, d, k, (T*)h->gram_part, h->gchunks_t, H, st);
-    launch_objective_identity<T>(G, H, k, acc, h->obj_out, st);
-    launch_norms<T>(W, n * k, h->obj_part, h->obj_out + 2, st);
-    launch_norms<T>(Tm, (int64_t)k * d, h->obj_part, h->obj_out + 4, st);
-    h->launches += 11;
+    launch_gram<T>(W, n, km, (T*)h->gram_part, h->gchunks_w, G, st, models, n * km);                 // IEEE Gram products
+    launch_gram<T>((const T*)h->Tt, d, km, (T*)h->gram_part, h->gchunks_t, H, st, models, d * km);
+    for (int z = 0; z < models; ++z) {
+        double* out = h->obj_out + 8 * z;
+        const size_t g = (size_t)z * km * km;
+        launch_objective_identity<T>(G + g, H + g, km, xsq, cross + z, out, st);
+        launch_norms<T>(W + (int64_t)z * n * km, n * km, h->obj_part, out + 2, st);
+        launch_norms<T>(Tm + (int64_t)z * km * d, (int64_t)km * d, h->obj_part, out + 4, st);
+    }
+    h->launches += 4 + 7 * models;
     CKL();
     return 0;
 }
@@ -1722,9 +1811,7 @@ extern "C" int rri_objective_contraction(rri_handle_t h, const void* W_dev, cons
     int rc = h->dtype == RRI_F32 ? objective_contraction_impl<float>(h, (const float*)W_dev, (const float*)T_dev, reuse_last_sweep != 0, st)
                                  : objective_contraction_impl<double>(h, (const double*)W_dev, (const double*)T_dev, reuse_last_sweep != 0, st);
     if (rc) return rc;
-    CK(cudaMemcpyAsync(out_host, h->obj_out, sizeof(double) * 6, cudaMemcpyDeviceToHost, st));
-    CK(cudaStreamSynchronize(st));
-    return 0;
+    return copy_objective(h, out_host, st);
 }
 
 // p[c * pstride] = (X' w_t)[c], g[j] = (W' w_t)[j]
@@ -1798,6 +1885,7 @@ extern "C" int rri_partials_T(rri_handle_t h, const void* W_dev, const void* T_d
     if (!h) return fail("null handle");
     if (!h->X) return fail("rri_bind has not been called");
     if (t < 0 || t >= h->k) return fail("bad topic %d", t);
+    if (h->models > 1) return fail("rri_partials_T does not serve a handle of several models");
     CK(cudaSetDevice(h->device));
     cudaStream_t st = (cudaStream_t)stream;
     return h->dtype == RRI_F32
@@ -1911,15 +1999,12 @@ extern "C" int rri_gemm_nt(rri_handle_t h, const void* A_dev, int64_t lda, const
 template <typename T>
 static int profile_impl(rri_handle_t h, int which, const T* W, const T* Tm, int iters, float* avg_ms, cudaStream_t st)
 {
-    const int64_t n = h->n, d = h->d;
+    const int64_t d = h->d;
     const int k = h->k;
     cudaEvent_t e0, e1;
     CK(cudaEventCreate(&e0));
     CK(cudaEventCreate(&e1));
-    if (which == 2 && h->mk == MK_NONE && h->order == RRI_ORDER_HALS) {
-        launch_transpose<T>(W, n, k, k, (T*)h->Wt, h->ldwt, st);
-        h->launches++;
-    }
+    if (which == 2 && h->mk == MK_NONE && h->order == RRI_ORDER_HALS) transpose_W<T>(h, W, st);
     if (which == 1 && h->zero_csr) {              // the W-half contraction gathers rows of T'
         launch_transpose<T>(Tm, k, d, d, (T*)h->Tt, k, st);
         h->launches++;
@@ -1932,9 +2017,8 @@ static int profile_impl(rri_handle_t h, int which, const T* W, const T* Tm, int 
     int64_t ldtk = d;
     if (halves) {
         if (h->mk != MK_NONE || h->order != RRI_ORDER_HALS) return fail("which=3/4 need an unmasked hals-order handle");
-        launch_transpose<T>(Tm, k, d, d, (T*)h->Tt, k, st);
-        launch_transpose<T>(W, n, k, k, (T*)h->Wt, h->ldwt, st);
-        h->launches += 2;
+        transpose_T<T>(h, Tm, st);
+        transpose_W<T>(h, W, st);
         if (h->world > 1 && h->p2p) {
             Tk = (T*)((char*)h->xbuf + h->x_off_tk); ldtk = h->ldtk;
             CK(cudaMemcpy2DAsync(Tk, (size_t)ldtk * sizeof(T), Tm, (size_t)d * sizeof(T), (size_t)d * sizeof(T), (size_t)k,

@@ -156,18 +156,27 @@ update_rows_kernel(T* __restrict__ F, int64_t m, int k, const T* __restrict__ Cp
                    int64_t part_stride, const T* const* __restrict__ srcs, const T* __restrict__ S,
                    T reg_l1, T reg_l2, T eps, T ub, int has_ub,
                    T* __restrict__ Ft, int64_t ldft, T* __restrict__ colsum_part, int* __restrict__ flags,
-                   double* __restrict__ sums, int sums_off, int zero_flag, unsigned* __restrict__ counter)
+                   double* __restrict__ sums, int sums_off, int zero_flag, unsigned* __restrict__ counter,
+                   int64_t ldc, int64_t lds, int64_t s_stride)
 {
     extern __shared__ __align__(16) unsigned char smem_raw[];
     T* ftile = reinterpret_cast<T*>(smem_raw);                 // [k][U_GROUP+1]
     T* csm = ftile + (size_t)k * (U_GROUP + 1);                // [U_NW][k]
     T* Ss = csm + (size_t)U_NW * k;                            // [k][k] when S_SMEM
     const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
+    const int z = blockIdx.y;                                  // model (RowBatch)
+    F += (int64_t)z * m * k;
+    S += (int64_t)z * s_stride;
+    if (Ft) Ft += (int64_t)z * k * ldft;
+    flags += z;
+    colsum_part += (int64_t)z * gridDim.x * k;
+    const int64_t coff = (int64_t)z * k;
     if (S_SMEM) {
-        for (int e = tid; e < k * k; e += U_THREADS) Ss[e] = S[e];
+        for (int e = tid; e < k * k; e += U_THREADS) Ss[e] = S[(e / k) * lds + e % k];
         __syncthreads();
     }
     const T* Sp = S_SMEM ? Ss : S;
+    const int64_t sld = S_SMEM ? k : lds;
 
     T csum[KL];
 #pragma unroll
@@ -191,7 +200,7 @@ update_rows_kernel(T* __restrict__ F, int64_t m, int k, const T* __restrict__ Cp
                         f[l] = F[i * k + tp];
                         T c = T(0);
                         for (int p = 0; p < parts; ++p)
-                            c += (srcs ? srcs[p] : Cpart + (int64_t)p * part_stride)[i * k + tp];
+                            c += (srcs ? srcs[p] : Cpart + (int64_t)p * part_stride)[coff + i * ldc + tp];
                         r[l] = c;
                     }
                 }
@@ -205,7 +214,7 @@ update_rows_kernel(T* __restrict__ F, int64_t m, int k, const T* __restrict__ Cp
 #pragma unroll
                         for (int l = 0; l < KL; ++l) {
                             const int tp = lane + 32 * l;
-                            if (tp < k && tp != j) r[l] = fma(-fj, Sp[j * k + tp], r[l]);
+                            if (tp < k && tp != j) r[l] = fma(-fj, Sp[j * sld + tp], r[l]);
                         }
                     }
                 }
@@ -217,7 +226,7 @@ update_rows_kernel(T* __restrict__ F, int64_t m, int k, const T* __restrict__ Cp
                         if (t >= k) break;
                         T delta = T(0);
                         if (lane == tt) {
-                            const T x = solve_scalar_c<T>(r[l0] - reg_l1, Sp[t * k + t] + reg_l2, eps, ub,
+                            const T x = solve_scalar_c<T>(r[l0] - reg_l1, Sp[t * sld + t] + reg_l2, eps, ub,
                                                           has_ub != 0, unb);
                             delta = x - f[l0];
                             f[l0] = x;
@@ -226,7 +235,7 @@ update_rows_kernel(T* __restrict__ F, int64_t m, int k, const T* __restrict__ Cp
 #pragma unroll
                         for (int l = 0; l < KL; ++l) {
                             const int tp = lane + 32 * l;
-                            if (tp < k && tp != t) r[l] = fma(-delta, Sp[t * k + tp], r[l]);
+                            if (tp < k && tp != t) r[l] = fma(-delta, Sp[t * sld + tp], r[l]);
                         }
                     }
                 }
@@ -269,22 +278,25 @@ update_rows_kernel(T* __restrict__ F, int64_t m, int k, const T* __restrict__ Cp
 template <typename T, int KL>
 static void launch_update_rows_kl(T* F, int64_t m, int k, const T* Cpart, int parts, int64_t part_stride,
                                   const T* const* srcs, const T* S, const SolveArgs& a, T* Ft, int64_t ldft, T* colsum_part,
-                                  int* flags, int blocks, const ColsumOut& co, cudaStream_t st)
+                                  int* flags, int blocks, const ColsumOut& co, const RowBatch& rb, cudaStream_t st)
 {
+    const dim3 grid((unsigned)blocks, (unsigned)rb.models);
     size_t base = sizeof(T) * ((size_t)k * (U_GROUP + 1) + (size_t)U_NW * k);
     size_t with_s = base + sizeof(T) * (size_t)k * k;
     if (with_s <= 200 * 1024) {
         auto kern = update_rows_kernel<T, KL, true>;
         if (with_s > 48 * 1024) cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)with_s);
-        kern<<<blocks, U_THREADS, with_s, st>>>(F, m, k, Cpart, parts, part_stride, srcs, S, (T)a.reg_l1,
-                                                 (T)a.reg_l2, (T)a.eps, (T)a.ub, a.has_ub, Ft, ldft,
-                                                 colsum_part, flags, co.sums, co.off, co.zero_flag, co.counter);
+        kern<<<grid, U_THREADS, with_s, st>>>(F, m, k, Cpart, parts, part_stride, srcs, S, (T)a.reg_l1,
+                                               (T)a.reg_l2, (T)a.eps, (T)a.ub, a.has_ub, Ft, ldft,
+                                               colsum_part, flags, co.sums, co.off, co.zero_flag, co.counter,
+                                               rb.ldc, rb.lds, rb.s_stride);
     } else {
         auto kern = update_rows_kernel<T, KL, false>;
         if (base > 48 * 1024) cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)base);
-        kern<<<blocks, U_THREADS, base, st>>>(F, m, k, Cpart, parts, part_stride, srcs, S, (T)a.reg_l1,
-                                               (T)a.reg_l2, (T)a.eps, (T)a.ub, a.has_ub, Ft, ldft,
-                                               colsum_part, flags, co.sums, co.off, co.zero_flag, co.counter);
+        kern<<<grid, U_THREADS, base, st>>>(F, m, k, Cpart, parts, part_stride, srcs, S, (T)a.reg_l1,
+                                             (T)a.reg_l2, (T)a.eps, (T)a.ub, a.has_ub, Ft, ldft,
+                                             colsum_part, flags, co.sums, co.off, co.zero_flag, co.counter,
+                                             rb.ldc, rb.lds, rb.s_stride);
     }
 }
 
@@ -345,7 +357,8 @@ update_rows_tpr_kernel(T* __restrict__ F, int64_t m, int k, const T* __restrict_
                        int64_t part_stride, const T* const* __restrict__ srcs, const T* __restrict__ S,
                        T reg_l1, T reg_l2, T eps, T ub, int has_ub,
                        T* __restrict__ Ft, int64_t ldft, T* __restrict__ colsum_part, int* __restrict__ flags,
-                       double* __restrict__ sums, int sums_off, int zero_flag, unsigned* __restrict__ counter)
+                       double* __restrict__ sums, int sums_off, int zero_flag, unsigned* __restrict__ counter,
+                       int64_t ldc, int64_t lds, int64_t s_stride)
 {
     constexpr int LD = KM + 1;                              // padded row stride of the tiles
     extern __shared__ __align__(16) unsigned char smem_raw[];
@@ -353,9 +366,16 @@ update_rows_tpr_kernel(T* __restrict__ F, int64_t m, int k, const T* __restrict_
     T* ctile = Ss + KM * KM;                                // [TPR_ROWS][LD]  contraction rows
     T* ftile = ctile + TPR_ROWS * LD;                       // [TPR_ROWS][LD]  factor rows
     const int tid = threadIdx.x;
+    const int z = blockIdx.y;                               // model (RowBatch)
+    F += (int64_t)z * m * k;
+    S += (int64_t)z * s_stride;
+    if (Ft) Ft += (int64_t)z * k * ldft;
+    flags += z;
+    colsum_part += (int64_t)z * gridDim.x * k;
+    const int64_t coff = (int64_t)z * k;
     for (int e = tid; e < KM * KM; e += TPR_ROWS) {
         const int a = e / KM, b = e % KM;
-        Ss[e] = (a < k && b < k) ? S[a * k + b] : T(0);
+        Ss[e] = (a < k && b < k) ? S[a * lds + b] : T(0);
     }
     T csum = T(0);          // thread j < k accumulates the sum of column j over this block's rows
     bool unb = false;
@@ -371,25 +391,35 @@ update_rows_tpr_kernel(T* __restrict__ F, int64_t m, int k, const T* __restrict_
             int rr = tid / k, cc = tid - rr * k;
             const int dr = TPR_ROWS / k, dc = TPR_ROWS - dr * k;
             const T* Frow = F + i0 * k;
-            const T* Crow = (srcs ? srcs[0] : Cpart) + i0 * k;
+            const T* Crow = (srcs ? srcs[0] : Cpart) + coff + i0 * ldc;
             constexpr int UB = 8;
             for (int e0 = tid; e0 < tot; e0 += UB * TPR_ROWS) {
                 T cv[UB], fv[UB];
+                int co[UB];                                 // offset of element e in the contraction rows (row stride ldc)
+                {
+                    int r2 = rr, c2 = cc;
+#pragma unroll
+                    for (int u = 0; u < UB; ++u) {
+                        co[u] = r2 * (int)ldc + c2;
+                        r2 += dr; c2 += dc;
+                        if (c2 >= k) { c2 -= k; ++r2; }
+                    }
+                }
 #pragma unroll
                 for (int u = 0; u < UB; ++u) {
                     const int e = e0 + u * TPR_ROWS;
                     cv[u] = T(0); fv[u] = T(0);
                     if (e < tot) {
-                        cv[u] = Crow[e];
+                        cv[u] = Crow[co[u]];
                         fv[u] = Frow[e];
                     }
                 }
                 for (int p = 1; p < parts; ++p) {
-                    const T* Cp = srcs ? srcs[p] + i0 * k : Crow + (int64_t)p * part_stride;
+                    const T* Cp = srcs ? srcs[p] + coff + i0 * ldc : Crow + (int64_t)p * part_stride;
 #pragma unroll
                     for (int u = 0; u < UB; ++u) {
                         const int e = e0 + u * TPR_ROWS;
-                        if (e < tot) cv[u] += Cp[e];
+                        if (e < tot) cv[u] += Cp[co[u]];
                     }
                 }
 #pragma unroll
@@ -439,14 +469,14 @@ update_rows_tpr_kernel(T* __restrict__ F, int64_t m, int k, const T* __restrict_
 template <typename T, int KM>
 static void launch_update_rows_tpr(T* F, int64_t m, int k, const T* Cpart, int parts, int64_t part_stride,
                                    const T* const* srcs, const T* S, const SolveArgs& a, T* Ft, int64_t ldft, T* colsum_part,
-                                   int* flags, int blocks, const ColsumOut& co, cudaStream_t st)
+                                   int* flags, int blocks, const ColsumOut& co, const RowBatch& rb, cudaStream_t st)
 {
     const size_t smem = sizeof(T) * ((size_t)KM * KM + 2 * (size_t)TPR_ROWS * (KM + 1));
     auto kern = update_rows_tpr_kernel<T, KM>;
     if (smem > 48 * 1024) cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-    kern<<<blocks, TPR_ROWS, smem, st>>>(F, m, k, Cpart, parts, part_stride, srcs, S, (T)a.reg_l1, (T)a.reg_l2,
-                                        (T)a.eps, (T)a.ub, a.has_ub, Ft, ldft, colsum_part, flags, co.sums, co.off,
-                                        co.zero_flag, co.counter);
+    kern<<<dim3((unsigned)blocks, (unsigned)rb.models), TPR_ROWS, smem, st>>>(
+        F, m, k, Cpart, parts, part_stride, srcs, S, (T)a.reg_l1, (T)a.reg_l2, (T)a.eps, (T)a.ub, a.has_ub, Ft, ldft,
+        colsum_part, flags, co.sums, co.off, co.zero_flag, co.counter, rb.ldc, rb.lds, rb.s_stride);
 }
 
 // ------------------------------------------------------------------------------------------------
@@ -463,16 +493,22 @@ template <typename T, int KM>
 __global__ void __launch_bounds__(128)
 update_rows_reg_kernel(T* __restrict__ F, int64_t m, int k, const T* __restrict__ C, const T* __restrict__ S,
                        T reg_l1, T reg_l2, T eps, T ub, int has_ub, T* __restrict__ Ft, int64_t ldft,
-                       int* __restrict__ flags)
+                       int* __restrict__ flags, int64_t ldc, int64_t lds, int64_t s_stride)
 {
     using V = typename Vec<T>::type;
     constexpr int VN = Vec<T>::N;
     extern __shared__ __align__(16) unsigned char smem_raw[];
     T* Ss = reinterpret_cast<T*>(smem_raw);                  // [KM][KM], zero padded
     const int tid = threadIdx.x;
+    const int z = blockIdx.y;                                // model (RowBatch)
+    F += (int64_t)z * m * k;
+    C += (int64_t)z * k;
+    S += (int64_t)z * s_stride;
+    if (Ft) Ft += (int64_t)z * k * ldft;
+    flags += z;
     for (int e = tid; e < KM * KM; e += 128) {
         const int a = e / KM, b = e % KM;
-        Ss[e] = (a < k && b < k) ? S[a * k + b] : T(0);
+        Ss[e] = (a < k && b < k) ? S[a * lds + b] : T(0);
     }
     __syncthreads();
     bool unb = false;
@@ -491,7 +527,7 @@ update_rows_reg_kernel(T* __restrict__ F, int64_t m, int k, const T* __restrict_
         // the contraction entries of 8 steps come as 16-byte loads, requested one group of steps ahead (a scalar load
         // per step leaves its line in L1 for the next 31 steps of the same thread -- with 16 warps per SM walking 32
         // rows each the lines do not survive, and every step waits for L2)
-        const V* crowv = reinterpret_cast<const V*>(C + row * k);
+        const V* crowv = reinterpret_cast<const V*>(C + row * ldc);
         constexpr int GV = 8 / VN;                                                  // vectors per group of 8 steps
         T cn[8];
 #pragma unroll
@@ -580,15 +616,21 @@ template <int KM>
 __global__ void __launch_bounds__(128)
 update_rows_reg_x2_kernel(float* __restrict__ F, int64_t m, int k, const float* __restrict__ C, const float* __restrict__ S,
                           float reg_l1, float reg_l2, float eps, float ub, int has_ub, float* __restrict__ Ft, int64_t ldft,
-                          int* __restrict__ flags)
+                          int* __restrict__ flags, int64_t ldc, int64_t lds, int64_t s_stride)
 {
     using U64 = unsigned long long;
     extern __shared__ __align__(16) unsigned char smem_raw[];
     float* Ss = reinterpret_cast<float*>(smem_raw);           // [KM][KM], zero padded
     const int tid = threadIdx.x;
+    const int z = blockIdx.y;                                 // model (RowBatch)
+    F += (int64_t)z * m * k;
+    C += (int64_t)z * k;
+    S += (int64_t)z * s_stride;
+    if (Ft) Ft += (int64_t)z * k * ldft;
+    flags += z;
     for (int e = tid; e < KM * KM; e += 128) {
         const int a = e / KM, b = e % KM;
-        Ss[e] = (a < k && b < k) ? S[a * k + b] : 0.f;
+        Ss[e] = (a < k && b < k) ? S[a * lds + b] : 0.f;
     }
     __syncthreads();
     bool unb = false;
@@ -601,7 +643,7 @@ update_rows_reg_x2_kernel(float* __restrict__ F, int64_t m, int k, const float* 
             if (4 * jv < k) v = frowv[jv];
             fp[2 * jv] = v.x; fp[2 * jv + 1] = v.y;
         }
-        const float4* crowv = reinterpret_cast<const float4*>(C + row * k);
+        const float4* crowv = reinterpret_cast<const float4*>(C + row * ldc);
         float cn[8];
 #pragma unroll
         for (int v = 0; v < 2; ++v) {
@@ -666,23 +708,25 @@ update_rows_reg_x2_kernel(float* __restrict__ F, int64_t m, int k, const float* 
 
 template <typename T, int KM>
 static void launch_update_rows_reg(T* F, int64_t m, int k, const T* C, const T* S, const SolveArgs& a, T* Ft, int64_t ldft,
-                                   int* flags, const ColsumOut& co, cudaStream_t st)
+                                   int* flags, const ColsumOut& co, const RowBatch& rb, cudaStream_t st)
 {
     const size_t smem = sizeof(T) * KM * KM;
-    const int64_t nb = (m + 127) / 128;
+    const dim3 nb((unsigned)((m + 127) / 128), (unsigned)rb.models);
     if constexpr (sizeof(T) == 4) {
         static const bool x2 = [] { const char* e = getenv("RRI_UPDATE_X2"); return !(e && *e == '0'); }();
         if (x2) {
             auto kx = update_rows_reg_x2_kernel<KM>;
             if (smem > 48 * 1024) cudaFuncSetAttribute(kx, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-            kx<<<(unsigned)nb, 128, smem, st>>>(F, m, k, C, S, (T)a.reg_l1, (T)a.reg_l2, (T)a.eps, (T)a.ub, a.has_ub, Ft, ldft, flags);
+            kx<<<nb, 128, smem, st>>>(F, m, k, C, S, (T)a.reg_l1, (T)a.reg_l2, (T)a.eps, (T)a.ub, a.has_ub, Ft, ldft, flags,
+                                      rb.ldc, rb.lds, rb.s_stride);
             if (co.sums) launch_rowsum_flag<T>(Ft, k, m, ldft, co.sums, co.off, co.zero_flag, flags, st);
             return;
         }
     }
     auto kern = update_rows_reg_kernel<T, KM>;
     if (smem > 48 * 1024) cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-    kern<<<(unsigned)nb, 128, smem, st>>>(F, m, k, C, S, (T)a.reg_l1, (T)a.reg_l2, (T)a.eps, (T)a.ub, a.has_ub, Ft, ldft, flags);
+    kern<<<nb, 128, smem, st>>>(F, m, k, C, S, (T)a.reg_l1, (T)a.reg_l2, (T)a.eps, (T)a.ub, a.has_ub, Ft, ldft, flags,
+                                rb.ldc, rb.lds, rb.s_stride);
     if (co.sums) launch_rowsum_flag<T>(Ft, k, m, ldft, co.sums, co.off, co.zero_flag, flags, st);
 }
 
@@ -947,32 +991,33 @@ int launch_peer_update_rows(const PeerExchange& px, int64_t d, int k, const Solv
 template <typename T>
 void launch_update_rows(T* F, int64_t m, int k, const T* Cpart, int parts, int64_t part_stride,
                         const T* const* srcs, const T* S, const SolveArgs& a, T* Ft, int64_t ldft,
-                        T* colsum_part, int* flags, int blocks, const ColsumOut& co, cudaStream_t st)
+                        T* colsum_part, int* flags, int blocks, const ColsumOut& co, const RowBatch& rb,
+                        cudaStream_t st)
 {
     // thread-per-row variants while the row fits in registers / the tiles in shared memory
     // (fp32: k <= 128, fp64: k <= 64); wider ranks use the warp-per-row kernel
     {
         static const bool reg_off = [] { const char* e = getenv("RRI_UPDATE_REG"); return e && *e == '0'; }();
         constexpr int VN = Vec<T>::N;
-        if (!reg_off && parts == 1 && !srcs && Ft && (k % VN) == 0 && k <= (sizeof(T) == 4 ? 128 : 64)) {
-            if (k <= 16) launch_update_rows_reg<T, 16>(F, m, k, Cpart, S, a, Ft, ldft, flags, co, st);
-            else if (k <= 32) launch_update_rows_reg<T, 32>(F, m, k, Cpart, S, a, Ft, ldft, flags, co, st);
-            else if (k <= 64) launch_update_rows_reg<T, 64>(F, m, k, Cpart, S, a, Ft, ldft, flags, co, st);
-            else if constexpr (sizeof(T) == 4) launch_update_rows_reg<T, 128>(F, m, k, Cpart, S, a, Ft, ldft, flags, co, st);
+        if (!reg_off && parts == 1 && !srcs && Ft && (k % VN) == 0 && (rb.ldc % VN) == 0 && k <= (sizeof(T) == 4 ? 128 : 64)) {
+            if (k <= 16) launch_update_rows_reg<T, 16>(F, m, k, Cpart, S, a, Ft, ldft, flags, co, rb, st);
+            else if (k <= 32) launch_update_rows_reg<T, 32>(F, m, k, Cpart, S, a, Ft, ldft, flags, co, rb, st);
+            else if (k <= 64) launch_update_rows_reg<T, 64>(F, m, k, Cpart, S, a, Ft, ldft, flags, co, rb, st);
+            else if constexpr (sizeof(T) == 4) launch_update_rows_reg<T, 128>(F, m, k, Cpart, S, a, Ft, ldft, flags, co, rb, st);
             return;
         }
     }
-#define RRI_TPR(KM) launch_update_rows_tpr<T, KM>(F, m, k, Cpart, parts, part_stride, srcs, S, a, Ft, ldft, colsum_part, flags, blocks, co, st)
+#define RRI_TPR(KM) launch_update_rows_tpr<T, KM>(F, m, k, Cpart, parts, part_stride, srcs, S, a, Ft, ldft, colsum_part, flags, blocks, co, rb, st)
     if (k <= 16) { RRI_TPR(16); return; }
     if (k <= 32) { RRI_TPR(32); return; }
     if (k <= 64) { RRI_TPR(64); return; }
     if (k <= 128 && sizeof(T) == 4) { RRI_TPR(128); return; }
 #undef RRI_TPR
     const int kl = (k + 31) / 32;
-    if (kl <= 1) launch_update_rows_kl<T, 1>(F, m, k, Cpart, parts, part_stride, srcs, S, a, Ft, ldft, colsum_part, flags, blocks, co, st);
-    else if (kl <= 2) launch_update_rows_kl<T, 2>(F, m, k, Cpart, parts, part_stride, srcs, S, a, Ft, ldft, colsum_part, flags, blocks, co, st);
-    else if (kl <= 4) launch_update_rows_kl<T, 4>(F, m, k, Cpart, parts, part_stride, srcs, S, a, Ft, ldft, colsum_part, flags, blocks, co, st);
-    else launch_update_rows_kl<T, 8>(F, m, k, Cpart, parts, part_stride, srcs, S, a, Ft, ldft, colsum_part, flags, blocks, co, st);
+    if (kl <= 1) launch_update_rows_kl<T, 1>(F, m, k, Cpart, parts, part_stride, srcs, S, a, Ft, ldft, colsum_part, flags, blocks, co, rb, st);
+    else if (kl <= 2) launch_update_rows_kl<T, 2>(F, m, k, Cpart, parts, part_stride, srcs, S, a, Ft, ldft, colsum_part, flags, blocks, co, rb, st);
+    else if (kl <= 4) launch_update_rows_kl<T, 4>(F, m, k, Cpart, parts, part_stride, srcs, S, a, Ft, ldft, colsum_part, flags, blocks, co, rb, st);
+    else launch_update_rows_kl<T, 8>(F, m, k, Cpart, parts, part_stride, srcs, S, a, Ft, ldft, colsum_part, flags, blocks, co, rb, st);
 }
 
 // ------------------------------------------------------------------------------------------------
@@ -991,8 +1036,9 @@ int gram_chunks(int64_t m, int k, int sm_count)
 
 template <typename T>
 __global__ void __launch_bounds__(256)
-gram_kernel(const T* __restrict__ F, int64_t m, int k, T* __restrict__ part)
+gram_kernel(const T* __restrict__ F, int64_t m, int k, T* __restrict__ part, int64_t f_stride)
 {
+    F += (int64_t)blockIdx.z * f_stride;                   // model z (launch_gram with models > 1)
     __shared__ T Fa[GR_ROWS][64 + 1];
     __shared__ T Fb[GR_ROWS][64 + 1];
     const int kb = (k + 63) / 64;
@@ -1038,7 +1084,7 @@ gram_kernel(const T* __restrict__ F, int64_t m, int k, T* __restrict__ part)
         }
         __syncthreads();
     }
-    T* P = part + (int64_t)blockIdx.x * k * k;
+    T* P = part + ((int64_t)blockIdx.x * gridDim.z + blockIdx.z) * k * k;      // [chunks][models][k*k]
 #pragma unroll
     for (int i = 0; i < 4; ++i)
 #pragma unroll
@@ -1102,12 +1148,14 @@ void launch_sum_sources(const T* const* srcs, int parts, int64_t len, T* out, cu
 }
 
 template <typename T>
-void launch_gram(const T* F, int64_t m, int k, T* part, int chunks, T* G, cudaStream_t st)
+void launch_gram(const T* F, int64_t m, int k, T* part, int chunks, T* G, cudaStream_t st, int models, int64_t f_stride)
 {
     const int kb = (k + 63) / 64;
-    dim3 grid(chunks, kb * kb);
-    gram_kernel<T><<<grid, 256, 0, st>>>(F, m, k, part);
-    launch_reduce_parts<T>(part, chunks, (int64_t)k * k, (int64_t)k * k, G, st);
+    dim3 grid(chunks, kb * kb, models);
+    gram_kernel<T><<<grid, 256, 0, st>>>(F, m, k, part, f_stride);
+    // (models * k * k <= 256 * 256: the reduction kernel, and with it the order of the sums, is the one model's)
+    const int64_t len = (int64_t)models * k * k;
+    launch_reduce_parts<T>(part, chunks, len, len, G, st);
 }
 
 template <typename T>
@@ -1181,11 +1229,11 @@ void launch_transpose(const T* A, int64_t rows, int64_t cols, int64_t lda, T* B,
                                          int, cudaStream_t);                                              \
     template void launch_update_rows<T>(T*, int64_t, int, const T*, int, int64_t, const T* const*,        \
                                         const T*, const SolveArgs&, T*, int64_t, T*, int*, int,            \
-                                        const ColsumOut&, cudaStream_t);                                   \
+                                        const ColsumOut&, const RowBatch&, cudaStream_t);                  \
     template int launch_peer_update_rows<T>(const PeerExchange&, int64_t, int, const SolveArgs&, T*, T*,    \
                                             int*, double*, unsigned*, int, cudaStream_t);                  \
     template void launch_sum_sources<T>(const T* const*, int, int64_t, T*, cudaStream_t);                  \
-    template void launch_gram<T>(const T*, int64_t, int, T*, int, T*, cudaStream_t);                      \
+    template void launch_gram<T>(const T*, int64_t, int, T*, int, T*, cudaStream_t, int, int64_t);        \
     template void launch_reduce_parts<T>(const T*, int, int64_t, int64_t, T*, cudaStream_t);              \
     template void launch_colsum_finalize<T>(const T*, int, int, double*, int, int, int*, cudaStream_t);   \
     template void launch_transpose<T>(const T*, int64_t, int64_t, int64_t, T*, int64_t, cudaStream_t);

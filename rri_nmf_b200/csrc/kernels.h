@@ -78,11 +78,20 @@ struct ColsumOut {
     int off, zero_flag;
     unsigned* counter;
 };
+// Models of rank k updated side by side in one launch (blockIdx.y = model z < models): F + z*m*k, Ft + z*k*ldft,
+// flags + z and colsum_part + z*blocks*k are model z's own; its contraction is the column block z*k of C (row stride
+// ldc) and its Gram matrix the block S + z*s_stride (row stride lds).  One model: {1, k, k, 0}.
+struct RowBatch {
+    int models;
+    int64_t ldc, lds, s_stride;
+};
 // srcs (optional, device array of `parts` pointers): slice p is srcs[p] instead of Cpart + p*part_stride.
+// With rb.models > 1, co.sums must be null (the column sums are taken from Ft afterwards).
 template <typename T>
 void launch_update_rows(T* F, int64_t m, int k, const T* Cpart, int parts, int64_t part_stride,
                         const T* const* srcs, const T* S, const SolveArgs& a, T* Ft, int64_t ldft,
-                        T* colsum_part, int* flags, int blocks, const ColsumOut& co, cudaStream_t st);
+                        T* colsum_part, int* flags, int blocks, const ColsumOut& co, const RowBatch& rb,
+                        cudaStream_t st);
 
 // Multi-GPU T half-step fused with its exchange over NVLink peer memory (hals_kernels.cu: peer_update_rows_kernel).
 // Pointers of rank r's exchange buffer as mapped in THIS process; flag arrays hold one 128-byte slot per rank.
@@ -110,10 +119,13 @@ int launch_peer_update_rows(const PeerExchange& px, int64_t d, int k, const Solv
 template <typename T>
 void launch_sum_sources(const T* const* srcs, int parts, int64_t len, T* out, cudaStream_t st);
 
-// Gram matrix G[k,k] = F'F of a row-major F[m,k]: per-chunk partials + fixed-order finalize.
+// Gram matrix G[k,k] = F'F of a row-major F[m,k]: per-chunk partials + fixed-order finalize.  models > 1: the Gram
+// matrices G[z] (G + z*k*k) of F_z = F + z*f_stride for z < models in the same two launches, each summed exactly as
+// a single one (part: chunks * models * k * k elements).
 int gram_chunks(int64_t m, int k, int sm_count);
 template <typename T>
-void launch_gram(const T* F, int64_t m, int k, T* part, int chunks, T* G, cudaStream_t st);
+void launch_gram(const T* F, int64_t m, int k, T* part, int chunks, T* G, cudaStream_t st, int models = 1,
+                 int64_t f_stride = 0);
 
 // out[c] = sum_b part[b][c]  (c < len) -- generic fixed-order reduction of per-block partials
 template <typename T>
@@ -178,10 +190,11 @@ void launch_wrri_final(const T* numer_part, const T* denom_part, int parts, int6
 template <typename T>
 void launch_vec_sum_flag(const T* v, int64_t len, int64_t stride, double* sums, int slot, int zero_flag,
                          int* flags, cudaStream_t st);
-// sums[slot0 + r] = sum of row r of A[rows, ld] over len elements; zero / non-finite flags (one launch per sweep)
+// sums[slot0 + r] = sum of row r of A[rows, ld] over len elements; zero / non-finite flags (one launch per sweep).
+// flag_rows > 0: row r raises its flags in word flags[r / flag_rows] (one word per model of flag_rows topics)
 template <typename T>
 void launch_rowsum_flag(const T* A, int rows, int64_t len, int64_t ld, double* sums, int slot0, int zero_flag,
-                        int* flags, cudaStream_t st);
+                        int* flags, cudaStream_t st, int flag_rows = 0);
 // v[i*stride] *= scale / sums[slot]   (vector-c branch with a sum constraint, optimization.py:85-87)
 template <typename T>
 void launch_vec_scale_to_sum(T* v, int64_t len, int64_t stride, const double* sums, int slot, double s,
@@ -198,13 +211,15 @@ void launch_objective(const T* X, int64_t ldx, const void* M, int mk, int64_t ld
 template <typename T>
 void launch_sumsq_rows(const T* A, int64_t rows, int64_t cols, int64_t lda, double* part, double* out, int sm_count,
                        cudaStream_t st);
-//   out[0] = sum_e (sum_p C[p*stride + e]) * W[e]
+//   out[0] = sum_e (sum_p C[p*stride + c(e)]) * W[e] with c(e) = e, or, when ldc > width, the entry (e / width, e % width)
+//   of a column block of C [., ldc] (one model's block of a stacked contraction)
 template <typename T>
 void launch_dot_parts(const T* C, int parts, int64_t stride, const T* W, int64_t len, double* part, double* out,
-                      int sm_count, cudaStream_t st);
-//   out[0] = 0.5 * (acc[0] - 2 acc[1] + sum G o H), out[1] = acc[0]
+                      int sm_count, cudaStream_t st, int64_t ldc = 0, int width = 0);
+//   out[0] = 0.5 * (xsq[0] - 2 cross[0] + sum G o H), out[1] = xsq[0]
 template <typename T>
-void launch_objective_identity(const T* G, const T* H, int k, const double* acc, double* out, cudaStream_t st);
+void launch_objective_identity(const T* G, const T* H, int k, const double* xsq, const double* cross, double* out,
+                               cudaStream_t st);
 // out[0] = sum v^2, out[1] = sum |v| over len contiguous elements (regulariser terms, nmf.py:72-75)
 template <typename T>
 void launch_norms(const T* v, int64_t len, double* part, double* out, cudaStream_t st);

@@ -284,7 +284,7 @@ void launch_vec_sum_flag(const T* v, int64_t len, int64_t stride, double* sums, 
 template <typename T>
 __global__ void __launch_bounds__(1024)
 rowsum_flag_kernel(const T* __restrict__ A, int64_t len, int64_t ld, double* __restrict__ sums, int slot0,
-                   int zero_flag, int* __restrict__ flags)
+                   int zero_flag, int* __restrict__ flags, int flag_rows)
 {
     __shared__ double red[32];
     const T* __restrict__ v = A + (int64_t)blockIdx.x * ld;
@@ -297,16 +297,17 @@ rowsum_flag_kernel(const T* __restrict__ A, int64_t len, int64_t ld, double* __r
         double tot = 0.0;
         for (int w = 0; w < (int)(blockDim.x >> 5); ++w) tot += red[w];
         sums[slot0 + blockIdx.x] = tot;
-        if (zero_flag && !(tot > 1e-10)) atomicOr(flags, zero_flag);
-        if (!isfinite(tot)) atomicOr(flags, 8);
+        int* f = flag_rows > 0 ? flags + blockIdx.x / flag_rows : flags;
+        if (zero_flag && !(tot > 1e-10)) atomicOr(f, zero_flag);
+        if (!isfinite(tot)) atomicOr(f, 8);
     }
 }
 
 template <typename T>
 void launch_rowsum_flag(const T* A, int rows, int64_t len, int64_t ld, double* sums, int slot0, int zero_flag,
-                        int* flags, cudaStream_t st)
+                        int* flags, cudaStream_t st, int flag_rows)
 {
-    if (rows > 0) rowsum_flag_kernel<T><<<rows, 1024, 0, st>>>(A, len, ld, sums, slot0, zero_flag, flags);
+    if (rows > 0) rowsum_flag_kernel<T><<<rows, 1024, 0, st>>>(A, len, ld, sums, slot0, zero_flag, flags, flag_rows);
 }
 
 template <typename T>
@@ -474,17 +475,19 @@ sumsq_rows_kernel(const T* __restrict__ A, int64_t rows, int64_t cols, int64_t l
     }
 }
 
-// part[b] = partial of sum_e (sum_p C[p*stride + e]) * W[e]
+// part[b] = partial of sum_e (sum_p C[p*stride + c(e)]) * W[e]; c(e) = e, or (width > 0) the entry (e / width, e % width)
+// of C [., ldc]
 template <typename T>
 __global__ void __launch_bounds__(256)
 dot_parts_kernel(const T* __restrict__ C, int parts, int64_t stride, const T* __restrict__ W, int64_t len,
-                 double* __restrict__ part)
+                 double* __restrict__ part, int64_t ldc, int width)
 {
     __shared__ double red[8];
     double s = 0.0;
     for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < len; i += (int64_t)gridDim.x * blockDim.x) {
+        const int64_t ci = width > 0 ? (i / width) * ldc + i % width : i;
         double c = 0.0;
-        for (int p = 0; p < parts; ++p) c += (double)C[(int64_t)p * stride + i];
+        for (int p = 0; p < parts; ++p) c += (double)C[(int64_t)p * stride + ci];
         s += c * (double)W[i];
     }
     s = warp_sum(s);
@@ -526,20 +529,20 @@ void launch_sumsq_rows(const T* A, int64_t rows, int64_t cols, int64_t lda, doub
 
 template <typename T>
 void launch_dot_parts(const T* C, int parts, int64_t stride, const T* W, int64_t len, double* part, double* out,
-                      int sm_count, cudaStream_t st)
+                      int sm_count, cudaStream_t st, int64_t ldc, int width)
 {
     int64_t blocks = (len + 256 * 8 - 1) / (256 * 8);
     if (blocks > 8 * sm_count) blocks = 8 * sm_count;
     if (blocks < 1) blocks = 1;
-    dot_parts_kernel<T><<<(unsigned)blocks, 256, 0, st>>>(C, parts, stride, W, len, part);
+    dot_parts_kernel<T><<<(unsigned)blocks, 256, 0, st>>>(C, parts, stride, W, len, part, ldc, ldc > width ? width : 0);
     sum_partials_kernel<<<1, 256, 0, st>>>(part, (int)blocks, out);
 }
 
-// out[0] = 0.5 * (xsq - 2 cross + sum_ab G[a,b] H[a,b]),  out[1] = xsq      (acc = {xsq, cross})
+// out[0] = 0.5 * (xsq - 2 cross + sum_ab G[a,b] H[a,b]),  out[1] = xsq
 template <typename T>
 __global__ void __launch_bounds__(256)
-objective_identity_kernel(const T* __restrict__ G, const T* __restrict__ H, int kk, const double* __restrict__ acc,
-                          double* __restrict__ out)
+objective_identity_kernel(const T* __restrict__ G, const T* __restrict__ H, int kk, const double* __restrict__ xsq,
+                          const double* __restrict__ cross, double* __restrict__ out)
 {
     __shared__ double red[8];
     double s = 0.0;
@@ -550,21 +553,24 @@ objective_identity_kernel(const T* __restrict__ G, const T* __restrict__ H, int 
     if (threadIdx.x == 0) {
         double q = 0.0;
         for (int w = 0; w < 8; ++w) q += red[w];
-        out[0] = 0.5 * (acc[0] - 2.0 * acc[1] + q);
-        out[1] = acc[0];
+        out[0] = 0.5 * (xsq[0] - 2.0 * cross[0] + q);
+        out[1] = xsq[0];
     }
 }
 
 template <typename T>
-void launch_objective_identity(const T* G, const T* H, int k, const double* acc, double* out, cudaStream_t st)
+void launch_objective_identity(const T* G, const T* H, int k, const double* xsq, const double* cross, double* out,
+                               cudaStream_t st)
 {
-    objective_identity_kernel<T><<<1, 256, 0, st>>>(G, H, k * k, acc, out);
+    objective_identity_kernel<T><<<1, 256, 0, st>>>(G, H, k * k, xsq, cross, out);
 }
 
 #define RRI_INST(T)                                                                                         \
     template void launch_sumsq_rows<T>(const T*, int64_t, int64_t, int64_t, double*, double*, int, cudaStream_t); \
-    template void launch_dot_parts<T>(const T*, int, int64_t, const T*, int64_t, double*, double*, int, cudaStream_t); \
-    template void launch_objective_identity<T>(const T*, const T*, int, const double*, double*, cudaStream_t); \
+    template void launch_dot_parts<T>(const T*, int, int64_t, const T*, int64_t, double*, double*, int, cudaStream_t, \
+                                      int64_t, int);                                                        \
+    template void launch_objective_identity<T>(const T*, const T*, int, const double*, const double*, double*, \
+                                               cudaStream_t);                                               \
     template void launch_wrri_tstats<T>(const T*, int64_t, const void*, int, int64_t, const T*, const T*,   \
                                         int64_t, int64_t, int, int, T*, T*, const TilePlan&, cudaStream_t); \
     template void launch_wrri_wstats<T>(const T*, int64_t, const void*, int, int64_t, const T*, const T*,   \
@@ -572,7 +578,7 @@ void launch_objective_identity(const T* G, const T* H, int k, const double* acc,
     template void launch_wrri_final<T>(const T*, const T*, int, int64_t, const SolveArgs&, T*, int64_t,     \
                                        T*, int64_t, int*, cudaStream_t);                                    \
     template void launch_vec_sum_flag<T>(const T*, int64_t, int64_t, double*, int, int, int*, cudaStream_t);\
-    template void launch_rowsum_flag<T>(const T*, int, int64_t, int64_t, double*, int, int, int*, cudaStream_t);\
+    template void launch_rowsum_flag<T>(const T*, int, int64_t, int64_t, double*, int, int, int*, cudaStream_t, int);\
     template void launch_vec_scale_to_sum<T>(T*, int64_t, int64_t, const double*, int, double, cudaStream_t);\
     template void launch_objective<T>(const T*, int64_t, const void*, int, int64_t, const T*, const T*,     \
                                       int64_t, int64_t, int, double*, int, double*, cudaStream_t);          \

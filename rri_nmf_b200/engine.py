@@ -59,9 +59,13 @@ class RRIEngine(object):
     order='rri' makes one pass over the rows and the columns per topic).
     order: 'rri' (reference-exact interleaved order, nmf.py:415-476) or 'hals' (block order).
     math : 'ieee' or 'tf32' (tcgen05 tensor-core contraction; float32 + hals only).
+    models: None (one model), or b >= 1 models of rank k each on the same binding (rri_set_models: dense unmasked X,
+           order='hals', one GPU, b * k <= 256).  Every block-order half-step contracts X once against the factors of
+           all b models.  The factors are then W [b, n, k] and T [b, k, d]; `sweeps` returns b flag words,
+           `topic_sums` two [b, k] arrays and `objective_terms` a [b, 6] array.
     """
 
-    def __init__(self, X, k, W_mat=None, order='rri', math='ieee', comm=None, unstored='missing'):
+    def __init__(self, X, k, W_mat=None, order='rri', math='ieee', comm=None, unstored='missing', models=None):
         if not isinstance(X, torch.Tensor) or not X.is_cuda:
             raise _lib.RriError('RRIEngine needs X resident on a CUDA device (no CPU fallback)')
         if X.dim() != 2:
@@ -85,6 +89,10 @@ class RRIEngine(object):
         self.X = X
         self.n, self.d = int(X.shape[0]), int(X.shape[1])
         self.k = int(k)
+        self.models = None if models is None else int(models)
+        if self.models is not None and self.models < 1:
+            raise ValueError('models must be >= 1')
+        width = self.k * (self.models or 1)
         self.dtype = X.dtype
         self.device = X.device
         self.order = order
@@ -96,7 +104,7 @@ class RRIEngine(object):
         self.h = C.c_void_p()
         dev_index = self.device.index if self.device.index is not None else torch.cuda.current_device()
         self.dev_index = dev_index
-        check(self.lib.rri_create(C.byref(self.h), self.n, self.d, self.k,
+        check(self.lib.rri_create(C.byref(self.h), self.n, self.d, width,
                                   _lib.RRI_F32 if self.dtype == torch.float32 else _lib.RRI_F64,
                                   {'ieee': _lib.RRI_MATH_IEEE, 'tf32': _lib.RRI_MATH_TF32}[math],
                                   {'rri': _lib.RRI_ORDER_RRI, 'hals': _lib.RRI_ORDER_HALS}[order],
@@ -104,6 +112,8 @@ class RRIEngine(object):
         if comm is not None and comm.world > 1:
             path = comm.nccl_path.encode() if comm.nccl_path else None
             check(self.lib.rri_set_comm(self.h, comm.comm, comm.rank, comm.world, path))
+        if self.models is not None:
+            check(self.lib.rri_set_models(self.h, self.models))
         if self.sparse:
             self._bind_csr(X, W_mat)
             return
@@ -242,19 +252,26 @@ class RRIEngine(object):
         return p
 
     def _check_factors(self, W, T):
-        if tuple(W.shape) != (self.n, self.k) or tuple(T.shape) != (self.k, self.d):
+        if self.models is not None:
+            b = self.models
+            if tuple(W.shape) != (b, self.n, self.k) or tuple(T.shape) != (b, self.k, self.d):
+                raise ValueError('W must be models*n*k and T must be models*k*d')
+        elif tuple(W.shape) != (self.n, self.k) or tuple(T.shape) != (self.k, self.d):
             raise ValueError('W must be n*k and T must be k*d')
         for a in (W, T):
             if a.dtype != self.dtype or a.device != self.device or not a.is_contiguous():
                 raise ValueError('factors must be contiguous %s tensors on %s' % (self.dtype, self.device))
 
     def sweeps(self, W, T, n_sweeps, params, want_flags=True):
-        """n_sweeps sweeps in place on W, T.  Returns the flags word (0 if want_flags is False)."""
+        """n_sweeps sweeps in place on W, T.  Returns the flags word (0 if want_flags is False); on a models engine
+        a list of one word per model."""
         self._check_factors(W, T)
-        flags = C.c_int32(0)
+        flags = (C.c_int32 * (self.models or 1))()
         check(self.lib.rri_sweeps(self.h, _ptr(W), _ptr(T), int(n_sweeps), C.byref(params),
-                                  C.byref(flags) if want_flags else None, self._stream()))
-        return int(flags.value)
+                                  flags if want_flags else None, self._stream()))
+        if self.models is not None:
+            return [int(f) for f in flags]
+        return int(flags[0])
 
     def topics(self, W, T, t_begin, t_end, params):
         self._check_factors(W, T)
@@ -264,24 +281,30 @@ class RRIEngine(object):
         return int(flags.value)
 
     def topic_sums(self):
-        sT = (C.c_double * self.k)()
-        sW = (C.c_double * self.k)()
+        width = self.k * (self.models or 1)
+        sT = (C.c_double * width)()
+        sW = (C.c_double * width)()
         check(self.lib.rri_topic_sums(self.h, sT, sW, self._stream()))
+        if self.models is not None:
+            return np.array(sT[:]).reshape(self.models, self.k), np.array(sW[:]).reshape(self.models, self.k)
         return np.array(sT[:]), np.array(sW[:])
 
     def objective_terms(self, W, T, via_contraction=False, reuse_last_sweep=False):
         """[0.5*sum M(X-WT)^2, sum M X^2, sum W^2, sum |W|, sum T^2, sum |T|]; the first four are
         all-reduced over the row shards when a communicator is attached.
         via_contraction (unmasked dense data): ||X||^2 - 2<X T', W> + <W'W, T T'> instead of an explicit pass over X;
-        reuse_last_sweep: W, T are exactly what the last block-order `sweeps` call left (its contraction is reused)."""
+        reuse_last_sweep: W, T are exactly what the last block-order `sweeps` call left (its contraction is reused).
+        On a models engine: one row of six per model."""
         self._check_factors(W, T)
-        out = (C.c_double * 6)()
+        out = (C.c_double * (6 * (self.models or 1)))()
         if via_contraction:
             check(self.lib.rri_objective_contraction(self.h, _ptr(W), _ptr(T), int(bool(reuse_last_sweep)), out,
                                                      self._stream()))
         else:
             check(self.lib.rri_objective(self.h, _ptr(W), _ptr(T), out, self._stream()))
         v = np.array(out[:])
+        if self.models is not None:
+            return v.reshape(self.models, 6)
         if self.comm is not None and self.comm.world > 1:
             import torch.distributed as dist
             t = torch.tensor(v[:4], dtype=torch.float64, device=self.device)
@@ -293,11 +316,16 @@ class RRIEngine(object):
                   reuse_last_sweep=False):
         """nmf.py:71-94"""
         v = self.objective_terms(W, T, via_contraction, reuse_last_sweep)
+        if self.models is not None:       # one objective per model
+            return [float(r[0] + 0.5 * reg_w_l2 * r[2] + 0.5 * reg_t_l2 * r[4] + reg_t_l1 * r[5] + reg_w_l1 * r[3])
+                    for r in v]
         return float(v[0] + 0.5 * reg_w_l2 * v[2] + 0.5 * reg_t_l2 * v[4] + reg_t_l1 * v[5] + reg_w_l1 * v[3])
 
     def rel_error(self, W, T):
-        """||M^(1/2) o (X - WT)||_F / ||M^(1/2) o X||_F"""
+        """||M^(1/2) o (X - WT)||_F / ||M^(1/2) o X||_F (a list of one per model on a models engine)"""
         v = self.objective_terms(W, T)
+        if self.models is not None:
+            return [float(np.sqrt(2.0 * r[0] / r[1])) for r in v]
         return float(np.sqrt(2.0 * v[0] / v[1]))
 
     def partials_T(self, W, T, t):

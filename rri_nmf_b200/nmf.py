@@ -412,13 +412,321 @@ def nmf(X, k, w_row=None, W_mat=None, fix_W=False, fix_T=False, random_state=Non
         dtype = torch.float32 if (X.dtype if sparse_in else np.asarray(X).dtype) == np.float32 else torch.float64
 
     # ---- initialisation and validation, as nmf.py:819-880
+    init_on_device = _init_on_device_rule(X, n, d, W_in, T_in, init_on_device, comm)
+    W0, T0 = _host_start(X, W_mat, k, init, random_state, t_row_sum, w_row_sum, W_in, T_in, init_on_device)
+    timing = {}
+    _t0 = time.perf_counter()
+    a_W_mat_user = W_mat
+    with torch.cuda.device(device):
+        if sparse_in:
+            Xd, W_mat = _sparse_to_device(X, W_mat, device, dtype)
+        else:
+            Xd = _to_device(X, device, dtype)
+        W_mat_user = a_W_mat_user
+        Md = W_mat if sparse_in else _mask_to_device(W_mat, device, dtype)   # sparse: 1-D entry weights, already there
+        # (no synchronisation here: the host -> device copy of X keeps running while the engine allocates its
+        # workspace; the first kernel is stream-ordered behind it)
+        timing['to_device_enqueue_s'] = time.perf_counter() - _t0   # host -> device copies of X (and W_mat) issued
+        _t1 = time.perf_counter()
+        own_engine = engine is None
+        if engine is None:
+            # (fix_T: the W-only sweeps are the same in both orders; on zero-filled data they run on a block-order
+            # binding, which holds no interleaved-order partials)
+            engine = RRIEngine(Xd, k, W_mat=Md, order='hals' if zero_filled and fix_T else update_order, math=math,
+                               comm=comm, unstored=unstored)
+        timing['engine_setup_s'] = time.perf_counter() - _t1       # workspace, transposed copy of X, peer mapping
+        try:
+            W, T = _device_start(engine, Xd, W_mat, Md, k, init, random_state, t_row_sum, w_row_sum, W0, T0,
+                                 init_on_device, timing)
+            if sharded:
+                import torch.distributed as dist
+                dist.broadcast(T, src=0)
+            _t2 = time.perf_counter()
+            out = _solve(engine, X if sparse_in else Xd, W, T, rtv, locals())
+            timing['solve_s'] = time.perf_counter() - _t2           # (rest of the H2D copy,) sweeps, device -> host copy of W, T
+            out['timing'] = timing
+            if return_reconstruction_err:
+                Wd = W if isinstance(out['W'], np.ndarray) else out['W']
+                Td = T if isinstance(out['T'], np.ndarray) else out['T']
+                out['reconstruction_err'] = float(np.sqrt(2.0 * engine.objective_terms(Wd, Td)[0]))
+            if 'obj_calculator' in out and own_engine:
+                # the calculator outlives this call without pinning device memory (and stays picklable)
+                out['obj_calculator']._detach(X, W_mat_user, out['W'], out['T'], device, dtype, engine.order,
+                                              engine.unstored)
+            return out
+        finally:
+            if own_engine:
+                _t3 = time.perf_counter()
+                engine.close()
+                timing['teardown_s'] = time.perf_counter() - _t3
+
+
+# Widest stacked factor operand (models * k) of one models engine; more models run as groups one after another on the
+# same device copy of X.  See DESIGN.md §6 for the measurement that chose it.
+MODELS_WIDTH_CAP = 256
+
+
+def _model_groups(n_models, k, cap=None):
+    """sizes of the groups the models are run in: as many models of rank k per group as fit the width cap"""
+    per = max(1, (MODELS_WIDTH_CAP if cap is None else cap) // int(k))
+    return [min(per, n_models - i) for i in range(0, n_models, per)]
+
+
+def nmf_models(X, k, random_state=None, W_in=None, T_in=None, **kwargs):
+    """Several block-order factorisations of one matrix, X ~ W_m T_m for m = 0..b-1, sharing every pass over X.
+
+    Restarts and consensus runs fit many models of one X.  Here the factors of up to MODELS_WIDTH_CAP / k models are
+    stacked into one operand, so each block-order half-step reads X once for all of them (two passes per sweep instead
+    of 2b); the row updates stay per model.  X is uploaded once.
+
+    random_state: a list of seeds, one per model, and/or W_in, T_in: lists of starting factors (n x k, k x d).  The
+    number of models is the length of the list(s) given.  Every other keyword argument is nmf()'s.  Each model starts
+    exactly as nmf() would start it (host or device initialisation by the same rule, or its W_in / T_in), and returns
+    what `nmf(X, k, random_state=s_m, update_order='hals', ...)` returns for it: a dict with 'W', 'T', 'iter_cputime',
+    'random_state' and, with compute_obj_each_iter, 'obj_history'.  NNDSVD hardly depends on the seed: for restarts use
+    init='random', 'smart_random' or 'nndsvdar', or pass starts.
+
+    Each model stops on its own (the stopping rule of nmf() on its own objective history); the batch sweeps on until all
+    have stopped or max_iter is reached.  A model whose sweep fails (an emptied topic, an unbounded objective,
+    non-finite values) gets the dict {'error': <the exception nmf() would raise>, 'random_state': ...} and no factors;
+    its factors are zeroed on the device and the others carry on.  With math='ieee' every model is bit-identical to its
+    own nmf() run; with math='tf32' the models share the contraction's operand (and, with 16-bit copies of X, its
+    power-of-two scale), which changes their rounding, not their accuracy.  The flags are read after every engine
+    call: a model that produces non-finite values inside a call of several sweeps (sweeps_per_call) can disturb that
+    shared scale for the rest of the call.
+
+    Supported: dense unmasked X (fp32 / fp64), update_order='hals', math 'ieee' / 'tf32', the four regularisers,
+    w_row_sum / t_row_sum as upper bounds, project_W_each_iter, do_final_project_W, compute_obj_each_iter, objective,
+    eps_stop, max_iter, max_time, sweeps_per_call, init_on_device, device.  Everything else raises before any device
+    work: NotImplementedError for W_mat, sparse X, comm, update_order='rri', fix_W / fix_T, project_T_each_iter with
+    t_row_sum, early_stop, diagnostics, w_row, the Gaussian mechanism, store_gradients, an engine, and
+    return_reconstruction_err; ValueError for lists of different lengths and for k > 256.
+    """
+    import inspect
+    defaults = {name: p.default for name, p in inspect.signature(nmf).parameters.items()
+                if p.default is not inspect.Parameter.empty}
+    unknown = sorted(set(kwargs) - set(defaults))
+    if unknown:
+        raise TypeError('nmf_models() got unexpected keyword arguments %s' % unknown)
+    a = dict(defaults)
+    a['update_order'] = 'hals'
+    a.update(kwargs)
+    lib = _lib.load()
+    del lib
+
+    # ---- what the shared contraction does not serve: refuse before any device work
+    if a['W_mat'] is not None:
+        raise NotImplementedError('nmf_models takes unmasked data (no W_mat)')
+    if _is_sparse(X):
+        raise NotImplementedError('nmf_models takes dense X')
+    if a['comm'] is not None:
+        raise NotImplementedError('nmf_models runs on one GPU (no comm)')
+    if a['update_order'] == 'rri':
+        raise NotImplementedError("nmf_models runs the block order (update_order='hals')")
+    if a['update_order'] != 'hals':
+        raise ValueError("update_order must be 'hals'")
+    if a['fix_W'] or a['fix_T']:
+        raise NotImplementedError('nmf_models does not take fix_W / fix_T')
+    if a['project_T_each_iter'] and a['t_row_sum'] and not (a['reg_w_l1'] or a['reg_t_l1']):
+        raise NotImplementedError('nmf_models does not take project_T_each_iter with t_row_sum')
+    if a['early_stop']:
+        raise NotImplementedError('nmf_models does not take early_stop')
+    diagnostics = a['diagnostics'] if type(a['diagnostics']) is list else [a['diagnostics']]
+    if diagnostics:
+        raise NotImplementedError('nmf_models does not take diagnostics')
+    if a['w_row'] is not None:
+        raise NotImplementedError('w_row is not on the device path; pre-scale X by sqrt(w_row) on the host')
+    if a['eps_gauss_t'] or a['delta_gauss_t']:
+        raise NotImplementedError('the Gaussian DP mechanism (nmf.py:422-435) is not on the device path')
+    if a['store_gradients']:
+        raise NotImplementedError('nmf_models does not take store_gradients')
+    if a['engine'] is not None:
+        raise NotImplementedError('nmf_models builds its own engines (no engine=)')
+    if a['return_reconstruction_err']:
+        raise NotImplementedError('nmf_models does not take return_reconstruction_err')
+    if a['w_row_sum'] is not None and not np.isscalar(a['w_row_sum']):
+        raise NotImplementedError('vector w_row_sum is not on the device path')
+    if a['math'] not in ('ieee', 'tf32'):
+        raise ValueError("math must be 'ieee' or 'tf32'")
+    if a['objective'] not in ('auto', 'exact', 'contraction'):
+        raise ValueError("objective must be 'auto', 'exact' or 'contraction'")
+    k = int(k)
+    if k < 1 or k > 256:
+        raise ValueError('k must be in [1, 256] (got %d)' % k)
+    lists = {name: v for name, v in (('random_state', random_state), ('W_in', W_in), ('T_in', T_in)) if v is not None}
+    if not lists:
+        raise ValueError('nmf_models needs a list of random_state seeds and/or lists W_in, T_in (one entry per model)')
+    lengths = {name: len(v) for name, v in lists.items()}
+    if len(set(lengths.values())) != 1:
+        raise ValueError('random_state, W_in and T_in must have one entry per model (lengths %s)' % lengths)
+    b = next(iter(lengths.values()))
+    if b < 1:
+        raise ValueError('nmf_models needs at least one model')
+    seeds = list(random_state) if random_state is not None else [None] * b
+    W_ins = list(W_in) if W_in is not None else [[]] * b
+    T_ins = list(T_in) if T_in is not None else [[]] * b
+    n, d = X.shape
+    # ---- argument policy of nmf() (nmf.py:280-315)
+    project_T = a['project_T_each_iter']
+    if project_T and np.any([a['reg_w_l1'], a['reg_t_l1']]):
+        logger.warning('This implementation can not solve project_T_each_iter=True with regularization. '
+                       'Setting project_T_each_iter to False.')
+        project_T = False
+    if (not project_T and not a['t_row_sum']) and (a['reg_t_l1'] < 0 or a['reg_t_l2'] < 0):
+        logger.error('Unbounded objective. reg_t_l1=%s, reg_t_l2=%s', a['reg_t_l1'], a['reg_t_l2'])
+        return [{'W': np.ones((n, k)), 'T': np.ones((k, d)) * 1e6, 'obj_history': [-np.inf], 'iter_cputime': [0]}
+                for _ in range(b)]
+    if (not a['project_W_each_iter'] and not a['w_row_sum']) and (a['reg_w_l1'] < 0 or a['reg_w_l2'] < 0):
+        logger.error('Unbounded objective. reg_w_l1=%s, reg_w_l2=%s', a['reg_w_l1'], a['reg_w_l2'])
+        return [{'W': np.ones((n, k)) * 1e6, 'T': np.ones((k, d)), 'obj_history': [-np.inf], 'iter_cputime': [0]}
+                for _ in range(b)]
+    seeds = [int(time.time()) % 4294967296 if s is None else s for s in seeds]
+    t_global_start = time.time()
+    max_time = a['max_time'] - 10                                 # nmf.py:333
+    init = 'random' if n <= k else a['init']                      # nmf.py:346-347
+    start_time = time.process_time()
+    device = a['device']
+    if device is None:
+        device = X.device if isinstance(X, torch.Tensor) and X.is_cuda else torch.device('cuda')
+    device = torch.device(device)
+    if not torch.cuda.is_available():
+        raise _lib.RriError('no CUDA device is available: rri_nmf_b200.nmf_models has no CPU fallback')
+    if device.type != 'cuda':
+        raise _lib.RriError('rri_nmf_b200.nmf_models runs on CUDA devices only (no CPU fallback)')
+    if device.index is None:
+        device = torch.device('cuda', torch.cuda.current_device())
+    if isinstance(X, torch.Tensor):
+        dtype = X.dtype if X.dtype in (torch.float32, torch.float64) else torch.float64
+    else:
+        dtype = torch.float32 if np.asarray(X).dtype == np.float32 else torch.float64
+    numpy_io = not isinstance(X, torch.Tensor)
+    w_row_sum, t_row_sum = a['w_row_sum'], a['t_row_sum']
+    on_device = [_init_on_device_rule(X, n, d, W_ins[m], T_ins[m], a['init_on_device'], None) for m in range(b)]
+    starts = [_host_start(X, None, k, init, seeds[m], t_row_sum, w_row_sum, W_ins[m], T_ins[m], on_device[m])
+              for m in range(b)]
+    results = [None] * b
+    with torch.cuda.device(device):
+        Xd = _to_device(X, device, dtype)
+        first = 0
+        for g in _model_groups(b, k):
+            idx = list(range(first, first + g))
+            first += g
+            engine = RRIEngine(Xd, k, order='hals', math=a['math'], models=g)
+            try:
+                out = _solve_models(engine, idx, starts, on_device, seeds, init, a, start_time, t_global_start,
+                                    max_time, numpy_io)
+            finally:
+                engine.close()
+            for m, r in zip(idx, out):
+                results[m] = r
+    return results
+
+
+def _solve_models(engine, idx, starts, on_device, seeds, init, a, start_time, t_global_start, max_time, numpy_io):
+    """The sweep loop of _solve for the models `idx` of one models engine, each stopping on its own."""
+    k, g = engine.k, len(idx)
+    w_row_sum, t_row_sum = a['w_row_sum'], a['t_row_sum']
+    regs = dict(reg_w_l1=a['reg_w_l1'], reg_w_l2=a['reg_w_l2'], reg_t_l1=a['reg_t_l1'], reg_t_l2=a['reg_t_l2'])
+    W = torch.empty((g, engine.n, k), dtype=engine.dtype, device=engine.device)
+    T = torch.empty((g, k, engine.d), dtype=engine.dtype, device=engine.device)
+    for j, m in enumerate(idx):
+        Wj, Tj = _device_start(engine, engine.X, None, None, k, init, seeds[m], t_row_sum, w_row_sum, starts[m][0],
+                               starts[m][1], on_device[m], {})
+        W[j].copy_(Wj)
+        T[j].copy_(Tj)
+        del Wj, Tj
+    project_W = a['project_W_each_iter'] and w_row_sum is not None
+    if project_W:                                                                 # nmf.py:870-873
+        for j in range(g):
+            engine.project_rows_simplex(W[j], w_row_sum)
+    params = engine.params(ub_w=w_row_sum, ub_t=t_row_sum, **regs)
+    obj_mode = a['objective']
+    via_contraction = obj_mode == 'contraction' or (obj_mode == 'auto' and engine.math == 'ieee')
+    compute_obj = a['compute_obj_each_iter']
+    unapplied_reset = a['reset_topic_method']
+    chunk = 1 if (compute_obj or project_W) else max(1, int(a['sweeps_per_call']))
+    active = [True] * g
+    final = [None] * g                      # (W, T) of a model that stopped before the others
+    errors = [None] * g
+    hist = [[] for _ in range(g)]
+    cpu = [[] for _ in range(g)]
+    iter_no, max_iter = 0, a['max_iter']
+    while iter_no < max_iter and any(active):
+        ns = min(chunk, max_iter - iter_no)
+        flags = engine.sweeps(W, T, ns, params, want_flags=True)
+        sums = []
+
+        def topic_sums(j):
+            if not sums:
+                sums.extend(engine.topic_sums())
+            return sums[0][j], sums[1][j]
+        for j in range(g):
+            if not active[j]:
+                if flags[j] & (_lib.FLAG_UNBOUNDED | _lib.FLAG_NONFINITE):
+                    W[j].zero_()            # (a model that already stopped: its result was taken when it stopped)
+                    T[j].zero_()
+                continue
+            exc = _flags_error(flags[j], lambda: topic_sums(j), unapplied_reset)
+            if exc is not None:
+                # only this model fails; zero factors keep it out of the shared operand's scale from here on
+                errors[j] = exc
+                active[j] = False
+                W[j].zero_()
+                T[j].zero_()
+        iter_no += ns
+        if project_W:                                                             # nmf.py:481-484
+            for j in range(g):
+                if active[j]:
+                    engine.project_rows_simplex(W[j], w_row_sum)
+        if compute_obj:                                                           # nmf.py:488-489
+            objs = engine.objective(W, T, via_contraction=via_contraction, reuse_last_sweep=not project_W, **regs)
+        now = time.process_time()
+        for j in range(g):
+            if active[j]:
+                if compute_obj:
+                    hist[j].append(objs[j])
+                cpu[j].extend([now] * ns)
+        if time.time() - t_global_start >= max_time:                             # nmf.py:506-508
+            break
+        if compute_obj:
+            for j in range(g):
+                if active[j] and _universal_stopping_condition(hist[j], a['eps_stop']):     # :510-514
+                    final[j] = (W[j].clone(), T[j].clone())
+                    active[j] = False
+    out = []
+    for j, m in enumerate(idx):
+        if errors[j] is not None:
+            out.append({'error': errors[j], 'random_state': seeds[m]})
+            continue
+        Wj, Tj = final[j] if final[j] is not None else (W[j].clone(), T[j].clone())
+        if not project_W and w_row_sum is not None and a['do_final_project_W']:   # nmf.py:519-529
+            engine.project_rows_simplex(Wj, w_row_sum)
+        torch.cuda.current_stream(Wj.device).synchronize()
+        r = {'W': Wj.cpu().numpy() if numpy_io else Wj, 'T': Tj.cpu().numpy() if numpy_io else Tj}
+        if compute_obj:
+            r['obj_history'] = hist[j]
+        r['iter_cputime'] = [x - start_time for x in cpu[j]]
+        r['random_state'] = seeds[m]
+        out.append(r)
+    return out
+
+
+def _init_on_device_rule(X, n, d, W_in, T_in, init_on_device, comm):
+    """Whether the NNDSVD initialisation runs on the device (see `init_on_device` in the module docstring)."""
     need_init = _is_empty(W_in) or _is_empty(T_in)
     if init_on_device is None:
         init_on_device = (isinstance(X, torch.Tensor) and X.is_cuda) or n * d >= (1 << 26)
-    init_on_device = bool(init_on_device) and need_init and comm is None
+    return bool(init_on_device) and need_init and comm is None
+
+
+def _host_start(X, W_mat, k, init, random_state, t_row_sum, w_row_sum, W_in, T_in, init_on_device):
+    """(W0, T0) of nmf.py:819-868 as far as the host makes them: the host NNDSVD (unless it runs on the device) and the
+    caller's W_in / T_in after their shape check.  A factor left to the device initialisation is None."""
+    n, d = X.shape
+    need_init = _is_empty(W_in) or _is_empty(T_in)
     W0 = T0 = None
     if need_init and not init_on_device:
-        if sparse_in:
+        if _is_sparse(X):
             # M o X is the sparse matrix itself (entry weights folded in): the SVD never densifies it
             if isinstance(X, torch.Tensor):
                 Xc = X.detach().to_sparse_csr().cpu()
@@ -450,67 +758,31 @@ def nmf(X, k, w_row=None, W_mat=None, fix_W=False, fix_T=False, random_state=Non
         if tuple(np.shape(T_in)) != (k, d):
             raise ValueError('T_in has wrong dimensions, must be k*d')
         T0 = T_in
-    timing = {}
-    _t0 = time.perf_counter()
-    a_W_mat_user = W_mat
-    with torch.cuda.device(device):
-        if sparse_in:
-            Xd, W_mat = _sparse_to_device(X, W_mat, device, dtype)
-        else:
-            Xd = _to_device(X, device, dtype)
-        W_mat_user = a_W_mat_user
-        Md = W_mat if sparse_in else _mask_to_device(W_mat, device, dtype)   # sparse: 1-D entry weights, already there
-        # (no synchronisation here: the host -> device copy of X keeps running while the engine allocates its
-        # workspace; the first kernel is stream-ordered behind it)
-        timing['to_device_enqueue_s'] = time.perf_counter() - _t0   # host -> device copies of X (and W_mat) issued
-        _t1 = time.perf_counter()
-        own_engine = engine is None
-        if engine is None:
-            # (fix_T: the W-only sweeps are the same in both orders; on zero-filled data they run on a block-order
-            # binding, which holds no interleaved-order partials)
-            engine = RRIEngine(Xd, k, W_mat=Md, order='hals' if zero_filled and fix_T else update_order, math=math,
-                               comm=comm, unstored=unstored)
-        timing['engine_setup_s'] = time.perf_counter() - _t1       # workspace, transposed copy of X, peer mapping
-        try:
-            if init_on_device:
-                # NNDSVD where X lives; its passes over X go through the engine's own contraction kernel
-                _ti = time.perf_counter()
-                Wi, Ti = _initialize_on_device(Xd, W_mat, k, init, random_state, t_row_sum, w_row_sum,
-                                               products=engine.products() if (Md is None or sparse_in) else None)
-                torch.cuda.current_stream(device).synchronize()
-                timing['init_on_device_s'] = time.perf_counter() - _ti
-                W0 = Wi if W0 is None else W0
-                T0 = Ti if T0 is None else T0
-            # np.maximum(W_in, 0) makes copies: the caller's arrays are never mutated (nmf.py:867-868)
-            W = _to_device(W0, device, dtype).clamp(min=0).contiguous()
-            T = _to_device(T0, device, dtype).clamp(min=0).contiguous()
-            if sharded:
-                import torch.distributed as dist
-                if T.data_ptr() == (T0.data_ptr() if isinstance(T0, torch.Tensor) else 0):
-                    T = T.clone()
-                dist.broadcast(T, src=0)
-            if W.data_ptr() == (W0.data_ptr() if isinstance(W0, torch.Tensor) else 0):
-                W = W.clone()
-            if T.data_ptr() == (T0.data_ptr() if isinstance(T0, torch.Tensor) else 0):
-                T = T.clone()
-            _t2 = time.perf_counter()
-            out = _solve(engine, X if sparse_in else Xd, W, T, rtv, locals())
-            timing['solve_s'] = time.perf_counter() - _t2           # (rest of the H2D copy,) sweeps, device -> host copy of W, T
-            out['timing'] = timing
-            if return_reconstruction_err:
-                Wd = W if isinstance(out['W'], np.ndarray) else out['W']
-                Td = T if isinstance(out['T'], np.ndarray) else out['T']
-                out['reconstruction_err'] = float(np.sqrt(2.0 * engine.objective_terms(Wd, Td)[0]))
-            if 'obj_calculator' in out and own_engine:
-                # the calculator outlives this call without pinning device memory (and stays picklable)
-                out['obj_calculator']._detach(X, W_mat_user, out['W'], out['T'], device, dtype, engine.order,
-                                              engine.unstored)
-            return out
-        finally:
-            if own_engine:
-                _t3 = time.perf_counter()
-                engine.close()
-                timing['teardown_s'] = time.perf_counter() - _t3
+    return W0, T0
+
+
+def _device_start(engine, Xd, W_mat, Md, k, init, random_state, t_row_sum, w_row_sum, W0, T0, init_on_device,
+                  timing):
+    """The device factors nmf() starts from: the device NNDSVD where `init_on_device` says so (its passes over X go
+    through the engine's own contraction kernel), then W0 / T0 clipped at 0 in fresh device tensors."""
+    device, dtype = engine.device, engine.dtype
+    if init_on_device:
+        _ti = time.perf_counter()
+        sparse_in = Xd.layout == torch.sparse_csr
+        Wi, Ti = _initialize_on_device(Xd, W_mat, k, init, random_state, t_row_sum, w_row_sum,
+                                       products=engine.products() if (Md is None or sparse_in) else None)
+        torch.cuda.current_stream(device).synchronize()
+        timing['init_on_device_s'] = timing.get('init_on_device_s', 0.0) + time.perf_counter() - _ti
+        W0 = Wi if W0 is None else W0
+        T0 = Ti if T0 is None else T0
+    # np.maximum(W_in, 0) makes copies: the caller's arrays are never mutated (nmf.py:867-868)
+    W = _to_device(W0, device, dtype).clamp(min=0).contiguous()
+    T = _to_device(T0, device, dtype).clamp(min=0).contiguous()
+    if W.data_ptr() == (W0.data_ptr() if isinstance(W0, torch.Tensor) else 0):
+        W = W.clone()
+    if T.data_ptr() == (T0.data_ptr() if isinstance(T0, torch.Tensor) else 0):
+        T = T.clone()
+    return W, T
 
 
 def _solve(engine, Xd, W, T, rtv, a):
@@ -718,21 +990,29 @@ def _sweep_fix_W(engine, W, T, a):
 
 
 def _raise_on_flags(flags, engine, unapplied_reset=None):
+    exc = _flags_error(flags, engine.topic_sums, unapplied_reset)
+    if exc is not None:
+        raise exc
+
+
+def _flags_error(flags, topic_sums, unapplied_reset=None):
+    """The exception a sweep's flags word stands for (None: carry on); topic_sums() -> (sum_T[k], sum_W[k])"""
     if unapplied_reset is not None and flags & (_lib.FLAG_ZERO_T | _lib.FLAG_ZERO_W):
-        sT, sW = engine.topic_sums()
+        sT, sW = topic_sums()
         if np.any(sT <= 1e-10) or np.any(sW <= 1e-10):
-            raise ValueError("a topic emptied (sum <= 1e-10) and reset_topic_method=%r is not applied on this engine "
-                             "(resets exist for update_order='rri' on unmasked, unsharded data; nmf.py:762-816): "
-                             "use that mode, other initial factors, or reset_topic_method=None" % (unapplied_reset,))
+            return ValueError("a topic emptied (sum <= 1e-10) and reset_topic_method=%r is not applied on this engine "
+                              "(resets exist for update_order='rri' on unmasked, unsharded data; nmf.py:762-816): "
+                              "use that mode, other initial factors, or reset_topic_method=None" % (unapplied_reset,))
     if flags & _lib.FLAG_UNBOUNDED:
         # optimization.py:60-67 / :76-77 -> _unbounded_objective (:105-107)
-        raise ValueError('Minimum objective is unbounded. (a denominator became <= 0 with no upper bound; '
-                         'typically a topic collapsed to zero while reset_topic_method is None)')
+        return ValueError('Minimum objective is unbounded. (a denominator became <= 0 with no upper bound; '
+                          'typically a topic collapsed to zero while reset_topic_method is None)')
     if flags & _lib.FLAG_NONFINITE:
-        raise FloatingPointError('non-finite values produced in the sweep')
+        return FloatingPointError('non-finite values produced in the sweep')
     if flags & _lib.FLAG_ZERO_W:
-        if np.any(engine.topic_sums()[1] <= 0):
-            raise AssertionError('W[:, t] sums to 0')                              # nmf.py:476
+        if np.any(topic_sums()[1] <= 0):
+            return AssertionError('W[:, t] sums to 0')                              # nmf.py:476
+    return None
 
 
 def _sweep_with_resets(engine, Xd, W, T, params, a, state):
