@@ -96,8 +96,18 @@ int rri_peer_close(rri_handle_t h);
  *     W_dev [models][n_local][k_m],   T_dev [models][k_m][d]  (= the stacked [k, d] operand of the W half-step).
  * Per model: rri_sweeps writes `models` flag words to flags_host, rri_topic_sums returns k sums per factor (model-major),
  * rri_objective and rri_objective_contraction write 6 doubles per model.  rri_topics, rri_partials_T and the peer-memory
- * entry points refuse the handle; sweeps take no simplex_T.  models == 1 is a handle as rri_create makes it. */
+ * entry points refuse the handle; sweeps take no simplex_T.  models == 1 is a handle as rri_create makes it.
+ * rri_set_models(h, b) is rri_set_model_ranks with b equal ranks k / b. */
 int rri_set_models(rri_handle_t h, int32_t models);
+/* Models of different ranks on one binding (choosing k: one fit per candidate rank): ranks[z] >= 1 for z < models,
+ * sum ranks == k (rri_create's k, <= 256), models <= k; the same conditions and refusals as rri_set_models.  With
+ * o_z = ranks[0] + ... + ranks[z-1] the layouts are the ones above with o_z in place of z * k_m:
+ *     W_dev: model z is [n_local, ranks[z]] at offset n_local * o_z,
+ *     T_dev: the stacked [k, d] operand, model z in rows o_z .. o_z + ranks[z] - 1 (offset d * o_z);
+ * rri_topic_sums returns the k sums per factor in the same stacked order.  Every model's rows are updated by the kernel
+ * a handle of its rank alone would use (consecutive models of equal rank share a launch); with RRI_MATH_IEEE every model is
+ * bit-identical to a handle of its own. */
+int rri_set_model_ranks(rri_handle_t h, int32_t models, const int32_t* ranks);
 
 /* Optional, before rri_bind on a hals handle: storage [d, ldXt] (ldXt >= n rounded up to 16 bytes) owned by the
  * caller for the engine's transposed copy of X, so that it comes from the caller's allocator (torch's caching

@@ -40,6 +40,7 @@ SYMBOLS = {
     'rri_peer_enable': (C.c_int, [_vp, _i32]),
     'rri_peer_close': (C.c_int, [_vp]),
     'rri_set_models': (C.c_int, [_vp, _i32]),
+    'rri_set_model_ranks': (C.c_int, [_vp, _i32, C.POINTER(_i32)]),
     'rri_set_transpose_storage': (C.c_int, [_vp, _vp, _i64]),
     'rri_bind': (C.c_int, [_vp, _vp, _i64, _vp, _i32, _i64, _vp]),
     'rri_x_operand_bits': (C.c_int, [_vp, C.POINTER(_i32)]),

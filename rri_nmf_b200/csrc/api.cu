@@ -120,12 +120,22 @@ struct PeerGroup {
 };
 
 
+// One model of a handle's stacked factors (rri_set_model_ranks): rank k, first row o of its block of the stacked
+// [k, .] factor (= its first column of the stacked contraction), and offset q of its IEEE Gram matrix (the sum of the
+// squared ranks of the models before it).  A handle of one model is {k, 0, 0}.
+struct ModelRows {
+    int k, o, q;
+};
+
 struct rri_handle_s {
     int64_t n = 0, d = 0;
     int k = 0, dtype = 0, math = 0, order = 0, device = 0, sm_count = 148;
-    // several models of rank km = k / models on one binding (rri_set_models): W [models][n][km], T [models][km][d] (the
-    // stacked [k, d] operand of the W-half contraction), Tt [models][d][km], Wt the stacked [k, ldwt]
-    int models = 1, km = 0;
+    // several models on one binding (rri_set_model_ranks), model z of rank k_z at offset o_z = sum of the ranks before
+    // it: W holds [n, k_z] at n o_z, T is the stacked [k, d] operand of the W-half contraction (model z in rows o_z..),
+    // Tt holds [d, k_z] at d o_z, Wt is the stacked [k, ldwt]
+    int models = 1;
+    std::vector<ModelRows> mrows;      // [models]: rank, offset, offset of the IEEE Gram matrix
+    int* topic_model = nullptr;        // device [k]: the model owning each topic (flag words of the column sums)
     size_t es = 4;
     // data
     const void* X = nullptr; int64_t ldx = 0;
@@ -245,15 +255,17 @@ extern "C" int rri_create(rri_handle_t* out, int64_t n_local, int64_t d, int32_t
     if (prop.major != 10)
         return fail("device %d is sm_%d%d; this build contains sm_100a code only", device, prop.major, prop.minor);
     rri_handle_t h = new rri_handle_s();
-    h->n = n_local; h->d = d; h->k = k; h->km = k; h->dtype = dtype; h->math = math; h->order = order;
+    h->n = n_local; h->d = d; h->k = k; h->dtype = dtype; h->math = math; h->order = order;
     h->device = device; h->sm_count = prop.multiProcessorCount;
     h->es = dtype == RRI_F32 ? 4 : 8;
     if (ws_alloc(h, (void**)&h->sums, sizeof(double) * 2 * k) || ws_alloc(h, (void**)&h->flags, sizeof(int) * 4) ||
-        ws_alloc(h, (void**)&h->counters, sizeof(unsigned) * 8)) {
+        ws_alloc(h, (void**)&h->counters, sizeof(unsigned) * 8) ||
+        ws_alloc(h, (void**)&h->topic_model, sizeof(int) * k)) {
         rri_destroy(h);
         return 1;
     }
     cudaStreamSynchronize(0);
+    h->mrows.assign(1, ModelRows{k, 0, 0});
     *out = h;
     return 0;
 }
@@ -481,6 +493,14 @@ static int allreduce(rri_handle_t h, void* buf, size_t count, cudaStream_t st)
     return 0;
 }
 
+// the end of the run of consecutive models of the same rank that starts at model z0
+static int equal_rank_run(rri_handle_t h, int z0)
+{
+    int z1 = z0 + 1;
+    while (z1 < h->models && h->mrows[z1].k == h->mrows[z0].k) ++z1;
+    return z1;
+}
+
 // Workspace of the block-order half-steps downstream of the contraction (and of the contraction's output): both the
 // dense binding and the zero-filled sparse one.  splits_w / splits_t (K-slices of the two contractions) are set first.
 static int alloc_halfstep_ws(rri_handle_t h)
@@ -498,11 +518,18 @@ static int alloc_halfstep_ws(rri_handle_t h)
         h->ldwt = (n + v - 1) / v * v;
     }
     if (ws_alloc(h, &h->Wt, es * (size_t)k * h->ldwt) || ws_alloc(h, &h->Tt, es * (size_t)d * k)) return 1;
-    // (IEEE Gram products: per model, chunked as a handle of one model of rank km would chunk them)
-    h->gchunks_w = gram_chunks(n, h->km, h->sm_count);
-    h->gchunks_t = gram_chunks(d, h->km, h->sm_count);
-    const int gc = h->gchunks_w > h->gchunks_t ? h->gchunks_w : h->gchunks_t;
-    if (ws_alloc(h, &h->gram_part, es * (size_t)gc * k * h->km)) return 1;
+    // (IEEE Gram products: per model, chunked as a handle of that model alone would chunk them -- model_grams)
+    h->gchunks_w = gram_chunks(n, k, h->sm_count);
+    h->gchunks_t = gram_chunks(d, k, h->sm_count);
+    size_t gp = 0;
+    for (int64_t m : {n, d})
+        for (int z0 = 0, z1; z0 < h->models; z0 = z1) {
+            z1 = equal_rank_run(h, z0);
+            const size_t kz = (size_t)h->mrows[z0].k;
+            const size_t e = (size_t)gram_chunks(m, (int)kz, h->sm_count) * (z1 - z0) * kz * kz;
+            if (e > gp) gp = e;
+        }
+    if (ws_alloc(h, &h->gram_part, es * gp)) return 1;
     h->ub_blocks_w = update_rows_blocks(n, h->sm_count);
     h->ub_blocks_t = update_rows_blocks(d, h->sm_count);
     int ubm = h->ub_blocks_w > h->ub_blocks_t ? h->ub_blocks_w : h->ub_blocks_t;
@@ -633,23 +660,47 @@ static int bind_impl(rri_handle_t h, cudaStream_t st)
     return 0;
 }
 
-extern "C" int rri_set_models(rri_handle_t h, int32_t models)
+extern "C" int rri_set_model_ranks(rri_handle_t h, int32_t models, const int32_t* ranks)
 {
     if (!h) return fail("null handle");
-    if (h->X) return fail("rri_set_models must be called before the data are bound");
+    if (h->X) return fail("the models must be set before the data are bound");
     if (models < 1) return fail("models must be >= 1 (got %d)", models);
     if (h->order != RRI_ORDER_HALS) return fail("several models per handle need RRI_ORDER_HALS");
     if (h->world != 1) return fail("several models per handle run on one GPU (world == 1)");
-    if (h->k % models != 0) return fail("k (%d) must be a multiple of models (%d)", h->k, models);
+    if (models > h->k) return fail("models (%d) must be <= k (%d)", models, h->k);
+    if (!ranks) return fail("ranks is null");
+    std::vector<ModelRows> mr((size_t)models);
+    std::vector<int> tm((size_t)h->k);
+    int o = 0, q = 0;
+    for (int z = 0; z < models; ++z) {
+        const int kz = ranks[z];
+        if (kz < 1) return fail("rank %d of model %d must be >= 1", kz, z);
+        if (kz > h->k - o) return fail("the ranks must add up to k (%d)", h->k);
+        mr[z] = ModelRows{kz, o, q};
+        for (int t = o; t < o + kz; ++t) tm[t] = z;
+        o += kz;
+        q += kz * kz;
+    }
+    if (o != h->k) return fail("the ranks add up to %d, not to k (%d)", o, h->k);
     if (models > 4) {       // one flags word per model (rri_create allocates 4)
         ws_release(h, h->flags, sizeof(int) * 4);
         h->flags = nullptr;
         if (ws_alloc(h, (void**)&h->flags, sizeof(int) * (size_t)models)) return 1;
         CK(cudaStreamSynchronize(0));
     }
+    CK(cudaMemcpy(h->topic_model, tm.data(), sizeof(int) * tm.size(), cudaMemcpyHostToDevice));
     h->models = models;
-    h->km = h->k / models;
+    h->mrows = mr;
     return 0;
+}
+
+extern "C" int rri_set_models(rri_handle_t h, int32_t models)
+{
+    if (!h) return fail("null handle");
+    if (models < 1) return fail("models must be >= 1 (got %d)", models);
+    if (h->k % models != 0) return fail("k (%d) must be a multiple of models (%d)", h->k, models);
+    const std::vector<int32_t> ranks((size_t)models, h->k / models);
+    return rri_set_model_ranks(h, models, ranks.data());
 }
 
 extern "C" int rri_set_transpose_storage(rri_handle_t h, void* Xt_dev, int64_t ldXt)
@@ -1145,51 +1196,70 @@ static int data_contraction(rri_handle_t h, bool transpose, const T* B, int64_t 
     return 0;
 }
 
-// Tt [models][d][km] <- the transpose of every model's T [km, d]
+// Tt <- the transpose of every model's T: model z's rows o_z.. of the stacked T [k, d] become [d, k_z] at d o_z
 template <typename T>
 static void transpose_T(rri_handle_t h, const T* Tm, cudaStream_t st)
 {
-    const int km = h->km;
-    for (int z = 0; z < h->models; ++z)
-        launch_transpose<T>(Tm + (int64_t)z * km * h->d, km, h->d, h->d, (T*)h->Tt + (int64_t)z * h->d * km, km, st);
+    for (const ModelRows& r : h->mrows)
+        launch_transpose<T>(Tm + (int64_t)r.o * h->d, r.k, h->d, h->d, (T*)h->Tt + (int64_t)r.o * h->d, r.k, st);
     h->launches += h->models;
 }
 
-// Wt [k, ldwt] (stacked, model-major rows) <- the transpose of every model's W [n, km]
+// Wt [k, ldwt] (stacked, model-major rows) <- the transpose of every model's W [n, k_z] (at n o_z)
 template <typename T>
 static void transpose_W(rri_handle_t h, const T* W, cudaStream_t st)
 {
-    const int km = h->km;
-    for (int z = 0; z < h->models; ++z)
-        launch_transpose<T>(W + (int64_t)z * h->n * km, h->n, km, km, (T*)h->Wt + (int64_t)z * km * h->ldwt, h->ldwt, st);
+    for (const ModelRows& r : h->mrows)
+        launch_transpose<T>(W + (int64_t)r.o * h->n, h->n, r.k, r.k, (T*)h->Wt + (int64_t)r.o * h->ldwt, h->ldwt, st);
     h->launches += h->models;
 }
 
-// The row updates of all models of a handle in one launch: model z reads the column block z*km of the stacked contraction
-// and its Gram matrix -- the diagonal block z of the k x k Gram tile of the tensor-core contraction, or the z-th of the
-// per-model IEEE Gram products
-static RowBatch row_batch(rri_handle_t h, bool tc_gram)
+// The IEEE Gram matrices of every model's block F + m o_z [m, k_z] into G + q_z, each chunked as a handle of that model
+// alone would chunk it (so each is bit-identical to its own): one launch pair per run of consecutive models of equal rank
+template <typename T>
+static void model_grams(rri_handle_t h, const T* F, int64_t m, T* G, cudaStream_t st)
 {
-    RowBatch rb;
-    rb.models = h->models;
-    rb.ldc = h->k;
-    rb.lds = tc_gram ? h->k : h->km;
-    rb.s_stride = tc_gram ? (int64_t)h->km * (h->k + 1) : (int64_t)h->km * h->km;
-    return rb;
+    for (int z0 = 0, z1; z0 < h->models; z0 = z1) {
+        z1 = equal_rank_run(h, z0);
+        const ModelRows& r = h->mrows[z0];
+        launch_gram<T>(F + (int64_t)r.o * m, m, r.k, (T*)h->gram_part, gram_chunks(m, r.k, h->sm_count), G + r.q, st,
+                       z1 - z0, m * r.k);
+        h->launches += 2;
+    }
+}
+
+// The row updates of all models of a handle: one launch per run of consecutive models of equal rank k_r, each a batch of
+// models of rank k_r whose factor rows, transposed copy, contraction columns (block o of C, row stride k), Gram matrix
+// (the diagonal block (o, o) of the k x k Gram tile of the tensor-core contraction, or its own IEEE Gram product at q),
+// flag word and column-sum partials start at the run's first model.  Every model thus gets the kernel, and the rank as
+// a launch argument, that a handle of its rank alone gets; equal ranks make one launch.
+template <typename T>
+static void update_models(rri_handle_t h, T* F, int64_t m, const T* C, int parts, int64_t part_stride, const T* S,
+                          bool tc_gram, const SolveArgs& a, T* Ft, int64_t ldft, int blocks, const ColsumOut& co,
+                          cudaStream_t st)
+{
+    const int64_t K = h->k;
+    for (int z0 = 0, z1; z0 < h->models; z0 = z1) {
+        z1 = equal_rank_run(h, z0);
+        const ModelRows& r = h->mrows[z0];
+        const int64_t o = r.o, kr = r.k;
+        const RowBatch rb{z1 - z0, K, tc_gram ? K : kr, tc_gram ? kr * (K + 1) : kr * kr};
+        launch_update_rows<T>(F + o * m, m, r.k, C + o, parts, part_stride, nullptr, S + (tc_gram ? o * (K + 1) : r.q), a,
+                              Ft ? Ft + o * ldft : nullptr, ldft, (T*)h->colsum_part + o * blocks, h->flags + z0, blocks,
+                              co, rb, st);
+        h->launches++;
+    }
 }
 
 template <typename T>
 static int hals_W_half(rri_handle_t h, T* W, const T* Tk, int64_t ldtk, const rri_params_t* p, bool recompute, cudaStream_t st)
 {
-    const int k = h->k, km = h->km;
+    const int k = h->k;
     const int64_t n = h->n, d = h->d;
     const bool tc_gram = gram_in_contraction(h);
     if (recompute) {
         // C2 = X T' and H = T T' (from the d x k transposed copy, or as the Gram tile of the contraction)
-        if (!tc_gram) {
-            launch_gram<T>((const T*)h->Tt, d, km, (T*)h->gram_part, h->gchunks_t, (T*)h->Hm, st, h->models, d * km);
-            h->launches += 2;
-        }
+        if (!tc_gram) model_grams<T>(h, (const T*)h->Tt, d, (T*)h->Hm, st);
         if (h->zero_csr) {
             launch_spmm<T>(h->zrow, (const T*)h->Tt, k, k, (T*)h->Cpart, k, st);
             h->launches++;
@@ -1200,10 +1270,8 @@ static int hals_W_half(rri_handle_t h, T* W, const T* Tk, int64_t ldtk, const rr
     const int parts = h->math == RRI_MATH_TF32 ? 1 : h->splits_w;
     // the zero-column test of nmf.py:793 is over ALL rows: with row shards the sums are all-reduced once per call
     // (the per-topic sums and the zero-topic flags are taken once per call from W' and T: hals_finish_sums)
-    launch_update_rows<T>(W, n, km, (const T*)h->Cpart, parts, n * k, nullptr, (const T*)h->Hm, solve_args(p, false),
-                          (T*)h->Wt, h->ldwt, (T*)h->colsum_part, h->flags, h->ub_blocks_w,
-                          ColsumOut{nullptr, k, 0, h->counters + 0}, row_batch(h, tc_gram), st);
-    h->launches++;
+    update_models<T>(h, W, n, (const T*)h->Cpart, parts, n * k, (const T*)h->Hm, tc_gram, solve_args(p, false), (T*)h->Wt,
+                     h->ldwt, h->ub_blocks_w, ColsumOut{nullptr, k, 0, h->counters + 0}, st);
     CKL();
     return 0;
 }
@@ -1239,7 +1307,7 @@ static int hals_T_half(rri_handle_t h, T* W, T* Tk, int64_t ldtk, const rri_para
         CKL();
         return 0;
     }
-    if (!tc_gram) { launch_gram<T>(W, n, h->km, (T*)h->gram_part, h->gchunks_w, G, st, h->models, n * h->km); h->launches += 2; }
+    if (!tc_gram) model_grams<T>(h, W, n, G, st);
     // (one rank, TF32: the Gram tile lands right behind the contraction output, as the all-reduce wants it)
     T* Cout = (h->world > 1 && psplits == 1) ? cg : (T*)h->Cpart;
     if (h->zero_csr) {
@@ -1268,9 +1336,8 @@ static int hals_T_half(rri_handle_t h, T* W, T* Tk, int64_t ldtk, const rri_para
         return 0;
     }
     // Tt (d x k) is updated in place; its transpose is written straight into the caller's T (k x d)
-    launch_update_rows<T>((T*)h->Tt, d, h->km, C, parts, d * k, nullptr, G, solve_args(p, true), Tk, ldtk, (T*)h->colsum_part,
-                          h->flags, h->ub_blocks_t, ColsumOut{nullptr, 0, 0, h->counters + 2}, row_batch(h, tc_gram), st);
-    h->launches++;
+    update_models<T>(h, (T*)h->Tt, d, C, parts, d * k, G, tc_gram, solve_args(p, true), Tk, ldtk, h->ub_blocks_t,
+                     ColsumOut{nullptr, 0, 0, h->counters + 2}, st);
     CKL();
     return 0;
 }
@@ -1282,10 +1349,11 @@ static int hals_T_half(rri_handle_t h, T* W, T* Tk, int64_t ldtk, const rri_para
 template <typename T>
 static int hals_finish_sums(rri_handle_t h, const T* Tm, bool t_sums, cudaStream_t st)
 {
-    launch_rowsum_flag<T>((const T*)h->Wt, h->k, h->n, h->ldwt, h->sums, h->k, h->world > 1 ? 0 : 2, h->flags, st, h->km);
+    launch_rowsum_flag<T>((const T*)h->Wt, h->k, h->n, h->ldwt, h->sums, h->k, h->world > 1 ? 0 : 2, h->flags, st,
+                          h->topic_model);
     h->launches++;
     if (t_sums) {
-        launch_rowsum_flag<T>(Tm, h->k, h->d, h->d, h->sums, 0, 1, h->flags, st, h->km);
+        launch_rowsum_flag<T>(Tm, h->k, h->d, h->d, h->sums, 0, 1, h->flags, st, h->topic_model);
         h->launches++;
     }
     if (h->world <= 1) return 0;
@@ -1709,15 +1777,15 @@ static int objective_impl(rri_handle_t h, const T* W, const T* Tm, cudaStream_t 
         return 0;
     }
     // one explicit pass per model over its own W and T, as separate fits make it
-    const int km = h->km;
     for (int z = 0; z < h->models; ++z) {
-        const T* Wz = W + (int64_t)z * h->n * km;
-        const T* Tz = Tm + (int64_t)z * km * h->d;
+        const ModelRows& r = h->mrows[z];
+        const T* Wz = W + (int64_t)r.o * h->n;
+        const T* Tz = Tm + (int64_t)r.o * h->d;
         double* out = h->obj_out + 8 * z;
-        launch_objective<T>((const T*)h->X, h->ldx, h->M, h->mk, h->ldm, Wz, Tz, h->n, h->d, km, h->obj_part,
+        launch_objective<T>((const T*)h->X, h->ldx, h->M, h->mk, h->ldm, Wz, Tz, h->n, h->d, r.k, h->obj_part,
                             h->oblocks, out, st);
-        launch_norms<T>(Wz, h->n * km, h->obj_part, out + 2, st);
-        launch_norms<T>(Tz, (int64_t)km * h->d, h->obj_part, out + 4, st);
+        launch_norms<T>(Wz, h->n * r.k, h->obj_part, out + 2, st);
+        launch_norms<T>(Tz, (int64_t)r.k * h->d, h->obj_part, out + 4, st);
         h->launches += 6;
     }
     CKL();
@@ -1754,7 +1822,7 @@ template <typename T>
 static int objective_contraction_impl(rri_handle_t h, const T* W, const T* Tm, bool reuse, cudaStream_t st)
 {
     const int64_t n = h->n, d = h->d;
-    const int k = h->k, km = h->km, models = h->models;
+    const int k = h->k, models = h->models;
     if (!h->Gobj && ws_alloc(h, &h->Gobj, sizeof(T) * 2 * (size_t)k * k)) return 1;
     CK(cudaStreamSynchronize(0));
     double* xsq = h->obj_out + 8 * models;              // ||X||^2, then <X T', W> of every model
@@ -1777,21 +1845,23 @@ static int objective_contraction_impl(rri_handle_t h, const T* W, const T* Tm, b
     }
     const int parts = h->math == RRI_MATH_TF32 ? 1 : h->splits_w;      // (1 on zero-filled sparse handles)
     // model z: its column block of X T' against its own W
-    for (int z = 0; z < models; ++z)
-        launch_dot_parts<T>((const T*)h->Cpart + (int64_t)z * km, parts, n * k, W + (int64_t)z * n * km, n * km, h->obj_part,
-                            cross + z, h->sm_count, st, k, km);
+    for (int z = 0; z < models; ++z) {
+        const ModelRows& r = h->mrows[z];
+        launch_dot_parts<T>((const T*)h->Cpart + r.o, parts, n * k, W + (int64_t)r.o * n, n * r.k, h->obj_part,
+                            cross + z, h->sm_count, st, k, r.k);
+    }
     T* G = (T*)h->Gobj;
     T* H = G + (size_t)k * k;
-    launch_gram<T>(W, n, km, (T*)h->gram_part, h->gchunks_w, G, st, models, n * km);                 // IEEE Gram products
-    launch_gram<T>((const T*)h->Tt, d, km, (T*)h->gram_part, h->gchunks_t, H, st, models, d * km);
+    model_grams<T>(h, W, n, G, st);                     // IEEE Gram products
+    model_grams<T>(h, (const T*)h->Tt, d, H, st);
     for (int z = 0; z < models; ++z) {
+        const ModelRows& r = h->mrows[z];
         double* out = h->obj_out + 8 * z;
-        const size_t g = (size_t)z * km * km;
-        launch_objective_identity<T>(G + g, H + g, km, xsq, cross + z, out, st);
-        launch_norms<T>(W + (int64_t)z * n * km, n * km, h->obj_part, out + 2, st);
-        launch_norms<T>(Tm + (int64_t)z * km * d, (int64_t)km * d, h->obj_part, out + 4, st);
+        launch_objective_identity<T>(G + r.q, H + r.q, r.k, xsq, cross + z, out, st);
+        launch_norms<T>(W + (int64_t)r.o * n, n * r.k, h->obj_part, out + 2, st);
+        launch_norms<T>(Tm + (int64_t)r.o * d, (int64_t)r.k * d, h->obj_part, out + 4, st);
     }
-    h->launches += 4 + 7 * models;
+    h->launches += 7 * models;
     CKL();
     return 0;
 }

@@ -999,7 +999,11 @@ void launch_update_rows(T* F, int64_t m, int k, const T* Cpart, int parts, int64
     {
         static const bool reg_off = [] { const char* e = getenv("RRI_UPDATE_REG"); return e && *e == '0'; }();
         constexpr int VN = Vec<T>::N;
-        if (!reg_off && parts == 1 && !srcs && Ft && (k % VN) == 0 && (rb.ldc % VN) == 0 && k <= (sizeof(T) == 4 ? 128 : 64)) {
+        // (16-byte loads of the factor and contraction rows: F and Cpart point at a model of a handle of several, which
+        // need not start on a 16-byte boundary; such a model takes the staged kernel, which gives the same bits)
+        const bool vec = (k % VN) == 0 && (rb.ldc % VN) == 0 && (reinterpret_cast<uintptr_t>(F) & 15) == 0 &&
+                         (reinterpret_cast<uintptr_t>(Cpart) & 15) == 0;
+        if (!reg_off && parts == 1 && !srcs && Ft && vec && k <= (sizeof(T) == 4 ? 128 : 64)) {
             if (k <= 16) launch_update_rows_reg<T, 16>(F, m, k, Cpart, S, a, Ft, ldft, flags, co, rb, st);
             else if (k <= 32) launch_update_rows_reg<T, 32>(F, m, k, Cpart, S, a, Ft, ldft, flags, co, rb, st);
             else if (k <= 64) launch_update_rows_reg<T, 64>(F, m, k, Cpart, S, a, Ft, ldft, flags, co, rb, st);

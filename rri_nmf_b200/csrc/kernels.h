@@ -191,10 +191,10 @@ template <typename T>
 void launch_vec_sum_flag(const T* v, int64_t len, int64_t stride, double* sums, int slot, int zero_flag,
                          int* flags, cudaStream_t st);
 // sums[slot0 + r] = sum of row r of A[rows, ld] over len elements; zero / non-finite flags (one launch per sweep).
-// flag_rows > 0: row r raises its flags in word flags[r / flag_rows] (one word per model of flag_rows topics)
+// topic_model (optional, device [rows]): row r raises its flags in word flags[topic_model[r]] (the model owning it)
 template <typename T>
 void launch_rowsum_flag(const T* A, int rows, int64_t len, int64_t ld, double* sums, int slot0, int zero_flag,
-                        int* flags, cudaStream_t st, int flag_rows = 0);
+                        int* flags, cudaStream_t st, const int* topic_model = nullptr);
 // v[i*stride] *= scale / sums[slot]   (vector-c branch with a sum constraint, optimization.py:85-87)
 template <typename T>
 void launch_vec_scale_to_sum(T* v, int64_t len, int64_t stride, const double* sums, int slot, double s,

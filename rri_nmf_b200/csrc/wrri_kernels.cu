@@ -284,7 +284,7 @@ void launch_vec_sum_flag(const T* v, int64_t len, int64_t stride, double* sums, 
 template <typename T>
 __global__ void __launch_bounds__(1024)
 rowsum_flag_kernel(const T* __restrict__ A, int64_t len, int64_t ld, double* __restrict__ sums, int slot0,
-                   int zero_flag, int* __restrict__ flags, int flag_rows)
+                   int zero_flag, int* __restrict__ flags, const int* __restrict__ topic_model)
 {
     __shared__ double red[32];
     const T* __restrict__ v = A + (int64_t)blockIdx.x * ld;
@@ -297,7 +297,7 @@ rowsum_flag_kernel(const T* __restrict__ A, int64_t len, int64_t ld, double* __r
         double tot = 0.0;
         for (int w = 0; w < (int)(blockDim.x >> 5); ++w) tot += red[w];
         sums[slot0 + blockIdx.x] = tot;
-        int* f = flag_rows > 0 ? flags + blockIdx.x / flag_rows : flags;
+        int* f = topic_model ? flags + topic_model[blockIdx.x] : flags;
         if (zero_flag && !(tot > 1e-10)) atomicOr(f, zero_flag);
         if (!isfinite(tot)) atomicOr(f, 8);
     }
@@ -305,9 +305,9 @@ rowsum_flag_kernel(const T* __restrict__ A, int64_t len, int64_t ld, double* __r
 
 template <typename T>
 void launch_rowsum_flag(const T* A, int rows, int64_t len, int64_t ld, double* sums, int slot0, int zero_flag,
-                        int* flags, cudaStream_t st, int flag_rows)
+                        int* flags, cudaStream_t st, const int* topic_model)
 {
-    if (rows > 0) rowsum_flag_kernel<T><<<rows, 1024, 0, st>>>(A, len, ld, sums, slot0, zero_flag, flags, flag_rows);
+    if (rows > 0) rowsum_flag_kernel<T><<<rows, 1024, 0, st>>>(A, len, ld, sums, slot0, zero_flag, flags, topic_model);
 }
 
 template <typename T>
@@ -578,7 +578,8 @@ void launch_objective_identity(const T* G, const T* H, int k, const double* xsq,
     template void launch_wrri_final<T>(const T*, const T*, int, int64_t, const SolveArgs&, T*, int64_t,     \
                                        T*, int64_t, int*, cudaStream_t);                                    \
     template void launch_vec_sum_flag<T>(const T*, int64_t, int64_t, double*, int, int, int*, cudaStream_t);\
-    template void launch_rowsum_flag<T>(const T*, int, int64_t, int64_t, double*, int, int, int*, cudaStream_t, int);\
+    template void launch_rowsum_flag<T>(const T*, int, int64_t, int64_t, double*, int, int, int*, cudaStream_t, \
+                                        const int*);                                                        \
     template void launch_vec_scale_to_sum<T>(T*, int64_t, int64_t, const double*, int, double, cudaStream_t);\
     template void launch_objective<T>(const T*, int64_t, const void*, int, int64_t, const T*, const T*,     \
                                       int64_t, int64_t, int, double*, int, double*, cudaStream_t);          \

@@ -63,6 +63,11 @@ class RRIEngine(object):
            order='hals', one GPU, b * k <= 256).  Every block-order half-step contracts X once against the factors of
            all b models.  The factors are then W [b, n, k] and T [b, k, d]; `sweeps` returns b flag words,
            `topic_sums` two [b, k] arrays and `objective_terms` a [b, 6] array.
+    k may also be a sequence of ranks (k_0, ..., k_{b-1}), sum <= 256, with models=None: b models of different ranks on
+           one binding (rri_set_model_ranks; same conditions as `models`).  W is then one flat buffer of n * sum(k)
+           elements and T the stacked [sum(k), d] matrix (`pack` makes them, `views` splits them into the per-model
+           [n, k_z] / [k_z, d] views); `sweeps` returns b flag words, `topic_sums` two lists of b arrays,
+           `objective_terms` a [b, 6] array.
     """
 
     def __init__(self, X, k, W_mat=None, order='rri', math='ieee', comm=None, unstored='missing', models=None):
@@ -88,11 +93,23 @@ class RRIEngine(object):
         self.lib = _lib.load()
         self.X = X
         self.n, self.d = int(X.shape[0]), int(X.shape[1])
-        self.k = int(k)
+        self.ranks = None
+        if isinstance(k, (list, tuple)):
+            if models is not None:
+                raise ValueError('models must be None when k is a sequence of ranks')
+            self.ranks = tuple(int(r) for r in k)
+            if not self.ranks:
+                raise ValueError('k must hold at least one rank')
+            models = len(self.ranks)
+            width = sum(self.ranks)
+            self.k = width
+        else:
+            self.k = int(k)
         self.models = None if models is None else int(models)
         if self.models is not None and self.models < 1:
             raise ValueError('models must be >= 1')
-        width = self.k * (self.models or 1)
+        if self.ranks is None:
+            width = self.k * (self.models or 1)
         self.dtype = X.dtype
         self.device = X.device
         self.order = order
@@ -112,7 +129,9 @@ class RRIEngine(object):
         if comm is not None and comm.world > 1:
             path = comm.nccl_path.encode() if comm.nccl_path else None
             check(self.lib.rri_set_comm(self.h, comm.comm, comm.rank, comm.world, path))
-        if self.models is not None:
+        if self.ranks is not None:
+            check(self.lib.rri_set_model_ranks(self.h, self.models, (C.c_int32 * self.models)(*self.ranks)))
+        elif self.models is not None:
             check(self.lib.rri_set_models(self.h, self.models))
         if self.sparse:
             self._bind_csr(X, W_mat)
@@ -251,8 +270,27 @@ class RRIEngine(object):
         p.sp_refresh_every = int(sp_refresh_every)
         return p
 
+    def pack(self, Ws, Ts):
+        """Ranks engine: the flat W (n * sum(k)) and the stacked T [sum(k), d] of per-model [n, k_z] / [k_z, d]
+        factors (torch tensors of the engine's dtype and device)."""
+        if len(Ws) != self.models or len(Ts) != self.models:
+            raise ValueError('one W and one T per model')
+        return (torch.cat([w.reshape(-1) for w in Ws]).contiguous(), torch.cat(list(Ts), 0).contiguous())
+
+    def views(self, W, T):
+        """Ranks engine: the per-model views [n, k_z] of the flat W and [k_z, d] of the stacked T."""
+        Wv, Tv, o = [], [], 0
+        for r in self.ranks:
+            Wv.append(W[self.n * o:self.n * (o + r)].view(self.n, r))
+            Tv.append(T[o:o + r])
+            o += r
+        return Wv, Tv
+
     def _check_factors(self, W, T):
-        if self.models is not None:
+        if self.ranks is not None:
+            if tuple(W.shape) != (self.n * self.k,) or tuple(T.shape) != (self.k, self.d):
+                raise ValueError('W must be flat of n*sum(k) elements and T must be sum(k)*d')
+        elif self.models is not None:
             b = self.models
             if tuple(W.shape) != (b, self.n, self.k) or tuple(T.shape) != (b, self.k, self.d):
                 raise ValueError('W must be models*n*k and T must be models*k*d')
@@ -281,10 +319,13 @@ class RRIEngine(object):
         return int(flags.value)
 
     def topic_sums(self):
-        width = self.k * (self.models or 1)
+        width = self.k * (self.models or 1) if self.ranks is None else self.k
         sT = (C.c_double * width)()
         sW = (C.c_double * width)()
         check(self.lib.rri_topic_sums(self.h, sT, sW, self._stream()))
+        if self.ranks is not None:
+            cut = np.cumsum(self.ranks)[:-1]
+            return np.split(np.array(sT[:]), cut), np.split(np.array(sW[:]), cut)
         if self.models is not None:
             return np.array(sT[:]).reshape(self.models, self.k), np.array(sW[:]).reshape(self.models, self.k)
         return np.array(sT[:]), np.array(sW[:])

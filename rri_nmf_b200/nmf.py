@@ -472,6 +472,23 @@ def _model_groups(n_models, k, cap=None):
     return [min(per, n_models - i) for i in range(0, n_models, per)]
 
 
+def _rank_groups(ranks, cap=None):
+    """the groups (lists of model indices, each in caller order) that models of the given ranks run in: first fit by
+    decreasing rank (ties in caller order) under the width cap"""
+    cap = MODELS_WIDTH_CAP if cap is None else cap
+    groups, widths = [], []
+    for m in sorted(range(len(ranks)), key=lambda m: -ranks[m]):
+        for g in range(len(groups)):
+            if widths[g] + ranks[m] <= cap:
+                groups[g].append(m)
+                widths[g] += ranks[m]
+                break
+        else:
+            groups.append([m])
+            widths.append(ranks[m])
+    return [sorted(g) for g in groups]
+
+
 def nmf_models(X, k, random_state=None, W_in=None, T_in=None, **kwargs):
     """Several block-order factorisations of one matrix, X ~ W_m T_m for m = 0..b-1, sharing every pass over X.
 
@@ -489,7 +506,12 @@ def nmf_models(X, k, random_state=None, W_in=None, T_in=None, **kwargs):
     Each model stops on its own (the stopping rule of nmf() on its own objective history); the batch sweeps on until all
     have stopped or max_iter is reached.  A model whose sweep fails (an emptied topic, an unbounded objective,
     non-finite values) gets the dict {'error': <the exception nmf() would raise>, 'random_state': ...} and no factors;
-    its factors are zeroed on the device and the others carry on.  With math='ieee' every model is bit-identical to its
+    its factors are zeroed on the device and the others carry on.
+
+    k may also be a sequence of ranks, one per model (choosing k: fit k = 2..20 in one call).  The lists given must then
+    have its length (they may all be omitted: every model takes the time-based seed nmf() would take), W_in[m] is
+    n x k[m], and the models run in groups of total width <= MODELS_WIDTH_CAP, packed first fit by decreasing rank; the
+    results come back in the order of k.  With math='ieee' every model is bit-identical to its
     own nmf() run; with math='tf32' the models share the contraction's operand (and, with 16-bit copies of X, its
     power-of-two scale), which changes their rounding, not their accuracy.  The flags are read after every engine
     call: a model that produces non-finite values inside a call of several sweeps (sweeps_per_call) can disturb that
@@ -500,7 +522,7 @@ def nmf_models(X, k, random_state=None, W_in=None, T_in=None, **kwargs):
     eps_stop, max_iter, max_time, sweeps_per_call, init_on_device, device.  Everything else raises before any device
     work: NotImplementedError for W_mat, sparse X, comm, update_order='rri', fix_W / fix_T, project_T_each_iter with
     t_row_sum, early_stop, diagnostics, w_row, the Gaussian mechanism, store_gradients, an engine, and
-    return_reconstruction_err; ValueError for lists of different lengths and for k > 256.
+    return_reconstruction_err; ValueError for lists of different lengths and for ranks outside [1, 256].
     """
     import inspect
     defaults = {name: p.default for name, p in inspect.signature(nmf).parameters.items()
@@ -550,18 +572,30 @@ def nmf_models(X, k, random_state=None, W_in=None, T_in=None, **kwargs):
         raise ValueError("math must be 'ieee' or 'tf32'")
     if a['objective'] not in ('auto', 'exact', 'contraction'):
         raise ValueError("objective must be 'auto', 'exact' or 'contraction'")
-    k = int(k)
-    if k < 1 or k > 256:
-        raise ValueError('k must be in [1, 256] (got %d)' % k)
+    rank_list = isinstance(k, (list, tuple, np.ndarray))
+    ks = [int(r) for r in k] if rank_list else [int(k)]
+    for r in ks:
+        if r < 1 or r > 256:
+            raise ValueError('k must be in [1, 256] (got %d)' % r)
     lists = {name: v for name, v in (('random_state', random_state), ('W_in', W_in), ('T_in', T_in)) if v is not None}
-    if not lists:
+    if not lists and not rank_list:
         raise ValueError('nmf_models needs a list of random_state seeds and/or lists W_in, T_in (one entry per model)')
     lengths = {name: len(v) for name, v in lists.items()}
+    if rank_list:
+        lengths['k'] = len(ks)
     if len(set(lengths.values())) != 1:
         raise ValueError('random_state, W_in and T_in must have one entry per model (lengths %s)' % lengths)
     b = next(iter(lengths.values()))
     if b < 1:
         raise ValueError('nmf_models needs at least one model')
+    if not rank_list:
+        ks = ks * b
+    if rank_list:                           # (each start must have its model's rank)
+        for m in range(b):
+            if W_in is not None and not _is_empty(W_in[m]) and tuple(np.shape(W_in[m])) != (X.shape[0], ks[m]):
+                raise ValueError('W_in[%d] must be n x k[%d] = %d x %d' % (m, m, X.shape[0], ks[m]))
+            if T_in is not None and not _is_empty(T_in[m]) and tuple(np.shape(T_in[m])) != (ks[m], X.shape[1]):
+                raise ValueError('T_in[%d] must be k[%d] x d = %d x %d' % (m, m, ks[m], X.shape[1]))
     seeds = list(random_state) if random_state is not None else [None] * b
     W_ins = list(W_in) if W_in is not None else [[]] * b
     T_ins = list(T_in) if T_in is not None else [[]] * b
@@ -574,16 +608,16 @@ def nmf_models(X, k, random_state=None, W_in=None, T_in=None, **kwargs):
         project_T = False
     if (not project_T and not a['t_row_sum']) and (a['reg_t_l1'] < 0 or a['reg_t_l2'] < 0):
         logger.error('Unbounded objective. reg_t_l1=%s, reg_t_l2=%s', a['reg_t_l1'], a['reg_t_l2'])
-        return [{'W': np.ones((n, k)), 'T': np.ones((k, d)) * 1e6, 'obj_history': [-np.inf], 'iter_cputime': [0]}
-                for _ in range(b)]
+        return [{'W': np.ones((n, r)), 'T': np.ones((r, d)) * 1e6, 'obj_history': [-np.inf], 'iter_cputime': [0]}
+                for r in ks]
     if (not a['project_W_each_iter'] and not a['w_row_sum']) and (a['reg_w_l1'] < 0 or a['reg_w_l2'] < 0):
         logger.error('Unbounded objective. reg_w_l1=%s, reg_w_l2=%s', a['reg_w_l1'], a['reg_w_l2'])
-        return [{'W': np.ones((n, k)) * 1e6, 'T': np.ones((k, d)), 'obj_history': [-np.inf], 'iter_cputime': [0]}
-                for _ in range(b)]
+        return [{'W': np.ones((n, r)) * 1e6, 'T': np.ones((r, d)), 'obj_history': [-np.inf], 'iter_cputime': [0]}
+                for r in ks]
     seeds = [int(time.time()) % 4294967296 if s is None else s for s in seeds]
     t_global_start = time.time()
     max_time = a['max_time'] - 10                                 # nmf.py:333
-    init = 'random' if n <= k else a['init']                      # nmf.py:346-347
+    inits = ['random' if n <= r else a['init'] for r in ks]       # nmf.py:346-347
     start_time = time.process_time()
     device = a['device']
     if device is None:
@@ -602,18 +636,23 @@ def nmf_models(X, k, random_state=None, W_in=None, T_in=None, **kwargs):
     numpy_io = not isinstance(X, torch.Tensor)
     w_row_sum, t_row_sum = a['w_row_sum'], a['t_row_sum']
     on_device = [_init_on_device_rule(X, n, d, W_ins[m], T_ins[m], a['init_on_device'], None) for m in range(b)]
-    starts = [_host_start(X, None, k, init, seeds[m], t_row_sum, w_row_sum, W_ins[m], T_ins[m], on_device[m])
+    starts = [_host_start(X, None, ks[m], inits[m], seeds[m], t_row_sum, w_row_sum, W_ins[m], T_ins[m], on_device[m])
               for m in range(b)]
+    if rank_list:
+        groups = _rank_groups(ks)
+    else:
+        sizes = _model_groups(b, ks[0])
+        groups = [list(range(sum(sizes[:i]), sum(sizes[:i + 1]))) for i in range(len(sizes))]
     results = [None] * b
     with torch.cuda.device(device):
         Xd = _to_device(X, device, dtype)
-        first = 0
-        for g in _model_groups(b, k):
-            idx = list(range(first, first + g))
-            first += g
-            engine = RRIEngine(Xd, k, order='hals', math=a['math'], models=g)
+        for idx in groups:
+            if rank_list:
+                engine = RRIEngine(Xd, [ks[m] for m in idx], order='hals', math=a['math'])
+            else:
+                engine = RRIEngine(Xd, ks[0], order='hals', math=a['math'], models=len(idx))
             try:
-                out = _solve_models(engine, idx, starts, on_device, seeds, init, a, start_time, t_global_start,
+                out = _solve_models(engine, idx, starts, on_device, seeds, inits, a, start_time, t_global_start,
                                     max_time, numpy_io)
             finally:
                 engine.close()
@@ -622,16 +661,25 @@ def nmf_models(X, k, random_state=None, W_in=None, T_in=None, **kwargs):
     return results
 
 
-def _solve_models(engine, idx, starts, on_device, seeds, init, a, start_time, t_global_start, max_time, numpy_io):
-    """The sweep loop of _solve for the models `idx` of one models engine, each stopping on its own."""
-    k, g = engine.k, len(idx)
+def _solve_models(engine, idx, starts, on_device, seeds, inits, a, start_time, t_global_start, max_time, numpy_io):
+    """The sweep loop of _solve for the models `idx` of one models engine (equal ranks, or a ranks engine), each
+    stopping on its own.  Wbuf, Tbuf are the engine's buffers; W[j], T[j] below are model j's views of them."""
+    g = len(idx)
     w_row_sum, t_row_sum = a['w_row_sum'], a['t_row_sum']
     regs = dict(reg_w_l1=a['reg_w_l1'], reg_w_l2=a['reg_w_l2'], reg_t_l1=a['reg_t_l1'], reg_t_l2=a['reg_t_l2'])
-    W = torch.empty((g, engine.n, k), dtype=engine.dtype, device=engine.device)
-    T = torch.empty((g, k, engine.d), dtype=engine.dtype, device=engine.device)
+    if engine.ranks is not None:
+        Wbuf = torch.empty((engine.n * engine.k,), dtype=engine.dtype, device=engine.device)
+        Tbuf = torch.empty((engine.k, engine.d), dtype=engine.dtype, device=engine.device)
+        W, T = engine.views(Wbuf, Tbuf)
+        ranks = engine.ranks
+    else:
+        Wbuf = torch.empty((g, engine.n, engine.k), dtype=engine.dtype, device=engine.device)
+        Tbuf = torch.empty((g, engine.k, engine.d), dtype=engine.dtype, device=engine.device)
+        W, T = list(Wbuf), list(Tbuf)
+        ranks = [engine.k] * g
     for j, m in enumerate(idx):
-        Wj, Tj = _device_start(engine, engine.X, None, None, k, init, seeds[m], t_row_sum, w_row_sum, starts[m][0],
-                               starts[m][1], on_device[m], {})
+        Wj, Tj = _device_start(engine, engine.X, None, None, ranks[j], inits[m], seeds[m], t_row_sum, w_row_sum,
+                               starts[m][0], starts[m][1], on_device[m], {})
         W[j].copy_(Wj)
         T[j].copy_(Tj)
         del Wj, Tj
@@ -653,7 +701,7 @@ def _solve_models(engine, idx, starts, on_device, seeds, init, a, start_time, t_
     iter_no, max_iter = 0, a['max_iter']
     while iter_no < max_iter and any(active):
         ns = min(chunk, max_iter - iter_no)
-        flags = engine.sweeps(W, T, ns, params, want_flags=True)
+        flags = engine.sweeps(Wbuf, Tbuf, ns, params, want_flags=True)
         sums = []
 
         def topic_sums(j):
@@ -679,7 +727,7 @@ def _solve_models(engine, idx, starts, on_device, seeds, init, a, start_time, t_
                 if active[j]:
                     engine.project_rows_simplex(W[j], w_row_sum)
         if compute_obj:                                                           # nmf.py:488-489
-            objs = engine.objective(W, T, via_contraction=via_contraction, reuse_last_sweep=not project_W, **regs)
+            objs = engine.objective(Wbuf, Tbuf, via_contraction=via_contraction, reuse_last_sweep=not project_W, **regs)
         now = time.process_time()
         for j in range(g):
             if active[j]:
