@@ -139,6 +139,20 @@ int rri_x_operand_bits(rri_handle_t h, int32_t* bits);
 int rri_bind_csr(rri_handle_t h, int64_t nnz, const int64_t* rowptr_dev, const int32_t* col_dev,
                  const void* val_dev, const void* weight_dev, void* stream);
 
+/* Weight w0 of the UNSTORED entries of an observed-entries binding (implicit feedback, one-class recommenders;
+ * DESIGN.md §1 f7): call after rri_create and before rri_bind_csr.  The handle then fits
+ *     0.5 sum_{all i,j} M_ij (X - W T)_ij^2,   M = w0 at every unstored entry (where X is 0), the entry weight (or 1)
+ *                                              at every stored one,
+ * i.e. the dense masked problem of nmf.py:687-701 / :735-746 with that M, without any n x d object: the residual
+ * copies hold the shifted residual (m - w0) E + w0 x at the stored entries (the same bytes per entry as w0 = 0) and
+ * each half-step adds the rank-k part -w0 sum_{s!=t} G_ts F_s, +w0 G_tt from one Gram row G_t. of its topic.
+ * w0 must be finite and >= 0; 0 is the plain observed-entries handle (same launches, same bits).  With w0 > 0:
+ * rri_sweeps (both orders, fix_T), rri_topics, rri_objective (<W'W, T T'> in fp64), rri_topic_sums, rri_spmm (which
+ * keeps applying the stored entry weights, not m - w0), rri_stats and rri_profile_kernel serve the handle;
+ * rri_bind, rri_bind_csr_zero, rri_set_models / rri_set_model_ranks, rri_set_comm with world > 1 and rri_partials_T
+ * refuse it. */
+int rri_set_unstored_weight(rri_handle_t h, double w0);
+
 /* Zero-filled sparse binding: the CSR matrix is an ordinary non-negative matrix stored sparsely (a tf-idf
  * document-term matrix); every entry is fitted, the unstored ones as 0.  Same CSR contract as rri_bind_csr
  * (int64 rowptr, int32 strictly ascending columns, nnz < 2^31, the three arrays stay alive while the handle is

@@ -1,5 +1,6 @@
 // api.cu -- C-ABI (include/rri_b200.h) and sweep orchestration of the B200-native RRI engine.
 #include <dlfcn.h>
+#include <math.h>
 #include <stdarg.h>
 #include <stdio.h>
 #include <string.h>
@@ -194,6 +195,13 @@ struct rri_handle_s {
     bool sp_refresh_v2 = true;         // residual restart: row copy from the factors, column copy gathered from it
     bool sp_batched_sums = true;       // per-topic sums once per sweep (2 launches) instead of once per half-step (2k)
     int* sp_err = nullptr;
+    // unstored weight (rri_set_unstored_weight): the copies hold the shifted residual S = (m - w0) E + w0 x, and every
+    // half-step adds the rank-k part of the statistic from one Gram row of its topic
+    double sp_w0 = 0.0;
+    void* sp_gpart = nullptr;          // [max(gc_w, gc_t)][k] Gram-row partials of one half-step
+    int sp_gc_w = 1, sp_gc_t = 1;      // their chunks over the rows of W (T-steps) / the columns of T (W-steps)
+    double* sp_gobj = nullptr;         // [k][oc_w][k] + [k][oc_t][k] fp64 Gram partials of the objective
+    int sp_oc_w = 1, sp_oc_t = 1;
     // zero-filled sparse binding (rri_bind_csr_zero): the rows and the columns with their chunk plans; the block-order
     // half-steps take X T' / X' W from launch_spmm instead of the dense contraction
     bool zero_csr = false;
@@ -291,6 +299,7 @@ extern "C" int rri_set_comm(rri_handle_t h, void* nccl_comm, int32_t rank, int32
 {
     if (!h) return fail("null handle");
     if (world > 1 && h->models > 1) return fail("a handle of several models runs on one GPU (world == 1)");
+    if (world > 1 && h->sp_w0 > 0) return fail("a handle with an unstored weight runs on one GPU (world == 1)");
     if (world > 1) {
         if (!nccl_comm) return fail("world > 1 needs a communicator");
         if (nccl_load(nccl_lib_path)) return 1;
@@ -667,6 +676,7 @@ extern "C" int rri_set_model_ranks(rri_handle_t h, int32_t models, const int32_t
     if (models < 1) return fail("models must be >= 1 (got %d)", models);
     if (h->order != RRI_ORDER_HALS) return fail("several models per handle need RRI_ORDER_HALS");
     if (h->world != 1) return fail("several models per handle run on one GPU (world == 1)");
+    if (h->sp_w0 > 0) return fail("several models per handle take dense data; this handle has an unstored weight");
     if (models > h->k) return fail("models (%d) must be <= k (%d)", models, h->k);
     if (!ranks) return fail("ranks is null");
     std::vector<ModelRows> mr((size_t)models);
@@ -722,6 +732,7 @@ extern "C" int rri_bind(rri_handle_t h, const void* X_dev, int64_t ldX, const vo
     if (mask_kind < 0 || mask_kind > 2) return fail("bad mask kind %d", mask_kind);
     if (h->sparse) return fail("this handle is bound to observed-entries (CSR) data; create a new one for dense data");
     if (h->zero_csr) return fail("this handle is bound to zero-filled sparse (CSR) data; create a new one for dense data");
+    if (h->sp_w0 > 0) return fail("an unstored weight applies to observed-entries data (rri_bind_csr), not to dense data");
     if (h->X && ((h->mk != MK_NONE) != (mask_kind != RRI_MASK_NONE)))
         return fail("a handle cannot switch between masked and unmasked data; create a new one");
     if (h->models > 1 && mask_kind != RRI_MASK_NONE) return fail("a handle of several models takes unmasked data");
@@ -753,7 +764,19 @@ static int bind_csr_impl(rri_handle_t h, const int64_t* rowptr, const int32_t* c
     const int64_t m = n > d ? n : d;
     const size_t ne = (size_t)(nnz > 0 ? nnz : 1);
     void *E_csr = nullptr, *E_csc = nullptr, *x_csc = nullptr, *w_csc = nullptr, *csc_row = nullptr, *colptr = nullptr;
-    if (ws_alloc(h, (void**)&h->obj_part, sizeof(double) * 2 * 256) || ws_alloc(h, (void**)&h->obj_out, sizeof(double) * 8)) return 1;
+    if (ws_alloc(h, (void**)&h->obj_part, sizeof(double) * (h->sp_w0 > 0 ? 3 : 2) * 256) ||
+        ws_alloc(h, (void**)&h->obj_out, sizeof(double) * 8))
+        return 1;
+    if (h->sp_w0 > 0) {
+        h->sp_gc_w = sp_gram_chunks(n, k, h->sm_count);
+        h->sp_gc_t = sp_gram_chunks(d, k, h->sm_count);
+        h->sp_oc_w = sp_gram_chunks(n, k * k, h->sm_count);
+        h->sp_oc_t = sp_gram_chunks(d, k * k, h->sm_count);
+        const int gc = h->sp_gc_w > h->sp_gc_t ? h->sp_gc_w : h->sp_gc_t;
+        if (ws_alloc(h, &h->sp_gpart, es * (size_t)gc * k) ||
+            ws_alloc(h, (void**)&h->sp_gobj, sizeof(double) * (size_t)k * k * (h->sp_oc_w + h->sp_oc_t)))
+            return 1;
+    }
     if (ws_alloc(h, &E_csr, es * ne) || ws_alloc(h, &E_csc, es * ne) || ws_alloc(h, &x_csc, es * ne)) return 1;
     if (wgt && ws_alloc(h, &w_csc, es * ne)) return 1;
     if (ws_alloc(h, &csc_row, sizeof(int32_t) * ne) || ws_alloc(h, &colptr, sizeof(int64_t) * (size_t)(d + 1))) return 1;
@@ -816,6 +839,17 @@ static int bind_csr_impl(rri_handle_t h, const int64_t* rowptr, const int32_t* c
     CK(cudaStreamSynchronize(0));
     CKL();
     CK(cudaStreamSynchronize(st));
+    return 0;
+}
+
+extern "C" int rri_set_unstored_weight(rri_handle_t h, double w0)
+{
+    if (!h) return fail("null handle");
+    if (h->X) return fail("rri_set_unstored_weight must be called before rri_bind_csr");
+    if (!isfinite(w0) || w0 < 0) return fail("the unstored weight must be finite and >= 0 (got %g)", w0);
+    if (w0 > 0 && h->models > 1) return fail("a handle of several models takes no unstored weight");
+    if (w0 > 0 && h->world > 1) return fail("an unstored weight is served on one GPU (world == 1)");
+    h->sp_w0 = w0;
     return 0;
 }
 
@@ -936,6 +970,8 @@ extern "C" int rri_bind_csr_zero(rri_handle_t h, int64_t nnz, const int64_t* row
     if (!h) return fail("null handle");
     if (h->X) return fail("the handle is already bound; create a new one");
     if (h->models > 1) return fail("a handle of several models takes dense data (rri_bind)");
+    if (h->sp_w0 > 0)
+        return fail("a zero-filled binding gives every unstored entry weight 1; an unstored weight needs rri_bind_csr");
     if (nnz < 0 || nnz >= ((int64_t)1 << 31)) return fail("nnz must be in [0, 2^31) (got %lld)", (long long)nnz);
     if (!rowptr_dev) return fail("rowptr is null");
     if (nnz > 0 && (!col_dev || !val_dev)) return fail("col/val is null");
@@ -1455,12 +1491,14 @@ struct SpState {
 };
 
 template <typename T>
-static void sp_refresh(rri_handle_t h, bool need_csr, bool need_csc, const T* W, cudaStream_t st)
+static void sp_refresh(rri_handle_t h, bool need_csr, bool need_csc, const T* W, cudaStream_t st, bool plain = false)
 {
-    // E = X - W T on the observed entries, from the current factors
+    // E = X - W T on the observed entries, from the current factors (with an unstored weight, unless `plain`: the
+    // shifted residual (m - w0) E + w0 x)
+    const double w0 = plain ? 0.0 : h->sp_w0;
     if (h->sp_refresh_v2) {
         // the row copy from the factors (16-byte gathers of T' rows), the column copy as a permutation of it
-        launch_sp_residual_rows<T>(h->csr, W, h->k, (const T*)h->Tt, h->sp_ldt, h->k, h->sm_count, st);
+        launch_sp_residual_rows<T>(h->csr, W, h->k, (const T*)h->Tt, h->sp_ldt, h->k, w0, h->sm_count, st);
         h->launches++;
         if (need_csc && h->nnz > 0) {
             launch_sp_gather<T>(h->sp_perm, (const T*)h->csr.E, (T*)h->csc.E, h->nnz, h->sm_count, st);
@@ -1468,8 +1506,8 @@ static void sp_refresh(rri_handle_t h, bool need_csr, bool need_csc, const T* W,
         }
         return;
     }
-    if (need_csc) { launch_sp_residual<T>(h->csc, (const T*)h->Tt, W, h->k, h->sm_count, st); h->launches++; }
-    if (need_csr) { launch_sp_residual<T>(h->csr, W, (const T*)h->Tt, h->k, h->sm_count, st); h->launches++; }
+    if (need_csc) { launch_sp_residual<T>(h->csc, (const T*)h->Tt, W, h->k, w0, h->sm_count, st); h->launches++; }
+    if (need_csr) { launch_sp_residual<T>(h->csr, W, (const T*)h->Tt, h->k, w0, h->sm_count, st); h->launches++; }
 }
 
 template <typename T>
@@ -1483,17 +1521,25 @@ static int sp_T_step(rri_handle_t h, T* W, T* Tm, int t, const rri_params_t* p, 
     launch_sp_pack<T>((const T*)S.csc.wo, (const T*)S.csc.wn, wt, wt, h->sp_quad, n, st);
     const T* nu = (const T*)h->sp_npart; const T* de = (const T*)h->sp_dpart;
     int parts = launch_sp_pass<T>(h->csc, h->sp_quad, (const T*)S.csc.to, (const T*)S.csc.tn, trow, told, (T*)h->sp_npart,
-                                  (T*)h->sp_dpart, h->sm_count, st);
+                                  (T*)h->sp_dpart, h->sp_w0, h->sm_count, st);
     h->launches += 2;
-    if (h->world > 1) {
-        launch_reduce_parts<T>(nu, parts, d, d, ms, st);
-        launch_reduce_parts<T>(de, parts, d, d, ms + d, st);
+    if (h->sp_w0 > 0) {
+        // g = w_t' W (one row of W'W), then the solve with  -w0 sum_{s!=t} g_s T[s,:]  and  +w0 g_t  (world == 1 here)
+        launch_sp_gram_rows<T, T>((const T*)h->Wt, h->ldwt, n, h->k, t, 1, h->sp_gc_w, (T*)h->sp_gpart, st);
+        launch_sp_implicit_final<T>(nu, de, parts, d, (const T*)h->sp_gpart, h->sp_gc_w, h->k, t, Tm, d, h->sp_w0,
+                                    solve_args(p, true), trow, 1, (T*)h->Tt + t, h->sp_ldt, h->flags, st);
         h->launches += 2;
-        if (allreduce(h, ms, (size_t)2 * d, st)) return 1;
-        nu = ms; de = ms + d; parts = 1;
+    } else {
+        if (h->world > 1) {
+            launch_reduce_parts<T>(nu, parts, d, d, ms, st);
+            launch_reduce_parts<T>(de, parts, d, d, ms + d, st);
+            h->launches += 2;
+            if (allreduce(h, ms, (size_t)2 * d, st)) return 1;
+            nu = ms; de = ms + d; parts = 1;
+        }
+        launch_wrri_final<T>(nu, de, parts, d, solve_args(p, true), trow, 1, (T*)h->Tt + t, h->sp_ldt, h->flags, st);
+        h->launches++;
     }
-    launch_wrri_final<T>(nu, de, parts, d, solve_args(p, true), trow, 1, (T*)h->Tt + t, h->sp_ldt, h->flags, st);
-    h->launches++;
     if (!h->sp_batched_sums || p->simplex_T) {
         launch_vec_sum_flag<T>(trow, d, 1, h->sums, t, p->simplex_T ? 0 : 1, h->flags, st);
         h->launches++;
@@ -1515,9 +1561,18 @@ static int sp_W_step(rri_handle_t h, T* W, T* Tm, int t, const rri_params_t* p, 
     T* wold = (T*)h->sp_wold + (int64_t)(S.cw & 1) * n;
     launch_sp_pack<T>((const T*)S.csr.to, (const T*)S.csr.tn, told, trow, h->sp_quad, d, st);
     const int parts = launch_sp_pass<T>(h->csr, h->sp_quad, (const T*)S.csr.wo, (const T*)S.csr.wn, wt, wold,
-                                        (T*)h->sp_npart, (T*)h->sp_dpart, h->sm_count, st);
-    launch_wrri_final<T>((const T*)h->sp_npart, (const T*)h->sp_dpart, parts, n, solve_args(p, false), W + t, h->k, wt, 1,
-                         h->flags, st);
+                                        (T*)h->sp_npart, (T*)h->sp_dpart, h->sp_w0, h->sm_count, st);
+    if (h->sp_w0 > 0) {
+        // h = t_t T' (one row of T T', this topic's T row already updated), then the solve with -w0 sum_{s!=t} h_s W[:,s]
+        launch_sp_gram_rows<T, T>(Tm, d, d, h->k, t, 1, h->sp_gc_t, (T*)h->sp_gpart, st);
+        launch_sp_implicit_final<T>((const T*)h->sp_npart, (const T*)h->sp_dpart, parts, n, (const T*)h->sp_gpart, h->sp_gc_t,
+                                    h->k, t, (const T*)h->Wt, h->ldwt, h->sp_w0, solve_args(p, false), W + t, h->k, wt, 1,
+                                    h->flags, st);
+        h->launches++;
+    } else {
+        launch_wrri_final<T>((const T*)h->sp_npart, (const T*)h->sp_dpart, parts, n, solve_args(p, false), W + t, h->k, wt, 1,
+                             h->flags, st);
+    }
     h->launches += 3;
     if (!h->sp_batched_sums) {
         launch_vec_sum_flag<T>(wt, n, 1, h->sums, h->k + t, h->world > 1 ? 0 : 2, h->flags, st);
@@ -1768,8 +1823,18 @@ static int objective_impl(rri_handle_t h, const T* W, const T* Tm, cudaStream_t 
     if (h->zero_csr) return objective_contraction_impl<T>(h, W, Tm, false, st);     // (no pass over n x d entries)
     if (h->sparse) {
         launch_transpose<T>(Tm, h->k, h->d, h->d, (T*)h->Tt, h->sp_ldt, st);
-        sp_refresh<T>(h, true, false, W, st);
-        launch_sp_objective<T>(h->csr, h->nnz, h->obj_part, h->obj_out, st);
+        sp_refresh<T>(h, true, false, W, st, true);
+        const int k = h->k;
+        double* gw = h->sp_gobj;
+        double* gt = gw ? gw + (size_t)k * k * h->sp_oc_w : nullptr;
+        if (h->sp_w0 > 0) {
+            // <W'W, T T'> in fp64 from the Gram partials of W' and T (no pass over the n x d entries)
+            launch_transpose<T>(W, h->n, k, k, (T*)h->Wt, h->ldwt, st);
+            launch_sp_gram_rows<T, double>((const T*)h->Wt, h->ldwt, h->n, k, 0, k, h->sp_oc_w, gw, st);
+            launch_sp_gram_rows<T, double>(Tm, h->d, h->d, k, 0, k, h->sp_oc_t, gt, st);
+            h->launches += 3;
+        }
+        launch_sp_objective<T>(h->csr, h->nnz, h->obj_part, h->obj_out, h->sp_w0, gw, h->sp_oc_w, gt, h->sp_oc_t, k, st);
         launch_norms<T>(W, h->n * h->k, h->obj_part, h->obj_out + 2, st);
         launch_norms<T>(Tm, (int64_t)h->k * h->d, h->obj_part, h->obj_out + 4, st);
         h->launches += 7;
@@ -1912,7 +1977,7 @@ static int partials_impl(rri_handle_t h, const T* W, const T* Tm, int t, T* wR, 
         const T* wt = (const T*)h->Wt + (int64_t)t * h->ldwt;
         launch_sp_pack<T>(nullptr, nullptr, wt, wt, h->sp_quad, h->n, st);
         const int parts = launch_sp_pass<T>(h->csc, h->sp_quad, nullptr, nullptr, Tm + (int64_t)t * d, (T*)h->sp_told,
-                                            (T*)h->sp_npart, (T*)h->sp_dpart, h->sm_count, st);
+                                            (T*)h->sp_npart, (T*)h->sp_dpart, 0.0, h->sm_count, st);
         launch_reduce_parts<T>((const T*)h->sp_npart, parts, d, d, wR, st);
         launch_reduce_parts<T>((const T*)h->sp_dpart, parts, d, d, nw, st);
         h->launches += 4;
@@ -1956,6 +2021,7 @@ extern "C" int rri_partials_T(rri_handle_t h, const void* W_dev, const void* T_d
     if (!h->X) return fail("rri_bind has not been called");
     if (t < 0 || t >= h->k) return fail("bad topic %d", t);
     if (h->models > 1) return fail("rri_partials_T does not serve a handle of several models");
+    if (h->sp_w0 > 0) return fail("rri_partials_T does not serve a handle with an unstored weight");
     CK(cudaSetDevice(h->device));
     cudaStream_t st = (cudaStream_t)stream;
     return h->dtype == RRI_F32

@@ -277,14 +277,15 @@ int sp_build_csc(const int64_t* rowptr, const int32_t* col, const T* x, const T*
                  int64_t nnz, int64_t* colptr, int32_t* csc_row, T* x_csc, T* w_csc, uint32_t* perm, int sm_count,
                  int* err_dev, cudaStream_t st);
 
-// s.E[p] = s.x[p] - sum_l A[seg,l] * B[s.idx[p],l]   (A: own factor rows [nseg,k], B: other factor rows [.,k])
+// s.E[p] = s.x[p] - sum_l A[seg,l] * B[s.idx[p],l]   (A: own factor rows [nseg,k], B: other factor rows [.,k]).
+// w0 > 0 (unstored weight): the shifted residual (m - w0) E + w0 x is stored instead (m = s.wgt[p], or 1).
 template <typename T>
-void launch_sp_residual(const SpSide& s, const T* A, const T* B, int k, int sm_count, cudaStream_t st);
+void launch_sp_residual(const SpSide& s, const T* A, const T* B, int k, double w0, int sm_count, cudaStream_t st);
 
 // The same for the row orientation with 16-byte gathers: B[., ldb] has a padded row stride (multiple of 16 bytes, zero
 // pad columns); A[nseg, lda] is staged per segment through shared memory.
 template <typename T>
-void launch_sp_residual_rows(const SpSide& s, const T* A, int64_t lda, const T* B, int ldb, int k, int sm_count,
+void launch_sp_residual_rows(const SpSide& s, const T* A, int64_t lda, const T* B, int ldb, int k, double w0, int sm_count,
                              cudaStream_t st);
 // dst[p] = src[perm[p]]
 template <typename T>
@@ -297,13 +298,29 @@ void launch_sp_pack(const T* po, const T* pn, const T* vold, const T* vnew, void
 // One half-step statistic over one orientation (see sparse_kernels.cu): applies the pending rank-one change
 // (own_po/own_pn null -> none), writes own_save[seg] = own_cur[seg] and `parts` slices numer[p][seg], denom[p][seg]
 // (before the regularisers; the consumer adds the slices in order).  Returns parts (1, or s.nblk when blocked).
+// w0 > 0: the copies hold the shifted residual and the sums are its stored-entry part (sparse_kernels.cu, sp_entry).
 template <typename T>
 int launch_sp_pass(const SpSide& s, const void* quad, const T* own_po, const T* own_pn, const T* own_cur,
-                    T* own_save, T* numer, T* denom, int sm_count, cudaStream_t st);
+                    T* own_save, T* numer, T* denom, double w0, int sm_count, cudaStream_t st);
 
-// out[0] = 0.5 * sum m E^2, out[1] = sum m x^2 over the observed entries (fixed-order reduction)
+// out[0] = 0.5 * sum m E^2, out[1] = sum m x^2 over the observed entries (fixed-order reduction).  w0 > 0: out[0] =
+// 0.5 (sum m E^2 + w0 (<W'W, T T'> - sum (x - E)^2)) with the fp64 Gram partials gw [k][cw][k], gt [k][ct][k] of W' and T
+// (launch_sp_gram_rows<T, double>); part then holds 3 doubles per block (<= 256 blocks)
 template <typename T>
-void launch_sp_objective(const SpSide& s, int64_t nnz, double* part, double* out, cudaStream_t st);
+void launch_sp_objective(const SpSide& s, int64_t nnz, double* part, double* out, double w0, const double* gw, int cw,
+                         const double* gt, int ct, int k, cudaStream_t st);
+
+// Unstored weight w0 > 0: Gram rows part[z][c][s] = sum_{i in chunk c of [0,len)} F[t0+z, i] F[s, i] (F [k, ld]; grid
+// k x chunks x rows), chunks = sp_gram_chunks(len, pairs of one launch, ...); A = accumulation type
+int sp_gram_chunks(int64_t len, int pairs, int sm_count);
+template <typename T, typename A>
+void launch_sp_gram_rows(const T* F, int64_t ld, int64_t len, int k, int t0, int rows, int chunks, A* part, cudaStream_t st);
+// launch_wrri_final with the dense part of the statistic: numer -= w0 sum_{s!=t} g_s F[s, i], denom += w0 g_t, g = sum of
+// the gchunks Gram-row partials gpart [gchunks][k] of topic t (k <= 256), F [k, ldf] the factor being updated
+template <typename T>
+void launch_sp_implicit_final(const T* numer_part, const T* denom_part, int parts, int64_t len, const T* gpart, int gchunks,
+                              int k, int t, const T* F, int64_t ldf, double w0, const SolveArgs& a, T* out,
+                              int64_t out_stride, T* out2, int64_t out2_stride, int* flags, cudaStream_t st);
 }  // namespace rri
 
 namespace rri {

@@ -139,11 +139,20 @@ int sp_build_csc(const int64_t* rowptr, const int32_t* col, const T* x, const T*
 // ------------------------------------------------------------------------------------------------
 // residual from scratch:  E[p] = x[p] - sum_l A[seg,l] * B[idx[p],l]
 // (CSR: A = W, B = T';  CSC: A = T', B = W -- the products commute, the sums run in the same order)
+// Shifted mode (SH): the stored value is S[p] = (m[p] - w0) E[p] + w0 x[p]  (m = 1 without entry weights).
 // ------------------------------------------------------------------------------------------------
-template <typename T, int V, int G>
+template <typename T, bool SH>
+RRI_DEVINL T sp_stored(T e, T x, const T* __restrict__ wgt, int64_t p, T w0)
+{
+    if constexpr (SH) return fma(sub_rn(wgt ? wgt[p] : T(1), w0), e, mul_rn(w0, x));
+    return e;
+}
+
+template <typename T, int V, int G, bool SH>
 __global__ void __launch_bounds__(256)
 sp_residual_kernel(const int64_t* __restrict__ ptr, const int32_t* __restrict__ idx, const T* __restrict__ x,
-                   const T* __restrict__ A, const T* __restrict__ B, int k, T* __restrict__ E, int64_t nseg)
+                   const T* __restrict__ A, const T* __restrict__ B, int k, T* __restrict__ E, int64_t nseg,
+                   const T* __restrict__ wgt, T w0)
 {
     constexpr int GPB = 256 / G;
     const int lane = threadIdx.x % G, g = threadIdx.x / G;
@@ -167,31 +176,32 @@ sp_residual_kernel(const int64_t* __restrict__ ptr, const int32_t* __restrict__ 
                     for (int v = 0; v < V; ++v) acc = fma(-x1.v[v], x2.v[v], acc);
                 }
             }
-            E[p] = acc;
+            E[p] = sp_stored<T, SH>(acc, x[p], wgt, p, w0);
         }
     }
 }
 
-template <typename T, int V>
-static void residual_dispatch(const SpSide& s, const T* A, const T* B, int k, int sm_count, cudaStream_t st)
+template <typename T, int V, bool SH>
+static void residual_dispatch(const SpSide& s, const T* A, const T* B, int k, T w0, int sm_count, cudaStream_t st)
 {
+    const T* w = (const T*)s.wgt;
     if (s.group == 256) {
-        sp_residual_kernel<T, V, 256><<<cap_blocks(s.nseg, sm_count, 8), 256, 0, st>>>(s.ptr, s.idx, (const T*)s.x, A, B, k,
-                                                                                        (T*)s.E, s.nseg);
+        sp_residual_kernel<T, V, 256, SH><<<cap_blocks(s.nseg, sm_count, 8), 256, 0, st>>>(s.ptr, s.idx, (const T*)s.x, A, B, k,
+                                                                                            (T*)s.E, s.nseg, w, w0);
     } else {
-        sp_residual_kernel<T, V, 32><<<cap_blocks((s.nseg + 7) / 8, sm_count, 8), 256, 0, st>>>(s.ptr, s.idx, (const T*)s.x, A,
-                                                                                                 B, k, (T*)s.E, s.nseg);
+        sp_residual_kernel<T, V, 32, SH><<<cap_blocks((s.nseg + 7) / 8, sm_count, 8), 256, 0, st>>>(s.ptr, s.idx, (const T*)s.x, A,
+                                                                                                     B, k, (T*)s.E, s.nseg, w, w0);
     }
 }
 
 // Row-orientation residual with the segment's own factor row staged in shared memory and the gathered rows read
 // with 16-byte loads: B has a padded row stride ldb (multiple of 16 bytes, pad columns zero), so an entry costs
 // ceil(k/V) vector loads -- half the L1 tag look-ups of the 8-byte version at k = 50 -- and the own row costs none.
-template <typename T, int G>
+template <typename T, int G, bool SH>
 __global__ void __launch_bounds__(256)
 sp_residual_rows_kernel(const int64_t* __restrict__ ptr, const int32_t* __restrict__ idx, const T* __restrict__ x,
                         const T* __restrict__ A, int64_t lda, const T* __restrict__ B, int ldb, int k,
-                        T* __restrict__ E, int64_t nseg)
+                        T* __restrict__ E, int64_t nseg, const T* __restrict__ wgt, T w0)
 {
     using V = typename Vec<T>::type;
     constexpr int VN = Vec<T>::N;
@@ -216,21 +226,31 @@ sp_residual_rows_kernel(const int64_t* __restrict__ ptr, const int32_t* __restri
 #pragma unroll
                 for (int v = 0; v < VN; ++v) acc = fma(-a[v], c[v], acc);
             }
-            E[p] = acc;
+            E[p] = sp_stored<T, SH>(acc, x[p], wgt, p, w0);
         }
     }
 }
 
+template <typename T, bool SH>
+static void residual_rows_dispatch(const SpSide& s, const T* A, int64_t lda, const T* B, int ldb, int k, T w0, int sm_count,
+                                   cudaStream_t st)
+{
+    const T* w = (const T*)s.wgt;
+    if (s.group == 256)
+        sp_residual_rows_kernel<T, 256, SH><<<cap_blocks(s.nseg, sm_count, 8), 256, 0, st>>>(s.ptr, s.idx, (const T*)s.x, A, lda, B,
+                                                                                             ldb, k, (T*)s.E, s.nseg, w, w0);
+    else
+        sp_residual_rows_kernel<T, 32, SH><<<cap_blocks((s.nseg + 7) / 8, sm_count, 8), 256, 0, st>>>(s.ptr, s.idx, (const T*)s.x, A,
+                                                                                                      lda, B, ldb, k, (T*)s.E, s.nseg,
+                                                                                                      w, w0);
+}
+
 template <typename T>
-void launch_sp_residual_rows(const SpSide& s, const T* A, int64_t lda, const T* B, int ldb, int k, int sm_count,
+void launch_sp_residual_rows(const SpSide& s, const T* A, int64_t lda, const T* B, int ldb, int k, double w0, int sm_count,
                              cudaStream_t st)
 {
-    if (s.group == 256)
-        sp_residual_rows_kernel<T, 256><<<cap_blocks(s.nseg, sm_count, 8), 256, 0, st>>>(s.ptr, s.idx, (const T*)s.x, A, lda, B,
-                                                                                         ldb, k, (T*)s.E, s.nseg);
-    else
-        sp_residual_rows_kernel<T, 32><<<cap_blocks((s.nseg + 7) / 8, sm_count, 8), 256, 0, st>>>(s.ptr, s.idx, (const T*)s.x, A,
-                                                                                                  lda, B, ldb, k, (T*)s.E, s.nseg);
+    if (w0 > 0.0) residual_rows_dispatch<T, true>(s, A, lda, B, ldb, k, (T)w0, sm_count, st);
+    else residual_rows_dispatch<T, false>(s, A, lda, B, ldb, k, T(0), sm_count, st);
 }
 
 // dst[p] = src[perm[p]]: the column copy of the residual taken from the row copy (bit-identical by construction)
@@ -261,14 +281,21 @@ void launch_sp_gather(const uint32_t* perm, const T* src, T* dst, int64_t nnz, i
 // (A variant that staged the gathered k-vectors of 32 entries through shared memory was measured slower than this
 // direct kernel -- 9.5 ms against 5.9 ms at nnz = 1e8, k = 50, profiles/r01_sparse_bench_v2_staged.log -- and was
 // removed; the shipped restart path is sp_residual_rows_kernel + sp_gather_kernel above.)
-template <typename T>
-void launch_sp_residual(const SpSide& s, const T* A, const T* B, int k, int sm_count, cudaStream_t st)
+template <typename T, bool SH>
+static void residual_vec_dispatch(const SpSide& s, const T* A, const T* B, int k, T w0, int sm_count, cudaStream_t st)
 {
     const uintptr_t al = reinterpret_cast<uintptr_t>(A) | reinterpret_cast<uintptr_t>(B);
     constexpr int VMAX = 16 / (int)sizeof(T);
-    if (VMAX == 4 && k % 4 == 0 && (al & 15) == 0) residual_dispatch<T, VMAX>(s, A, B, k, sm_count, st);
-    else if (k % 2 == 0 && (al & (2 * sizeof(T) - 1)) == 0) residual_dispatch<T, 2>(s, A, B, k, sm_count, st);
-    else residual_dispatch<T, 1>(s, A, B, k, sm_count, st);
+    if (VMAX == 4 && k % 4 == 0 && (al & 15) == 0) residual_dispatch<T, VMAX, SH>(s, A, B, k, w0, sm_count, st);
+    else if (k % 2 == 0 && (al & (2 * sizeof(T) - 1)) == 0) residual_dispatch<T, 2, SH>(s, A, B, k, w0, sm_count, st);
+    else residual_dispatch<T, 1, SH>(s, A, B, k, w0, sm_count, st);
+}
+
+template <typename T>
+void launch_sp_residual(const SpSide& s, const T* A, const T* B, int k, double w0, int sm_count, cudaStream_t st)
+{
+    if (w0 > 0.0) residual_vec_dispatch<T, true>(s, A, B, k, (T)w0, sm_count, st);
+    else residual_vec_dispatch<T, false>(s, A, B, k, T(0), sm_count, st);
 }
 
 // ------------------------------------------------------------------------------------------------
@@ -303,10 +330,30 @@ void launch_sp_pack(const T* po, const T* pn, const T* vold, const T* vnew, void
 // T-step: segments = columns, own = T[t,:], other_old = other_new = W[:,t].
 // W-step: segments = rows, own = W[:,t], other_old / other_new = T[t,:] before / after this topic's T-step.
 // ------------------------------------------------------------------------------------------------
-template <typename T, bool HASW>
+//
+// Shifted mode (SH, a handle with unstored weight w0 > 0, DESIGN.md §1 row f7): the copies hold S = mt E + w0 x with
+// mt = m - w0 (m = 1 without entry weights), so that
+//   S'      = S + mt (w_po t_po - w_pn t_pn)
+//   numer_s = sum other_new * (S' + mt own_cur other_old)     = sum other_new (mt Eh + w0 x)
+//   denom_s = sum mt other_new^2
+// and the solve adds the dense rank-k part  -w0 sum_{s!=t} G_ts own_s,  +w0 G_tt  (sp_implicit_final_kernel).
+template <typename T, bool HASW, bool SH>
 RRI_DEVINL void sp_entry(T ev, const Quad<T>& q, T m, T opo, T opn, T oc, bool apply, T* __restrict__ Eout,
-                         T& num, T& den)
+                         T& num, T& den, T w0)
 {
+    if constexpr (SH) {
+        const T mt = sub_rn(m, w0);
+        if (apply) {
+            const T a = mul_rn(q.a, opo);
+            const T b = mul_rn(q.b, opn);
+            ev = fma(mt, sub_rn(a, b), ev);
+            *Eout = ev;
+        }
+        const T eh = fma(mul_rn(mt, q.c), oc, ev);
+        num = fma(q.d, eh, num);
+        den = fma(mul_rn(mt, q.d), q.d, den);
+        return;
+    }
     if (apply) {
         const T a = mul_rn(q.a, opo);
         const T b = mul_rn(q.b, opn);
@@ -319,12 +366,12 @@ RRI_DEVINL void sp_entry(T ev, const Quad<T>& q, T m, T opo, T opn, T oc, bool a
     den = fma(wn, q.d, den);
 }
 
-template <typename T, int G, bool HASW>
+template <typename T, int G, bool HASW, bool SH>
 __global__ void __launch_bounds__(256)
 sp_pass_kernel(const int64_t* __restrict__ ptr, const int32_t* __restrict__ idx, T* __restrict__ E,
                const T* __restrict__ wgt, const Quad<T>* __restrict__ Q, const T* __restrict__ own_po,
                const T* __restrict__ own_pn, const T* __restrict__ own_cur, T* __restrict__ own_save,
-               T* __restrict__ numer, T* __restrict__ denom, int64_t nseg)
+               T* __restrict__ numer, T* __restrict__ denom, int64_t nseg, T w0)
 {
     constexpr int GPB = 256 / G;
     constexpr int U = 4;
@@ -348,11 +395,12 @@ sp_pass_kernel(const int64_t* __restrict__ ptr, const int32_t* __restrict__ idx,
 #pragma unroll
             for (int u = 0; u < U; ++u) qq[u] = Q[q[u]];
 #pragma unroll
-            for (int u = 0; u < U; ++u) sp_entry<T, HASW>(ev[u], qq[u], m[u], opo, opn, oc, apply, E + p + u * G, num, den);
+            for (int u = 0; u < U; ++u)
+                sp_entry<T, HASW, SH>(ev[u], qq[u], m[u], opo, opn, oc, apply, E + p + u * G, num, den, w0);
         }
         for (; p < e; p += G) {
             const Quad<T> qq = Q[idx[p]];
-            sp_entry<T, HASW>(E[p], qq, HASW ? wgt[p] : T(1), opo, opn, oc, apply, E + p, num, den);
+            sp_entry<T, HASW, SH>(E[p], qq, HASW ? wgt[p] : T(1), opo, opn, oc, apply, E + p, num, den, w0);
         }
         num = warp_sum(num);
         den = warp_sum(den);
@@ -378,14 +426,14 @@ sp_pass_kernel(const int64_t* __restrict__ ptr, const int32_t* __restrict__ idx,
 // stages block b of Q once and walks the sub-segments [ptr2[s][b], ptr2[s][b+1]) of its chunk c of the segments, a
 // warp per sub-segment, so every gather is a shared-memory read.  Per-block partial sums are written to
 // numer_part[b][s], denom_part[b][s] and added in block order by the solve kernel (deterministic).
-template <typename T, bool HASW, int U, int THREADS, int MINB>
+template <typename T, bool HASW, bool SH, int U, int THREADS, int MINB>
 __global__ void __launch_bounds__(THREADS, MINB)
 sp_pass_blocked_kernel(const int64_t* __restrict__ ptr2, const int32_t* __restrict__ idx,
                        const uint16_t* __restrict__ idx16, T* __restrict__ E,
                        const T* __restrict__ wgt, const Quad<T>* __restrict__ Q, const T* __restrict__ own_po,
                        const T* __restrict__ own_pn, const T* __restrict__ own_cur, T* __restrict__ own_save,
                        T* __restrict__ numer_part, T* __restrict__ denom_part, int64_t nseg, int nblk, int nb,
-                       int64_t nother, int chunks)
+                       int64_t nother, int chunks, T w0)
 {
     extern __shared__ __align__(16) unsigned char sp_smem[];
     Quad<T>* __restrict__ qs = reinterpret_cast<Quad<T>*>(sp_smem);
@@ -432,7 +480,7 @@ sp_pass_blocked_kernel(const int64_t* __restrict__ ptr2, const int32_t* __restri
             for (int u = 0; u < U; ++u)
                 if (q[u] >= 0) {
                     const Quad<T> qq = qs[q[u]];
-                    sp_entry<T, HASW>(ev[u], qq, m[u], opo, opn, oc, apply, E + p0 + u * 32, num, den);
+                    sp_entry<T, HASW, SH>(ev[u], qq, m[u], opo, opn, oc, apply, E + p0 + u * 32, num, den, w0);
                 }
         }
         num = warp_sum(num);
@@ -452,13 +500,13 @@ sp_pass_blocked_kernel(const int64_t* __restrict__ ptr2, const int32_t* __restri
 //   * trips with all 32*U entries present run without any predicate,
 //   * the remainder issues only the slots the warp needs (warp-uniform tests) -- with U = 16 almost every sub-segment
 //     of a config-4 shaped problem (~330-390 entries) is ONE batch of loads with 11-13 slots in flight per lane.
-template <typename T, bool HASW, int U, int THREADS, int MINB>
+template <typename T, bool HASW, bool SH, int U, int THREADS, int MINB>
 __global__ void __launch_bounds__(THREADS, MINB)
 sp_pass_stream_kernel(const int64_t* __restrict__ ptr2, const uint16_t* __restrict__ idx16, T* __restrict__ E,
                       const T* __restrict__ wgt, const Quad<T>* __restrict__ Q, const T* __restrict__ own_po,
                       const T* __restrict__ own_pn, const T* __restrict__ own_cur, T* __restrict__ own_save,
                       T* __restrict__ numer_part, T* __restrict__ denom_part, int64_t nseg, int nblk, int nb,
-                      int64_t nother, int chunks)
+                      int64_t nother, int chunks, T w0)
 {
     extern __shared__ __align__(16) unsigned char sp_smem[];
     Quad<T>* __restrict__ qs = reinterpret_cast<Quad<T>*>(sp_smem);
@@ -505,7 +553,7 @@ sp_pass_stream_kernel(const int64_t* __restrict__ ptr2, const uint16_t* __restri
 #pragma unroll
             for (int u = 0; u < U; ++u) {
                 const Quad<T> qq = qs[q[u]];
-                sp_entry<T, HASW>(ev[u], qq, m[u], opo, opn, oc, apply, Ep + i + 32 * u, num, den);
+                sp_entry<T, HASW, SH>(ev[u], qq, m[u], opo, opn, oc, apply, Ep + i + 32 * u, num, den, w0);
             }
         }
         const int rem = len - i;                                  // < 32 * U entries left (warp-uniform)
@@ -528,7 +576,7 @@ sp_pass_stream_kernel(const int64_t* __restrict__ ptr2, const uint16_t* __restri
             for (int u = 0; u < U; ++u)
                 if (32 * u < lrem) {
                     const Quad<T> qq = qs[q[u]];
-                    sp_entry<T, HASW>(ev[u], qq, m[u], opo, opn, oc, apply, Ep + i + 32 * u, num, den);
+                    sp_entry<T, HASW, SH>(ev[u], qq, m[u], opo, opn, oc, apply, Ep + i + 32 * u, num, den, w0);
                 }
         }
         num = warp_sum(num);
@@ -595,11 +643,10 @@ void launch_sp_subptr(const int64_t* ptr, const int32_t* idx, int64_t nseg, int 
     sp_subptr_kernel<<<cap_blocks((total + 255) / 256, sm_count, 8), 256, 0, st>>>(ptr, idx, nseg, nblk, nb, ptr2);
 }
 
-template <typename T>
-int launch_sp_pass(const SpSide& s, const void* quad, const T* own_po, const T* own_pn, const T* own_cur,
-                   T* own_save, T* numer, T* denom, int sm_count, cudaStream_t st)
+template <typename T, bool SH>
+static int sp_pass_dispatch(const SpSide& s, const Quad<T>* Q, const T* own_po, const T* own_pn, const T* own_cur,
+                            T* own_save, T* numer, T* denom, T w0, int sm_count, cudaStream_t st)
 {
-    const Quad<T>* Q = (const Quad<T>*)quad;
     const T* w = (const T*)s.wgt;
     T* E = (T*)s.E;
     if (s.ptr2) {
@@ -616,10 +663,10 @@ int launch_sp_pass(const SpSide& s, const void* quad, const T* own_po, const T* 
             if (chunks < 1) chunks = 1;
             if ((int64_t)chunks * 16 > s.nseg) chunks = (int)((s.nseg + 15) / 16);
             if (chunks < 1) chunks = 1;
-            auto kern = w ? sp_pass_blocked_kernel<T, true, U, 512, 2> : sp_pass_blocked_kernel<T, false, U, 512, 2>;
+            auto kern = w ? sp_pass_blocked_kernel<T, true, SH, U, 512, 2> : sp_pass_blocked_kernel<T, false, SH, U, 512, 2>;
             if (smem > 48 * 1024) cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, 64 * 1024);
             kern<<<(unsigned)(s.nblk * chunks), 512, smem, st>>>(s.ptr2, s.idx, s.idx16, E, w, Q, own_po, own_pn, own_cur, own_save,
-                                                                numer, denom, s.nseg, s.nblk, s.nb, s.nother, chunks);
+                                                                numer, denom, s.nseg, s.nblk, s.nb, s.nother, chunks, w0);
             return s.nblk;
         }
         if constexpr (sizeof(T) == 4) {
@@ -629,60 +676,78 @@ int launch_sp_pass(const SpSide& s, const void* quad, const T* own_po, const T* 
             static const bool stream = [] { const char* e = getenv("RRI_SP_STREAM"); return !(e && *e == '0'); }();
             if (stream && s.idx16) {
                 if (w) {
-                    auto kv = sp_pass_stream_kernel<T, true, 8, 1024, 1>;
+                    auto kv = sp_pass_stream_kernel<T, true, SH, 8, 1024, 1>;
                     if (smem > 48 * 1024) cudaFuncSetAttribute(kv, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
                     kv<<<(unsigned)(s.nblk * chunks), 1024, smem, st>>>(s.ptr2, s.idx16, E, w, Q, own_po, own_pn, own_cur, own_save,
-                                                                       numer, denom, s.nseg, s.nblk, s.nb, s.nother, chunks);
+                                                                       numer, denom, s.nseg, s.nblk, s.nb, s.nother, chunks, w0);
                 } else {
-                    auto kv = sp_pass_stream_kernel<T, false, 16, 1024, 1>;
+                    // (shifted: 12 entries per lane and batch -- 16 spill there)
+                    auto kv = sp_pass_stream_kernel<T, false, SH, SH ? 12 : 16, 1024, 1>;
                     if (smem > 48 * 1024) cudaFuncSetAttribute(kv, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
                     kv<<<(unsigned)(s.nblk * chunks), 1024, smem, st>>>(s.ptr2, s.idx16, E, w, Q, own_po, own_pn, own_cur, own_save,
-                                                                       numer, denom, s.nseg, s.nblk, s.nb, s.nother, chunks);
+                                                                       numer, denom, s.nseg, s.nblk, s.nb, s.nother, chunks, w0);
                 }
                 return s.nblk;
             }
         }
-        auto kern = w ? sp_pass_blocked_kernel<T, true, U, 1024, 1> : sp_pass_blocked_kernel<T, false, U, 1024, 1>;
+        auto kern = w ? sp_pass_blocked_kernel<T, true, SH, U, 1024, 1> : sp_pass_blocked_kernel<T, false, SH, U, 1024, 1>;
         if (smem > 48 * 1024) cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
         kern<<<(unsigned)(s.nblk * chunks), 1024, smem, st>>>(s.ptr2, s.idx, s.idx16, E, w, Q, own_po, own_pn, own_cur, own_save, numer,
-                                                             denom, s.nseg, s.nblk, s.nb, s.nother, chunks);
+                                                             denom, s.nseg, s.nblk, s.nb, s.nother, chunks, w0);
         return s.nblk;
     }
     if (s.group == 256) {
         const int nb = cap_blocks(s.nseg, sm_count, 8);
-        if (w) sp_pass_kernel<T, 256, true><<<nb, 256, 0, st>>>(s.ptr, s.idx, E, w, Q, own_po, own_pn, own_cur, own_save, numer, denom, s.nseg);
-        else   sp_pass_kernel<T, 256, false><<<nb, 256, 0, st>>>(s.ptr, s.idx, E, w, Q, own_po, own_pn, own_cur, own_save, numer, denom, s.nseg);
+        if (w) sp_pass_kernel<T, 256, true, SH><<<nb, 256, 0, st>>>(s.ptr, s.idx, E, w, Q, own_po, own_pn, own_cur, own_save, numer, denom, s.nseg, w0);
+        else   sp_pass_kernel<T, 256, false, SH><<<nb, 256, 0, st>>>(s.ptr, s.idx, E, w, Q, own_po, own_pn, own_cur, own_save, numer, denom, s.nseg, w0);
     } else {
         const int nb = cap_blocks((s.nseg + 7) / 8, sm_count, 8);
-        if (w) sp_pass_kernel<T, 32, true><<<nb, 256, 0, st>>>(s.ptr, s.idx, E, w, Q, own_po, own_pn, own_cur, own_save, numer, denom, s.nseg);
-        else   sp_pass_kernel<T, 32, false><<<nb, 256, 0, st>>>(s.ptr, s.idx, E, w, Q, own_po, own_pn, own_cur, own_save, numer, denom, s.nseg);
+        if (w) sp_pass_kernel<T, 32, true, SH><<<nb, 256, 0, st>>>(s.ptr, s.idx, E, w, Q, own_po, own_pn, own_cur, own_save, numer, denom, s.nseg, w0);
+        else   sp_pass_kernel<T, 32, false, SH><<<nb, 256, 0, st>>>(s.ptr, s.idx, E, w, Q, own_po, own_pn, own_cur, own_save, numer, denom, s.nseg, w0);
     }
     return 1;
+}
+
+template <typename T>
+int launch_sp_pass(const SpSide& s, const void* quad, const T* own_po, const T* own_pn, const T* own_cur,
+                   T* own_save, T* numer, T* denom, double w0, int sm_count, cudaStream_t st)
+{
+    const Quad<T>* Q = (const Quad<T>*)quad;
+    if (w0 > 0.0) return sp_pass_dispatch<T, true>(s, Q, own_po, own_pn, own_cur, own_save, numer, denom, (T)w0, sm_count, st);
+    return sp_pass_dispatch<T, false>(s, Q, own_po, own_pn, own_cur, own_save, numer, denom, T(0), sm_count, st);
 }
 
 // ------------------------------------------------------------------------------------------------
 // objective pieces (nmf.py:71-94 on the observed entries): out[0] = 0.5 sum m E^2, out[1] = sum m x^2
 // ------------------------------------------------------------------------------------------------
-template <typename T>
+// SH (unstored weight w0 > 0): a third sum, out of the parts only, s2 = sum (x - E)^2 = sum (W T)^2 over the stored
+// entries (the part of <W'W, T T'> that the unstored weight does not apply to)
+template <typename T, bool SH>
 __global__ void __launch_bounds__(256)
 sp_objective_kernel(const T* __restrict__ E, const T* __restrict__ x, const T* __restrict__ wgt, int64_t nnz,
                     double* __restrict__ part)
 {
-    __shared__ double red[2][8];
-    double s0 = 0.0, s1 = 0.0;
+    constexpr int NS = SH ? 3 : 2;
+    __shared__ double red[NS][8];
+    double s0 = 0.0, s1 = 0.0, s2 = 0.0;
     for (int64_t p = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; p < nnz; p += (int64_t)gridDim.x * blockDim.x) {
         const double m = wgt ? (double)wgt[p] : 1.0;
         const double r = (double)E[p], v = (double)x[p];
         s0 += m * r * r;
         s1 += m * v * v;
+        if (SH) s2 += (v - r) * (v - r);
     }
     s0 = warp_sum(s0); s1 = warp_sum(s1);
-    if ((threadIdx.x & 31) == 0) { red[0][threadIdx.x >> 5] = s0; red[1][threadIdx.x >> 5] = s1; }
+    if (SH) s2 = warp_sum(s2);
+    if ((threadIdx.x & 31) == 0) {
+        red[0][threadIdx.x >> 5] = s0; red[1][threadIdx.x >> 5] = s1;
+        if (SH) red[NS - 1][threadIdx.x >> 5] = s2;
+    }
     __syncthreads();
-    if (threadIdx.x < 2) {
+    if (threadIdx.x < NS) {
         double s = 0.0;
         for (int w = 0; w < 8; ++w) s += red[threadIdx.x][w];
-        part[2 * (int64_t)blockIdx.x + threadIdx.x] = s;
+        part[NS * (int64_t)blockIdx.x + threadIdx.x] = s;
     }
 }
 
@@ -695,27 +760,160 @@ __global__ void sp_objective_finalize_kernel(const double* __restrict__ part, in
     }
 }
 
+// out[0] = 0.5 (sum m E^2 + w0 (<W'W, T T'> - sum (x - E)^2)) = 0.5 sum M (X - W T)^2 over all n x d entries,
+// out[1] = sum m x^2; <W'W, T T'> from the fp64 Gram partials gw [k][cw][k] and gt [k][ct][k] (fixed order)
+__global__ void __launch_bounds__(256)
+sp_objective_implicit_finalize_kernel(const double* __restrict__ part, int blocks, const double* __restrict__ gw, int cw,
+                                      const double* __restrict__ gt, int ct, int k, double w0, double* __restrict__ out)
+{
+    __shared__ double red[8];
+    double gh = 0.0;
+    for (int q = threadIdx.x; q < k * k; q += blockDim.x) {
+        const int a = q / k, b = q - a * k;
+        double x = 0.0, y = 0.0;
+        for (int c = 0; c < cw; ++c) x += gw[((int64_t)a * cw + c) * k + b];
+        for (int c = 0; c < ct; ++c) y += gt[((int64_t)a * ct + c) * k + b];
+        gh += x * y;
+    }
+    gh = warp_sum(gh);
+    if ((threadIdx.x & 31) == 0) red[threadIdx.x >> 5] = gh;
+    __syncthreads();
+    if (threadIdx.x == 0) {
+        double g = 0.0, s0 = 0.0, s1 = 0.0, s2 = 0.0;
+        for (int w = 0; w < 8; ++w) g += red[w];
+        for (int b = 0; b < blocks; ++b) { s0 += part[3 * (int64_t)b]; s1 += part[3 * (int64_t)b + 1]; s2 += part[3 * (int64_t)b + 2]; }
+        out[0] = 0.5 * (s0 + w0 * (g - s2));
+        out[1] = s1;
+    }
+}
+
 template <typename T>
-void launch_sp_objective(const SpSide& s, int64_t nnz, double* part, double* out, cudaStream_t st)
+void launch_sp_objective(const SpSide& s, int64_t nnz, double* part, double* out, double w0, const double* gw, int cw,
+                         const double* gt, int ct, int k, cudaStream_t st)
 {
     int blocks = (int)((nnz + 256 * 8 - 1) / (256 * 8));
     if (blocks > 256) blocks = 256;
     if (blocks < 1) blocks = 1;
-    sp_objective_kernel<T><<<blocks, 256, 0, st>>>((const T*)s.E, (const T*)s.x, (const T*)s.wgt, nnz, part);
+    if (w0 > 0.0) {
+        sp_objective_kernel<T, true><<<blocks, 256, 0, st>>>((const T*)s.E, (const T*)s.x, (const T*)s.wgt, nnz, part);
+        sp_objective_implicit_finalize_kernel<<<1, 256, 0, st>>>(part, blocks, gw, cw, gt, ct, k, w0, out);
+        return;
+    }
+    sp_objective_kernel<T, false><<<blocks, 256, 0, st>>>((const T*)s.E, (const T*)s.x, (const T*)s.wgt, nnz, part);
     sp_objective_finalize_kernel<<<1, 32, 0, st>>>(part, blocks, out);
+}
+
+// ------------------------------------------------------------------------------------------------
+// the dense rank-k part of a half-step on a handle with unstored weight w0 (DESIGN.md §1 row f7)
+// ------------------------------------------------------------------------------------------------
+// Gram rows of F [k, ld] (row r = topic r over len entries): for z < gridDim.z, with t = t0 + z,
+//   part[z][c][s] = sum_{i in chunk c} F[t, i] F[s, i]     (one block per (s, c, z); fixed-order block reduction)
+template <typename T, typename A>
+__global__ void __launch_bounds__(256)
+sp_gram_rows_kernel(const T* __restrict__ F, int64_t ld, int64_t len, int k, int t0, int chunks, A* __restrict__ part)
+{
+    __shared__ A red[8];
+    const int s = blockIdx.x, c = blockIdx.y, z = blockIdx.z;
+    int64_t b, e;
+    part_range(len, chunks, c, b, e);
+    const T* __restrict__ a = F + (int64_t)(t0 + z) * ld;
+    const T* __restrict__ f = F + (int64_t)s * ld;
+    A acc = A(0);
+    for (int64_t i = b + threadIdx.x; i < e; i += 256) acc = fma((A)a[i], (A)f[i], acc);
+    acc = warp_sum(acc);
+    if ((threadIdx.x & 31) == 0) red[threadIdx.x >> 5] = acc;
+    __syncthreads();
+    if (threadIdx.x == 0) {
+        A g = A(0);
+#pragma unroll
+        for (int w = 0; w < 8; ++w) g += red[w];
+        part[((int64_t)z * chunks + c) * k + s] = g;
+    }
+}
+
+int sp_gram_chunks(int64_t len, int pairs, int sm_count)
+{
+    int64_t c = (2 * (int64_t)sm_count + pairs - 1) / pairs;
+    const int64_t cap = (len + 2047) / 2048;
+    if (c > cap) c = cap;
+    if (c > 64) c = 64;
+    return (int)(c < 1 ? 1 : c);
+}
+
+template <typename T, typename A>
+void launch_sp_gram_rows(const T* F, int64_t ld, int64_t len, int k, int t0, int rows, int chunks, A* part, cudaStream_t st)
+{
+    sp_gram_rows_kernel<T, A><<<dim3((unsigned)k, (unsigned)chunks, (unsigned)rows), 256, 0, st>>>(F, ld, len, k, t0, chunks, part);
+}
+
+// The vector-c solve of wrri_final_kernel with the rank-k part of the statistic added first:
+//   numer_i = sum_p numer_part[p][i] - w0 sum_{s != t} g_s F[s, i],   denom_i = sum_p denom_part[p][i] + w0 g_t
+// g = the Gram row of topic t (sum of its `gchunks` partials), F [k, ldf] the factor being updated (rows s != t only:
+// row t is the one written).
+template <typename T>
+__global__ void __launch_bounds__(256)
+sp_implicit_final_kernel(const T* __restrict__ numer_part, const T* __restrict__ denom_part, int parts, int64_t len,
+                         const T* __restrict__ gpart, int gchunks, int k, int t, const T* __restrict__ F, int64_t ldf,
+                         T w0, T reg_l1, T reg_l2, T eps, T ub, int has_ub, T* __restrict__ out, int64_t out_stride,
+                         T* __restrict__ out2, int64_t out2_stride, int* __restrict__ flags)
+{
+    __shared__ T g[256];
+    for (int s = threadIdx.x; s < k; s += blockDim.x) {
+        T a = T(0);
+        for (int c = 0; c < gchunks; ++c) a += gpart[(int64_t)c * k + s];
+        g[s] = a;
+    }
+    __syncthreads();
+    const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= len) return;
+    T nu = T(0), de = T(0);
+#pragma unroll 4
+    for (int p = 0; p < parts; ++p) {
+        nu += numer_part[(int64_t)p * len + i];
+        de += denom_part[(int64_t)p * len + i];
+    }
+    T corr = T(0);
+    for (int s = 0; s < k; ++s)
+        if (s != t) corr = fma(g[s], F[(int64_t)s * ldf + i], corr);
+    nu = fma(-w0, corr, nu);
+    de = fma(w0, g[t], de);
+    bool unb = false;
+    const T x = solve_vector_c<T>(nu - reg_l1, de + reg_l2, eps, ub, has_ub != 0, unb);
+    out[i * out_stride] = x;
+    if (out2) out2[i * out2_stride] = x;
+    if (unb) atomicOr(flags, 4);
+}
+
+template <typename T>
+void launch_sp_implicit_final(const T* numer_part, const T* denom_part, int parts, int64_t len, const T* gpart, int gchunks,
+                              int k, int t, const T* F, int64_t ldf, double w0, const SolveArgs& a, T* out,
+                              int64_t out_stride, T* out2, int64_t out2_stride, int* flags, cudaStream_t st)
+{
+    sp_implicit_final_kernel<T><<<(unsigned)((len + 255) / 256), 256, 0, st>>>(numer_part, denom_part, parts, len, gpart,
+        gchunks, k, t, F, ldf, (T)w0, (T)a.reg_l1, (T)a.reg_l2, (T)a.eps, (T)a.ub, a.has_ub, out, out_stride, out2,
+        out2_stride, flags);
 }
 
 #define RRI_INST(T)                                                                                                 \
     template int sp_build_csc<T>(const int64_t*, const int32_t*, const T*, const T*, int64_t, int64_t, int64_t,    \
                                  int64_t*, int32_t*, T*, T*, uint32_t*, int, int*, cudaStream_t);                  \
-    template void launch_sp_residual<T>(const SpSide&, const T*, const T*, int, int, cudaStream_t);                \
-    template void launch_sp_residual_rows<T>(const SpSide&, const T*, int64_t, const T*, int, int, int, cudaStream_t); \
+    template void launch_sp_residual<T>(const SpSide&, const T*, const T*, int, double, int, cudaStream_t);        \
+    template void launch_sp_residual_rows<T>(const SpSide&, const T*, int64_t, const T*, int, int, double, int,    \
+                                             cudaStream_t);                                                        \
     template void launch_sp_gather<T>(const uint32_t*, const T*, T*, int64_t, int, cudaStream_t);                  \
     template void launch_sp_pack<T>(const T*, const T*, const T*, const T*, void*, int64_t, cudaStream_t);         \
-    template int launch_sp_pass<T>(const SpSide&, const void*, const T*, const T*, const T*, T*, T*, T*, int,      \
-                                   cudaStream_t);                                                                  \
-    template void launch_sp_objective<T>(const SpSide&, int64_t, double*, double*, cudaStream_t);
+    template int launch_sp_pass<T>(const SpSide&, const void*, const T*, const T*, const T*, T*, T*, T*, double,   \
+                                   int, cudaStream_t);                                                             \
+    template void launch_sp_objective<T>(const SpSide&, int64_t, double*, double*, double, const double*, int,      \
+                                         const double*, int, int, cudaStream_t);                                   \
+    template void launch_sp_implicit_final<T>(const T*, const T*, int, int64_t, const T*, int, int, int, const T*, \
+                                              int64_t, double, const SolveArgs&, T*, int64_t, T*, int64_t, int*,   \
+                                              cudaStream_t);
 RRI_INST(float)
 RRI_INST(double)
+// Gram rows: accumulated in the element type inside a half-step, in fp64 for the objective
+template void launch_sp_gram_rows<float, float>(const float*, int64_t, int64_t, int, int, int, int, float*, cudaStream_t);
+template void launch_sp_gram_rows<float, double>(const float*, int64_t, int64_t, int, int, int, int, double*, cudaStream_t);
+template void launch_sp_gram_rows<double, double>(const double*, int64_t, int64_t, int, int, int, int, double*, cudaStream_t);
 
 }  // namespace rri

@@ -17,6 +17,24 @@ def _ptr(t):
     return C.c_void_p(t.data_ptr()) if t is not None else C.c_void_p(0)
 
 
+def check_unstored_weight(w0, sparse, unstored):
+    """the unstored weight as a float; ValueError unless it is finite and >= 0 and, when > 0, X is sparse with
+    unstored='missing'"""
+    try:
+        w0 = float(w0)
+    except (TypeError, ValueError):
+        raise ValueError('unstored_weight must be a number (got %r)' % (w0,))
+    if not np.isfinite(w0) or w0 < 0:
+        raise ValueError('unstored_weight must be finite and >= 0 (got %r)' % (w0,))
+    if w0 > 0 and not sparse:
+        raise ValueError('unstored_weight applies to sparse X (its unstored entries); for dense X pass the weights '
+                         'as a dense W_mat')
+    if w0 > 0 and unstored != 'missing':
+        raise ValueError("unstored_weight needs unstored='missing' (with unstored='zero' every unstored entry has "
+                         "weight 1)")
+    return w0
+
+
 class NcclComm(object):
     """An ncclComm_t created by the engine library from an id broadcast over torch.distributed."""
 
@@ -57,6 +75,10 @@ class RRIEngine(object):
     unstored='zero': X is an ordinary non-negative matrix stored sparsely (a tf-idf document-term matrix), every entry
     is fitted, the unstored ones as 0 (rri_bind_csr_zero: math='ieee', no W_mat; order='hals' contracts X T' / X' W,
     order='rri' makes one pass over the rows and the columns per topic).
+    unstored_weight: w0 >= 0, sparse X with unstored='missing' only (implicit feedback): every unstored entry is fitted as
+           a 0 of weight w0, the stored ones with their W_mat weight (1 without W_mat) -- the dense masked problem with
+           M = w0 off the stored entries, without forming it (rri_set_unstored_weight).  0 (default) is the plain
+           observed-entries binding.  One GPU, one model.
     order: 'rri' (reference-exact interleaved order, nmf.py:415-476) or 'hals' (block order).
     math : 'ieee' or 'tf32' (tcgen05 tensor-core contraction; float32 + hals only).
     models: None (one model), or b >= 1 models of rank k each on the same binding (rri_set_models: dense unmasked X,
@@ -70,7 +92,8 @@ class RRIEngine(object):
            `objective_terms` a [b, 6] array.
     """
 
-    def __init__(self, X, k, W_mat=None, order='rri', math='ieee', comm=None, unstored='missing', models=None):
+    def __init__(self, X, k, W_mat=None, order='rri', math='ieee', comm=None, unstored='missing', models=None,
+                 unstored_weight=0.0):
         if not isinstance(X, torch.Tensor) or not X.is_cuda:
             raise _lib.RriError('RRIEngine needs X resident on a CUDA device (no CPU fallback)')
         if X.dim() != 2:
@@ -88,6 +111,11 @@ class RRIEngine(object):
             if W_mat is not None:
                 raise ValueError('zero-filled sparse X takes no W_mat (weights on every entry would be a dense n x d object)')
         self.unstored = unstored if self.sparse else 'missing'
+        self.unstored_weight = check_unstored_weight(unstored_weight, self.sparse, unstored)
+        if self.unstored_weight > 0 and (models is not None or isinstance(k, (list, tuple))):
+            raise ValueError('several models take dense data; unstored_weight needs one model')
+        if self.unstored_weight > 0 and comm is not None and comm.world > 1:
+            raise NotImplementedError('unstored_weight runs on one GPU (no row shards)')
         if not self.sparse and X.stride(1) != 1:
             X = X.contiguous()
         self.lib = _lib.load()
@@ -134,6 +162,8 @@ class RRIEngine(object):
         elif self.models is not None:
             check(self.lib.rri_set_models(self.h, self.models))
         if self.sparse:
+            if self.unstored_weight > 0:
+                check(self.lib.rri_set_unstored_weight(self.h, self.unstored_weight))
             self._bind_csr(X, W_mat)
             return
         mk = _lib.RRI_MASK_NONE

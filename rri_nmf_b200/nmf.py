@@ -47,6 +47,11 @@ set by the keyword-only argument `unstored`:
                           magnitude faster than the densified matrix).  Topic reset works as on dense data: the
                           residual document is found over the stored entries, never densifying X.
                   Traffic grows with the stored entries, not with n * d.
+With unstored='missing', the keyword-only `unstored_weight` w0 >= 0 (default 0) gives the unstored entries a weight of
+their own (implicit feedback, one-class recommenders: unobserved pairs count as zeros of small weight w0, observed
+ones with their W_mat weight, 1 without W_mat).  The result equals nmf(X.toarray(), ..., W_mat=M) with the dense M that
+holds w0 at every unstored entry, up to the summation order, in both orders -- but nothing of size n x d is formed:
+per entry the sweep moves the bytes of w0 = 0, plus O((n + d) k) per topic.  One GPU (no comm), no fix_W.
 """
 import logging
 import time
@@ -58,7 +63,7 @@ import torch
 from . import _lib
 from ._device_init import initialize_nmf_torch
 from ._host import initialize_nmf, normalize
-from .engine import RRIEngine, EPS_DIV_BY_ZERO
+from .engine import RRIEngine, EPS_DIV_BY_ZERO, check_unstored_weight
 
 logger = logging.getLogger(__name__)
 eps_div_by_zero = EPS_DIV_BY_ZERO          # nmf.py:52
@@ -85,7 +90,7 @@ class DeviceObjective(object):
                                              reuse_last_sweep=self._after_sweep, **self.regs)
             self._after_sweep = False
         elif self._rebuild is not None:
-            X, W_mat, device, dtype, order, unstored = self._rebuild
+            X, W_mat, device, dtype, order, unstored, unstored_weight = self._rebuild
             device = torch.device(device)
             with torch.cuda.device(device):
                 if _is_sparse(X):
@@ -94,7 +99,7 @@ class DeviceObjective(object):
                     Xd, Md = _to_device(X, device, dtype), _mask_to_device(W_mat, device, dtype)
                 # (a zero-filled sparse binding evaluates in the order of the fit; every other binding in 'rri')
                 eng = RRIEngine(Xd, int(np.shape(self.W)[1]), W_mat=Md, order=order if unstored == 'zero' else 'rri',
-                                unstored=unstored)
+                                unstored=unstored, unstored_weight=unstored_weight)
                 try:
                     self.obj = eng.objective(_to_device(self.W, device, dtype).contiguous(),
                                              _to_device(self.T, device, dtype).contiguous(), **self.regs)
@@ -102,11 +107,11 @@ class DeviceObjective(object):
                     eng.close()
         return self.obj
 
-    def _detach(self, X, W_mat, W, T, device, dtype, order, unstored='missing'):
+    def _detach(self, X, W_mat, W, T, device, dtype, order, unstored='missing', unstored_weight=0.0):
         """called by nmf() before it closes the engine"""
         self.engine = None
         self.W, self.T = W, T
-        self._rebuild = (X, W_mat, str(device), dtype, order, unstored)
+        self._rebuild = (X, W_mat, str(device), dtype, order, unstored, unstored_weight)
 
     def __getstate__(self):
         st = dict(self.__dict__)
@@ -313,7 +318,7 @@ def nmf(X, k, w_row=None, W_mat=None, fix_W=False, fix_T=False, random_state=Non
         ind_rows_to_store=None, eps_gauss_t=None, delta_gauss_t=None,
         *, device=None, update_order=None, math='ieee', comm=None, engine=None, sweeps_per_call=16,
         init_on_device=None, return_reconstruction_err=False, sparse_refresh_every=1, objective='auto',
-        unstored='missing'):
+        unstored='missing', unstored_weight=0.0):
     """Non-negative factorisation X ~ W T by rank-one residue iteration.  See the reference docstring
     (nmf.py:109-269) for the arguments; returns {'W', 'T', 'iter_cputime', 'random_state'[, 'obj_history',
     'obj_calculator', 'diagnostics']} (nmf.py:551-560).  W and T come back as the kind of array X was
@@ -325,6 +330,12 @@ def nmf(X, k, w_row=None, W_mat=None, fix_W=False, fix_T=False, random_state=Non
     if unstored not in ('missing', 'zero'):
         raise ValueError("unstored must be 'missing' or 'zero'")
     zero_filled = unstored == 'zero' and _is_sparse(X)
+    unstored_weight = check_unstored_weight(unstored_weight, _is_sparse(X), unstored)
+    if unstored_weight > 0:
+        if comm is not None:
+            raise NotImplementedError('unstored_weight runs on one GPU (row shards are not implemented)')
+        if fix_W:
+            raise NotImplementedError('fix_W=True is not available with unstored_weight')
     if zero_filled:
         if W_mat is not None:
             raise ValueError("unstored='zero' takes no W_mat: weights on a zero-filled matrix would be a dense n x d object")
@@ -433,7 +444,7 @@ def nmf(X, k, w_row=None, W_mat=None, fix_W=False, fix_T=False, random_state=Non
             # (fix_T: the W-only sweeps are the same in both orders; on zero-filled data they run on a block-order
             # binding, which holds no interleaved-order partials)
             engine = RRIEngine(Xd, k, W_mat=Md, order='hals' if zero_filled and fix_T else update_order, math=math,
-                               comm=comm, unstored=unstored)
+                               comm=comm, unstored=unstored, unstored_weight=unstored_weight)
         timing['engine_setup_s'] = time.perf_counter() - _t1       # workspace, transposed copy of X, peer mapping
         try:
             W, T = _device_start(engine, Xd, W_mat, Md, k, init, random_state, t_row_sum, w_row_sum, W0, T0,
@@ -452,7 +463,7 @@ def nmf(X, k, w_row=None, W_mat=None, fix_W=False, fix_T=False, random_state=Non
             if 'obj_calculator' in out and own_engine:
                 # the calculator outlives this call without pinning device memory (and stays picklable)
                 out['obj_calculator']._detach(X, W_mat_user, out['W'], out['T'], device, dtype, engine.order,
-                                              engine.unstored)
+                                              engine.unstored, engine.unstored_weight)
             return out
         finally:
             if own_engine:
