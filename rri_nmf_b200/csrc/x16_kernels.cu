@@ -100,31 +100,85 @@ __device__ __forceinline__ unsigned block_max(unsigned v, unsigned* sh)
     return sh[32];
 }
 
-__global__ void f16_absmax_kernel(const float* __restrict__ F, int rows, int64_t cols, int64_t ld, unsigned* __restrict__ part)
+// Both passes over the factor go four elements per load (VEC: rows of a multiple of 4 columns, 16-byte aligned) with
+// U loads in flight per thread before any of them is used: one dependent load per thread at a time left a 64 x 200 000
+// factor (the T half-step's W') latency-bound.  The maximum does not depend on which block sees which element, and every
+// element is converted on its own, so the copy and its scale are those of the one-element-at-a-time loops.
+constexpr int FU = 4;
+
+__device__ __forceinline__ unsigned absbits(float x) { return __float_as_uint(fabsf(to_tf32(x))); }
+
+template <bool VEC>
+__global__ void __launch_bounds__(256)
+f16_absmax_kernel(const float* __restrict__ F, int rows, int64_t cols, int64_t ld, unsigned* __restrict__ part)
 {
     __shared__ unsigned sh[33];
     unsigned m = 0u;
-    for (int r = 0; r < rows; ++r)
-        for (int64_t c = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; c < cols; c += (int64_t)gridDim.x * blockDim.x) {
-            const unsigned b = __float_as_uint(fabsf(to_tf32(F[(int64_t)r * ld + c])));
-            m = b > m ? b : m;
+    const int64_t stride = (int64_t)gridDim.x * blockDim.x;
+    const int64_t t0 = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (VEC) {
+        const int64_t cq = cols / 4, total = (int64_t)rows * cq;
+        for (int64_t e0 = t0; e0 < total; e0 += FU * stride) {
+            float4 v[FU];
+#pragma unroll
+            for (int u = 0; u < FU; ++u) {
+                const int64_t e = e0 + u * stride;
+                v[u] = make_float4(0.f, 0.f, 0.f, 0.f);
+                if (e < total) v[u] = __ldg(reinterpret_cast<const float4*>(F + (e / cq) * ld) + e % cq);
+            }
+#pragma unroll
+            for (int u = 0; u < FU; ++u)
+                m = max(m, max(max(absbits(v[u].x), absbits(v[u].y)), max(absbits(v[u].z), absbits(v[u].w))));
         }
+    } else {
+        for (int r = 0; r < rows; ++r)
+            for (int64_t c = t0; c < cols; c += stride) m = max(m, absbits(F[(int64_t)r * ld + c]));
+    }
     m = block_max(m, sh);
     if (threadIdx.x == 0) part[blockIdx.x] = m;
 }
 
-__global__ void f16_factor_kernel(const float* __restrict__ F, int rows, int64_t cols, int64_t ld,
-                                  const unsigned* __restrict__ part, int nparts, __half* __restrict__ out, int64_t ldo,
-                                  int* __restrict__ e_out)
+__device__ __forceinline__ __half2 to_h2(float a, float b, float s)
+{
+    return __halves2half2(__float2half_rn(to_tf32(a) * s), __float2half_rn(to_tf32(b) * s));
+}
+
+template <bool VEC>
+__global__ void __launch_bounds__(256)
+f16_factor_kernel(const float* __restrict__ F, int rows, int64_t cols, int64_t ld, const unsigned* __restrict__ part,
+                  int nparts, __half* __restrict__ out, int64_t ldo, int* __restrict__ e_out)
 {
     __shared__ unsigned sh[33];
     unsigned m = 0u;
     for (int i = threadIdx.x; i < nparts; i += blockDim.x) m = part[i] > m ? part[i] : m;
     const int e = factor_exp(block_max(m, sh));
     const float s = pow2(e);
-    for (int r = 0; r < rows; ++r)
-        for (int64_t c = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; c < cols; c += (int64_t)gridDim.x * blockDim.x)
-            out[(int64_t)r * ldo + c] = __float2half_rn(to_tf32(F[(int64_t)r * ld + c]) * s);
+    const int64_t stride = (int64_t)gridDim.x * blockDim.x;
+    const int64_t t0 = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (VEC) {
+        const int64_t cq = cols / 4, total = (int64_t)rows * cq;
+        for (int64_t e0 = t0; e0 < total; e0 += FU * stride) {
+            float4 v[FU];
+#pragma unroll
+            for (int u = 0; u < FU; ++u) {
+                const int64_t q = e0 + u * stride;
+                if (q < total) v[u] = __ldg(reinterpret_cast<const float4*>(F + (q / cq) * ld) + q % cq);
+            }
+#pragma unroll
+            for (int u = 0; u < FU; ++u) {
+                const int64_t q = e0 + u * stride;
+                if (q < total) {
+                    __half2* o = reinterpret_cast<__half2*>(out + (q / cq) * ldo + 4 * (q % cq));
+                    o[0] = to_h2(v[u].x, v[u].y, s);
+                    o[1] = to_h2(v[u].z, v[u].w, s);
+                }
+            }
+        }
+    } else {
+        for (int r = 0; r < rows; ++r)
+            for (int64_t c = t0; c < cols; c += stride)
+                out[(int64_t)r * ldo + c] = __float2half_rn(to_tf32(F[(int64_t)r * ld + c]) * s);
+    }
     if (blockIdx.x == 0 && threadIdx.x == 0) *e_out = e;
 }
 
@@ -168,8 +222,15 @@ int f16_factor_parts(int sm_count) { return 4 * sm_count < 1024 ? 4 * sm_count :
 void launch_f16_factor(const float* F, int rows, int64_t cols, int64_t ld, unsigned* part, int nparts, void* out,
                        int64_t ldo, int* e_out, cudaStream_t st)
 {
-    f16_absmax_kernel<<<nparts, 256, 0, st>>>(F, rows, cols, ld, part);
-    f16_factor_kernel<<<nparts, 256, 0, st>>>(F, rows, cols, ld, part, nparts, (__half*)out, ldo, e_out);
+    const bool vec = cols % 4 == 0 && ld % 4 == 0 && ldo % 4 == 0 && (reinterpret_cast<uintptr_t>(F) & 15) == 0 &&
+                     (reinterpret_cast<uintptr_t>(out) & 7) == 0;
+    if (vec) {
+        f16_absmax_kernel<true><<<nparts, 256, 0, st>>>(F, rows, cols, ld, part);
+        f16_factor_kernel<true><<<nparts, 256, 0, st>>>(F, rows, cols, ld, part, nparts, (__half*)out, ldo, e_out);
+    } else {
+        f16_absmax_kernel<false><<<nparts, 256, 0, st>>>(F, rows, cols, ld, part);
+        f16_factor_kernel<false><<<nparts, 256, 0, st>>>(F, rows, cols, ld, part, nparts, (__half*)out, ldo, e_out);
+    }
 }
 
 }  // namespace rri
