@@ -150,8 +150,21 @@ int rri_bind_csr(rri_handle_t h, int64_t nnz, const int64_t* rowptr_dev, const i
  * rri_sweeps (both orders, fix_T), rri_topics, rri_objective (<W'W, T T'> in fp64), rri_topic_sums, rri_spmm (which
  * keeps applying the stored entry weights, not m - w0), rri_stats and rri_profile_kernel serve the handle;
  * rri_bind, rri_bind_csr_zero, rri_set_models / rri_set_model_ranks, rri_set_comm with world > 1 and rri_partials_T
- * refuse it. */
+ * refuse it.  A later call with w0 = 0 also drops the vectors of rri_set_unstored_weight_vectors. */
 int rri_set_unstored_weight(rri_handle_t h, double w0);
+
+/* Rank-one unstored weights (user- / item-oriented and item-popularity schemes of one-class collaborative filtering;
+ * DESIGN.md §1 f8): the weight of unstored entry (i, j) becomes u_ij = w0 (a_i b_j) instead of w0.  a_dev [n_local]
+ * and b_dev [d] are device vectors of the handle's dtype; either may be NULL (all ones; both NULL is the scalar-w0
+ * handle: same launches, same bits).  Call after rri_set_unstored_weight with w0 > 0 and before rri_bind_csr.  The
+ * engine keeps its own copies (O(n + d)): the caller may free its vectors on return.  rri_bind_csr checks on the device
+ * that every entry is finite and >= 0 and fails otherwise.  The stored entries keep a shifted residual
+ * mt E + u x with mt = m - u computed once per entry at bind (two nnz-long copies, CSR and CSC order, streamed by the
+ * passes as their weights); each half-step scales its Gram row W' diag(a) W (T-steps) / T diag(b) T' (W-steps) by b_j /
+ * a_i.  The entry points that serve rri_set_unstored_weight serve this too (rri_spmm still applies the stored entry
+ * weights only).  Refused: a handle without w0 > 0, a bound handle, a handle of several models; rri_set_comm with
+ * world > 1 keeps refusing the handle. */
+int rri_set_unstored_weight_vectors(rri_handle_t h, const void* a_dev, const void* b_dev);
 
 /* Zero-filled sparse binding: the CSR matrix is an ordinary non-negative matrix stored sparsely (a tf-idf
  * document-term matrix); every entry is fitted, the unstored ones as 0.  Same CSR contract as rri_bind_csr

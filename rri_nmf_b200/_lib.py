@@ -47,6 +47,7 @@ SYMBOLS = {
     'rri_bind_csr': (C.c_int, [_vp, _i64, _vp, _vp, _vp, _vp, _vp]),
     'rri_bind_csr_zero': (C.c_int, [_vp, _i64, _vp, _vp, _vp, _vp]),
     'rri_set_unstored_weight': (C.c_int, [_vp, C.c_double]),
+    'rri_set_unstored_weight_vectors': (C.c_int, [_vp, _vp, _vp]),
     'rri_spmm': (C.c_int, [_vp, _i32, _vp, _i64, _vp, _i64, _i32, _vp]),
     'rri_sweeps': (C.c_int, [_vp, _vp, _vp, _i32, C.POINTER(RriParams), C.POINTER(_i32), _vp]),
     'rri_topics': (C.c_int, [_vp, _vp, _vp, _i32, _i32, C.POINTER(RriParams), C.POINTER(_i32), _vp]),

@@ -202,6 +202,11 @@ struct rri_handle_s {
     int sp_gc_w = 1, sp_gc_t = 1;      // their chunks over the rows of W (T-steps) / the columns of T (W-steps)
     double* sp_gobj = nullptr;         // [k][oc_w][k] + [k][oc_t][k] fp64 Gram partials of the objective
     int sp_oc_w = 1, sp_oc_t = 1;
+    // rank-one unstored weights u = w0 (a_i b_j) (rri_set_unstored_weight_vectors): the engine's copies of a [n] and b [d]
+    // (null: all ones; both null = the scalar w0 above), and mt = m - u per entry in both orders, the weight stream of
+    // every pass and restart (the stored entry weights m stay in csr.wgt / csc.wgt for the objective and rri_spmm)
+    void *sp_va = nullptr, *sp_vb = nullptr;
+    void *sp_mt_csr = nullptr, *sp_mt_csc = nullptr;
     // zero-filled sparse binding (rri_bind_csr_zero): the rows and the columns with their chunk plans; the block-order
     // half-steps take X T' / X' W from launch_spmm instead of the dense contraction
     bool zero_csr = false;
@@ -779,6 +784,8 @@ static int bind_csr_impl(rri_handle_t h, const int64_t* rowptr, const int32_t* c
     }
     if (ws_alloc(h, &E_csr, es * ne) || ws_alloc(h, &E_csc, es * ne) || ws_alloc(h, &x_csc, es * ne)) return 1;
     if (wgt && ws_alloc(h, &w_csc, es * ne)) return 1;
+    const bool vec = h->sp_w0 > 0 && (h->sp_va || h->sp_vb);
+    if (vec && (ws_alloc(h, &h->sp_mt_csr, es * ne) || ws_alloc(h, &h->sp_mt_csc, es * ne))) return 1;
     if (ws_alloc(h, &csc_row, sizeof(int32_t) * ne) || ws_alloc(h, &colptr, sizeof(int64_t) * (size_t)(d + 1))) return 1;
     if (ws_alloc(h, &h->sp_quad, 4 * es * (size_t)m) || ws_alloc(h, &h->sp_told, es * 2 * (size_t)d) ||
         ws_alloc(h, &h->sp_wold, es * 2 * (size_t)n) || ws_alloc(h, &h->mstat, es * 2 * (size_t)m) ||
@@ -799,17 +806,33 @@ static int bind_csr_impl(rri_handle_t h, const int64_t* rowptr, const int32_t* c
     if (ws_alloc(h, &h->Wt, es * (size_t)k * h->ldwt) || ws_alloc(h, &h->Tt, es * (size_t)d * h->sp_ldt)) return 1;
     if (ws_alloc(h, (void**)&h->sp_perm, sizeof(uint32_t) * ne)) return 1;
     CK(cudaStreamSynchronize(0));          // the zero-fills above ran on the legacy default stream
+    if (vec) {
+        // the rank-one vectors are checked with the CSR (bits 8 and 16 of the same error word)
+        launch_sp_check_weights<T>((const T*)h->sp_va, n, 8, h->sp_err, h->sm_count, st);
+        launch_sp_check_weights<T>((const T*)h->sp_vb, d, 16, h->sp_err, h->sm_count, st);
+        h->launches += 2;
+    }
     const int rc = sp_build_csc<T>(rowptr, col, val, wgt, n, d, nnz, (int64_t*)colptr, (int32_t*)csc_row, (T*)x_csc,
                                    (T*)w_csc, h->sp_perm, h->sm_count, h->sp_err, st);
-    if (rc < 0)
+    if (rc < 0 && (-rc & 7))
         return fail("malformed CSR input:%s%s%s", (-rc & 1) ? " rowptr is not a monotone [0..nnz] sequence;" : "",
                     (-rc & 2) ? " column index outside [0,d);" : "",
                     (-rc & 4) ? " column indices must be strictly ascending inside every row (sort and merge duplicates);" : "");
+    if (rc < 0)
+        return fail("the unstored weight vectors must be finite and >= 0:%s%s", (-rc & 8) ? " a (rows) is not;" : "",
+                    (-rc & 16) ? " b (columns) is not;" : "");
     if (rc > 0) return fail("building the column orientation failed: %s", cudaGetErrorString((cudaError_t)rc));
     h->csr = SpSide{n, rowptr, col, val, wgt, E_csr, nnz / n >= 512 ? 256 : 32, nullptr, 1, 0, d, nullptr};
     h->csc = SpSide{d, (const int64_t*)colptr, (const int32_t*)csc_row, x_csc, w_csc, E_csc, nnz / d >= 512 ? 256 : 32,
                     nullptr, 1, 0, n, nullptr};
     h->launches += 8;
+    if (vec && nnz > 0) {
+        // mt = m - w0 (a_i b_j) once, in CSR order; the column copy is its permutation (the same bits in both orders)
+        launch_sp_mtilde<T>(rowptr, col, wgt, n, (const T*)h->sp_va, (const T*)h->sp_vb, h->sp_w0, (T*)h->sp_mt_csr,
+                            h->sm_count, st);
+        launch_sp_gather<T>(h->sp_perm, (const T*)h->sp_mt_csr, (T*)h->sp_mt_csc, nnz, h->sm_count, st);
+        h->launches += 2;
+    }
     // blocked passes: the gathered factor is staged through shared memory in blocks of nb records
     const char* env = getenv("RRI_SP_BLOCKED");
     const bool blocked = !(env && *env == '0');
@@ -842,6 +865,13 @@ static int bind_csr_impl(rri_handle_t h, const int64_t* rowptr, const int32_t* c
     return 0;
 }
 
+static void release_weight_vectors(rri_handle_t h)
+{
+    if (h->sp_va) ws_release(h, h->sp_va, h->es * (size_t)h->n);
+    if (h->sp_vb) ws_release(h, h->sp_vb, h->es * (size_t)h->d);
+    h->sp_va = h->sp_vb = nullptr;
+}
+
 extern "C" int rri_set_unstored_weight(rri_handle_t h, double w0)
 {
     if (!h) return fail("null handle");
@@ -850,6 +880,28 @@ extern "C" int rri_set_unstored_weight(rri_handle_t h, double w0)
     if (w0 > 0 && h->models > 1) return fail("a handle of several models takes no unstored weight");
     if (w0 > 0 && h->world > 1) return fail("an unstored weight is served on one GPU (world == 1)");
     h->sp_w0 = w0;
+    if (w0 == 0) release_weight_vectors(h);        // (the weight vectors scale w0: none is left)
+    return 0;
+}
+
+extern "C" int rri_set_unstored_weight_vectors(rri_handle_t h, const void* a_dev, const void* b_dev)
+{
+    if (!h) return fail("null handle");
+    if (h->X) return fail("rri_set_unstored_weight_vectors must be called before rri_bind_csr");
+    if (h->models > 1) return fail("a handle of several models takes no unstored weight");
+    if (!(h->sp_w0 > 0)) return fail("unstored weight vectors scale w0: call rri_set_unstored_weight with w0 > 0 first");
+    CK(cudaSetDevice(h->device));
+    release_weight_vectors(h);             // (an unbound handle: nothing in flight reads them)
+    // the engine's own copies: the caller may free its vectors on return (checked on the device by rri_bind_csr)
+    if (a_dev) {
+        if (ws_alloc(h, &h->sp_va, h->es * (size_t)h->n)) return 1;
+        CK(cudaMemcpy(h->sp_va, a_dev, h->es * (size_t)h->n, cudaMemcpyDeviceToDevice));
+    }
+    if (b_dev) {
+        if (ws_alloc(h, &h->sp_vb, h->es * (size_t)h->d)) return 1;
+        CK(cudaMemcpy(h->sp_vb, b_dev, h->es * (size_t)h->d, cudaMemcpyDeviceToDevice));
+    }
+    CK(cudaStreamSynchronize(0));          // (a device-to-device cudaMemcpy may return before the copy has run)
     return 0;
 }
 
@@ -1490,15 +1542,28 @@ struct SpState {
     const void* told_cur = nullptr;     // T[t,:] before this topic's T-step (null: no T-step preceded the W-step)
 };
 
+// The orientation a pass or a restart of this handle reads: with rank-one unstored weights its weight stream is mt.
+static SpSide sp_pass_side(rri_handle_t h, const SpSide& s, const void* mt)
+{
+    SpSide r = s;
+    if (h->sp_mt_csr) r.wgt = mt;
+    return r;
+}
+
 template <typename T>
 static void sp_refresh(rri_handle_t h, bool need_csr, bool need_csc, const T* W, cudaStream_t st, bool plain = false)
 {
     // E = X - W T on the observed entries, from the current factors (with an unstored weight, unless `plain`: the
-    // shifted residual (m - w0) E + w0 x)
+    // shifted residual (m - w0) E + w0 x, or mt E + w0 (a_i b_j) x with rank-one weights)
     const double w0 = plain ? 0.0 : h->sp_w0;
+    const bool vec = !plain && h->sp_mt_csr;
+    const T* va = vec ? (const T*)h->sp_va : nullptr;
+    const T* vb = vec ? (const T*)h->sp_vb : nullptr;
+    const SpSide csr = vec ? sp_pass_side(h, h->csr, h->sp_mt_csr) : h->csr;
+    const SpSide csc = vec ? sp_pass_side(h, h->csc, h->sp_mt_csc) : h->csc;
     if (h->sp_refresh_v2) {
         // the row copy from the factors (16-byte gathers of T' rows), the column copy as a permutation of it
-        launch_sp_residual_rows<T>(h->csr, W, h->k, (const T*)h->Tt, h->sp_ldt, h->k, w0, h->sm_count, st);
+        launch_sp_residual_rows<T>(csr, W, h->k, (const T*)h->Tt, h->sp_ldt, h->k, w0, h->sm_count, st, va, vb);
         h->launches++;
         if (need_csc && h->nnz > 0) {
             launch_sp_gather<T>(h->sp_perm, (const T*)h->csr.E, (T*)h->csc.E, h->nnz, h->sm_count, st);
@@ -1506,8 +1571,8 @@ static void sp_refresh(rri_handle_t h, bool need_csr, bool need_csc, const T* W,
         }
         return;
     }
-    if (need_csc) { launch_sp_residual<T>(h->csc, (const T*)h->Tt, W, h->k, w0, h->sm_count, st); h->launches++; }
-    if (need_csr) { launch_sp_residual<T>(h->csr, W, (const T*)h->Tt, h->k, w0, h->sm_count, st); h->launches++; }
+    if (need_csc) { launch_sp_residual<T>(csc, (const T*)h->Tt, W, h->k, w0, h->sm_count, st, vb, va); h->launches++; }
+    if (need_csr) { launch_sp_residual<T>(csr, W, (const T*)h->Tt, h->k, w0, h->sm_count, st, va, vb); h->launches++; }
 }
 
 template <typename T>
@@ -1520,14 +1585,17 @@ static int sp_T_step(rri_handle_t h, T* W, T* Tm, int t, const rri_params_t* p, 
     T* ms = (T*)h->mstat;                                            // [numer(d) | denom(d)] for the all-reduce
     launch_sp_pack<T>((const T*)S.csc.wo, (const T*)S.csc.wn, wt, wt, h->sp_quad, n, st);
     const T* nu = (const T*)h->sp_npart; const T* de = (const T*)h->sp_dpart;
-    int parts = launch_sp_pass<T>(h->csc, h->sp_quad, (const T*)S.csc.to, (const T*)S.csc.tn, trow, told, (T*)h->sp_npart,
-                                  (T*)h->sp_dpart, h->sp_w0, h->sm_count, st);
+    // (rank-one weights: the pass streams mt itself as its weights, with no shift of its own)
+    const bool vec = h->sp_mt_csr != nullptr;
+    int parts = launch_sp_pass<T>(sp_pass_side(h, h->csc, h->sp_mt_csc), h->sp_quad, (const T*)S.csc.to, (const T*)S.csc.tn,
+                                  trow, told, (T*)h->sp_npart, (T*)h->sp_dpart, vec ? 0.0 : h->sp_w0, h->sm_count, st, vec);
     h->launches += 2;
     if (h->sp_w0 > 0) {
-        // g = w_t' W (one row of W'W), then the solve with  -w0 sum_{s!=t} g_s T[s,:]  and  +w0 g_t  (world == 1 here)
-        launch_sp_gram_rows<T, T>((const T*)h->Wt, h->ldwt, n, h->k, t, 1, h->sp_gc_w, (T*)h->sp_gpart, st);
+        // g = w_t' W (one row of W'W; W' diag(a) W with row weights), then the solve with  -w0 sum_{s!=t} g_s T[s,:]  and
+        // +w0 g_t, w0 scaled by b_j with column weights  (world == 1 here)
+        launch_sp_gram_rows<T, T>((const T*)h->Wt, h->ldwt, n, h->k, t, 1, h->sp_gc_w, (T*)h->sp_gpart, st, (const T*)h->sp_va);
         launch_sp_implicit_final<T>(nu, de, parts, d, (const T*)h->sp_gpart, h->sp_gc_w, h->k, t, Tm, d, h->sp_w0,
-                                    solve_args(p, true), trow, 1, (T*)h->Tt + t, h->sp_ldt, h->flags, st);
+                                    solve_args(p, true), trow, 1, (T*)h->Tt + t, h->sp_ldt, h->flags, st, (const T*)h->sp_vb);
         h->launches += 2;
     } else {
         if (h->world > 1) {
@@ -1560,14 +1628,17 @@ static int sp_W_step(rri_handle_t h, T* W, T* Tm, int t, const rri_params_t* p, 
     const T* told = S.told_cur ? (const T*)S.told_cur : trow;
     T* wold = (T*)h->sp_wold + (int64_t)(S.cw & 1) * n;
     launch_sp_pack<T>((const T*)S.csr.to, (const T*)S.csr.tn, told, trow, h->sp_quad, d, st);
-    const int parts = launch_sp_pass<T>(h->csr, h->sp_quad, (const T*)S.csr.wo, (const T*)S.csr.wn, wt, wold,
-                                        (T*)h->sp_npart, (T*)h->sp_dpart, h->sp_w0, h->sm_count, st);
+    const bool vec = h->sp_mt_csr != nullptr;
+    const int parts = launch_sp_pass<T>(sp_pass_side(h, h->csr, h->sp_mt_csr), h->sp_quad, (const T*)S.csr.wo,
+                                        (const T*)S.csr.wn, wt, wold, (T*)h->sp_npart, (T*)h->sp_dpart, vec ? 0.0 : h->sp_w0,
+                                        h->sm_count, st, vec);
     if (h->sp_w0 > 0) {
-        // h = t_t T' (one row of T T', this topic's T row already updated), then the solve with -w0 sum_{s!=t} h_s W[:,s]
-        launch_sp_gram_rows<T, T>(Tm, d, d, h->k, t, 1, h->sp_gc_t, (T*)h->sp_gpart, st);
+        // h = t_t T' (one row of T T', T diag(b) T' with column weights; this topic's T row already updated), then the
+        // solve with -w0 sum_{s!=t} h_s W[:,s], w0 scaled by a_i with row weights
+        launch_sp_gram_rows<T, T>(Tm, d, d, h->k, t, 1, h->sp_gc_t, (T*)h->sp_gpart, st, (const T*)h->sp_vb);
         launch_sp_implicit_final<T>((const T*)h->sp_npart, (const T*)h->sp_dpart, parts, n, (const T*)h->sp_gpart, h->sp_gc_t,
                                     h->k, t, (const T*)h->Wt, h->ldwt, h->sp_w0, solve_args(p, false), W + t, h->k, wt, 1,
-                                    h->flags, st);
+                                    h->flags, st, (const T*)h->sp_va);
         h->launches++;
     } else {
         launch_wrri_final<T>((const T*)h->sp_npart, (const T*)h->sp_dpart, parts, n, solve_args(p, false), W + t, h->k, wt, 1,
@@ -1828,13 +1899,15 @@ static int objective_impl(rri_handle_t h, const T* W, const T* Tm, cudaStream_t 
         double* gw = h->sp_gobj;
         double* gt = gw ? gw + (size_t)k * k * h->sp_oc_w : nullptr;
         if (h->sp_w0 > 0) {
-            // <W'W, T T'> in fp64 from the Gram partials of W' and T (no pass over the n x d entries)
+            // <W'W, T T'> in fp64 from the Gram partials of W' and T (no pass over the n x d entries); with rank-one
+            // weights <W' diag(a) W, T diag(b) T'>
             launch_transpose<T>(W, h->n, k, k, (T*)h->Wt, h->ldwt, st);
-            launch_sp_gram_rows<T, double>((const T*)h->Wt, h->ldwt, h->n, k, 0, k, h->sp_oc_w, gw, st);
-            launch_sp_gram_rows<T, double>(Tm, h->d, h->d, k, 0, k, h->sp_oc_t, gt, st);
+            launch_sp_gram_rows<T, double>((const T*)h->Wt, h->ldwt, h->n, k, 0, k, h->sp_oc_w, gw, st, (const T*)h->sp_va);
+            launch_sp_gram_rows<T, double>(Tm, h->d, h->d, k, 0, k, h->sp_oc_t, gt, st, (const T*)h->sp_vb);
             h->launches += 3;
         }
-        launch_sp_objective<T>(h->csr, h->nnz, h->obj_part, h->obj_out, h->sp_w0, gw, h->sp_oc_w, gt, h->sp_oc_t, k, st);
+        launch_sp_objective<T>(h->csr, h->nnz, h->obj_part, h->obj_out, h->sp_w0, gw, h->sp_oc_w, gt, h->sp_oc_t, k, st,
+                               (const T*)h->sp_va, (const T*)h->sp_vb);
         launch_norms<T>(W, h->n * h->k, h->obj_part, h->obj_out + 2, st);
         launch_norms<T>(Tm, (int64_t)h->k * h->d, h->obj_part, h->obj_out + 4, st);
         h->launches += 7;

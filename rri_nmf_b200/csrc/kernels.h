@@ -278,15 +278,18 @@ int sp_build_csc(const int64_t* rowptr, const int32_t* col, const T* x, const T*
                  int* err_dev, cudaStream_t st);
 
 // s.E[p] = s.x[p] - sum_l A[seg,l] * B[s.idx[p],l]   (A: own factor rows [nseg,k], B: other factor rows [.,k]).
-// w0 > 0 (unstored weight): the shifted residual (m - w0) E + w0 x is stored instead (m = s.wgt[p], or 1).
+// w0 > 0 (unstored weight): the shifted residual (m - w0) E + w0 x is stored instead (m = s.wgt[p], or 1).  With a
+// rank-one weight vector vseg (over the segments) or vidx (over the gathered index), u = w0 (a_i b_j): s.wgt then holds
+// mt = m - u (launch_sp_mtilde) and mt E + u x is stored.
 template <typename T>
-void launch_sp_residual(const SpSide& s, const T* A, const T* B, int k, double w0, int sm_count, cudaStream_t st);
+void launch_sp_residual(const SpSide& s, const T* A, const T* B, int k, double w0, int sm_count, cudaStream_t st,
+                        const T* vseg = nullptr, const T* vidx = nullptr);
 
 // The same for the row orientation with 16-byte gathers: B[., ldb] has a padded row stride (multiple of 16 bytes, zero
 // pad columns); A[nseg, lda] is staged per segment through shared memory.
 template <typename T>
 void launch_sp_residual_rows(const SpSide& s, const T* A, int64_t lda, const T* B, int ldb, int k, double w0, int sm_count,
-                             cudaStream_t st);
+                             cudaStream_t st, const T* vseg = nullptr, const T* vidx = nullptr);
 // dst[p] = src[perm[p]]
 template <typename T>
 void launch_sp_gather(const uint32_t* perm, const T* src, T* dst, int64_t nnz, int sm_count, cudaStream_t st);
@@ -299,28 +302,42 @@ void launch_sp_pack(const T* po, const T* pn, const T* vold, const T* vnew, void
 // (own_po/own_pn null -> none), writes own_save[seg] = own_cur[seg] and `parts` slices numer[p][seg], denom[p][seg]
 // (before the regularisers; the consumer adds the slices in order).  Returns parts (1, or s.nblk when blocked).
 // w0 > 0: the copies hold the shifted residual and the sums are its stored-entry part (sparse_kernels.cu, sp_entry).
+// shifted with w0 = 0: the same with s.wgt as mt itself (rank-one unstored weights: s.wgt is the mt copy).
 template <typename T>
 int launch_sp_pass(const SpSide& s, const void* quad, const T* own_po, const T* own_pn, const T* own_cur,
-                    T* own_save, T* numer, T* denom, double w0, int sm_count, cudaStream_t st);
+                    T* own_save, T* numer, T* denom, double w0, int sm_count, cudaStream_t st, bool shifted = false);
 
 // out[0] = 0.5 * sum m E^2, out[1] = sum m x^2 over the observed entries (fixed-order reduction).  w0 > 0: out[0] =
 // 0.5 (sum m E^2 + w0 (<W'W, T T'> - sum (x - E)^2)) with the fp64 Gram partials gw [k][cw][k], gt [k][ct][k] of W' and T
-// (launch_sp_gram_rows<T, double>); part then holds 3 doubles per block (<= 256 blocks)
+// (launch_sp_gram_rows<T, double>); part then holds 3 doubles per block (<= 256 blocks).  Rank-one weights va [n] / vb [d]
+// (s = the CSR side, either may be null = ones): the Grams are W' diag(a) W, T diag(b) T' and the stored-entry term
+// carries a_i b_j.
 template <typename T>
 void launch_sp_objective(const SpSide& s, int64_t nnz, double* part, double* out, double w0, const double* gw, int cw,
-                         const double* gt, int ct, int k, cudaStream_t st);
+                         const double* gt, int ct, int k, cudaStream_t st, const T* va = nullptr, const T* vb = nullptr);
 
 // Unstored weight w0 > 0: Gram rows part[z][c][s] = sum_{i in chunk c of [0,len)} F[t0+z, i] F[s, i] (F [k, ld]; grid
-// k x chunks x rows), chunks = sp_gram_chunks(len, pairs of one launch, ...); A = accumulation type
+// k x chunks x rows), chunks = sp_gram_chunks(len, pairs of one launch, ...); A = accumulation type.  wv [len] (optional):
+// the weighted Gram rows sum F[t0+z, i] wv[i] F[s, i] (rank-one unstored weights)
 int sp_gram_chunks(int64_t len, int pairs, int sm_count);
 template <typename T, typename A>
-void launch_sp_gram_rows(const T* F, int64_t ld, int64_t len, int k, int t0, int rows, int chunks, A* part, cudaStream_t st);
+void launch_sp_gram_rows(const T* F, int64_t ld, int64_t len, int k, int t0, int rows, int chunks, A* part, cudaStream_t st,
+                         const T* wv = nullptr);
 // launch_wrri_final with the dense part of the statistic: numer -= w0 sum_{s!=t} g_s F[s, i], denom += w0 g_t, g = sum of
-// the gchunks Gram-row partials gpart [gchunks][k] of topic t (k <= 256), F [k, ldf] the factor being updated
+// the gchunks Gram-row partials gpart [gchunks][k] of topic t (k <= 256), F [k, ldf] the factor being updated.  sc [len]
+// (optional): w0 sc[i] in place of w0 (rank-one unstored weights: b in a T-step, a in a W-step)
 template <typename T>
 void launch_sp_implicit_final(const T* numer_part, const T* denom_part, int parts, int64_t len, const T* gpart, int gchunks,
                               int k, int t, const T* F, int64_t ldf, double w0, const SolveArgs& a, T* out,
-                              int64_t out_stride, T* out2, int64_t out2_stride, int* flags, cudaStream_t st);
+                              int64_t out_stride, T* out2, int64_t out2_stride, int* flags, cudaStream_t st,
+                              const T* sc = nullptr);
+// Rank-one unstored weights (rri_set_unstored_weight_vectors): err |= bit unless every v[i] is finite and >= 0 (v null:
+// nothing); mt[p] = m[p] - w0 (a_i b_j) in CSR order (wgt / va / vb null: ones)
+template <typename T>
+void launch_sp_check_weights(const T* v, int64_t len, int bit, int* err, int sm_count, cudaStream_t st);
+template <typename T>
+void launch_sp_mtilde(const int64_t* rowptr, const int32_t* col, const T* wgt, int64_t n, const T* va, const T* vb,
+                      double w0, T* mt, int sm_count, cudaStream_t st);
 }  // namespace rri
 
 namespace rri {

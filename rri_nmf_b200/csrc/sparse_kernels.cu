@@ -139,20 +139,31 @@ int sp_build_csc(const int64_t* rowptr, const int32_t* col, const T* x, const T*
 // ------------------------------------------------------------------------------------------------
 // residual from scratch:  E[p] = x[p] - sum_l A[seg,l] * B[idx[p],l]
 // (CSR: A = W, B = T';  CSC: A = T', B = W -- the products commute, the sums run in the same order)
-// Shifted mode (SH): the stored value is S[p] = (m[p] - w0) E[p] + w0 x[p]  (m = 1 without entry weights).
+// Shifted mode (SH == 1): the stored value is S[p] = (m[p] - w0) E[p] + w0 x[p]  (m = 1 without entry weights).
+// Rank-one mode (SH == 2, unstored weights u = w0 (a_i b_j), DESIGN.md §1 row f8): wgt holds mt = m - u per entry
+// (sp_mtilde_kernel) and S[p] = mt E[p] + u x[p]; ab = a_i b_j from the segment's and the gathered entry's vector.
 // ------------------------------------------------------------------------------------------------
-template <typename T, bool SH>
-RRI_DEVINL T sp_stored(T e, T x, const T* __restrict__ wgt, int64_t p, T w0)
+template <typename T, int SH>
+RRI_DEVINL T sp_stored(T e, T x, const T* __restrict__ wgt, int64_t p, T w0, T ab)
 {
-    if constexpr (SH) return fma(sub_rn(wgt ? wgt[p] : T(1), w0), e, mul_rn(w0, x));
+    if constexpr (SH == 1) return fma(sub_rn(wgt ? wgt[p] : T(1), w0), e, mul_rn(w0, x));
+    if constexpr (SH == 2) return fma(wgt[p], e, mul_rn(mul_rn(w0, ab), x));
     return e;
 }
 
-template <typename T, int V, int G, bool SH>
+// a_i b_j of entry p of segment s (a missing vector is all ones); only the rank-one mode reads the vectors
+template <typename T, int SH>
+RRI_DEVINL T sp_ab(const T* __restrict__ vseg, const T* __restrict__ vidx, int64_t s, int32_t j)
+{
+    if constexpr (SH == 2) return mul_rn(vseg ? vseg[s] : T(1), vidx ? vidx[j] : T(1));
+    return T(1);
+}
+
+template <typename T, int V, int G, int SH>
 __global__ void __launch_bounds__(256)
 sp_residual_kernel(const int64_t* __restrict__ ptr, const int32_t* __restrict__ idx, const T* __restrict__ x,
                    const T* __restrict__ A, const T* __restrict__ B, int k, T* __restrict__ E, int64_t nseg,
-                   const T* __restrict__ wgt, T w0)
+                   const T* __restrict__ wgt, T w0, const T* __restrict__ vseg, const T* __restrict__ vidx)
 {
     constexpr int GPB = 256 / G;
     const int lane = threadIdx.x % G, g = threadIdx.x / G;
@@ -176,32 +187,35 @@ sp_residual_kernel(const int64_t* __restrict__ ptr, const int32_t* __restrict__ 
                     for (int v = 0; v < V; ++v) acc = fma(-x1.v[v], x2.v[v], acc);
                 }
             }
-            E[p] = sp_stored<T, SH>(acc, x[p], wgt, p, w0);
+            E[p] = sp_stored<T, SH>(acc, x[p], wgt, p, w0, sp_ab<T, SH>(vseg, vidx, s, idx[p]));
         }
     }
 }
 
-template <typename T, int V, bool SH>
-static void residual_dispatch(const SpSide& s, const T* A, const T* B, int k, T w0, int sm_count, cudaStream_t st)
+template <typename T, int V, int SH>
+static void residual_dispatch(const SpSide& s, const T* A, const T* B, int k, T w0, const T* vseg, const T* vidx,
+                              int sm_count, cudaStream_t st)
 {
     const T* w = (const T*)s.wgt;
     if (s.group == 256) {
         sp_residual_kernel<T, V, 256, SH><<<cap_blocks(s.nseg, sm_count, 8), 256, 0, st>>>(s.ptr, s.idx, (const T*)s.x, A, B, k,
-                                                                                            (T*)s.E, s.nseg, w, w0);
+                                                                                            (T*)s.E, s.nseg, w, w0, vseg, vidx);
     } else {
         sp_residual_kernel<T, V, 32, SH><<<cap_blocks((s.nseg + 7) / 8, sm_count, 8), 256, 0, st>>>(s.ptr, s.idx, (const T*)s.x, A,
-                                                                                                     B, k, (T*)s.E, s.nseg, w, w0);
+                                                                                                     B, k, (T*)s.E, s.nseg, w, w0,
+                                                                                                     vseg, vidx);
     }
 }
 
 // Row-orientation residual with the segment's own factor row staged in shared memory and the gathered rows read
 // with 16-byte loads: B has a padded row stride ldb (multiple of 16 bytes, pad columns zero), so an entry costs
 // ceil(k/V) vector loads -- half the L1 tag look-ups of the 8-byte version at k = 50 -- and the own row costs none.
-template <typename T, int G, bool SH>
+template <typename T, int G, int SH>
 __global__ void __launch_bounds__(256)
 sp_residual_rows_kernel(const int64_t* __restrict__ ptr, const int32_t* __restrict__ idx, const T* __restrict__ x,
                         const T* __restrict__ A, int64_t lda, const T* __restrict__ B, int ldb, int k,
-                        T* __restrict__ E, int64_t nseg, const T* __restrict__ wgt, T w0)
+                        T* __restrict__ E, int64_t nseg, const T* __restrict__ wgt, T w0, const T* __restrict__ vseg,
+                        const T* __restrict__ vidx)
 {
     using V = typename Vec<T>::type;
     constexpr int VN = Vec<T>::N;
@@ -226,31 +240,34 @@ sp_residual_rows_kernel(const int64_t* __restrict__ ptr, const int32_t* __restri
 #pragma unroll
                 for (int v = 0; v < VN; ++v) acc = fma(-a[v], c[v], acc);
             }
-            E[p] = sp_stored<T, SH>(acc, x[p], wgt, p, w0);
+            E[p] = sp_stored<T, SH>(acc, x[p], wgt, p, w0, sp_ab<T, SH>(vseg, vidx, s, idx[p]));
         }
     }
 }
 
-template <typename T, bool SH>
-static void residual_rows_dispatch(const SpSide& s, const T* A, int64_t lda, const T* B, int ldb, int k, T w0, int sm_count,
-                                   cudaStream_t st)
+template <typename T, int SH>
+static void residual_rows_dispatch(const SpSide& s, const T* A, int64_t lda, const T* B, int ldb, int k, T w0, const T* vseg,
+                                   const T* vidx, int sm_count, cudaStream_t st)
 {
     const T* w = (const T*)s.wgt;
     if (s.group == 256)
         sp_residual_rows_kernel<T, 256, SH><<<cap_blocks(s.nseg, sm_count, 8), 256, 0, st>>>(s.ptr, s.idx, (const T*)s.x, A, lda, B,
-                                                                                             ldb, k, (T*)s.E, s.nseg, w, w0);
+                                                                                             ldb, k, (T*)s.E, s.nseg, w, w0,
+                                                                                             vseg, vidx);
     else
         sp_residual_rows_kernel<T, 32, SH><<<cap_blocks((s.nseg + 7) / 8, sm_count, 8), 256, 0, st>>>(s.ptr, s.idx, (const T*)s.x, A,
                                                                                                       lda, B, ldb, k, (T*)s.E, s.nseg,
-                                                                                                      w, w0);
+                                                                                                      w, w0, vseg, vidx);
 }
 
+// (rank-one mode when a vector is given: s.wgt is then the mt copy of this orientation)
 template <typename T>
 void launch_sp_residual_rows(const SpSide& s, const T* A, int64_t lda, const T* B, int ldb, int k, double w0, int sm_count,
-                             cudaStream_t st)
+                             cudaStream_t st, const T* vseg, const T* vidx)
 {
-    if (w0 > 0.0) residual_rows_dispatch<T, true>(s, A, lda, B, ldb, k, (T)w0, sm_count, st);
-    else residual_rows_dispatch<T, false>(s, A, lda, B, ldb, k, T(0), sm_count, st);
+    if (w0 > 0.0 && (vseg || vidx)) residual_rows_dispatch<T, 2>(s, A, lda, B, ldb, k, (T)w0, vseg, vidx, sm_count, st);
+    else if (w0 > 0.0) residual_rows_dispatch<T, 1>(s, A, lda, B, ldb, k, (T)w0, nullptr, nullptr, sm_count, st);
+    else residual_rows_dispatch<T, 0>(s, A, lda, B, ldb, k, T(0), nullptr, nullptr, sm_count, st);
 }
 
 // dst[p] = src[perm[p]]: the column copy of the residual taken from the row copy (bit-identical by construction)
@@ -281,21 +298,24 @@ void launch_sp_gather(const uint32_t* perm, const T* src, T* dst, int64_t nnz, i
 // (A variant that staged the gathered k-vectors of 32 entries through shared memory was measured slower than this
 // direct kernel -- 9.5 ms against 5.9 ms at nnz = 1e8, k = 50, profiles/r01_sparse_bench_v2_staged.log -- and was
 // removed; the shipped restart path is sp_residual_rows_kernel + sp_gather_kernel above.)
-template <typename T, bool SH>
-static void residual_vec_dispatch(const SpSide& s, const T* A, const T* B, int k, T w0, int sm_count, cudaStream_t st)
+template <typename T, int SH>
+static void residual_vec_dispatch(const SpSide& s, const T* A, const T* B, int k, T w0, const T* vseg, const T* vidx,
+                                  int sm_count, cudaStream_t st)
 {
     const uintptr_t al = reinterpret_cast<uintptr_t>(A) | reinterpret_cast<uintptr_t>(B);
     constexpr int VMAX = 16 / (int)sizeof(T);
-    if (VMAX == 4 && k % 4 == 0 && (al & 15) == 0) residual_dispatch<T, VMAX, SH>(s, A, B, k, w0, sm_count, st);
-    else if (k % 2 == 0 && (al & (2 * sizeof(T) - 1)) == 0) residual_dispatch<T, 2, SH>(s, A, B, k, w0, sm_count, st);
-    else residual_dispatch<T, 1, SH>(s, A, B, k, w0, sm_count, st);
+    if (VMAX == 4 && k % 4 == 0 && (al & 15) == 0) residual_dispatch<T, VMAX, SH>(s, A, B, k, w0, vseg, vidx, sm_count, st);
+    else if (k % 2 == 0 && (al & (2 * sizeof(T) - 1)) == 0) residual_dispatch<T, 2, SH>(s, A, B, k, w0, vseg, vidx, sm_count, st);
+    else residual_dispatch<T, 1, SH>(s, A, B, k, w0, vseg, vidx, sm_count, st);
 }
 
 template <typename T>
-void launch_sp_residual(const SpSide& s, const T* A, const T* B, int k, double w0, int sm_count, cudaStream_t st)
+void launch_sp_residual(const SpSide& s, const T* A, const T* B, int k, double w0, int sm_count, cudaStream_t st,
+                        const T* vseg, const T* vidx)
 {
-    if (w0 > 0.0) residual_vec_dispatch<T, true>(s, A, B, k, (T)w0, sm_count, st);
-    else residual_vec_dispatch<T, false>(s, A, B, k, T(0), sm_count, st);
+    if (w0 > 0.0 && (vseg || vidx)) residual_vec_dispatch<T, 2>(s, A, B, k, (T)w0, vseg, vidx, sm_count, st);
+    else if (w0 > 0.0) residual_vec_dispatch<T, 1>(s, A, B, k, (T)w0, nullptr, nullptr, sm_count, st);
+    else residual_vec_dispatch<T, 0>(s, A, B, k, T(0), nullptr, nullptr, sm_count, st);
 }
 
 // ------------------------------------------------------------------------------------------------
@@ -710,10 +730,10 @@ static int sp_pass_dispatch(const SpSide& s, const Quad<T>* Q, const T* own_po, 
 
 template <typename T>
 int launch_sp_pass(const SpSide& s, const void* quad, const T* own_po, const T* own_pn, const T* own_cur,
-                   T* own_save, T* numer, T* denom, double w0, int sm_count, cudaStream_t st)
+                   T* own_save, T* numer, T* denom, double w0, int sm_count, cudaStream_t st, bool shifted)
 {
     const Quad<T>* Q = (const Quad<T>*)quad;
-    if (w0 > 0.0) return sp_pass_dispatch<T, true>(s, Q, own_po, own_pn, own_cur, own_save, numer, denom, (T)w0, sm_count, st);
+    if (w0 > 0.0 || shifted) return sp_pass_dispatch<T, true>(s, Q, own_po, own_pn, own_cur, own_save, numer, denom, (T)w0, sm_count, st);
     return sp_pass_dispatch<T, false>(s, Q, own_po, own_pn, own_cur, own_save, numer, denom, T(0), sm_count, st);
 }
 
@@ -751,6 +771,38 @@ sp_objective_kernel(const T* __restrict__ E, const T* __restrict__ x, const T* _
     }
 }
 
+// Rank-one unstored weights (DESIGN.md §1 row f8): the same three sums with s2 = sum a_i b_j (x - E)^2; a warp per row
+// (grid-stride over the rows, fixed order), b_j gathered by the column index
+template <typename T>
+__global__ void __launch_bounds__(256)
+sp_objective_rows_kernel(const int64_t* __restrict__ ptr, const int32_t* __restrict__ idx, const T* __restrict__ E,
+                         const T* __restrict__ x, const T* __restrict__ wgt, int64_t nseg, const T* __restrict__ va,
+                         const T* __restrict__ vb, double* __restrict__ part)
+{
+    __shared__ double red[3][8];
+    const int lane = threadIdx.x & 31;
+    double s0 = 0.0, s1 = 0.0, s2 = 0.0;
+    for (int64_t r = ((int64_t)blockIdx.x * blockDim.x + threadIdx.x) >> 5; r < nseg; r += ((int64_t)gridDim.x * blockDim.x) >> 5) {
+        const double ai = va ? (double)va[r] : 1.0;
+        for (int64_t p = ptr[r] + lane; p < ptr[r + 1]; p += 32) {
+            const double m = wgt ? (double)wgt[p] : 1.0;
+            const double e = (double)E[p], v = (double)x[p];
+            const double ab = vb ? ai * (double)vb[idx[p]] : ai;
+            s0 += m * e * e;
+            s1 += m * v * v;
+            s2 += ab * (v - e) * (v - e);
+        }
+    }
+    s0 = warp_sum(s0); s1 = warp_sum(s1); s2 = warp_sum(s2);
+    if (lane == 0) { red[0][threadIdx.x >> 5] = s0; red[1][threadIdx.x >> 5] = s1; red[2][threadIdx.x >> 5] = s2; }
+    __syncthreads();
+    if (threadIdx.x < 3) {
+        double s = 0.0;
+        for (int w = 0; w < 8; ++w) s += red[threadIdx.x][w];
+        part[3 * (int64_t)blockIdx.x + threadIdx.x] = s;
+    }
+}
+
 __global__ void sp_objective_finalize_kernel(const double* __restrict__ part, int blocks, double* __restrict__ out)
 {
     if (threadIdx.x < 2) {
@@ -761,7 +813,8 @@ __global__ void sp_objective_finalize_kernel(const double* __restrict__ part, in
 }
 
 // out[0] = 0.5 (sum m E^2 + w0 (<W'W, T T'> - sum (x - E)^2)) = 0.5 sum M (X - W T)^2 over all n x d entries,
-// out[1] = sum m x^2; <W'W, T T'> from the fp64 Gram partials gw [k][cw][k] and gt [k][ct][k] (fixed order)
+// out[1] = sum m x^2; <W'W, T T'> from the fp64 Gram partials gw [k][cw][k] and gt [k][ct][k] (fixed order).  With
+// rank-one weights the Grams are W' diag(a) W and T diag(b) T' and s2 carries a_i b_j.
 __global__ void __launch_bounds__(256)
 sp_objective_implicit_finalize_kernel(const double* __restrict__ part, int blocks, const double* __restrict__ gw, int cw,
                                       const double* __restrict__ gt, int ct, int k, double w0, double* __restrict__ out)
@@ -789,11 +842,17 @@ sp_objective_implicit_finalize_kernel(const double* __restrict__ part, int block
 
 template <typename T>
 void launch_sp_objective(const SpSide& s, int64_t nnz, double* part, double* out, double w0, const double* gw, int cw,
-                         const double* gt, int ct, int k, cudaStream_t st)
+                         const double* gt, int ct, int k, cudaStream_t st, const T* va, const T* vb)
 {
     int blocks = (int)((nnz + 256 * 8 - 1) / (256 * 8));
     if (blocks > 256) blocks = 256;
     if (blocks < 1) blocks = 1;
+    if (w0 > 0.0 && (va || vb)) {
+        sp_objective_rows_kernel<T><<<blocks, 256, 0, st>>>(s.ptr, s.idx, (const T*)s.E, (const T*)s.x, (const T*)s.wgt, s.nseg,
+                                                            va, vb, part);
+        sp_objective_implicit_finalize_kernel<<<1, 256, 0, st>>>(part, blocks, gw, cw, gt, ct, k, w0, out);
+        return;
+    }
     if (w0 > 0.0) {
         sp_objective_kernel<T, true><<<blocks, 256, 0, st>>>((const T*)s.E, (const T*)s.x, (const T*)s.wgt, nnz, part);
         sp_objective_implicit_finalize_kernel<<<1, 256, 0, st>>>(part, blocks, gw, cw, gt, ct, k, w0, out);
@@ -808,9 +867,12 @@ void launch_sp_objective(const SpSide& s, int64_t nnz, double* part, double* out
 // ------------------------------------------------------------------------------------------------
 // Gram rows of F [k, ld] (row r = topic r over len entries): for z < gridDim.z, with t = t0 + z,
 //   part[z][c][s] = sum_{i in chunk c} F[t, i] F[s, i]     (one block per (s, c, z); fixed-order block reduction)
-template <typename T, typename A>
+// WV (rank-one unstored weights, row f8): sum F[t, i] v_i F[s, i] with the weight vector v over the len entries
+// (a for W' diag(a) W, b for T diag(b) T'), the product F[t, i] v_i rounded in A first.
+template <typename T, typename A, bool WV>
 __global__ void __launch_bounds__(256)
-sp_gram_rows_kernel(const T* __restrict__ F, int64_t ld, int64_t len, int k, int t0, int chunks, A* __restrict__ part)
+sp_gram_rows_kernel(const T* __restrict__ F, int64_t ld, int64_t len, int k, int t0, int chunks, A* __restrict__ part,
+                    const T* __restrict__ wv)
 {
     __shared__ A red[8];
     const int s = blockIdx.x, c = blockIdx.y, z = blockIdx.z;
@@ -819,7 +881,11 @@ sp_gram_rows_kernel(const T* __restrict__ F, int64_t ld, int64_t len, int k, int
     const T* __restrict__ a = F + (int64_t)(t0 + z) * ld;
     const T* __restrict__ f = F + (int64_t)s * ld;
     A acc = A(0);
-    for (int64_t i = b + threadIdx.x; i < e; i += 256) acc = fma((A)a[i], (A)f[i], acc);
+    if constexpr (WV) {
+        for (int64_t i = b + threadIdx.x; i < e; i += 256) acc = fma((A)a[i] * (A)wv[i], (A)f[i], acc);
+    } else {
+        for (int64_t i = b + threadIdx.x; i < e; i += 256) acc = fma((A)a[i], (A)f[i], acc);
+    }
     acc = warp_sum(acc);
     if ((threadIdx.x & 31) == 0) red[threadIdx.x >> 5] = acc;
     __syncthreads();
@@ -841,21 +907,25 @@ int sp_gram_chunks(int64_t len, int pairs, int sm_count)
 }
 
 template <typename T, typename A>
-void launch_sp_gram_rows(const T* F, int64_t ld, int64_t len, int k, int t0, int rows, int chunks, A* part, cudaStream_t st)
+void launch_sp_gram_rows(const T* F, int64_t ld, int64_t len, int k, int t0, int rows, int chunks, A* part, cudaStream_t st,
+                         const T* wv)
 {
-    sp_gram_rows_kernel<T, A><<<dim3((unsigned)k, (unsigned)chunks, (unsigned)rows), 256, 0, st>>>(F, ld, len, k, t0, chunks, part);
+    const dim3 grid((unsigned)k, (unsigned)chunks, (unsigned)rows);
+    if (wv) sp_gram_rows_kernel<T, A, true><<<grid, 256, 0, st>>>(F, ld, len, k, t0, chunks, part, wv);
+    else sp_gram_rows_kernel<T, A, false><<<grid, 256, 0, st>>>(F, ld, len, k, t0, chunks, part, nullptr);
 }
 
 // The vector-c solve of wrri_final_kernel with the rank-k part of the statistic added first:
 //   numer_i = sum_p numer_part[p][i] - w0 sum_{s != t} g_s F[s, i],   denom_i = sum_p denom_part[p][i] + w0 g_t
 // g = the Gram row of topic t (sum of its `gchunks` partials), F [k, ldf] the factor being updated (rows s != t only:
-// row t is the one written).
+// row t is the one written).  sc (rank-one unstored weights, row f8): w0 is w0 sc_i for entry i -- b_j in a T-step,
+// a_i in a W-step -- in both terms.
 template <typename T>
 __global__ void __launch_bounds__(256)
 sp_implicit_final_kernel(const T* __restrict__ numer_part, const T* __restrict__ denom_part, int parts, int64_t len,
                          const T* __restrict__ gpart, int gchunks, int k, int t, const T* __restrict__ F, int64_t ldf,
                          T w0, T reg_l1, T reg_l2, T eps, T ub, int has_ub, T* __restrict__ out, int64_t out_stride,
-                         T* __restrict__ out2, int64_t out2_stride, int* __restrict__ flags)
+                         T* __restrict__ out2, int64_t out2_stride, int* __restrict__ flags, const T* __restrict__ sc)
 {
     __shared__ T g[256];
     for (int s = threadIdx.x; s < k; s += blockDim.x) {
@@ -875,8 +945,9 @@ sp_implicit_final_kernel(const T* __restrict__ numer_part, const T* __restrict__
     T corr = T(0);
     for (int s = 0; s < k; ++s)
         if (s != t) corr = fma(g[s], F[(int64_t)s * ldf + i], corr);
-    nu = fma(-w0, corr, nu);
-    de = fma(w0, g[t], de);
+    const T wi = sc ? mul_rn(w0, sc[i]) : w0;
+    nu = fma(-wi, corr, nu);
+    de = fma(wi, g[t], de);
     bool unb = false;
     const T x = solve_vector_c<T>(nu - reg_l1, de + reg_l2, eps, ub, has_ub != 0, unb);
     out[i * out_stride] = x;
@@ -887,33 +958,83 @@ sp_implicit_final_kernel(const T* __restrict__ numer_part, const T* __restrict__
 template <typename T>
 void launch_sp_implicit_final(const T* numer_part, const T* denom_part, int parts, int64_t len, const T* gpart, int gchunks,
                               int k, int t, const T* F, int64_t ldf, double w0, const SolveArgs& a, T* out,
-                              int64_t out_stride, T* out2, int64_t out2_stride, int* flags, cudaStream_t st)
+                              int64_t out_stride, T* out2, int64_t out2_stride, int* flags, cudaStream_t st, const T* sc)
 {
     sp_implicit_final_kernel<T><<<(unsigned)((len + 255) / 256), 256, 0, st>>>(numer_part, denom_part, parts, len, gpart,
         gchunks, k, t, F, ldf, (T)w0, (T)a.reg_l1, (T)a.reg_l2, (T)a.eps, (T)a.ub, a.has_ub, out, out_stride, out2,
-        out2_stride, flags);
+        out2_stride, flags, sc);
+}
+
+// ------------------------------------------------------------------------------------------------
+// rank-one unstored weights u_ij = w0 (a_i b_j) (rri_set_unstored_weight_vectors, DESIGN.md §1 row f8), once per bind
+// ------------------------------------------------------------------------------------------------
+// err |= bit unless every v[i] is finite and >= 0
+template <typename T>
+__global__ void sp_check_weights_kernel(const T* __restrict__ v, int64_t len, int bit, int* __restrict__ err)
+{
+    bool bad = false;
+    for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < len; i += (int64_t)gridDim.x * blockDim.x)
+        bad |= !(isfinite((double)v[i]) && v[i] >= T(0));
+    if (__syncthreads_or(bad) && threadIdx.x == 0) atomicOr(err, bit);
+}
+
+template <typename T>
+void launch_sp_check_weights(const T* v, int64_t len, int bit, int* err, int sm_count, cudaStream_t st)
+{
+    if (v && len > 0) sp_check_weights_kernel<T><<<cap_blocks((len + 255) / 256, sm_count, 4), 256, 0, st>>>(v, len, bit, err);
+}
+
+// mt[p] = m[p] - w0 (a_i b_j) in CSR order (m = 1 without entry weights; a warp per row).  The column copy is the
+// permutation of it (launch_sp_gather), so both orientations hold the same bits.
+template <typename T>
+__global__ void __launch_bounds__(256)
+sp_mtilde_kernel(const int64_t* __restrict__ rowptr, const int32_t* __restrict__ col, const T* __restrict__ wgt, int64_t n,
+                 const T* __restrict__ va, const T* __restrict__ vb, T w0, T* __restrict__ mt)
+{
+    const int lane = threadIdx.x & 31;
+    for (int64_t r = ((int64_t)blockIdx.x * blockDim.x + threadIdx.x) >> 5; r < n; r += ((int64_t)gridDim.x * blockDim.x) >> 5) {
+        const T ai = va ? va[r] : T(1);
+        for (int64_t p = rowptr[r] + lane; p < rowptr[r + 1]; p += 32) {
+            const T u = mul_rn(w0, mul_rn(ai, vb ? vb[col[p]] : T(1)));
+            mt[p] = sub_rn(wgt ? wgt[p] : T(1), u);
+        }
+    }
+}
+
+template <typename T>
+void launch_sp_mtilde(const int64_t* rowptr, const int32_t* col, const T* wgt, int64_t n, const T* va, const T* vb,
+                      double w0, T* mt, int sm_count, cudaStream_t st)
+{
+    sp_mtilde_kernel<T><<<cap_blocks((n + 7) / 8, sm_count, 8), 256, 0, st>>>(rowptr, col, wgt, n, va, vb, (T)w0, mt);
 }
 
 #define RRI_INST(T)                                                                                                 \
     template int sp_build_csc<T>(const int64_t*, const int32_t*, const T*, const T*, int64_t, int64_t, int64_t,    \
                                  int64_t*, int32_t*, T*, T*, uint32_t*, int, int*, cudaStream_t);                  \
-    template void launch_sp_residual<T>(const SpSide&, const T*, const T*, int, double, int, cudaStream_t);        \
+    template void launch_sp_residual<T>(const SpSide&, const T*, const T*, int, double, int, cudaStream_t, const T*, \
+                                        const T*);                                                                 \
     template void launch_sp_residual_rows<T>(const SpSide&, const T*, int64_t, const T*, int, int, double, int,    \
-                                             cudaStream_t);                                                        \
+                                             cudaStream_t, const T*, const T*);                                    \
     template void launch_sp_gather<T>(const uint32_t*, const T*, T*, int64_t, int, cudaStream_t);                  \
     template void launch_sp_pack<T>(const T*, const T*, const T*, const T*, void*, int64_t, cudaStream_t);         \
     template int launch_sp_pass<T>(const SpSide&, const void*, const T*, const T*, const T*, T*, T*, T*, double,   \
-                                   int, cudaStream_t);                                                             \
+                                   int, cudaStream_t, bool);                                                       \
     template void launch_sp_objective<T>(const SpSide&, int64_t, double*, double*, double, const double*, int,      \
-                                         const double*, int, int, cudaStream_t);                                   \
+                                         const double*, int, int, cudaStream_t, const T*, const T*);               \
     template void launch_sp_implicit_final<T>(const T*, const T*, int, int64_t, const T*, int, int, int, const T*, \
                                               int64_t, double, const SolveArgs&, T*, int64_t, T*, int64_t, int*,   \
-                                              cudaStream_t);
+                                              cudaStream_t, const T*);                                             \
+    template void launch_sp_check_weights<T>(const T*, int64_t, int, int*, int, cudaStream_t);                     \
+    template void launch_sp_mtilde<T>(const int64_t*, const int32_t*, const T*, int64_t, const T*, const T*, double, \
+                                      T*, int, cudaStream_t);
 RRI_INST(float)
 RRI_INST(double)
 // Gram rows: accumulated in the element type inside a half-step, in fp64 for the objective
-template void launch_sp_gram_rows<float, float>(const float*, int64_t, int64_t, int, int, int, int, float*, cudaStream_t);
-template void launch_sp_gram_rows<float, double>(const float*, int64_t, int64_t, int, int, int, int, double*, cudaStream_t);
-template void launch_sp_gram_rows<double, double>(const double*, int64_t, int64_t, int, int, int, int, double*, cudaStream_t);
+template void launch_sp_gram_rows<float, float>(const float*, int64_t, int64_t, int, int, int, int, float*, cudaStream_t,
+                                                const float*);
+template void launch_sp_gram_rows<float, double>(const float*, int64_t, int64_t, int, int, int, int, double*, cudaStream_t,
+                                                 const float*);
+template void launch_sp_gram_rows<double, double>(const double*, int64_t, int64_t, int, int, int, int, double*, cudaStream_t,
+                                                  const double*);
 
 }  // namespace rri

@@ -35,6 +35,38 @@ def check_unstored_weight(w0, sparse, unstored):
     return w0
 
 
+def check_unstored_vectors(a, b, n, d, w0):
+    """the rank-one unstored weights u_ij = w0 a_i b_j: (a, b) with a over the n rows and b over the d columns, each None
+    (all ones), a CUDA tensor or a float64 NumPy array; ValueError for a vector without w0 > 0, a vector that is not 1-D
+    of the right length, or one with a negative or non-finite entry"""
+    out = []
+    for v, name, length in ((a, 'unstored_row_weight', n), (b, 'unstored_col_weight', d)):
+        if v is None:
+            out.append(None)
+            continue
+        if not w0 > 0:
+            raise ValueError('%s scales the unstored weight: it needs unstored_weight > 0' % name)
+        if isinstance(v, torch.Tensor) and v.is_cuda:
+            if v.dim() != 1 or int(v.numel()) != length:
+                raise ValueError('%s must be 1-D of length %d (got shape %s)' % (name, length, tuple(v.shape)))
+            if not v.is_floating_point() or not bool(torch.all(torch.isfinite(v) & (v >= 0))):
+                raise ValueError('%s must be finite and >= 0' % name)
+            out.append(v)
+            continue
+        if isinstance(v, torch.Tensor):
+            v = v.detach().numpy()
+        try:
+            v = np.asarray(v, dtype=np.float64)
+        except (TypeError, ValueError):
+            raise ValueError('%s must be a vector of numbers' % name)
+        if v.ndim != 1 or v.shape[0] != length:
+            raise ValueError('%s must be 1-D of length %d (got shape %s)' % (name, length, v.shape))
+        if not np.all(np.isfinite(v)) or np.any(v < 0):
+            raise ValueError('%s must be finite and >= 0' % name)
+        out.append(v)
+    return tuple(out)
+
+
 class NcclComm(object):
     """An ncclComm_t created by the engine library from an id broadcast over torch.distributed."""
 
@@ -79,6 +111,10 @@ class RRIEngine(object):
            a 0 of weight w0, the stored ones with their W_mat weight (1 without W_mat) -- the dense masked problem with
            M = w0 off the stored entries, without forming it (rri_set_unstored_weight).  0 (default) is the plain
            observed-entries binding.  One GPU, one model.
+    unstored_row_weight, unstored_col_weight: rank-one unstored weights (with unstored_weight > 0): the unstored entry
+           (i, j) weighs w0 a_i b_j, a over the n rows, b over the d columns (1-D NumPy arrays or tensors, >= 0; None =
+           ones) -- user- / item-oriented and item-popularity weights of one-class recommenders
+           (rri_set_unstored_weight_vectors).  The engine keeps its own copies.
     order: 'rri' (reference-exact interleaved order, nmf.py:415-476) or 'hals' (block order).
     math : 'ieee' or 'tf32' (tcgen05 tensor-core contraction; float32 + hals only).
     models: None (one model), or b >= 1 models of rank k each on the same binding (rri_set_models: dense unmasked X,
@@ -93,7 +129,7 @@ class RRIEngine(object):
     """
 
     def __init__(self, X, k, W_mat=None, order='rri', math='ieee', comm=None, unstored='missing', models=None,
-                 unstored_weight=0.0):
+                 unstored_weight=0.0, unstored_row_weight=None, unstored_col_weight=None):
         if not isinstance(X, torch.Tensor) or not X.is_cuda:
             raise _lib.RriError('RRIEngine needs X resident on a CUDA device (no CPU fallback)')
         if X.dim() != 2:
@@ -116,6 +152,8 @@ class RRIEngine(object):
             raise ValueError('several models take dense data; unstored_weight needs one model')
         if self.unstored_weight > 0 and comm is not None and comm.world > 1:
             raise NotImplementedError('unstored_weight runs on one GPU (no row shards)')
+        self.unstored_vectors = check_unstored_vectors(unstored_row_weight, unstored_col_weight, int(X.shape[0]),
+                                                       int(X.shape[1]), self.unstored_weight)
         if not self.sparse and X.stride(1) != 1:
             X = X.contiguous()
         self.lib = _lib.load()
@@ -164,6 +202,11 @@ class RRIEngine(object):
         if self.sparse:
             if self.unstored_weight > 0:
                 check(self.lib.rri_set_unstored_weight(self.h, self.unstored_weight))
+            if any(v is not None for v in self.unstored_vectors):
+                a, b = (None if v is None else torch.as_tensor(v).to(device=self.device, dtype=self.dtype).contiguous()
+                        for v in self.unstored_vectors)
+                torch.cuda.current_stream(self.device).synchronize()     # (the library copies them on the default stream)
+                check(self.lib.rri_set_unstored_weight_vectors(self.h, _ptr(a), _ptr(b)))
             self._bind_csr(X, W_mat)
             return
         mk = _lib.RRI_MASK_NONE

@@ -52,6 +52,10 @@ their own (implicit feedback, one-class recommenders: unobserved pairs count as 
 ones with their W_mat weight, 1 without W_mat).  The result equals nmf(X.toarray(), ..., W_mat=M) with the dense M that
 holds w0 at every unstored entry, up to the summation order, in both orders -- but nothing of size n x d is formed:
 per entry the sweep moves the bytes of w0 = 0, plus O((n + d) k) per topic.  One GPU (no comm), no fix_W.
+The keyword-only `unstored_row_weight` a (length n) and `unstored_col_weight` b (length d), NumPy or torch vectors >= 0,
+make that weight rank-one: the unstored entry (i, j) weighs w0 a_i b_j (user- / item-oriented and item-popularity
+schemes of one-class collaborative filtering; None = ones).  The result equals nmf(X.toarray(), ..., W_mat=M) with that
+M; an unweighted sweep then streams the bytes of a weighted one.  They need unstored_weight > 0.
 """
 import logging
 import time
@@ -63,7 +67,7 @@ import torch
 from . import _lib
 from ._device_init import initialize_nmf_torch
 from ._host import initialize_nmf, normalize
-from .engine import RRIEngine, EPS_DIV_BY_ZERO, check_unstored_weight
+from .engine import RRIEngine, EPS_DIV_BY_ZERO, check_unstored_weight, check_unstored_vectors
 
 logger = logging.getLogger(__name__)
 eps_div_by_zero = EPS_DIV_BY_ZERO          # nmf.py:52
@@ -90,7 +94,7 @@ class DeviceObjective(object):
                                              reuse_last_sweep=self._after_sweep, **self.regs)
             self._after_sweep = False
         elif self._rebuild is not None:
-            X, W_mat, device, dtype, order, unstored, unstored_weight = self._rebuild
+            X, W_mat, device, dtype, order, unstored, unstored_weight, vectors = self._rebuild
             device = torch.device(device)
             with torch.cuda.device(device):
                 if _is_sparse(X):
@@ -99,7 +103,8 @@ class DeviceObjective(object):
                     Xd, Md = _to_device(X, device, dtype), _mask_to_device(W_mat, device, dtype)
                 # (a zero-filled sparse binding evaluates in the order of the fit; every other binding in 'rri')
                 eng = RRIEngine(Xd, int(np.shape(self.W)[1]), W_mat=Md, order=order if unstored == 'zero' else 'rri',
-                                unstored=unstored, unstored_weight=unstored_weight)
+                                unstored=unstored, unstored_weight=unstored_weight, unstored_row_weight=vectors[0],
+                                unstored_col_weight=vectors[1])
                 try:
                     self.obj = eng.objective(_to_device(self.W, device, dtype).contiguous(),
                                              _to_device(self.T, device, dtype).contiguous(), **self.regs)
@@ -107,11 +112,14 @@ class DeviceObjective(object):
                     eng.close()
         return self.obj
 
-    def _detach(self, X, W_mat, W, T, device, dtype, order, unstored='missing', unstored_weight=0.0):
-        """called by nmf() before it closes the engine"""
+    def _detach(self, X, W_mat, W, T, device, dtype, order, unstored='missing', unstored_weight=0.0,
+                unstored_vectors=(None, None)):
+        """called by nmf() before it closes the engine (the rank-one unstored weights are kept as host arrays)"""
         self.engine = None
         self.W, self.T = W, T
-        self._rebuild = (X, W_mat, str(device), dtype, order, unstored, unstored_weight)
+        vectors = tuple(None if v is None else (v.detach().cpu().numpy() if isinstance(v, torch.Tensor) else np.asarray(v))
+                        for v in unstored_vectors)
+        self._rebuild = (X, W_mat, str(device), dtype, order, unstored, unstored_weight, vectors)
 
     def __getstate__(self):
         st = dict(self.__dict__)
@@ -318,7 +326,7 @@ def nmf(X, k, w_row=None, W_mat=None, fix_W=False, fix_T=False, random_state=Non
         ind_rows_to_store=None, eps_gauss_t=None, delta_gauss_t=None,
         *, device=None, update_order=None, math='ieee', comm=None, engine=None, sweeps_per_call=16,
         init_on_device=None, return_reconstruction_err=False, sparse_refresh_every=1, objective='auto',
-        unstored='missing', unstored_weight=0.0):
+        unstored='missing', unstored_weight=0.0, unstored_row_weight=None, unstored_col_weight=None):
     """Non-negative factorisation X ~ W T by rank-one residue iteration.  See the reference docstring
     (nmf.py:109-269) for the arguments; returns {'W', 'T', 'iter_cputime', 'random_state'[, 'obj_history',
     'obj_calculator', 'diagnostics']} (nmf.py:551-560).  W and T come back as the kind of array X was
@@ -336,6 +344,8 @@ def nmf(X, k, w_row=None, W_mat=None, fix_W=False, fix_T=False, random_state=Non
             raise NotImplementedError('unstored_weight runs on one GPU (row shards are not implemented)')
         if fix_W:
             raise NotImplementedError('fix_W=True is not available with unstored_weight')
+    unstored_vectors = check_unstored_vectors(unstored_row_weight, unstored_col_weight, X.shape[0], X.shape[1],
+                                              unstored_weight)
     if zero_filled:
         if W_mat is not None:
             raise ValueError("unstored='zero' takes no W_mat: weights on a zero-filled matrix would be a dense n x d object")
@@ -444,7 +454,8 @@ def nmf(X, k, w_row=None, W_mat=None, fix_W=False, fix_T=False, random_state=Non
             # (fix_T: the W-only sweeps are the same in both orders; on zero-filled data they run on a block-order
             # binding, which holds no interleaved-order partials)
             engine = RRIEngine(Xd, k, W_mat=Md, order='hals' if zero_filled and fix_T else update_order, math=math,
-                               comm=comm, unstored=unstored, unstored_weight=unstored_weight)
+                               comm=comm, unstored=unstored, unstored_weight=unstored_weight,
+                               unstored_row_weight=unstored_vectors[0], unstored_col_weight=unstored_vectors[1])
         timing['engine_setup_s'] = time.perf_counter() - _t1       # workspace, transposed copy of X, peer mapping
         try:
             W, T = _device_start(engine, Xd, W_mat, Md, k, init, random_state, t_row_sum, w_row_sum, W0, T0,
@@ -463,7 +474,7 @@ def nmf(X, k, w_row=None, W_mat=None, fix_W=False, fix_T=False, random_state=Non
             if 'obj_calculator' in out and own_engine:
                 # the calculator outlives this call without pinning device memory (and stays picklable)
                 out['obj_calculator']._detach(X, W_mat_user, out['W'], out['T'], device, dtype, engine.order,
-                                              engine.unstored, engine.unstored_weight)
+                                              engine.unstored, engine.unstored_weight, engine.unstored_vectors)
             return out
         finally:
             if own_engine:
@@ -531,7 +542,7 @@ def nmf_models(X, k, random_state=None, W_in=None, T_in=None, **kwargs):
     Supported: dense unmasked X (fp32 / fp64), update_order='hals', math 'ieee' / 'tf32', the four regularisers,
     w_row_sum / t_row_sum as upper bounds, project_W_each_iter, do_final_project_W, compute_obj_each_iter, objective,
     eps_stop, max_iter, max_time, sweeps_per_call, init_on_device, device.  Everything else raises before any device
-    work: NotImplementedError for W_mat, sparse X, comm, update_order='rri', fix_W / fix_T, project_T_each_iter with
+    work: NotImplementedError for W_mat, sparse X, unstored weight vectors, comm, update_order='rri', fix_W / fix_T, project_T_each_iter with
     t_row_sum, early_stop, diagnostics, w_row, the Gaussian mechanism, store_gradients, an engine, and
     return_reconstruction_err; ValueError for lists of different lengths and for ranks outside [1, 256].
     """
@@ -550,6 +561,8 @@ def nmf_models(X, k, random_state=None, W_in=None, T_in=None, **kwargs):
     # ---- what the shared contraction does not serve: refuse before any device work
     if a['W_mat'] is not None:
         raise NotImplementedError('nmf_models takes unmasked data (no W_mat)')
+    if a['unstored_row_weight'] is not None or a['unstored_col_weight'] is not None:
+        raise NotImplementedError('nmf_models takes dense X (no unstored weights)')
     if _is_sparse(X):
         raise NotImplementedError('nmf_models takes dense X')
     if a['comm'] is not None:

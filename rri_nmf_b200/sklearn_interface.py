@@ -277,7 +277,9 @@ class NMF_RS_Estimator(_FactorMixin, sklearn.base.BaseEstimator):
         return self.fit(np.column_stack([I, J]), np.asarray(Xtr[I, J]).ravel())
 
     def transform(self, Xnew):
-        """express Xnew in terms of the fitted topics (sklearn_interface.py:144-156)"""
+        """express Xnew in terms of the fitted topics (sklearn_interface.py:144-156).  Of the rank-one unstored weights
+        in nmf_kwargs, the new rows keep unstored_weight and unstored_col_weight (the items); unstored_row_weight belongs
+        to the fitted rows and is dropped."""
         if self.sparse:
             Xnew = sp.csr_matrix(Xnew, dtype=np.float64)
             Xnew.eliminate_zeros()
@@ -288,7 +290,8 @@ class NMF_RS_Estimator(_FactorMixin, sklearn.base.BaseEstimator):
         soln = nmf(Xnew, self.k, max_iter=4, max_time=7200, project_W_each_iter=False,
                    project_T_each_iter=False, W_mat=mask, T_in=self.T, fix_T=True, reg_w_l1=self.wr1,
                    reg_t_l1=self.tr1, t_row_sum=1.0, w_row_sum=None, reset_topic_method='random',
-                   random_state=self.random_state, **dict(self._device_kwargs(), **self.nmf_kwargs))
+                   random_state=self.random_state,
+                   **dict(self._device_kwargs(), **{a: b for a, b in self.nmf_kwargs.items() if a != 'unstored_row_weight'}))
         return soln['W']
 
     def make_Xpred(self):
