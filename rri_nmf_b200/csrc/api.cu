@@ -192,8 +192,6 @@ struct rri_handle_s {
     void *sp_npart = nullptr, *sp_dpart = nullptr;     // per-block partial sums of a pass: [nblk][nseg] each
     uint32_t* sp_perm = nullptr;       // [nnz] CSR position of every CSC entry
     int sp_ldt = 0;                    // row stride of T' [d, sp_ldt] (k rounded up to 16 bytes: vector gathers)
-    bool sp_refresh_v2 = true;         // residual restart: row copy from the factors, column copy gathered from it
-    bool sp_batched_sums = true;       // per-topic sums once per sweep (2 launches) instead of once per half-step (2k)
     int* sp_err = nullptr;
     // unstored weight (rri_set_unstored_weight): the copies hold the shifted residual S = (m - w0) E + w0 x, and every
     // half-step adds the rank-k part of the statistic from one Gram row of its topic
@@ -792,16 +790,9 @@ static int bind_csr_impl(rri_handle_t h, const int64_t* rowptr, const int32_t* c
         ws_alloc(h, (void**)&h->sp_err, sizeof(int)))
         return 1;
     {
-        const int64_t v = 16 / (int64_t)es;
-        h->ldwt = (n + v - 1) / v * v;
-    }
-    {
-        const char* env = getenv("RRI_SP_REFRESH_V2");
-        h->sp_refresh_v2 = !(env && *env == '0');
-        const char* envb = getenv("RRI_SP_BATCHED_SUMS");
-        h->sp_batched_sums = !(envb && *envb == '0');        // measured: 30.8 -> 29.8 ms per config-4 sweep
         const int v = 16 / (int)es;
-        h->sp_ldt = h->sp_refresh_v2 ? (k + v - 1) / v * v : k;
+        h->ldwt = (n + v - 1) / v * v;
+        h->sp_ldt = (k + v - 1) / v * v;
     }
     if (ws_alloc(h, &h->Wt, es * (size_t)k * h->ldwt) || ws_alloc(h, &h->Tt, es * (size_t)d * h->sp_ldt)) return 1;
     if (ws_alloc(h, (void**)&h->sp_perm, sizeof(uint32_t) * ne)) return 1;
@@ -833,28 +824,25 @@ static int bind_csr_impl(rri_handle_t h, const int64_t* rowptr, const int32_t* c
         launch_sp_gather<T>(h->sp_perm, (const T*)h->sp_mt_csr, (T*)h->sp_mt_csc, nnz, h->sm_count, st);
         h->launches += 2;
     }
-    // blocked passes: the gathered factor is staged through shared memory in blocks of nb records
-    const char* env = getenv("RRI_SP_BLOCKED");
-    const bool blocked = !(env && *env == '0');
-    const char* env16 = getenv("RRI_SP_IDX16");
-    const bool use16 = !(env16 && *env16 == '0');
+    // blocked passes: the gathered factor is staged through shared memory in blocks of nb records, addressed by
+    // 16-bit block-local indices
     size_t part_elems = (size_t)m;
     for (SpSide* sd : {&h->csr, &h->csc}) {
         int nblk = 1;
         const int nb = sp_block_len((int)es, sd->nother, &nblk);
-        if (!blocked || nblk > 64) continue;          // (a very long factor would make the sub-segments too short)
+        if (nblk > 64) continue;                      // (a very long factor would make the sub-segments too short)
         void* p2 = nullptr;
         void* i16 = nullptr;
-        if (ws_alloc(h, &p2, sizeof(int64_t) * (size_t)sd->nseg * (size_t)(nblk + 1))) return 1;
-        if (use16 && ws_alloc(h, &i16, sizeof(uint16_t) * ne)) return 1;
+        if (ws_alloc(h, &p2, sizeof(int64_t) * (size_t)sd->nseg * (size_t)(nblk + 1)) ||
+            ws_alloc(h, &i16, sizeof(uint16_t) * ne))
+            return 1;
         CK(cudaStreamSynchronize(0));
         launch_sp_subptr(sd->ptr, sd->idx, sd->nseg, nblk, nb, (int64_t*)p2, h->sm_count, st);
-        if (use16 && nnz > 0) {
+        if (nnz > 0) {
             launch_sp_local_index(sd->idx, nnz, nb, (uint16_t*)i16, h->sm_count, st);
-            sd->idx16 = (const uint16_t*)i16;
             h->launches++;
         }
-        sd->ptr2 = (const int64_t*)p2; sd->nblk = nblk; sd->nb = nb;
+        sd->ptr2 = (const int64_t*)p2; sd->nblk = nblk; sd->nb = nb; sd->idx16 = (const uint16_t*)i16;
         if ((size_t)nblk * (size_t)sd->nseg > part_elems) part_elems = (size_t)nblk * (size_t)sd->nseg;
         h->launches++;
     }
@@ -1250,12 +1238,11 @@ static int contraction(rri_handle_t h, const T* A, int64_t lda, const T* B, int6
     return 0;
 }
 
-// the Gram matrix of a half-step: on the tensor cores inside the contraction launch (TF32 math, RRI_TC_GRAM=0 to
-// switch off), otherwise the IEEE gram_kernel + fixed-order reduce
+// the Gram matrix of a half-step: on the tensor cores inside the contraction launch (TF32 math), otherwise the IEEE
+// gram_kernel + fixed-order reduce
 static bool gram_in_contraction(rri_handle_t h)
 {
-    static const bool off = [] { const char* e = getenv("RRI_TC_GRAM"); return e && *e == '0'; }();
-    return h->math == RRI_MATH_TF32 && !off;
+    return h->math == RRI_MATH_TF32;
 }
 
 // C = A B' over the data of a block-order half-step: A = X (transpose = false, n x d) or X' (d x n), B [N, K] factor
@@ -1551,28 +1538,22 @@ static SpSide sp_pass_side(rri_handle_t h, const SpSide& s, const void* mt)
 }
 
 template <typename T>
-static void sp_refresh(rri_handle_t h, bool need_csr, bool need_csc, const T* W, cudaStream_t st, bool plain = false)
+static void sp_refresh(rri_handle_t h, bool need_csc, const T* W, cudaStream_t st, bool plain = false)
 {
     // E = X - W T on the observed entries, from the current factors (with an unstored weight, unless `plain`: the
-    // shifted residual (m - w0) E + w0 x, or mt E + w0 (a_i b_j) x with rank-one weights)
+    // shifted residual (m - w0) E + w0 x, or mt E + w0 (a_i b_j) x with rank-one weights).  The row copy is computed
+    // from the factors (16-byte gathers of T' rows), the column copy as a permutation of it.
     const double w0 = plain ? 0.0 : h->sp_w0;
     const bool vec = !plain && h->sp_mt_csr;
     const T* va = vec ? (const T*)h->sp_va : nullptr;
     const T* vb = vec ? (const T*)h->sp_vb : nullptr;
     const SpSide csr = vec ? sp_pass_side(h, h->csr, h->sp_mt_csr) : h->csr;
-    const SpSide csc = vec ? sp_pass_side(h, h->csc, h->sp_mt_csc) : h->csc;
-    if (h->sp_refresh_v2) {
-        // the row copy from the factors (16-byte gathers of T' rows), the column copy as a permutation of it
-        launch_sp_residual_rows<T>(csr, W, h->k, (const T*)h->Tt, h->sp_ldt, h->k, w0, h->sm_count, st, va, vb);
+    launch_sp_residual_rows<T>(csr, W, h->k, (const T*)h->Tt, h->sp_ldt, h->k, w0, h->sm_count, st, va, vb);
+    h->launches++;
+    if (need_csc && h->nnz > 0) {
+        launch_sp_gather<T>(h->sp_perm, (const T*)h->csr.E, (T*)h->csc.E, h->nnz, h->sm_count, st);
         h->launches++;
-        if (need_csc && h->nnz > 0) {
-            launch_sp_gather<T>(h->sp_perm, (const T*)h->csr.E, (T*)h->csc.E, h->nnz, h->sm_count, st);
-            h->launches++;
-        }
-        return;
     }
-    if (need_csc) { launch_sp_residual<T>(csc, (const T*)h->Tt, W, h->k, w0, h->sm_count, st, vb, va); h->launches++; }
-    if (need_csr) { launch_sp_residual<T>(csr, W, (const T*)h->Tt, h->k, w0, h->sm_count, st, va, vb); h->launches++; }
 }
 
 template <typename T>
@@ -1608,11 +1589,11 @@ static int sp_T_step(rri_handle_t h, T* W, T* Tm, int t, const rri_params_t* p, 
         launch_wrri_final<T>(nu, de, parts, d, solve_args(p, true), trow, 1, (T*)h->Tt + t, h->sp_ldt, h->flags, st);
         h->launches++;
     }
-    if (!h->sp_batched_sums || p->simplex_T) {
-        launch_vec_sum_flag<T>(trow, d, 1, h->sums, t, p->simplex_T ? 0 : 1, h->flags, st);
+    if (p->simplex_T) {
+        launch_vec_sum_flag<T>(trow, d, 1, h->sums, t, 0, h->flags, st);
         h->launches++;
+        scale_row_to_sum<T>(h, trow, (T*)h->Tt + t, h->sp_ldt, t, p, st);
     }
-    if (p->simplex_T) scale_row_to_sum<T>(h, trow, (T*)h->Tt + t, h->sp_ldt, t, p, st);
     S.csc = SpPending{wt, wt, told, trow};       // w_t (told - tnew)'; merged with the W-step's change if one follows
     S.told_cur = told;
     S.ct++;
@@ -1645,15 +1626,6 @@ static int sp_W_step(rri_handle_t h, T* W, T* Tm, int t, const rri_params_t* p, 
                              h->flags, st);
     }
     h->launches += 3;
-    if (!h->sp_batched_sums) {
-        launch_vec_sum_flag<T>(wt, n, 1, h->sums, h->k + t, h->world > 1 ? 0 : 2, h->flags, st);
-        h->launches++;
-        if (h->world > 1) {
-            NCK(g_nccl.AllReduce(h->sums + h->k + t, h->sums + h->k + t, 1, 8, 0, h->comm, st));
-            launch_flag_from_sums(h->sums, h->k + t, 1, 2, h->flags, st);
-            h->launches += 2;
-        }
-    }
     // both copies now lag by  wold told' - wnew tnew'  (one record even when a T-step preceded: the terms in
     // w_old t_new' cancel)
     S.csr = SpPending{wold, wt, told, trow};
@@ -1663,12 +1635,11 @@ static int sp_W_step(rri_handle_t h, T* W, T* Tm, int t, const rri_params_t* p, 
     return 0;
 }
 
-// The 2k single-block column-sum launches of a sweep (13.6 us each at config-4 shape) replaced by two launches at its
-// end -- row t of T and of W' is final once its step has run (RRI_SP_BATCHED_SUMS=0 restores the per-step sums).
+// The per-topic sums of a sweep in two launches at its end (instead of 2k single-block column sums, 13.6 us each at
+// config-4 shape): row t of T and of W' is final once its step has run.
 template <typename T>
 static int sp_topic_sums(rri_handle_t h, const T* Tm, int t0, int t1, bool did_T, bool did_W, cudaStream_t st)
 {
-    if (!h->sp_batched_sums) return 0;
     if (did_T) { launch_rowsum_flag<T>(Tm + (int64_t)t0 * h->d, t1 - t0, h->d, h->d, h->sums, t0, 1, h->flags, st); h->launches++; }
     if (did_W) {
         launch_rowsum_flag<T>((const T*)h->Wt + (int64_t)t0 * h->ldwt, t1 - t0, h->n, h->ldwt, h->sums, h->k + t0,
@@ -1701,7 +1672,7 @@ static int sp_topic_range(rri_handle_t h, T* W, T* Tm, int t0, int t1, const rri
     // the start of a call); otherwise they continue from the previous sweep with its pending rank-one record
     SpState local;
     SpState& S = carried ? *carried : local;
-    if (restart) { S = SpState(); sp_refresh<T>(h, true, true, W, st); }
+    if (restart) { S = SpState(); sp_refresh<T>(h, true, W, st); }
     for (int t = t0; t < t1; ++t) {
         if (sp_T_step<T>(h, W, Tm, t, p, S, st)) return 1;
         if (sp_W_step<T>(h, W, Tm, t, p, S, st)) return 1;
@@ -1729,14 +1700,14 @@ static int sp_sweeps(rri_handle_t h, T* W, T* Tm, int n_sweeps, const rri_params
         }
         if (!p->fix_T) {                       // block order, T half: only the column copy is read
             SpState S;
-            sp_refresh<T>(h, false, true, W, st);
+            sp_refresh<T>(h, true, W, st);
             for (int t = 0; t < k; ++t) {
                 if (sp_T_step<T>(h, W, Tm, t, p, S, st)) return 1;
                 S.told_cur = nullptr;
             }
         }
         SpState S;                             // W half (also transform(): fix_T): only the row copy is read
-        sp_refresh<T>(h, true, false, W, st);
+        sp_refresh<T>(h, false, W, st);
         for (int t = 0; t < k; ++t)
             if (sp_W_step<T>(h, W, Tm, t, p, S, st)) return 1;
         if (sp_topic_sums<T>(h, Tm, 0, k, !p->fix_T, true, st)) return 1;
@@ -1894,7 +1865,7 @@ static int objective_impl(rri_handle_t h, const T* W, const T* Tm, cudaStream_t 
     if (h->zero_csr) return objective_contraction_impl<T>(h, W, Tm, false, st);     // (no pass over n x d entries)
     if (h->sparse) {
         launch_transpose<T>(Tm, h->k, h->d, h->d, (T*)h->Tt, h->sp_ldt, st);
-        sp_refresh<T>(h, true, false, W, st, true);
+        sp_refresh<T>(h, false, W, st, true);
         const int k = h->k;
         double* gw = h->sp_gobj;
         double* gt = gw ? gw + (size_t)k * k * h->sp_oc_w : nullptr;
@@ -2046,7 +2017,7 @@ static int partials_impl(rri_handle_t h, const T* W, const T* Tm, int t, T* wR, 
     memset(&p, 0, sizeof(p));
     if (h->sparse) {
         if (sp_load_factors<T>(h, W, Tm, st)) return 1;
-        sp_refresh<T>(h, false, true, W, st);
+        sp_refresh<T>(h, true, W, st);
         const T* wt = (const T*)h->Wt + (int64_t)t * h->ldwt;
         launch_sp_pack<T>(nullptr, nullptr, wt, wt, h->sp_quad, h->n, st);
         const int parts = launch_sp_pass<T>(h->csc, h->sp_quad, nullptr, nullptr, Tm + (int64_t)t * d, (T*)h->sp_told,
@@ -2241,7 +2212,7 @@ static int profile_impl(rri_handle_t h, int which, const T* W, const T* Tm, int 
         prm.ub_t = 1.0;
         if (h->sparse) {
             if (sp_load_factors<T>(h, W, Tm, st)) return 1;
-            sp_refresh<T>(h, true, true, W, st);
+            sp_refresh<T>(h, true, W, st);
         } else if (h->wtc) {
             wrri_tc_load_factors(h->wtc, (const float*)W, (const float*)Tm, st);
             h->launches += 2;

@@ -36,7 +36,6 @@
 #include <cuda.h>
 #include <cuda_runtime.h>
 #include <stdio.h>
-#include <stdlib.h>
 
 #include "devmem.h"
 #include "gemm_tf32_sm100.h"
@@ -371,10 +370,6 @@ struct Tf32Gemm {
     float* ws = nullptr;
     size_t ws_bytes = 0;
     int* err = nullptr;
-    CUtensorMapDataType dtype = CU_TENSOR_MAP_DATA_TYPE_TFLOAT32;
-    int force_mt = 0;
-    int flush = FLUSH;
-    int reverse_tail = -1;             // -1: automatic (on for N > 64), 0 / 1: forced by RRI_GEMM_REVERSE_TAIL
     int* ctr = nullptr;
     size_t ctr_len = 0;
 };
@@ -401,16 +396,6 @@ Tf32Gemm* tf32_gemm_create(int sm_count, int nmax, std::string& err)
         return nullptr;
     }
     cudaMemset(g->err, 0, sizeof(int));
-    // operand element type seen by TMA: TFLOAT32 (default) or plain FLOAT32 (RRI_TMA_F32=1), for the
-    // rounding experiment described in DESIGN.md
-    const char* ev = getenv("RRI_TMA_F32");
-    if (ev && ev[0] == '1') g->dtype = CU_TENSOR_MAP_DATA_TYPE_FLOAT32;
-    const char* mt = getenv("RRI_GEMM_MT");
-    if (mt) g->force_mt = atoi(mt);
-    const char* rt = getenv("RRI_GEMM_REVERSE_TAIL");
-    if (rt) g->reverse_tail = atoi(rt);
-    const char* fl = getenv("RRI_GEMM_FLUSH");       // 0 = never flush (one TMEM accumulation per segment)
-    if (fl) g->flush = atoi(fl);
     return g;
 }
 
@@ -423,7 +408,7 @@ void tf32_gemm_destroy(Tf32Gemm* g)
     delete g;
 }
 
-// f16: a matrix of fp16 elements (box of 64 per 128-byte row), otherwise fp32 (the handle's TFLOAT32 / FLOAT32 map)
+// f16: a matrix of fp16 elements (box of 64 per 128-byte row), otherwise fp32 seen by TMA as TFLOAT32
 static bool encode_2d(Tf32Gemm* g, CUtensorMap* tm, const void* base, int64_t rows, int64_t cols, int64_t ld,
                       int box_rows, bool f16, std::string& err)
 {
@@ -436,7 +421,7 @@ static bool encode_2d(Tf32Gemm* g, CUtensorMap* tm, const void* base, int64_t ro
     cuuint64_t gstr[1] = {(cuuint64_t)(ld * es)};
     cuuint32_t box[2] = {(cuuint32_t)(ROW_BYTES / es), (cuuint32_t)box_rows};
     cuuint32_t estr[2] = {1, 1};
-    CUresult r = g->encode(tm, f16 ? CU_TENSOR_MAP_DATA_TYPE_FLOAT16 : g->dtype, 2, const_cast<void*>(base), gdim, gstr, box,
+    CUresult r = g->encode(tm, f16 ? CU_TENSOR_MAP_DATA_TYPE_FLOAT16 : CU_TENSOR_MAP_DATA_TYPE_TFLOAT32, 2, const_cast<void*>(base), gdim, gstr, box,
                            estr, CU_TENSOR_MAP_INTERLEAVE_NONE,
                            CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
     if (r != CUDA_SUCCESS) {
@@ -464,12 +449,12 @@ static int run_cfg(Tf32Gemm* g, const CUtensorMap& tmA, const CUtensorMap& tmB, 
     int cols = 32;
     while (cols < p.nbuf * MT * NPAD) cols <<= 1;
     p.tmem_cols = cols;
-    // the flush period is a K length (RRI_GEMM_FLUSH counts 32-wide chunks): two 64-wide chunks of 16-bit operands
-    p.flush = g->flush > 0 ? (F16 ? (g->flush + 1) / 2 : g->flush) : (1 << 30);
+    // the flush period is a K length (FLUSH counts 32-wide chunks): two 64-wide chunks of 16-bit operands
+    p.flush = F16 ? FLUSH / 2 : FLUSH;
     // Measured (profiles/r02_gemm_reverse_tail_ab.txt): the shared B stream wins where B is half of A's traffic (k = 128:
     // T half-step of a config-5 shard 1.91 -> 1.76 ms) and loses where it is a quarter (k = 64: 2.49 -> 2.71 ms; streaming
     // all CTAs through the same columns at the same time costs more than the re-reads it saves).
-    p.reverse_tail = g->reverse_tail >= 0 ? g->reverse_tail : (NPAD >= 128 ? 1 : 0);
+    p.reverse_tail = NPAD >= 128 ? 1 : 0;
     int64_t grid = p.units < g->sm_count ? p.units : g->sm_count;
     constexpr int EWQ = NPAD >= 128 ? 4 : 2;
     auto kern = tf32_gemm_kernel<MT, NPAD, EWQ, F16>;
@@ -498,7 +483,6 @@ static int gemm_run(Tf32Gemm* g, bool f16, const void* A, int64_t lda, int a_exp
     // M = 20 000, N = 64, K = 25 000 / 50 000 (profiles/r02_gemm_tile_height_ab.txt).  At K = 200 000 (B = 51 MB) the
     // doubled re-reads cost 0.16 ms, and N = 128 gains nothing.
     if (npad <= 64 && (M + 2 * BM - 1) / (2 * BM) < g->sm_count && (int64_t)npad * K * 4 <= ((int64_t)16 << 20)) mt = 1;
-    if (g->force_mt == 1 || (g->force_mt == 2 && npad < 256)) mt = g->force_mt;
     CUtensorMap tmA, tmB, tmA2;
     if (!encode_2d(g, &tmA, A, M, K, lda, mt * BM, f16, err)) return -1;
     if (!encode_2d(g, &tmB, B, N, K, ldb, npad, f16, err)) return -1;

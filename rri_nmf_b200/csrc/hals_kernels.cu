@@ -713,20 +713,16 @@ static void launch_update_rows_reg(T* F, int64_t m, int k, const T* C, const T* 
     const size_t smem = sizeof(T) * KM * KM;
     const dim3 nb((unsigned)((m + 127) / 128), (unsigned)rb.models);
     if constexpr (sizeof(T) == 4) {
-        static const bool x2 = [] { const char* e = getenv("RRI_UPDATE_X2"); return !(e && *e == '0'); }();
-        if (x2) {
-            auto kx = update_rows_reg_x2_kernel<KM>;
-            if (smem > 48 * 1024) cudaFuncSetAttribute(kx, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-            kx<<<nb, 128, smem, st>>>(F, m, k, C, S, (T)a.reg_l1, (T)a.reg_l2, (T)a.eps, (T)a.ub, a.has_ub, Ft, ldft, flags,
-                                      rb.ldc, rb.lds, rb.s_stride);
-            if (co.sums) launch_rowsum_flag<T>(Ft, k, m, ldft, co.sums, co.off, co.zero_flag, flags, st);
-            return;
-        }
+        auto kx = update_rows_reg_x2_kernel<KM>;
+        if (smem > 48 * 1024) cudaFuncSetAttribute(kx, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+        kx<<<nb, 128, smem, st>>>(F, m, k, C, S, (T)a.reg_l1, (T)a.reg_l2, (T)a.eps, (T)a.ub, a.has_ub, Ft, ldft, flags,
+                                  rb.ldc, rb.lds, rb.s_stride);
+    } else {
+        auto kern = update_rows_reg_kernel<T, KM>;
+        if (smem > 48 * 1024) cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+        kern<<<nb, 128, smem, st>>>(F, m, k, C, S, (T)a.reg_l1, (T)a.reg_l2, (T)a.eps, (T)a.ub, a.has_ub, Ft, ldft, flags,
+                                    rb.ldc, rb.lds, rb.s_stride);
     }
-    auto kern = update_rows_reg_kernel<T, KM>;
-    if (smem > 48 * 1024) cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-    kern<<<nb, 128, smem, st>>>(F, m, k, C, S, (T)a.reg_l1, (T)a.reg_l2, (T)a.eps, (T)a.ub, a.has_ub, Ft, ldft, flags,
-                                rb.ldc, rb.lds, rb.s_stride);
     if (co.sums) launch_rowsum_flag<T>(Ft, k, m, ldft, co.sums, co.off, co.zero_flag, flags, st);
 }
 
@@ -997,13 +993,12 @@ void launch_update_rows(T* F, int64_t m, int k, const T* Cpart, int parts, int64
     // thread-per-row variants while the row fits in registers / the tiles in shared memory
     // (fp32: k <= 128, fp64: k <= 64); wider ranks use the warp-per-row kernel
     {
-        static const bool reg_off = [] { const char* e = getenv("RRI_UPDATE_REG"); return e && *e == '0'; }();
         constexpr int VN = Vec<T>::N;
         // (16-byte loads of the factor and contraction rows: F and Cpart point at a model of a handle of several, which
         // need not start on a 16-byte boundary; such a model takes the staged kernel, which gives the same bits)
         const bool vec = (k % VN) == 0 && (rb.ldc % VN) == 0 && (reinterpret_cast<uintptr_t>(F) & 15) == 0 &&
                          (reinterpret_cast<uintptr_t>(Cpart) & 15) == 0;
-        if (!reg_off && parts == 1 && !srcs && Ft && vec && k <= (sizeof(T) == 4 ? 128 : 64)) {
+        if (parts == 1 && !srcs && Ft && vec && k <= (sizeof(T) == 4 ? 128 : 64)) {
             if (k <= 16) launch_update_rows_reg<T, 16>(F, m, k, Cpart, S, a, Ft, ldft, flags, co, rb, st);
             else if (k <= 32) launch_update_rows_reg<T, 32>(F, m, k, Cpart, S, a, Ft, ldft, flags, co, rb, st);
             else if (k <= 64) launch_update_rows_reg<T, 64>(F, m, k, Cpart, S, a, Ft, ldft, flags, co, rb, st);

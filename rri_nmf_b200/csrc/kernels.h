@@ -262,7 +262,7 @@ struct SpSide {            // one compressed orientation of the observed entries
     const int64_t* ptr2;   // [nseg][nblk + 1] first entry of segment s with index >= b * nb, or null
     int nblk, nb;
     int64_t nother;        // length of the other factor's index range (d for CSR, n for CSC)
-    const uint16_t* idx16; // [nnz] idx % nb (2 bytes instead of 4 per entry and pass), or null
+    const uint16_t* idx16; // [nnz] idx % nb (2 bytes instead of 4 per entry and pass), with ptr2
 };
 int sp_block_len(int elem_size, int64_t nother, int* nblk_out);
 void launch_sp_local_index(const int32_t* idx, int64_t nnz, int nb, uint16_t* out, int sm_count, cudaStream_t st);
@@ -277,16 +277,11 @@ int sp_build_csc(const int64_t* rowptr, const int32_t* col, const T* x, const T*
                  int64_t nnz, int64_t* colptr, int32_t* csc_row, T* x_csc, T* w_csc, uint32_t* perm, int sm_count,
                  int* err_dev, cudaStream_t st);
 
-// s.E[p] = s.x[p] - sum_l A[seg,l] * B[s.idx[p],l]   (A: own factor rows [nseg,k], B: other factor rows [.,k]).
+// s.E[p] = s.x[p] - sum_l A[seg,l] * B[s.idx[p],l]   (A: own factor rows [nseg, lda], staged per segment through shared
+// memory; B: other factor rows [., ldb] read with 16-byte gathers, ldb a multiple of 16 bytes with zero pad columns).
 // w0 > 0 (unstored weight): the shifted residual (m - w0) E + w0 x is stored instead (m = s.wgt[p], or 1).  With a
 // rank-one weight vector vseg (over the segments) or vidx (over the gathered index), u = w0 (a_i b_j): s.wgt then holds
 // mt = m - u (launch_sp_mtilde) and mt E + u x is stored.
-template <typename T>
-void launch_sp_residual(const SpSide& s, const T* A, const T* B, int k, double w0, int sm_count, cudaStream_t st,
-                        const T* vseg = nullptr, const T* vidx = nullptr);
-
-// The same for the row orientation with 16-byte gathers: B[., ldb] has a padded row stride (multiple of 16 bytes, zero
-// pad columns); A[nseg, lda] is staged per segment through shared memory.
 template <typename T>
 void launch_sp_residual_rows(const SpSide& s, const T* A, int64_t lda, const T* B, int ldb, int k, double w0, int sm_count,
                              cudaStream_t st, const T* vseg = nullptr, const T* vidx = nullptr);

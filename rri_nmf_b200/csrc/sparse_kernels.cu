@@ -12,7 +12,6 @@
 // rebuilt from X, W, T at the start of every sweep (so N sweeps == N x 1 sweep bit for bit, and rounding drift
 // cannot accumulate).  No atomics: one warp (or one block) owns a whole segment.
 #include <cub/device/device_radix_sort.cuh>
-#include <stdlib.h>
 
 #include "common.cuh"
 #include "kernels.h"
@@ -137,8 +136,8 @@ int sp_build_csc(const int64_t* rowptr, const int32_t* col, const T* x, const T*
 }
 
 // ------------------------------------------------------------------------------------------------
-// residual from scratch:  E[p] = x[p] - sum_l A[seg,l] * B[idx[p],l]
-// (CSR: A = W, B = T';  CSC: A = T', B = W -- the products commute, the sums run in the same order)
+// residual from scratch:  E[p] = x[p] - sum_l A[seg,l] * B[idx[p],l]  in the row orientation (A = W, B = T'); the
+// column copy is its permutation (sp_gather_kernel)
 // Shifted mode (SH == 1): the stored value is S[p] = (m[p] - w0) E[p] + w0 x[p]  (m = 1 without entry weights).
 // Rank-one mode (SH == 2, unstored weights u = w0 (a_i b_j), DESIGN.md §1 row f8): wgt holds mt = m - u per entry
 // (sp_mtilde_kernel) and S[p] = mt E[p] + u x[p]; ab = a_i b_j from the segment's and the gathered entry's vector.
@@ -157,54 +156,6 @@ RRI_DEVINL T sp_ab(const T* __restrict__ vseg, const T* __restrict__ vidx, int64
 {
     if constexpr (SH == 2) return mul_rn(vseg ? vseg[s] : T(1), vidx ? vidx[j] : T(1));
     return T(1);
-}
-
-template <typename T, int V, int G, int SH>
-__global__ void __launch_bounds__(256)
-sp_residual_kernel(const int64_t* __restrict__ ptr, const int32_t* __restrict__ idx, const T* __restrict__ x,
-                   const T* __restrict__ A, const T* __restrict__ B, int k, T* __restrict__ E, int64_t nseg,
-                   const T* __restrict__ wgt, T w0, const T* __restrict__ vseg, const T* __restrict__ vidx)
-{
-    constexpr int GPB = 256 / G;
-    const int lane = threadIdx.x % G, g = threadIdx.x / G;
-    for (int64_t s = (int64_t)blockIdx.x * GPB + g; s < nseg; s += (int64_t)gridDim.x * GPB) {
-        const int64_t b = ptr[s], e = ptr[s + 1];
-        const T* __restrict__ a = A + s * k;
-        for (int64_t p = b + lane; p < e; p += G) {
-            const T* __restrict__ bb = B + (int64_t)idx[p] * k;
-            T acc = x[p];
-            if constexpr (V == 1) {
-#pragma unroll 4
-                for (int l = 0; l < k; ++l) acc = fma(-a[l], bb[l], acc);
-            } else {
-                struct alignas(sizeof(T) * V) Pk { T v[V]; };
-                const Pk* __restrict__ av = reinterpret_cast<const Pk*>(a);
-                const Pk* __restrict__ bv = reinterpret_cast<const Pk*>(bb);
-#pragma unroll 2
-                for (int l = 0; l < k / V; ++l) {
-                    const Pk x1 = av[l], x2 = bv[l];
-#pragma unroll
-                    for (int v = 0; v < V; ++v) acc = fma(-x1.v[v], x2.v[v], acc);
-                }
-            }
-            E[p] = sp_stored<T, SH>(acc, x[p], wgt, p, w0, sp_ab<T, SH>(vseg, vidx, s, idx[p]));
-        }
-    }
-}
-
-template <typename T, int V, int SH>
-static void residual_dispatch(const SpSide& s, const T* A, const T* B, int k, T w0, const T* vseg, const T* vidx,
-                              int sm_count, cudaStream_t st)
-{
-    const T* w = (const T*)s.wgt;
-    if (s.group == 256) {
-        sp_residual_kernel<T, V, 256, SH><<<cap_blocks(s.nseg, sm_count, 8), 256, 0, st>>>(s.ptr, s.idx, (const T*)s.x, A, B, k,
-                                                                                            (T*)s.E, s.nseg, w, w0, vseg, vidx);
-    } else {
-        sp_residual_kernel<T, V, 32, SH><<<cap_blocks((s.nseg + 7) / 8, sm_count, 8), 256, 0, st>>>(s.ptr, s.idx, (const T*)s.x, A,
-                                                                                                     B, k, (T*)s.E, s.nseg, w, w0,
-                                                                                                     vseg, vidx);
-    }
 }
 
 // Row-orientation residual with the segment's own factor row staged in shared memory and the gathered rows read
@@ -293,29 +244,6 @@ template <typename T>
 void launch_sp_gather(const uint32_t* perm, const T* src, T* dst, int64_t nnz, int sm_count, cudaStream_t st)
 {
     sp_gather_kernel<T><<<cap_blocks((nnz + 1023) / 1024, sm_count, 8), 256, 0, st>>>(perm, src, dst, nnz);
-}
-
-// (A variant that staged the gathered k-vectors of 32 entries through shared memory was measured slower than this
-// direct kernel -- 9.5 ms against 5.9 ms at nnz = 1e8, k = 50, profiles/r01_sparse_bench_v2_staged.log -- and was
-// removed; the shipped restart path is sp_residual_rows_kernel + sp_gather_kernel above.)
-template <typename T, int SH>
-static void residual_vec_dispatch(const SpSide& s, const T* A, const T* B, int k, T w0, const T* vseg, const T* vidx,
-                                  int sm_count, cudaStream_t st)
-{
-    const uintptr_t al = reinterpret_cast<uintptr_t>(A) | reinterpret_cast<uintptr_t>(B);
-    constexpr int VMAX = 16 / (int)sizeof(T);
-    if (VMAX == 4 && k % 4 == 0 && (al & 15) == 0) residual_dispatch<T, VMAX, SH>(s, A, B, k, w0, vseg, vidx, sm_count, st);
-    else if (k % 2 == 0 && (al & (2 * sizeof(T) - 1)) == 0) residual_dispatch<T, 2, SH>(s, A, B, k, w0, vseg, vidx, sm_count, st);
-    else residual_dispatch<T, 1, SH>(s, A, B, k, w0, vseg, vidx, sm_count, st);
-}
-
-template <typename T>
-void launch_sp_residual(const SpSide& s, const T* A, const T* B, int k, double w0, int sm_count, cudaStream_t st,
-                        const T* vseg, const T* vidx)
-{
-    if (w0 > 0.0 && (vseg || vidx)) residual_vec_dispatch<T, 2>(s, A, B, k, (T)w0, vseg, vidx, sm_count, st);
-    else if (w0 > 0.0) residual_vec_dispatch<T, 1>(s, A, B, k, (T)w0, nullptr, nullptr, sm_count, st);
-    else residual_vec_dispatch<T, 0>(s, A, B, k, T(0), nullptr, nullptr, sm_count, st);
 }
 
 // ------------------------------------------------------------------------------------------------
@@ -448,8 +376,7 @@ sp_pass_kernel(const int64_t* __restrict__ ptr, const int32_t* __restrict__ idx,
 // numer_part[b][s], denom_part[b][s] and added in block order by the solve kernel (deterministic).
 template <typename T, bool HASW, bool SH, int U, int THREADS, int MINB>
 __global__ void __launch_bounds__(THREADS, MINB)
-sp_pass_blocked_kernel(const int64_t* __restrict__ ptr2, const int32_t* __restrict__ idx,
-                       const uint16_t* __restrict__ idx16, T* __restrict__ E,
+sp_pass_blocked_kernel(const int64_t* __restrict__ ptr2, const uint16_t* __restrict__ idx16, T* __restrict__ E,
                        const T* __restrict__ wgt, const Quad<T>* __restrict__ Q, const T* __restrict__ own_po,
                        const T* __restrict__ own_pn, const T* __restrict__ own_cur, T* __restrict__ own_save,
                        T* __restrict__ numer_part, T* __restrict__ denom_part, int64_t nseg, int nblk, int nb,
@@ -466,7 +393,6 @@ sp_pass_blocked_kernel(const int64_t* __restrict__ ptr2, const int32_t* __restri
     int64_t s0, s1;
     part_range(nseg, chunks, c, s0, s1);
     const bool apply = own_po != nullptr;
-    const int32_t ibase = (int32_t)base;
     const int64_t pstride = (int64_t)nblk + 1;
     // the bounds and the per-segment scalars of the NEXT sub-segment are requested before this one is streamed: the
     // pointer load would otherwise sit in front of every sub-segment's first batch (two dependent round trips per ~3 KB)
@@ -492,7 +418,7 @@ sp_pass_blocked_kernel(const int64_t* __restrict__ ptr2, const int32_t* __restri
             for (int u = 0; u < U; ++u) {
                 const int64_t p = p0 + u * 32;
                 const bool ok = p < end;
-                q[u] = ok ? (idx16 ? (int32_t)idx16[p] : idx[p] - ibase) : -1;     // block-local record index
+                q[u] = ok ? (int32_t)idx16[p] : -1;                                // block-local record index
                 ev[u] = ok ? E[p] : T(0);
                 m[u] = (HASW && ok) ? wgt[p] : T(1);
             }
@@ -628,14 +554,15 @@ __global__ void sp_subptr_kernel(const int64_t* __restrict__ ptr, const int32_t*
     }
 }
 
-// Records per staged block of Q: at most 128 KB of shared memory, and all blocks equally long (a short last block
-// would leave its CTAs with a fraction of the work of the others).
+// Records per staged block of Q: at most SP_BLOCK_BYTES of shared memory (one 1024-thread CTA per SM; a block of
+// <= 64 KB runs as two 512-thread CTAs per SM), and all blocks equally long (a short last block would leave its CTAs
+// with a fraction of the work of the others).
+constexpr int64_t SP_BLOCK_BYTES = 128 * 1024;
+static_assert(SP_BLOCK_BYTES / (4 * sizeof(float)) <= 65536, "block-local indices must fit 16 bits (SpSide::idx16)");
+
 int sp_block_len(int elem_size, int64_t nother, int* nblk_out)
 {
-    // RRI_SP_BLOCK_KB: shared-memory staging block (default 128 KB: one 1024-thread CTA per SM; <= 64 KB: two
-    // 512-thread CTAs per SM, shorter sub-segments)
-    static const int kb = [] { const char* e = getenv("RRI_SP_BLOCK_KB"); const int v = e ? atoi(e) : 128; return v >= 8 && v <= 216 ? v : 128; }();
-    const int64_t cap = ((int64_t)kb * 1024) / (4 * elem_size);
+    const int64_t cap = SP_BLOCK_BYTES / (4 * elem_size);
     const int64_t nblk = nother > 0 ? (nother + cap - 1) / cap : 1;
     int64_t nb = (nother + nblk - 1) / nblk;
     nb = (nb + 31) / 32 * 32;
@@ -685,35 +612,31 @@ static int sp_pass_dispatch(const SpSide& s, const Quad<T>* Q, const T* own_po, 
             if (chunks < 1) chunks = 1;
             auto kern = w ? sp_pass_blocked_kernel<T, true, SH, U, 512, 2> : sp_pass_blocked_kernel<T, false, SH, U, 512, 2>;
             if (smem > 48 * 1024) cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, 64 * 1024);
-            kern<<<(unsigned)(s.nblk * chunks), 512, smem, st>>>(s.ptr2, s.idx, s.idx16, E, w, Q, own_po, own_pn, own_cur, own_save,
+            kern<<<(unsigned)(s.nblk * chunks), 512, smem, st>>>(s.ptr2, s.idx16, E, w, Q, own_po, own_pn, own_cur, own_save,
                                                                 numer, denom, s.nseg, s.nblk, s.nb, s.nother, chunks, w0);
             return s.nblk;
         }
         if constexpr (sizeof(T) == 4) {
-            // fp32 with 16-bit block-local indices: the streamlined kernel, 16 entries per lane and batch where no
-            // weights are read (64 registers, no spills), 8 with weights.  RRI_SP_STREAM=0 selects the general kernel
-            // below (A/B in profiles/r02_sparse_shape_ab_call16.txt, r02_sparse_pass_experiments.txt).
-            static const bool stream = [] { const char* e = getenv("RRI_SP_STREAM"); return !(e && *e == '0'); }();
-            if (stream && s.idx16) {
-                if (w) {
-                    auto kv = sp_pass_stream_kernel<T, true, SH, 8, 1024, 1>;
-                    if (smem > 48 * 1024) cudaFuncSetAttribute(kv, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-                    kv<<<(unsigned)(s.nblk * chunks), 1024, smem, st>>>(s.ptr2, s.idx16, E, w, Q, own_po, own_pn, own_cur, own_save,
-                                                                       numer, denom, s.nseg, s.nblk, s.nb, s.nother, chunks, w0);
-                } else {
-                    // (shifted: 12 entries per lane and batch -- 16 spill there)
-                    auto kv = sp_pass_stream_kernel<T, false, SH, SH ? 12 : 16, 1024, 1>;
-                    if (smem > 48 * 1024) cudaFuncSetAttribute(kv, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-                    kv<<<(unsigned)(s.nblk * chunks), 1024, smem, st>>>(s.ptr2, s.idx16, E, w, Q, own_po, own_pn, own_cur, own_save,
-                                                                       numer, denom, s.nseg, s.nblk, s.nb, s.nother, chunks, w0);
-                }
-                return s.nblk;
+            // fp32: the streamlined kernel, 16 entries per lane and batch where no weights are read (64 registers, no
+            // spills), 8 with weights
+            if (w) {
+                auto kv = sp_pass_stream_kernel<T, true, SH, 8, 1024, 1>;
+                if (smem > 48 * 1024) cudaFuncSetAttribute(kv, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+                kv<<<(unsigned)(s.nblk * chunks), 1024, smem, st>>>(s.ptr2, s.idx16, E, w, Q, own_po, own_pn, own_cur, own_save,
+                                                                   numer, denom, s.nseg, s.nblk, s.nb, s.nother, chunks, w0);
+            } else {
+                // (shifted: 12 entries per lane and batch -- 16 spill there)
+                auto kv = sp_pass_stream_kernel<T, false, SH, SH ? 12 : 16, 1024, 1>;
+                if (smem > 48 * 1024) cudaFuncSetAttribute(kv, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+                kv<<<(unsigned)(s.nblk * chunks), 1024, smem, st>>>(s.ptr2, s.idx16, E, w, Q, own_po, own_pn, own_cur, own_save,
+                                                                   numer, denom, s.nseg, s.nblk, s.nb, s.nother, chunks, w0);
             }
+        } else {
+            auto kern = w ? sp_pass_blocked_kernel<T, true, SH, U, 1024, 1> : sp_pass_blocked_kernel<T, false, SH, U, 1024, 1>;
+            if (smem > 48 * 1024) cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+            kern<<<(unsigned)(s.nblk * chunks), 1024, smem, st>>>(s.ptr2, s.idx16, E, w, Q, own_po, own_pn, own_cur, own_save,
+                                                                 numer, denom, s.nseg, s.nblk, s.nb, s.nother, chunks, w0);
         }
-        auto kern = w ? sp_pass_blocked_kernel<T, true, SH, U, 1024, 1> : sp_pass_blocked_kernel<T, false, SH, U, 1024, 1>;
-        if (smem > 48 * 1024) cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-        kern<<<(unsigned)(s.nblk * chunks), 1024, smem, st>>>(s.ptr2, s.idx, s.idx16, E, w, Q, own_po, own_pn, own_cur, own_save, numer,
-                                                             denom, s.nseg, s.nblk, s.nb, s.nother, chunks, w0);
         return s.nblk;
     }
     if (s.group == 256) {
@@ -1011,8 +934,6 @@ void launch_sp_mtilde(const int64_t* rowptr, const int32_t* col, const T* wgt, i
 #define RRI_INST(T)                                                                                                 \
     template int sp_build_csc<T>(const int64_t*, const int32_t*, const T*, const T*, int64_t, int64_t, int64_t,    \
                                  int64_t*, int32_t*, T*, T*, uint32_t*, int, int*, cudaStream_t);                  \
-    template void launch_sp_residual<T>(const SpSide&, const T*, const T*, int, double, int, cudaStream_t, const T*, \
-                                        const T*);                                                                 \
     template void launch_sp_residual_rows<T>(const SpSide&, const T*, int64_t, const T*, int, int, double, int,    \
                                              cudaStream_t, const T*, const T*);                                    \
     template void launch_sp_gather<T>(const uint32_t*, const T*, T*, int64_t, int, cudaStream_t);                  \

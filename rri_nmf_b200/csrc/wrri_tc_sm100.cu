@@ -17,7 +17,6 @@
 #include <cuda.h>
 #include <cuda_runtime.h>
 #include <stdio.h>
-#include <stdlib.h>
 
 #include "devmem.h"
 #include "kernels.h"
@@ -811,9 +810,7 @@ static bool tma_prepare(WrriTc* g, const float* X, int64_t ldx, const void* M, i
         // previous MMA retires), then as many X/mask stages as still fit (>= 2; the end-of-CTA reduction needs 64 KB)
         const size_t room = (size_t)227 * 1024;
         int S = 0, ns = 0;
-        static const char* force_s = getenv("RRI_WRRI_OPERAND_STAGES");
         for (int s_try = 2; s_try >= 1; --s_try) {
-            if (force_s && atoi(force_s) != s_try) continue;
             const size_t base = fixed + (size_t)s_try * var + extra;
             if (base >= room) continue;
             int n_try = (int)((room - base) / xm);
@@ -841,8 +838,7 @@ static int launch_mode(WrriTc* g, const float* X, int64_t ldx, const void* M, in
     dim3 grid(MODE == 0 ? p.tiles_c : p.tiles_r, groups);
     if (mk != MK_U8 && mk != MK_REAL) { err = "the tensor-core WRRI path needs a mask"; return -1; }
     if (ldm % 4 != 0) { err = "mask rows need a stride that is a multiple of 4 elements"; return -1; }
-    static const bool no_tma = getenv("RRI_WRRI_NO_TMA") != nullptr;
-    if (!no_tma && Trow && (reinterpret_cast<uintptr_t>(Trow) & 15) == 0 && tma_prepare(g, X, ldx, M, mk, ldm) &&
+    if (Trow && (reinterpret_cast<uintptr_t>(Trow) & 15) == 0 && tma_prepare(g, X, ldx, M, mk, ldm) &&
         g->tma_xm[MODE][mk] >= 2) {
         p.stages = g->tma_stages[MODE][mk];
         p.xm_stages = g->tma_xm[MODE][mk];

@@ -66,10 +66,12 @@ def test_sparse_entry_weights_both_orders(R):
                                           (1900, 700, 0.3),     # the other way round
                                           (257, 131, 0.05),     # short, ragged segments; empty rows and columns
                                           (9000, 300, 0.05),    # the gathered factor spans several shared-memory blocks
-                                          (300, 9000, 0.05)])   # (4096 records each in fp64), in either orientation
+                                          (300, 9000, 0.05),    # (4096 records each in fp64), in either orientation
+                                          (48, 270000, 0.001),  # more than 64 such blocks: the direct pass, gathering
+                                          (270000, 48, 0.001)]) # from global memory, in either orientation
 @pytest.mark.parametrize('order', ['rri', 'hals'])
 def test_sparse_matches_oracle_fp64(R, n, d, density, order):
-    k = 8 if n > 500 else 7        # odd k: the residual kernel's scalar path
+    k = 8 if n > 500 else 7        # odd k: zero pad columns in the restart's 16-byte gathers of T' rows
     X, W0, T0, M = orc.synth(n, d, k, k, sigma=0.05, seed=n + d, mask_density=density)
     M[5, :] = 0
     M[:, 3] = 0                                               # an unobserved row and column

@@ -165,7 +165,7 @@ def test_n_sweeps_in_one_call_equal_n_calls(R, order, weighted):
         eng.close()
 
 
-def test_refresh_every_8_and_the_v1_restart_fp64(R, monkeypatch):
+def test_refresh_every_8_fp64(R):
     X, Wm, Xd, M, W0, T0, a, b = _case(600, 450, 8, 0.1, True, 'ab', seed=9)
     kw = dict(W_mat=Wm, W_in=W0, T_in=T0, max_iter=10, reset_topic_method=None, unstored_weight=0.1,
               unstored_row_weight=a, unstored_col_weight=b, sweeps_per_call=10)
@@ -174,9 +174,6 @@ def test_refresh_every_8_and_the_v1_restart_fp64(R, monkeypatch):
     assert relfro(g['W'], o['W']) <= 1e-9 and relfro(g['T'], o['T']) <= 1e-9
     e8 = R.nmf(X, 8, sparse_refresh_every=8, **kw)
     assert relfro(e8['W'], g['W']) <= 1e-9 and relfro(e8['T'], g['T']) <= 1e-9
-    monkeypatch.setenv('RRI_SP_REFRESH_V2', '0')              # the restart from both orientations (read at bind)
-    v1 = R.nmf(X, 8, **kw)
-    assert relfro(v1['W'], o['W']) <= 1e-9 and relfro(v1['T'], o['T']) <= 1e-9
 
 
 def test_topics_in_two_ranges(R):

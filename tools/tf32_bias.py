@@ -1,5 +1,5 @@
 """Signed bias of the TF32 contraction against an fp64 product for long K (accumulation-chain check).
-python tools/tf32_bias.py      (RRI_GEMM_FLUSH=0 disables the periodic TMEM -> register flush)"""
+python tools/tf32_bias.py"""
 import os, sys
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 import torch

@@ -1,8 +1,8 @@
 """Signed bias of the block-order contraction over long K with both storages of X: the fp32 tensor map (TF32 rounding on
 the way into shared memory, tcgen05.mma kind::tf32) and the 16-bit copies (kind::f16), against the fp64 product of the
-same TF32-rounded operands.  The TMEM flush period (RRI_GEMM_FLUSH, in 32-wide chunks; 4 = every 128 K) bounds the
+same TF32-rounded operands.  The TMEM flush period (FLUSH in gemm_tf32_sm100.cu, in 32-wide chunks; 4 = every 128 K) bounds the
 accumulation chain of either kind.
-python tools/x16_bias.py      (RRI_GEMM_FLUSH=0 disables the flush)"""
+python tools/x16_bias.py"""
 import os
 import sys
 
